@@ -14,15 +14,21 @@ does the full Newton work on fresh rays.  Inputs (6 GB/GPU) are far larger than 
 flush is needed between steps.
 
 Prints ONE JSON line (rank 0).  See DESIGN.md "Measurement" for every field.
+``--dump-outputs DIR`` also writes what the last timed step computed as DIR/<name>.npy (see ``dump_outputs``).
+The benchmark writes nothing into the repository tree, which may be read-only.
 """
 import argparse
+import atexit
 import json
 import os
+import shutil
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
+sys.dont_write_bytecode = True
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
@@ -51,7 +57,51 @@ def parse():
     ap.add_argument("--ref-rays", type=float, default=2.0e7, help="rays per step of the reference arm")
     ap.add_argument("--no-configs", action="store_true", help="skip the BASELINE configs 1-5 sub-results")
     ap.add_argument("--configs-scale", type=float, default=1., help="scale the configs' ray counts (smoke runs)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the last step's traced rows (a fixed sample of rays) and HPD "
+                         "to DIR/<name>.npy, float64 (N > 1: rank 0's shard and the global HPD)")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    return a
+
+
+DUMP_ROWS = ("x", "y", "z", "l", "m", "n", "ux", "uy", "uz")
+DUMP_RAYS = 1 << 18          # rays per dumped row: 9 rows x 2 MB
+
+
+def dump_sample(n):
+    """Indices of the rays --dump-outputs writes: all of a small bundle, else a fixed seeded sample in ascending
+    order, so that two builds run with the same arguments dump the same rays."""
+    import numpy as np
+    if n <= DUMP_RAYS:
+        return np.arange(n)
+    return np.sort(np.random.default_rng(20261020).choice(n, DUMP_RAYS, replace=False))
+
+
+def dump_outputs(path, rows, hpd):
+    """What the timed path hands its caller after its last step: rows x..uz of the traced bundle at the
+    ``dump_sample`` rays, and the HPD."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    for name, row in zip(DUMP_ROWS, rows):
+        np.save(os.path.join(path, name + ".npy"), np.asarray(row, dtype=np.float64))
+    np.save(os.path.join(path, "hpd.npy"), np.array([hpd], dtype=np.float64))
+
+
+def private_jit_cache():
+    """Specialised kernels compiled at run time are cached in a temporary directory instead of the tree: the
+    kernels build() cached under pyxfocus_b200/_jit are copied there and PXF_JIT_CACHE points at it."""
+    if "PXF_JIT_CACHE" in os.environ:
+        return
+    tmp = tempfile.mkdtemp(prefix="pxf_jit_")
+    atexit.register(shutil.rmtree, tmp, ignore_errors=True)
+    built = os.path.join(ROOT, "pyxfocus_b200", "_jit")
+    if os.path.isdir(built):
+        for f in os.listdir(built):
+            if f.endswith(".cubin"):
+                shutil.copy(os.path.join(built, f), tmp)
+    os.environ["PXF_JIT_CACHE"] = tmp
 
 
 # ------------------------------------------------------------------------------- clocks
@@ -194,6 +244,9 @@ def run_reference(args):
         t0 = time.perf_counter()
         hp = step(rays)
         t += time.perf_counter() - t0
+    if args.dump_outputs:
+        idx = dump_sample(n)
+        dump_outputs(args.dump_outputs, [rays[k][idx] for k in range(1, 10)], hp)
     val = n * args.steps / t
     sample = "%d steps x %.3g rays (same chain + hpd), C oracle port with OpenMP" % (args.steps, n)
     line = {
@@ -280,6 +333,7 @@ def run_engine(args):
     if world > 1:
         os.environ.setdefault("MASTER_ADDR", "127.0.0.1")
         td.init_process_group("nccl", device_id=dev)
+    private_jit_cache()
     import pyxfocus_b200 as pxf
     from pyxfocus_b200 import dist as pdist
     from pyxfocus_b200._call import bundle_alloc
@@ -382,6 +436,9 @@ def run_engine(args):
         ms, hp_t = timed_loop(False)
     assert hp_t == hp or (hp_t != hp_t and hp != hp), "HPD changed between warm-up and timed steps"
     launches = pxf.launch_count() - launches0
+    if args.dump_outputs and rank == 0:
+        idx = torch.from_numpy(dump_sample(n)).to(dev)
+        dump_outputs(args.dump_outputs, [out[k].index_select(0, idx).cpu().numpy() for k in range(1, 10)], hp_t)
     kname = pxf.last_trace_kernel()             # the kernel the timed steps launched
     clocks = clk.stop() if rank == 0 else None
     trace_ms = sum(a.elapsed_time(b) for a, b in kev) / K

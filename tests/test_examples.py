@@ -1,6 +1,7 @@
 """Whole-chain BASELINE configurations on the CPU oracle (no GPU): ``oracle.refapi`` -- the restatement that
 travels to the GPU box -- against the committed goldens (``tests/golden/configs.npz``, produced by the reference's
-own Python layer) and, when the reference tree is present, against that layer live, bit for bit."""
+own Python layer, and ``tests/golden/reference_api.npz``) and, when the reference tree is present, against that layer
+live, bit for bit."""
 import os
 import sys
 
@@ -13,6 +14,8 @@ sys.path.insert(0, os.path.join(ROOT, "tests", "golden"))
 from oracle import refapi, refload  # noqa: E402
 from pyxfocus_b200 import examples as ex  # noqa: E402
 from make_golden_configs import SIZES, stack  # noqa: E402
+import make_golden_reference_calls as rc  # noqa: E402
+from make_golden_reference_calls import assert_pinned  # noqa: E402
 
 C4_CASES = ((-1, 4.8), (-3, 2.4), (-8, .6), (-1, "uniform"))
 
@@ -68,22 +71,11 @@ def test_config5_matches_golden(api, gold):
     assert r["kept"] < SIZES["c5_n"] * SIZES["c5_shells"]
 
 
-@pytest.mark.skipif(not refload.available(), reason="reference tree not present (GPU box)")
-def test_restated_api_equals_the_live_reference_layer(api):
-    """Other sizes / seeds than the goldens: every configuration on the reference's own Python layer and on the
-    restatement, same bits."""
-    ref = ex.make_api(refload.load(), ex.NumpyXP, "reference")
-    ap = ex.ws_aperture(ref)
-    assert ap == ex.ws_aperture(api)
-    pairs = [(ex.config1(ref, 5000, 3), ex.config1(api, 5000, 3)),
-             (ex.config2_point(ref, 2000, 24. / 60. * np.pi / 180., ap, 5), ex.config2_point(api, 2000, 24. / 60. * np.pi / 180., ap, 5)),
-             (ex.config3(ref, 3000, 2), ex.config3(api, 3000, 2)),
-             (ex.config4(ref, 15, 30, order=-2, wave=2.4, rng_seed=4, offX=1e-4, offY=-2e-4),
-              ex.config4(api, 15, 30, order=-2, wave=2.4, rng_seed=4, offX=1e-4, offY=-2e-4)),
-             (ex.config5(ref, 60, 25, offaxis=2e-4, rng_seed=7), ex.config5(api, 60, 25, offaxis=2e-4, rng_seed=7))]
-    for a, b in pairs:
-        for k in a:
-            if isinstance(a[k], list):
-                assert all(same(x, y) for x, y in zip(a[k], b[k])), k
-            else:
-                assert same(a[k], b[k]), k
+def test_restated_api_equals_the_live_reference_layer(api, golden):
+    """Other sizes / seeds than the goldens: every configuration on the restatement against the bits the reference's own
+    Python layer gave for the same calls (tests/golden/reference_api.npz); where the reference tree
+    is present, that layer live as well."""
+    assert_pinned(rc.api_runs(api), golden("reference_api"), what="refapi")
+    if refload.available():
+        assert_pinned(rc.api_runs(ex.make_api(refload.load(), ex.NumpyXP, "reference")), golden("reference_api"),
+                      what="reference")

@@ -20,6 +20,8 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.join(HERE, "golden"))
 from oracle import f2py as of, f95run, refload  # noqa: E402
 from util import ROWS, assert_bit_equal, assert_close  # noqa: E402
+import make_golden_reference_calls as rc  # noqa: E402
+from make_golden_reference_calls import assert_pinned  # noqa: E402
 
 HIDDEN = {"num", "arrsize", "arrsize1", "arrsize2", "cnum", "nc", "np"}
 # Fortran dummy-argument order of every routine (from the .f95 headers; the fixture does not need the reference tree)
@@ -202,38 +204,23 @@ def test_libpxf_reproduces_the_fortran_source(fixture):
     assert n >= 53
 
 
-@pytest.mark.skipif(not refload.available(), reason="reference tree not present (GPU box)")
 def test_whole_reference_runs_here_and_equals_the_oracle_driven_reference():
-    """The reference ITSELF, end to end, in a container without a Fortran compiler: its unmodified Python layer
-    (sources / surfaces / transformations / analyses, imported from /root/reference) over its unmodified Fortran text
-    executed by oracle/f95run.py (``oracle.f95mods`` in the f2py slots) -- against the same layer over the C oracle,
-    which is how every golden fixture under tests/golden/ was produced.  All five BASELINE configurations at small
-    sizes: every ray row, surviving-index set and merit figure bit for bit."""
-    from oracle import f95mods
+    """All five BASELINE configurations at small sizes: the restatement (``oracle.refapi``) against the bits the
+    reference ITSELF gave for them -- its unmodified Python layer over its unmodified Fortran text executed by
+    oracle/f95run.py (``oracle.f95mods`` in the f2py slots) -- stored in tests/golden/reference_f95.npz: every ray
+    row, surviving-index set and merit figure bit for bit.  Where the reference tree is present, the reference over its
+    own Fortran and over the C oracle (how every golden fixture under tests/golden/ was produced) are run live and
+    compared with the fixture as well."""
+    from oracle import refapi
     from pyxfocus_b200 import examples as ex
-    src_api = ex.make_api(refload.load(f2py_modules=f95mods.modules()), ex.NumpyXP, "reference over its own Fortran")
-    runs_src = [ex.config1(src_api, 400, 3),
-                ex.config2_point(src_api, 150, 5. / 60. * np.pi / 180., ex.ws_aperture(src_api), 5),
-                ex.config2_point(src_api, 60, 24. / 60. * np.pi / 180., ex.ws_aperture(src_api), 6),
-                ex.config3(src_api, 300, 2),
-                ex.config4(src_api, 6, 20, order=-2, wave=2.4, rng_seed=4, offX=1e-4, offY=-2e-4),
-                ex.config5(src_api, 12, 20, offaxis=2e-4, rng_seed=7)]
-    orc_api = ex.make_api(refload.load(), ex.NumpyXP, "reference over the C oracle")
-    runs_orc = [ex.config1(orc_api, 400, 3),
-                ex.config2_point(orc_api, 150, 5. / 60. * np.pi / 180., ex.ws_aperture(orc_api), 5),
-                ex.config2_point(orc_api, 60, 24. / 60. * np.pi / 180., ex.ws_aperture(orc_api), 6),
-                ex.config3(orc_api, 300, 2),
-                ex.config4(orc_api, 6, 20, order=-2, wave=2.4, rng_seed=4, offX=1e-4, offY=-2e-4),
-                ex.config5(orc_api, 12, 20, offaxis=2e-4, rng_seed=7)]
-
-    def same(a, b):
-        return np.array_equal(np.asarray(a), np.asarray(b), equal_nan=True)
-    for k, (a, b) in enumerate(zip(runs_src, runs_orc)):
-        for key in a:
-            if isinstance(a[key], list):
-                assert all(same(x, y) for x, y in zip(a[key], b[key])), (k, key)
-            else:
-                assert same(a[key], b[key]), (k, key)
+    gold = np.load(os.path.join(HERE, "golden", "reference_f95.npz"))
+    assert_pinned(rc.f95_runs(ex.make_api(refapi.load(), ex.NumpyXP, "refapi")), gold, what="refapi")
+    if refload.available():
+        from oracle import f95mods
+        assert_pinned(rc.f95_runs(ex.make_api(refload.load(f2py_modules=f95mods.modules()), ex.NumpyXP,
+                                              "reference over its own Fortran")), gold, what="reference over its Fortran")
+        assert_pinned(rc.f95_runs(ex.make_api(refload.load(), ex.NumpyXP, "reference over the C oracle")), gold,
+                      what="reference over the C oracle")
 
 
 def test_translator_control_flow_and_precedence():

@@ -1,13 +1,21 @@
 """The oracle restatement (oracle/pyref.py + oracle/chains.py over the C oracle) against
 (a) the committed golden vectors, which were produced by the reference's own unmodified
-Python layer (tests/golden/make_golden.py), and (b) the live reference Python when
-/root/reference is present (build container only)."""
+Python layer (tests/golden/make_golden.py), and (b) the bits that layer gave for further calls
+(tests/golden/reference_*.npz, tests/golden/make_golden_reference_calls.py), re-checked against
+the layer live when its tree is present."""
+import os
+import sys
+
 import numpy as np
 import pytest
 
 from oracle import chains, pyref, refload
 from oracle import f2py as of
-from util import assert_bit_equal, copy, rows_of
+from util import assert_bit_equal, rows_of
+
+sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden"))
+import make_golden_reference_calls as rc  # noqa: E402
+from make_golden_reference_calls import assert_pinned  # noqa: E402
 
 
 def test_golden_wolter1_reproduced_by_restatement(golden):
@@ -55,78 +63,18 @@ def test_golden_vignette_reproduced_by_restatement(golden):
     assert_bit_equal(rays, rows_of(g["after_evan"]), what="masked radgrat")
 
 
-@pytest.mark.skipif(not refload.available(), reason="reference tree not present (GPU box)")
-def test_restatement_matches_live_reference_python():
-    """Every numpy restatement in oracle/pyref.py against the reference's own function."""
-    ref = refload.load()
-    src, tran, anal, surf, con = ref.sources, ref.transformations, ref.analyses, ref.surfaces, ref.conicsolve
-    for name, args in (("subannulus", (220., 220.6, 1.3, 5001, -1.)), ("annulus", (200., 230., 5001, 1.)),
-                       ("circularbeam", (12.5, 5001)), ("pointsource", (.03, 5001))):
-        np.random.seed(11)
-        a = getattr(src, name)(*args)
-        np.random.seed(11)
-        b = getattr(pyref, name)(*args)
-        assert_bit_equal(b, a, what=name)
-    # the set-up sources (the product generates them on the device; tests/test_gpu_parity.py compares with these)
-    for name, args in (("xslit", (-3., 5., 257, 1.)), ("rectArray", (4., 2.5, 33)),
-                       ("convergingbeam", (8400., 200., 230., -.1, .3, 4001, 1.5)),
-                       ("convergingbeam2", (8400., -20., 30., 190., 240., 4001, .5)),
-                       ("rectbeam", (12., 7., 4001)), ("gaussianBeam", (.01, 4001)),
-                       ("fanBeam", (.02, .03, 21)), ("circFan", (.05, 7, 12))):
-        np.random.seed(13)
-        a = getattr(src, name)(*args)
-        np.random.seed(13)
-        b = getattr(pyref, name)(*args)
-        assert_bit_equal(b, a, what=name)
-    rays = chains.wolter1_source(5001, 12)
-    chains.run_steps_cpu(rays, chains.wolter1_steps())
-    rays[6][::13] = np.nan
-    rays[4][::17] = 0.; rays[5][::17] = 0.; rays[6][::17] = 0.
-    assert_bit_equal(pyref.vignette(copy(rays)), tran.vignette(copy(rays)), what="vignette")
-    good = pyref.vignette(copy(rays))
-    w = np.random.default_rng(12).uniform(.2, 3., good[1].size)
-    for fn in ("centroid", "rmsCentroid", "hpd", "analyticImagePlane"):
-        for ww in (None, w):
-            assert np.array_equal(np.array(getattr(pyref, fn)(good, weights=ww)),
-                                  np.array(getattr(anal, fn)(good, weights=ww))), fn
-    ra, ca = anal.rhocdf(good, weights=w)
-    rb, cb = pyref.rhocdf(good, weights=w)
-    assert np.array_equal(ra, rb) and np.array_equal(ca, cb)
-    assert pyref.woltparam(220., 8400.) == con.woltparam(220., 8400.)
-    a, b = copy(good), copy(good)
-    assert pyref.focusI(a) == surf.focusI(b)
-    assert_bit_equal(a, b, what="focusI")
-    # the two scalar set-up formulas of analyses.py
-    from pyxfocus_b200 import analyses as panal
-    xs, ys = np.linspace(-3., 4., 11), np.linspace(1., 9., 11)
-    for u, v in zip(panal.radialGrad(xs, ys, 2e-4, .03, 11832.), anal.radialGrad(xs, ys, 2e-4, .03, 11832.)):
-        assert np.array_equal(u, v)
-    assert np.array_equal(panal.sellmeier([.5, .6, .7], [1.03, .23, 1.01], [6e-3, 2e-2, 103.]),
-                          anal.sellmeier([.5, .6, .7], [1.03, .23, 1.01], [6e-3, 2e-2, 103.]))
-    # the mirrored host-side helpers of the product package
-    import importlib
-    import sys
-    import types
-    # import the pure-numpy product modules without touching CUDA: they only need _lib lazily
-    from pyxfocus_b200 import conicsolve as pcon
-    from pyxfocus_b200 import transformations as ptran
-    for f, a in (("primrad", (8450., 220., 8400.)), ("secrad", (8350., 220., 8400.)), ("woltparam", (220., 8400.)),
-                 ("primfocus", (220., 8400.)), ("wsRMS", (1., 1e-3, 6e-3, 200., 1e4)), ("wsFoc", (3., 1., 200., 1e4, 6e-3))):
-        assert np.array_equal(np.array(getattr(pcon, f)(*a)), np.array(getattr(con, f)(*a))), f
-    for f, a in (("primsag", (8500., 220., 8400.)), ("secsag", (8300., 8400., 220., 8400.)), ("rGoal_to_rMax", (221., 8400., 8500.)),
-                 ("ellipsoidRad", (1e5, 1., 220., 8400., 8450.)), ("ehSecRad", (1e5, 1., 220., 8400., 8350.)),
-                 ("ellipsoidSag", (1e5, 1., 220., 8400., 8500., 8400.)),
-                 ("solveS", (8500., 9000., 30., .99, 8900., 0., 0., -1., 0., 0., 1.))):
-        got, want = np.array(getattr(pcon, f)(*a)), np.array(getattr(con, f)(*a))
-        assert np.all(np.isfinite(want)) and np.array_equal(got, want), f
-    for inv in (False, True):
-        assert np.allclose(ptran.rotationM(.1, -.2, .3, inverse=inv), tran.rotationM(.1, -.2, .3, inverse=inv),
-                           rtol=0, atol=1e-16)
-    assert np.array_equal(ptran.translationM(1., 2., 3.), tran.translationM(1., 2., 3.))
-    c1, c2 = ptran.newCoords(), tran.newCoords()
-    ptran._update_coords_fwd(c1, 1., 2., 3., .1, .2, .3)
-    rotm, tranm = tran.rotationM(.1, .2, .3), tran.translationM(1., 2., 3.)
-    assert np.allclose(c1[1], np.dot(np.dot(rotm, tranm), c2[1]), atol=1e-15)
+def test_restatement_matches_live_reference_python(golden):
+    """Every numpy restatement in oracle/pyref.py, and the product's mirrored host helpers, against the bits the
+    reference's own functions gave for the same calls (tests/golden/reference_python.npz); where the reference tree is
+    present, those functions live as well."""
+    gold = golden("reference_python")
+    values = rc.python_layer_values(rc.restated_python_layer())
+    for f, _ in rc.CONIC_FINITE:
+        assert np.all(np.isfinite(values["py.con." + f])), f
+    assert_pinned(values, gold, atol=rc.PYTHON_ATOL, what="restatement")
+    if refload.available():
+        assert_pinned(rc.python_layer_values(rc.reference_python_layer(refload.load())), gold, atol=rc.PYTHON_ATOL,
+                      what="reference")
 
 
 def test_golden_southwell_reproduced_by_the_oracle(golden):
@@ -158,41 +106,16 @@ def test_golden_southwell_reproduced_by_the_oracle(golden):
         assert np.array_equal(xa, g["bin_%s_xang" % tag]) and np.array_equal(ph, g["bin_%s_phase" % tag])
 
 
-@pytest.mark.skipif(not refload.available(), reason="reference tree not present (GPU box)")
-def test_interpolatevec_and_wavefront_restatements_match_the_live_reference():
-    """oracle/refapi.py interpolateVec against the reference's own function (analyses.py:189-230; both call scipy's
-    griddata) bit for bit, and wavefront (:305-334) against the reference's text run with the two things it lacks as
-    shipped supplied from outside: ``man.padRect`` (un-vendored; a one-pixel NaN frame) and a ``reconstruct`` whose
-    ``maxiter`` has a default (the reference omits the required argument, :327)."""
+def test_interpolatevec_and_wavefront_restatements_match_the_live_reference(golden):
+    """oracle/refapi.py interpolateVec (analyses.py:189-230; both call scipy's griddata) and wavefront (:305-334)
+    against the bits the reference's text gave for the same calls (tests/golden/reference_interp.npz), run with the
+    two things it lacks as shipped supplied from outside (``make_golden_reference_calls.reference_interp``); where the
+    reference tree is present, that text live as well."""
     pytest.importorskip("scipy.interpolate")
-    from oracle import f2py as of, refapi
-    ref = refload.load()
-    anal = ref.analyses
-    rng = np.random.default_rng(4)
-    n = 3000
-    r, t = 12.5 * np.sqrt(rng.uniform(0, 1, n)), rng.uniform(0, 2 * np.pi, n)
-    x, y = r * np.cos(t), r * np.sin(t)
-    l, m = 1e-3 * np.sin(x / 5.) + 1e-5 * rng.normal(size=n), 1e-3 * np.cos(y / 7.) + 1e-5 * rng.normal(size=n)
-    zero = np.zeros(n)
-    rays = [zero.copy(), x, y, zero.copy(), l, m, np.sqrt(1 - l ** 2 - m ** 2), zero.copy(), zero.copy(), zero + 1.]
-    for kw in (dict(method="linear"), dict(method="nearest"), dict(method="cubic"), dict(method="linear", polar=True),
-               dict(method="linear", xr=[-3., 9.], yr=[-14., 2.], interpVec=x * y)):
-        import warnings
-        with warnings.catch_warnings():
-            warnings.simplefilter("ignore")
-            a = anal.interpolateVec(copy(rays), 4, 31, 23, **kw)
-        b = refapi.interpolateVec(copy(rays), 4, 31, 23, **kw)
-        assert np.array_equal(a[0], b[0], equal_nan=True) and a[1] == b[1] and a[2] == b[2], kw
-
-    def pad_rect(img):
-        out = np.full((img.shape[0] + 2, img.shape[1] + 2), np.nan)
-        out[1:-1, 1:-1] = img
-        return out
-    anal.man.padRect = pad_rect
-    anal.reconstruct.reconstruct = lambda xa, ya, crit, h, ph, maxiter=500: of.reconstruct.reconstruct(xa, ya, crit, h, ph, maxiter)
+    gold = golden("reference_interp")
+    values = rc.interp_values(*rc.restated_interp())
     for method in ("linear", "cubic"):
-        a = anal.wavefront(copy(rays), 20, 16, method=method)
-        b = refapi.wavefront(copy(rays), 20, 16, method=method, maxiter=500)
-        for u, v in zip(a, b):
-            assert np.array_equal(u, v, equal_nan=True), method
-        assert np.isfinite(a[0]).sum() > 50
+        assert np.isfinite(values["interp.wf.%s.0" % method]).sum() > 50, method
+    assert_pinned(values, gold, what="restatement")
+    if refload.available():
+        assert_pinned(rc.interp_values(*rc.reference_interp(refload.load())), gold, what="reference")
