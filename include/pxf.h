@@ -512,6 +512,44 @@ int pxf_hpd_from_sums_dev(const double *x, const double *y, int64_t num, const d
 /* host-result convenience of the above (synchronises; falls back to the five-pass select itself) */
 int pxf_hpd_with_sums(const double *x, const double *y, int64_t num, const double *sums_dev,
                       double *hpd_host, pxf_stream_t stream);
+/* ---- per-segment analyses of a segmented bundle -------------------------------------------------
+ * The bundle is a concatenation of nseg segments, segment s = rays [seg_start[s], seg_start[s+1]) with
+ * seg_start_dev a device int64[nseg+1], seg_start[0] == 0 (the layout of pxf_trace_program_segmented).  Each call
+ * does what the single-bundle call does, once per segment, in a number of launches that does not depend on nseg.
+ *   pxf_segment_counts : counts_dev[s] = #(flags != 0) in segment s (device int64[nseg]); one pass over the flags.
+ *                        The segments of the bundle pxf_compact_scatter makes are the exclusive scan of the counts.
+ *   pxf_sums_segmented : the PXF_SUMS_* sums of every segment, out_dev = device double[nseg][16] (entries past the
+ *                        mode's count are 0).  z is needed by PXF_SUMS_IMAGEPLANE_Z / PXF_SUMS_POINT; ab_dev is the
+ *                        per-segment centre, double[nseg][2] for PXF_SUMS_RMS, (px,py,pz) double[nseg][3] for
+ *                        PXF_SUMS_POINT.  The per-ray arithmetic is that of pxf_sums; each segment's sums are
+ *                        folded in a fixed order (same bits on every run for the same bundle and layout, no
+ *                        floating-point atomics).  scratch: pxf_sums_segmented_scratch_bytes(num, nseg).
+ *   pxf_centroids_segmented : cxy_dev[s] = {sums[s][1] / sums[s][0], sums[s][2] / sums[s][0]}.
+ *   pxf_hpd_segmented  : analyses.hpd (analyses.py:88-97) of every segment, out_dev = device double[nseg][4] =
+ *                        {HPD, lower, upper, valid}.  sums_dev = pxf_sums_segmented(PXF_SUMS_CENTROID) output (with
+ *                        the same weights); radii are taken about exactly that centroid.
+ *                        Unweighted (w == NULL): 2*median of the radii (np.median: mean of the two middle values,
+ *                        NaN if the segment is empty or has a NaN radius); lower/upper = the middle order statistics.
+ *                        Segments of up to 8192 rays are sorted in shared memory; larger ones are bracketed from a
+ *                        strided sample, ONE pass over the bundle collects the radii inside every bracket and the
+ *                        exact pair is selected among them.  valid == 0 flags a segment whose bracket missed or whose
+ *                        candidates overflowed: resolve it with pxf_hpd_from_sums_dev(mode 1) on its slice.
+ *                        mode 1 runs that five-pass select for every segment (reads seg_start back; for tests).
+ *                        Weighted: r[argmin|cdf-.75|] - r[argmin|cdf-.25|] with the cdf taken within the segment
+ *                        (stable sort by (segment, radius), cumulative weights restarted per segment, first
+ *                        minimisers); upper/lower = r75/r25.  A segment with no rays or zero total weight gives NaN.
+ *                        workspace: pxf_hpd_segmented_workspace_bytes(num, nseg, w != NULL). */
+int pxf_segment_counts(const uint8_t *flags, int64_t num, const int64_t *seg_start_dev, int32_t nseg,
+                       int64_t *counts_dev, pxf_stream_t stream);
+size_t pxf_sums_segmented_scratch_bytes(int64_t num, int32_t nseg);
+int pxf_sums_segmented(int32_t mode, const double *x, const double *y, const double *z, const double *l,
+                       const double *m, const double *n, const double *w, int64_t num, const int64_t *seg_start_dev,
+                       int32_t nseg, const double *ab_dev, double *out_dev, void *scratch, pxf_stream_t stream);
+int pxf_centroids_segmented(const double *sums_dev, int32_t nseg, double *cxy_dev, pxf_stream_t stream);
+size_t pxf_hpd_segmented_workspace_bytes(int64_t num, int32_t nseg, int32_t weighted);
+int pxf_hpd_segmented(const double *x, const double *y, const double *w, int64_t num, const int64_t *seg_start_dev,
+                      int32_t nseg, const double *sums_dev, double *out_dev, void *workspace, int32_t mode,
+                      pxf_stream_t stream);
 /* rows_out[r][i] = rows_in[r][idx[i]] for nrows <= 16 rows (vignette with an index array,
  * transformations.py:225).  rows_in/rows_out are HOST arrays of device pointers;
  * table_scratch: >= 256 B device. */

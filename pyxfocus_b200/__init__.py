@@ -20,7 +20,7 @@ _lib.lib()      # fail loudly if libpxf.so is missing
 
 from . import conicsolve, program, sources, transformations, surfaces, analyses, dist, host  # noqa: E402,F401
 from . import transformationsf, surfacesf, woltsurf, zernsurf, reconstruct, southwell, examples  # noqa: E402,F401
-from .program import FanAux, Program, SegmentedProgram, fused  # noqa: E402,F401
+from .program import FanAux, Program, SegmentedProgram, Segments, fused  # noqa: E402,F401
 from ._lib import OPT_WS_LIBM, OPT_WS_RETRACE, OPT_WS_GRAZE_PPM, PxfError, jit_status, last_trace_kernel, launch_count, set_option  # noqa: E402,F401
 
 __version__ = "0.1.0"

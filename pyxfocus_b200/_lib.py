@@ -139,6 +139,12 @@ SIGNATURES = {
     "pxf_hpd_unweighted_dev": (_c.c_int, [_dp, _dp, _i64, _dp, _vp, _i32, _st]),
     "pxf_hpd_from_sums_dev": (_c.c_int, [_dp, _dp, _i64, _dp, _dp, _vp, _i32, _st]),
     "pxf_hpd_with_sums": (_c.c_int, [_dp, _dp, _i64, _dp, _vp, _st]),
+    "pxf_segment_counts": (_c.c_int, [_vp, _i64, _vp, _i32, _vp, _st]),
+    "pxf_sums_segmented_scratch_bytes": (_sz, [_i64, _i32]),
+    "pxf_sums_segmented": (_c.c_int, [_i32] + [_dp] * 7 + [_i64, _vp, _i32, _dp, _dp, _vp, _st]),
+    "pxf_centroids_segmented": (_c.c_int, [_dp, _i32, _dp, _st]),
+    "pxf_hpd_segmented_workspace_bytes": (_sz, [_i64, _i32, _i32]),
+    "pxf_hpd_segmented": (_c.c_int, [_dp, _dp, _dp, _i64, _vp, _i32, _dp, _dp, _vp, _i32, _st]),
     "pxf_centroid": (_c.c_int, [_dp, _dp, _dp, _i64, _vp, _vp, _st]),
     "pxf_rmscentroid": (_c.c_int, [_dp, _dp, _dp, _i64, _vp, _st]),
     "pxf_hpd": (_c.c_int, [_dp, _dp, _dp, _i64, _vp, _st]),

@@ -31,11 +31,49 @@ def _ptr(t):
     return t.data_ptr() if t is not None else None
 
 
-def centroid(rays, weights=None):
-    """Centroid of the rays in the xy plane (np.average semantics)."""
+# ---- segmented bundles: ``segments=`` (a ``program.Segments``) gives every quantity per segment, as an
+# np.ndarray[nseg], in a number of launches that does not depend on nseg and ONE read-back of the nseg results.
+# A segment with no rays, or with zero total weight, gives NaN for every quantity.
+def _seg_sums(mode, x, y, w, segments, z=None, l=None, m=None, n=None, ab=None):
+    """Device [nseg, 16] per-segment sums of ``pxf_sums_segmented``."""
+    segments.check(x.shape[0], x.device)
+    dev = x.device
+    L = _lib.lib()
+    out = torch.empty((segments.nseg, 16), dtype=torch.float64, device=dev)
+    with torch.cuda.device(dev):
+        scratch = torch.empty(int(L.pxf_sums_segmented_scratch_bytes(x.shape[0], segments.nseg)), dtype=torch.uint8,
+                              device=dev)
+        _lib.check(L.pxf_sums_segmented(mode, x.data_ptr(), y.data_ptr(), _ptr(z), _ptr(l), _ptr(m), _ptr(n), _ptr(w),
+                                        x.shape[0], segments.start_dev.data_ptr(), segments.nseg, _ptr(ab), out.data_ptr(),
+                                        scratch.data_ptr(), stream_ptr(dev)))
+    return out
+
+
+def _nan_where_empty(v, S0):
+    v = np.array(v, dtype=np.float64)
+    v[S0 == 0] = np.nan
+    return v
+
+
+def _seg_rms(x, y, w, segments):
+    sums = _seg_sums(0, x, y, w, segments)
+    cxy = torch.empty((segments.nseg, 2), dtype=torch.float64, device=x.device)
+    with torch.cuda.device(x.device):
+        _lib.check(_lib.lib().pxf_centroids_segmented(sums.data_ptr(), segments.nseg, cxy.data_ptr(), stream_ptr(x.device)))
+    S = _seg_sums(1, x, y, w, segments, ab=cxy).cpu().numpy()
+    with np.errstate(divide="ignore", invalid="ignore"):
+        return _nan_where_empty(np.sqrt(S[:, 1] / S[:, 0]), S[:, 0])
+
+
+def centroid(rays, weights=None, segments=None):
+    """Centroid of the rays in the xy plane (np.average semantics).  ``segments``: ``(cx[nseg], cy[nseg])``."""
     flush(rays)
     x, y = rays[1:3]
     w = _w(weights, x)
+    if segments is not None:
+        S = _seg_sums(0, x, y, w, segments).cpu().numpy()
+        with np.errstate(divide="ignore", invalid="ignore"):
+            return _nan_where_empty(S[:, 1] / S[:, 0], S[:, 0]), _nan_where_empty(S[:, 2] / S[:, 0], S[:, 0])
     cx, cy = ctypes.c_double(), ctypes.c_double()
     with torch.cuda.device(x.device):
         _lib.check(_lib.lib().pxf_centroid(x.data_ptr(), y.data_ptr(), _ptr(w), x.shape[0], ctypes.byref(cx),
@@ -43,11 +81,14 @@ def centroid(rays, weights=None):
     return cx.value, cy.value
 
 
-def rmsCentroid(rays, weights=None):
-    """RMS distance of the rays from their centroid in the xy plane."""
+def rmsCentroid(rays, weights=None, segments=None):
+    """RMS distance of the rays from their centroid in the xy plane (``segments``: per segment, about its own
+    centroid)."""
     flush(rays)
     x, y = rays[1:3]
     w = _w(weights, x)
+    if segments is not None:
+        return _seg_rms(x, y, w, segments)
     out = ctypes.c_double()
     with torch.cuda.device(x.device):
         _lib.check(_lib.lib().pxf_rmscentroid(x.data_ptr(), y.data_ptr(), _ptr(w), x.shape[0], ctypes.byref(out),
@@ -55,10 +96,12 @@ def rmsCentroid(rays, weights=None):
     return out.value
 
 
-def _rms1(v, weights):
+def _rms1(v, weights, segments=None):
     # 1-D analogue of rmsCentroid: feed the same row as x and a zero-extent y
     w = _w(weights, v)
     zero = torch.zeros_like(v)
+    if segments is not None:
+        return _seg_rms(v, zero, w, segments)
     out = ctypes.c_double()
     with torch.cuda.device(v.device):
         _lib.check(_lib.lib().pxf_rmscentroid(v.data_ptr(), zero.data_ptr(), _ptr(w), v.shape[0],
@@ -66,16 +109,16 @@ def _rms1(v, weights):
     return out.value
 
 
-def rmsX(rays, weights=None):
+def rmsX(rays, weights=None, segments=None):
     """RMS from centroid in the X direction (analyses.py:46-51)."""
     flush(rays)
-    return _rms1(rays[1], weights)
+    return _rms1(rays[1], weights, segments)
 
 
-def rmsY(rays, weights=None):
+def rmsY(rays, weights=None, segments=None):
     """RMS from centroid in the Y direction (analyses.py:53-58)."""
     flush(rays)
-    return _rms1(rays[2], weights)
+    return _rms1(rays[2], weights, segments)
 
 
 def rho(rays, weights=None, cent=False):
@@ -127,15 +170,20 @@ def rhocdf(rays, weights=None, cent=True):
     return rs, cdf
 
 
-def hpd(rays, weights=None, cent=True, sums=None):
+def hpd(rays, weights=None, cent=True, sums=None, segments=None):
     """Half-power diameter about the centroid (the reference ignores ``cent``,
     analyses.py:90).  Unweighted: 2*median(r).  Weighted:
     r[argmin|cdf-.75|] - r[argmin|cdf-.25|].
     ``sums`` (unweighted only): the centroid sums ``Program.run(..., sums=...)`` produced for
-    this very bundle; saves the pass over x,y that computes them."""
+    this very bundle; saves the pass over x,y that computes them.
+    ``segments``: the HPD of every segment about its own centroid (np.ndarray[nseg]); not with ``sums``."""
     flush(rays)
     x, y = rays[1:3]
     w = _w(weights, x)
+    if segments is not None:
+        if sums is not None:
+            raise ValueError("hpd: segments= and sums= cannot be combined")
+        return _hpd_seg(x, y, w, segments)
     out = ctypes.c_double()
     with torch.cuda.device(x.device):
         if sums is not None and w is None:
@@ -145,6 +193,30 @@ def hpd(rays, weights=None, cent=True, sums=None):
             _lib.check(_lib.lib().pxf_hpd(x.data_ptr(), y.data_ptr(), _ptr(w), x.shape[0], ctypes.byref(out),
                                           stream_ptr(x.device)))
     return out.value
+
+
+def _hpd_seg(x, y, w, segments, mode=0, raw=False):
+    """Per-segment ``pxf_hpd_segmented``; segments it flags (bracket miss / candidate overflow: rare) are resolved
+    by the five-pass select on their slice.  ``raw``: the [nseg, 4] {HPD, lower, upper, valid} rows."""
+    sums = _seg_sums(0, x, y, w, segments)
+    dev, num, ns = x.device, x.shape[0], segments.nseg
+    L = _lib.lib()
+    out = torch.empty((ns, 4), dtype=torch.float64, device=dev)
+    with torch.cuda.device(dev):
+        ws = torch.empty(int(L.pxf_hpd_segmented_workspace_bytes(num, ns, 0 if w is None else 1)), dtype=torch.uint8,
+                         device=dev)
+        _lib.check(L.pxf_hpd_segmented(x.data_ptr(), y.data_ptr(), _ptr(w), num, segments.start_dev.data_ptr(), ns,
+                                       sums.data_ptr(), out.data_ptr(), ws.data_ptr(), mode, stream_ptr(dev)))
+        h = out.cpu().numpy()
+        bad = np.nonzero(h[:, 3] == 0)[0]
+        if bad.size:
+            fws = hpd_workspace(0, dev)
+            for k in bad:
+                a, b = int(segments.start[k]), int(segments.start[k + 1])
+                _lib.check(L.pxf_hpd_from_sums_dev(x[a:].data_ptr(), y[a:].data_ptr(), b - a, sums[k].data_ptr(),
+                                                   out[k].data_ptr(), fws.data_ptr(), 1, stream_ptr(dev)))
+            h[bad] = out[bad].cpu().numpy()
+    return h if raw else h[:, 0].copy()
 
 
 def hpd_workspace(num, device):
@@ -166,11 +238,22 @@ def hpd_enqueue(rays, out, workspace, sums=None, mode=0):
     return out
 
 
-def analyticImagePlane(rays, weights=None):
+def analyticImagePlane(rays, weights=None, segments=None):
     """Axial shift to the best image plane, Ron Elsner's analytic method (analyses.py:118-133)."""
     flush(rays)
     x, y, z, l, m, n = rays[1:7]
     w = _w(weights, x)
+    if segments is not None:
+        h = imageplane_sums(rays, weights, segments=segments).cpu().numpy()
+        W = h[:, 0]
+        with np.errstate(divide="ignore", invalid="ignore"):
+            # pxf_analyticimageplane's arithmetic, per segment
+            ax_, ay_, aln, amn = h[:, 1] / W, h[:, 2] / W, h[:, 3] / W, h[:, 4] / W
+            bx = h[:, 5] / W - ax_ * aln
+            ax = h[:, 7] / W - aln * aln
+            by = h[:, 6] / W - ay_ * amn
+            ay = h[:, 8] / W - amn * amn
+            return _nan_where_empty(-(bx + by) / (ax + ay), W)
     out = ctypes.c_double()
     with torch.cuda.device(x.device):
         _lib.check(_lib.lib().pxf_analyticimageplane(x.data_ptr(), y.data_ptr(), l.data_ptr(), m.data_ptr(),
@@ -179,14 +262,17 @@ def analyticImagePlane(rays, weights=None):
     return out.value
 
 
-def imageplane_sums(rays, weights=None, at_z0=False):
+def imageplane_sums(rays, weights=None, at_z0=False, segments=None):
     """The nine weighted sums behind ``analyticImagePlane`` / ``findimageplane`` as a device
     tensor [S0, Sx, Sy, Sa, Sb, Sxa, Syb, Saa, Sbb] with a=l/n, b=m/n (one pass, 40 B/ray).
     ``at_z0``: take x, y where each ray crosses z = 0, (x - z a, y - z b) (48 B/ray) -- what a plane scan needs
-    when the rays are not on the plane; ``analyticImagePlane`` itself ignores z (analyses.py:122-131)."""
+    when the rays are not on the plane; ``analyticImagePlane`` itself ignores z (analyses.py:122-131).
+    ``segments``: a device [nseg, 9] tensor, one row of sums per segment."""
     flush(rays)
     x, y, z, l, m, n = rays[1:7]
     w = _w(weights, x)
+    if segments is not None:
+        return _seg_sums(3 if at_z0 else 2, x, y, w, segments, z=z, l=l, m=m, n=n)[:, :9]
     L = _lib.lib()
     dev = x.device
     out = torch.zeros(16, dtype=torch.float64, device=dev)
@@ -201,7 +287,7 @@ def imageplane_sums(rays, weights=None, at_z0=False):
     return out[:9]
 
 
-def findimageplane(rays, zscan, num, weights=None, sums=None, moved=0.):
+def findimageplane(rays, zscan, num, weights=None, sums=None, moved=0., segments=None):
     """Scan the axial offset over ``linspace(-zscan, zscan, num)`` and return the offset of
     minimum RMS spot radius about the centroid.
 
@@ -214,7 +300,24 @@ def findimageplane(rays, zscan, num, weights=None, sums=None, moved=0.):
     after ``transform(rays,0,0,dz,...)`` without a ``flat`` -- scan as the literal loop would): one pass over the
     bundle instead of ``num`` passes.  ``sums`` / ``moved``: sums from an earlier ``imageplane_sums(rays,
     at_z0=True)`` and the z offset the frame has been moved by since (``transform(rays,0,0,moved,...)``): a second,
-    finer scan then costs no pass at all."""
+    finer scan then costs no pass at all.
+    ``segments``: the offset of every segment (np.ndarray[nseg]); ``sums`` is then the [nseg, 9] output of
+    ``imageplane_sums(rays, at_z0=True, segments=...)`` and ``moved`` a scalar or one offset per segment."""
+    if segments is not None:
+        S = (sums if sums is not None else imageplane_sums(rays, weights, at_z0=True, segments=segments)).cpu().numpy()
+        S = S.copy()
+        mv = np.broadcast_to(np.asarray(moved, dtype=np.float64), (S.shape[0],))
+        sh = mv != 0.
+        for k, j in ((1, 3), (2, 4), (5, 7), (6, 8)):
+            S[sh, k] += mv[sh] * S[sh, j]
+        W = S[:, 0]
+        with np.errstate(divide="ignore", invalid="ignore"):
+            mx, my, ma, mb = S[:, 1] / W, S[:, 2] / W, S[:, 3] / W, S[:, 4] / W
+            vxx = S[:, 7] / W - ma * ma + S[:, 8] / W - mb * mb
+            cxa = S[:, 5] / W - mx * ma + S[:, 6] / W - my * mb
+        dz = np.linspace(-zscan, zscan, int(num))
+        merit = 2 * dz[None, :] * cxa[:, None] + dz[None, :] ** 2 * vxx[:, None]
+        return _nan_where_empty(dz[np.argmin(merit, axis=1)], W)
     S = (sums if sums is not None else imageplane_sums(rays, weights, at_z0=True)).cpu().numpy().copy()
     if moved != 0.:
         # the new z = 0 plane lies `moved` further along: x0' = x0 + moved a, y0' = y0 + moved b
@@ -229,26 +332,36 @@ def findimageplane(rays, zscan, num, weights=None, sums=None, moved=0.):
     return float(dz[np.argmin(merit)])
 
 
-def _plane_sums(rays, weights):
+def _plane_sums(rays, weights, segments=None):
+    if segments is not None:
+        S = imageplane_sums(rays, weights, segments=segments).cpu().numpy().T      # [9, nseg]
+        with np.errstate(divide="ignore", invalid="ignore"):
+            return _nan_where_empty(S / S[0], np.broadcast_to(S[0], S.shape))
     S = imageplane_sums(rays, weights).cpu().numpy()
     W = S[0]
     return S / W
 
 
-def analyticYPlane(rays, weights=None):
+def analyticYPlane(rays, weights=None, segments=None):
     """Axial shift to the best line focus in y (analyses.py:135-144); same one-pass sums as
     ``analyticImagePlane``."""
-    a = _plane_sums(rays, weights)      # [1, <x>, <y>, <l/n>, <m/n>, <x l/n>, <y m/n>, <(l/n)^2>, <(m/n)^2>]
+    a = _plane_sums(rays, weights, segments)      # [1, <x>, <y>, <l/n>, <m/n>, <x l/n>, <y m/n>, <(l/n)^2>, <(m/n)^2>]
     by = a[6] - a[2] * a[4]
     ay = a[8] - a[4] ** 2
+    if segments is not None:
+        with np.errstate(divide="ignore", invalid="ignore"):
+            return -by / ay
     return float(-by / ay)
 
 
-def analyticXPlane(rays, weights=None):
+def analyticXPlane(rays, weights=None, segments=None):
     """Axial shift to the best line focus in x (analyses.py:146-155)."""
-    a = _plane_sums(rays, weights)
+    a = _plane_sums(rays, weights, segments)
     bx = a[5] - a[1] * a[3]
     ax = a[7] - a[3] ** 2
+    if segments is not None:
+        with np.errstate(divide="ignore", invalid="ignore"):
+            return -bx / ax
     return float(-bx / ax)
 
 

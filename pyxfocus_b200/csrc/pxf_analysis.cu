@@ -841,6 +841,24 @@ k_cand_scan(const unsigned int *__restrict__ fhist, const unsigned long long *__
     cand_scan_block(sh, counters, ~0ull, k0, k1, fs, wsum, found);
 }
 
+// ascending bitonic sort of m (a power of two) NaN-free keys in shared memory; all threads of the CTA call
+PXF_DEV void block_bitonic_sort(double *srt, unsigned int m)
+{
+    for (unsigned int k = 2; k <= m; k <<= 1) {
+        for (unsigned int j = k >> 1; j > 0; j >>= 1) {
+            for (unsigned int t = threadIdx.x; t < m; t += blockDim.x) {
+                const unsigned int u = t ^ j;
+                if (u > t) {
+                    const double a = srt[t], b = srt[u];
+                    const bool up = (t & k) == 0;
+                    if ((a > b) == up) { srt[t] = b; srt[u] = a; }
+                }
+            }
+            __syncthreads();
+        }
+    }
+}
+
 __global__ void __launch_bounds__(PXF_BLOCK)
 k_cand_finish(const double *__restrict__ cand, unsigned long long cap, const unsigned long long *__restrict__ ncand_ptr,
               const double *__restrict__ lohi, FastSel *__restrict__ fs, double *__restrict__ fin,
@@ -899,19 +917,7 @@ k_cand_finish(const double *__restrict__ cand, unsigned long long cap, const uns
     for (unsigned int t = threadIdx.x; t < m; t += blockDim.x)
         srt[t] = t < n ? __ldcg(&fin[t]) : __longlong_as_double(0x7ff0000000000000ll);
     __syncthreads();
-    for (unsigned int k = 2; k <= m; k <<= 1) {
-        for (unsigned int j = k >> 1; j > 0; j >>= 1) {
-            for (unsigned int t = threadIdx.x; t < m; t += blockDim.x) {
-                const unsigned int u = t ^ j;
-                if (u > t) {
-                    const double a = srt[t], b = srt[u];
-                    const bool up = (t & k) == 0;
-                    if ((a > b) == up) { srt[t] = b; srt[u] = a; }
-                }
-            }
-            __syncthreads();
-        }
-    }
+    block_bitonic_sort(srt, m);
     if (threadIdx.x == 0) {
         const double a = srt[i0], b = srt[i1];
         out[0] = ((a + b) / 2.) * 2.;
@@ -1073,6 +1079,362 @@ k_gather_rows(const __grid_constant__ RowTable T, int nrows, const long long *__
     for (int64_t i = tid; i < count; i += nthr) {
         const long long s = idx[i];
         for (int r = 0; r < nrows; r++) T.out[r][i] = T.in[r][s];
+    }
+}
+
+// ------------------------------------------------------------------ segmented bundles
+// Per-segment versions of the analyses for a bundle that is a concatenation of segments (seg_start[0..nseg],
+// the layout of SegmentedProgram).  Every kernel walks the bundle in tiles with seg_tile_pieces; the launch count
+// does not depend on nseg.
+//
+// Sums: a tile of SEGSUM_TILE rays splits into pieces (tile t, segment s); walking the bundle in order, each
+// piece advances t or s or both, so slot = t + s is unique and the slots of one segment are contiguous
+// ([start/T + s, (end-1)/T + s]).  One partial per slot, then one CTA per segment folds its slots in a fixed
+// tree: the same bits on every run for the same bundle and layout, whatever the grid.
+#define SEGSUM_TILE 4096
+
+PXF_DEV void block_sum_store(const double *acc, int ns, double *__restrict__ out, double (*sh)[PXF_BLOCK / 32])
+{
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    for (int k = 0; k < ns; k++) {
+        double v = acc[k];
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) v += __shfl_down_sync(0xffffffffu, v, o);
+        if (lane == 0) sh[k][warp] = v;
+    }
+    __syncthreads();
+    if (warp == 0) {
+        for (int k = 0; k < ns; k++) {
+            double v = lane < PXF_BLOCK / 32 ? sh[k][lane] : 0.;
+#pragma unroll
+            for (int o = 4; o > 0; o >>= 1) v += __shfl_down_sync(0xffffffffu, v, o);
+            if (lane == 0) out[k] = v;
+        }
+    }
+    __syncthreads();
+}
+
+template <int MODE, bool VEC2>
+__global__ void __launch_bounds__(PXF_BLOCK)
+k_sums_seg(const double *__restrict__ x, const double *__restrict__ y, const double *__restrict__ z,
+           const double *__restrict__ l, const double *__restrict__ m, const double *__restrict__ n,
+           const double *__restrict__ w, int64_t num, const long long *__restrict__ seg_start, int nseg,
+           const double *__restrict__ ab_dev, double *__restrict__ partial)
+{
+    constexpr int NS = MODE == PXF_SUMS_CENTROID ? 4 : ((MODE == PXF_SUMS_RMS || MODE == PXF_SUMS_POINT) ? 2 : 9);
+    constexpr bool IP = MODE == PXF_SUMS_IMAGEPLANE || MODE == PXF_SUMS_IMAGEPLANE_Z;
+    constexpr bool ZZ = MODE == PXF_SUMS_IMAGEPLANE_Z || MODE == PXF_SUMS_POINT;
+    constexpr int U = IP ? 2 : 4;
+    __shared__ double sh[NSUM][PXF_BLOCK / 32];
+    const bool has_w = w != nullptr;
+    // one ray through sums_accum, loaded with scalar loads (odd ends of a piece, unaligned rows)
+    auto one = [&](double *acc, int64_t i, double a, double b, double c) {
+        sums_accum<MODE>(acc, x[i], y[i], IP ? l[i] : 0., IP ? m[i] : 0., IP ? n[i] : 1., has_w ? w[i] : 1., has_w, a, b,
+                         ZZ ? z[i] : 0., c);
+    };
+    for (int64_t t0 = (int64_t)blockIdx.x * SEGSUM_TILE; t0 < num; t0 += (int64_t)gridDim.x * SEGSUM_TILE) {
+        const int64_t t1 = t0 + SEGSUM_TILE < num ? t0 + SEGSUM_TILE : num;
+        const int64_t tile = t0 / SEGSUM_TILE;
+        seg_tile_pieces(t0, t1, seg_start, nseg, [&](int seg, int64_t pa, int64_t pb) {
+            double a = 0., b = 0., c = 0.;
+            if (MODE == PXF_SUMS_RMS) { a = ab_dev[2 * seg]; b = ab_dev[2 * seg + 1]; }
+            if (MODE == PXF_SUMS_POINT) { a = ab_dev[3 * seg]; b = ab_dev[3 * seg + 1]; c = ab_dev[3 * seg + 2]; }
+            double acc[U][NSUM];
+#pragma unroll
+            for (int u = 0; u < U; u++)
+#pragma unroll
+                for (int k = 0; k < NSUM; k++) acc[u][k] = 0.;
+            if (VEC2) {
+                // pairs at even bundle indices (the 16-byte alignment of the rows), odd ends one by one
+                const int64_t q0 = (pa + 1) >> 1, q1 = pb >> 1;
+                for (int64_t qb = q0 + threadIdx.x; qb < q1; qb += U * blockDim.x) {
+                    double2 xv[U], yv[U], lv[U], mv[U], nv[U], wv[U], zv[U];
+#pragma unroll
+                    for (int u = 0; u < U; u++) {
+                        const int64_t q = qb + u * blockDim.x;
+                        const bool in = q < q1;
+                        const double2 z2 = make_double2(0., 0.), o2 = make_double2(1., 1.);
+                        xv[u] = in ? *reinterpret_cast<const double2 *>(x + 2 * q) : z2;
+                        yv[u] = in ? *reinterpret_cast<const double2 *>(y + 2 * q) : z2;
+                        if (IP) {
+                            lv[u] = in ? *reinterpret_cast<const double2 *>(l + 2 * q) : z2;
+                            mv[u] = in ? *reinterpret_cast<const double2 *>(m + 2 * q) : z2;
+                            nv[u] = in ? *reinterpret_cast<const double2 *>(n + 2 * q) : o2;
+                        } else { lv[u] = z2; mv[u] = z2; nv[u] = o2; }
+                        zv[u] = (ZZ && in) ? *reinterpret_cast<const double2 *>(z + 2 * q) : z2;
+                        wv[u] = (in && has_w) ? *reinterpret_cast<const double2 *>(w + 2 * q) : o2;
+                    }
+#pragma unroll
+                    for (int u = 0; u < U; u++)
+                        if (qb + u * blockDim.x < q1) {
+                            sums_accum<MODE>(acc[u], xv[u].x, yv[u].x, lv[u].x, mv[u].x, nv[u].x, wv[u].x, has_w, a, b, zv[u].x, c);
+                            sums_accum<MODE>(acc[u], xv[u].y, yv[u].y, lv[u].y, mv[u].y, nv[u].y, wv[u].y, has_w, a, b, zv[u].y, c);
+                        }
+                }
+                if (threadIdx.x == 0 && (pa & 1)) one(acc[0], pa, a, b, c);
+                if (threadIdx.x == 1 && (pb & 1) && pb - 1 >= 2 * q0) one(acc[0], pb - 1, a, b, c);
+            } else {
+                for (int64_t i = pa + threadIdx.x; i < pb; i += blockDim.x) one(acc[0], i, a, b, c);
+            }
+#pragma unroll
+            for (int k = 0; k < NS; k++) {
+                double t = acc[0][k];
+#pragma unroll
+                for (int u = 1; u < U; u++) t += acc[u][k];
+                acc[0][k] = t;
+            }
+            block_sum_store(acc[0], NS, partial + (tile + seg) * NSUM, sh);
+        });
+    }
+}
+
+// one CTA per segment: fixed-order fold of its slots; out[16 s + k], k >= ns zeroed
+__global__ void __launch_bounds__(PXF_BLOCK)
+k_sums_seg_fold(const double *__restrict__ partial, const long long *__restrict__ seg_start, int ns,
+                double *__restrict__ out)
+{
+    __shared__ double sh[NSUM][PXF_BLOCK / 32];
+    const int s = blockIdx.x;
+    const long long a = seg_start[s], b = seg_start[s + 1];
+    const long long first = b > a ? a / SEGSUM_TILE + s : 0, last = b > a ? (b - 1) / SEGSUM_TILE + s : -1;
+    double acc[NSUM];
+    for (int k = 0; k < NSUM; k++) acc[k] = 0.;
+    for (long long q = first + threadIdx.x; q <= last; q += blockDim.x)
+        for (int k = 0; k < ns; k++) acc[k] += partial[q * NSUM + k];
+    double v[NSUM];
+    block_sum_store(acc, ns, v, sh);
+    if (threadIdx.x == 0)
+        for (int k = 0; k < 16; k++) out[16 * (int64_t)s + k] = k < ns ? v[k] : 0.;
+}
+
+// cxy[2 s..] = sums[16 s + 1] / sums[16 s], sums[16 s + 2] / sums[16 s] (k_centroid_from_sums per segment)
+__global__ void k_centroids_seg(const double *__restrict__ sums, int nseg, double *__restrict__ cxy)
+{
+    for (int s = blockIdx.x * blockDim.x + threadIdx.x; s < nseg; s += gridDim.x * blockDim.x) {
+        cxy[2 * s] = sums[16 * (int64_t)s + 1] / sums[16 * (int64_t)s];
+        cxy[2 * s + 1] = sums[16 * (int64_t)s + 2] / sums[16 * (int64_t)s];
+    }
+}
+
+// survivors per segment: counts[s] += #flags != 0 (zeroed by the caller)
+__global__ void __launch_bounds__(PXF_BLOCK)
+k_seg_counts(const uint8_t *__restrict__ flags, int64_t num, const long long *__restrict__ seg_start, int nseg,
+             unsigned long long *__restrict__ counts)
+{
+    __shared__ unsigned int cnt;
+    for (int64_t t0 = (int64_t)blockIdx.x * SEGSUM_TILE; t0 < num; t0 += (int64_t)gridDim.x * SEGSUM_TILE) {
+        const int64_t t1 = t0 + SEGSUM_TILE < num ? t0 + SEGSUM_TILE : num;
+        seg_tile_pieces(t0, t1, seg_start, nseg, [&](int seg, int64_t pa, int64_t pb) {
+            if (threadIdx.x == 0) cnt = 0;
+            __syncthreads();
+            unsigned int c = 0;
+            for (int64_t i = pa + threadIdx.x; i < pb; i += blockDim.x) c += flags[i] != 0;
+#pragma unroll
+            for (int o = 16; o > 0; o >>= 1) c += __shfl_down_sync(0xffffffffu, c, o);
+            if ((threadIdx.x & 31) == 0 && c) atomicAdd(&cnt, c);
+            __syncthreads();
+            if (threadIdx.x == 0 && cnt) atomicAdd(&counts[seg], (unsigned long long)cnt);
+            __syncthreads();
+        });
+    }
+}
+
+// ---- segmented unweighted HPD: exact 2*median of every segment's radii about its own centroid
+// k_hpdseg_prepare  one CTA per segment.  Up to SEG_DIRECT rays: all radii in shared memory, bitonic sort, done.
+//                   Larger: a strided sample of SEG_DIRECT radii, sorted -> bracket [lo, hi] around the median
+//                   (sample ranks 0.5 +- 6 sigma, pxf_bracket_sample_ranks).
+// k_hpdseg_collect  ONE pass over the bundle: per bracketed segment, #(r < lo), #NaN, and the radii inside the
+//                   bracket appended to the segment's slice of the candidate buffer (capacity ~1/8 of the segment)
+// k_hpdseg_finish   one CTA per bracketed segment: 4096 linear bins over [lo, hi] locate the middle ranks, the
+//                   keys of those bins are sorted in shared memory.
+// A bracket miss, a candidate overflow or ties piling up in one bin leave valid = 0 for that segment only; the
+// caller resolves those segments with the five-pass select on their slice.
+#define SEG_DIRECT 8192
+#define SEG_CAND_DIV 8
+#define SEG_FINCAP 8192
+
+PXF_DEV double nan_d() { return __longlong_as_double(0x7ff8000000000000ll); }
+
+__global__ void __launch_bounds__(1024)
+k_hpdseg_prepare(const double *__restrict__ x, const double *__restrict__ y, const long long *__restrict__ seg_start,
+                 const double *__restrict__ sums, int ra, int rb, double *__restrict__ cxy, double *__restrict__ lohi,
+                 unsigned long long *__restrict__ counters, int *__restrict__ state, double *__restrict__ out)
+{
+    extern __shared__ double keys[];
+    const int s = blockIdx.x;
+    const long long a = seg_start[s], n = seg_start[s + 1] - a;
+    const double cx = sums[16 * (int64_t)s + 1] / sums[16 * (int64_t)s], cy = sums[16 * (int64_t)s + 2] / sums[16 * (int64_t)s];
+    double *o = out + 4 * (int64_t)s;
+    if (threadIdx.x == 0) {
+        cxy[2 * s] = cx; cxy[2 * s + 1] = cy;
+        counters[3 * (int64_t)s] = 0; counters[3 * (int64_t)s + 1] = 0; counters[3 * (int64_t)s + 2] = 0;
+        state[s] = 0;
+    }
+    if (n == 0) {                                       // np.median([]) is nan
+        if (threadIdx.x == 0) { o[0] = nan_d(); o[1] = nan_d(); o[2] = nan_d(); o[3] = 1.; }
+        return;
+    }
+    const int mcnt = n <= SEG_DIRECT ? (int)n : SEG_DIRECT;
+    bool nan = false;
+    for (int j = threadIdx.x; j < mcnt; j += blockDim.x) {
+        const long long i = a + (n <= SEG_DIRECT ? j : (long long)(((unsigned long long)j * (unsigned long long)n) / SEG_DIRECT));
+        const double r = sqrt(sq(x[i] - cx) + sq(y[i] - cy));
+        keys[j] = r;
+        nan = nan || r != r;
+    }
+    if (__syncthreads_or(nan)) {                        // a NaN radius: np.median is nan
+        if (threadIdx.x == 0) { o[0] = nan_d(); o[1] = nan_d(); o[2] = nan_d(); o[3] = 1.; }
+        return;
+    }
+    unsigned int m2 = 1;
+    while (m2 < (unsigned)mcnt) m2 <<= 1;
+    for (unsigned int t = mcnt + threadIdx.x; t < m2; t += blockDim.x) keys[t] = __longlong_as_double(0x7ff0000000000000ll);
+    __syncthreads();
+    block_bitonic_sort(keys, m2);
+    if (threadIdx.x == 0) {
+        if (n <= SEG_DIRECT) {
+            const double lo = keys[(n - 1) / 2], hi = keys[n / 2];
+            o[0] = ((lo + hi) / 2.) * 2.; o[1] = lo; o[2] = hi; o[3] = 1.;
+        } else {
+            lohi[2 * s] = keys[ra]; lohi[2 * s + 1] = keys[rb];
+            state[s] = 1;
+        }
+    }
+}
+
+#define SEGCOL_TILE 4096
+template <bool VEC2>
+__global__ void __launch_bounds__(PXF_BLOCK)
+k_hpdseg_collect(const double *__restrict__ x, const double *__restrict__ y, int64_t num,
+                 const long long *__restrict__ seg_start, int nseg, const int *__restrict__ state,
+                 const double *__restrict__ cxy, const double *__restrict__ lohi, double *__restrict__ cand,
+                 unsigned long long *__restrict__ counters)
+{
+    __shared__ double sbuf[SEGCOL_TILE];
+    __shared__ unsigned int scount, sbelow, snan;
+    __shared__ unsigned long long sbase;
+    for (int64_t t0 = (int64_t)blockIdx.x * SEGCOL_TILE; t0 < num; t0 += (int64_t)gridDim.x * SEGCOL_TILE) {
+        const int64_t t1 = t0 + SEGCOL_TILE < num ? t0 + SEGCOL_TILE : num;
+        seg_tile_pieces(t0, t1, seg_start, nseg, [&](int seg, int64_t pa, int64_t pb) {
+            if (state[seg] != 1) return;               // block-uniform
+            const double cx = cxy[2 * seg], cy = cxy[2 * seg + 1], lo = lohi[2 * seg], hi = lohi[2 * seg + 1];
+            if (threadIdx.x == 0) { scount = 0; sbelow = 0; snan = 0; }
+            __syncthreads();
+            unsigned int below = 0, nans = 0;
+            auto put = [&](double r) {
+                if (r != r) nans++;
+                else if (r < lo) below++;
+                else if (r <= hi) sbuf[atomicAdd(&scount, 1u)] = r;
+            };
+            if (VEC2) {
+                const int64_t q0 = (pa + 1) >> 1, q1 = pb >> 1;
+                for (int64_t qb = q0 + threadIdx.x; qb < q1; qb += 4 * blockDim.x) {
+                    double2 xv[4], yv[4];
+#pragma unroll
+                    for (int u = 0; u < 4; u++) {
+                        const int64_t q = qb + u * blockDim.x;
+                        xv[u] = q < q1 ? *reinterpret_cast<const double2 *>(x + 2 * q) : make_double2(0., 0.);
+                        yv[u] = q < q1 ? *reinterpret_cast<const double2 *>(y + 2 * q) : make_double2(0., 0.);
+                    }
+#pragma unroll
+                    for (int u = 0; u < 4; u++)
+                        if (qb + u * blockDim.x < q1) {
+                            put(sqrt(sq(xv[u].x - cx) + sq(yv[u].x - cy)));
+                            put(sqrt(sq(xv[u].y - cx) + sq(yv[u].y - cy)));
+                        }
+                }
+                if (threadIdx.x == 0 && (pa & 1)) put(sqrt(sq(x[pa] - cx) + sq(y[pa] - cy)));
+                if (threadIdx.x == 1 && (pb & 1) && pb - 1 >= 2 * q0) put(sqrt(sq(x[pb - 1] - cx) + sq(y[pb - 1] - cy)));
+            } else {
+                for (int64_t i = pa + threadIdx.x; i < pb; i += blockDim.x) put(sqrt(sq(x[i] - cx) + sq(y[i] - cy)));
+            }
+#pragma unroll
+            for (int o = 16; o > 0; o >>= 1) {
+                below += __shfl_down_sync(0xffffffffu, below, o);
+                nans += __shfl_down_sync(0xffffffffu, nans, o);
+            }
+            if ((threadIdx.x & 31) == 0) {
+                if (below) atomicAdd(&sbelow, below);
+                if (nans) atomicAdd(&snan, nans);
+            }
+            __syncthreads();
+            unsigned long long *c = counters + 3 * (int64_t)seg;
+            if (threadIdx.x == 0) {
+                sbase = scount ? atomicAdd(&c[1], (unsigned long long)scount) : 0ull;
+                if (sbelow) atomicAdd(&c[0], (unsigned long long)sbelow);
+                if (snan) atomicAdd(&c[2], (unsigned long long)snan);
+            }
+            __syncthreads();
+            const long long a = seg_start[seg];
+            const unsigned long long cap = (unsigned long long)(seg_start[seg + 1] / SEG_CAND_DIV - a / SEG_CAND_DIV);
+            double *dst = cand + a / SEG_CAND_DIV;
+            for (unsigned int t = threadIdx.x; t < scount; t += blockDim.x)
+                if (sbase + t < cap) dst[sbase + t] = sbuf[t];
+            __syncthreads();
+        });
+    }
+}
+
+__global__ void __launch_bounds__(1024)
+k_hpdseg_finish(const long long *__restrict__ seg_start, const int *__restrict__ state,
+                const unsigned long long *__restrict__ counters, const double *__restrict__ lohi,
+                const double *__restrict__ cand, double *__restrict__ out)
+{
+    extern __shared__ double fin[];                                   // [SEG_FINCAP] then the bins
+    unsigned int *h = reinterpret_cast<unsigned int *>(fin + SEG_FINCAP);
+    __shared__ unsigned long long wsum[32];
+    __shared__ unsigned long long found[2][2];
+    __shared__ unsigned int nfin;
+    const int s = blockIdx.x;
+    if (state[s] != 1) return;
+    double *o = out + 4 * (int64_t)s;
+    const long long a = seg_start[s], b = seg_start[s + 1], n = b - a;
+    const unsigned long long k0 = (n - 1) / 2, k1 = n / 2;
+    const unsigned long long below = counters[3 * (int64_t)s], nc = counters[3 * (int64_t)s + 1];
+    const unsigned long long cap = (unsigned long long)(b / SEG_CAND_DIV - a / SEG_CAND_DIV);
+    if (counters[3 * (int64_t)s + 2]) {
+        if (threadIdx.x == 0) { o[0] = nan_d(); o[1] = nan_d(); o[2] = nan_d(); o[3] = 1.; }
+        return;
+    }
+    if (!(nc <= cap && k0 >= below && k1 < below + nc)) {
+        if (threadIdx.x == 0) { o[0] = 0.; o[1] = 0.; o[2] = 0.; o[3] = 0.; }
+        return;
+    }
+    const double *c = cand + a / SEG_CAND_DIV;
+    const double lo = lohi[2 * s], scale = cand_scale(lo, lohi[2 * s + 1]);
+    for (int t = threadIdx.x; t < FAST_NBINS; t += blockDim.x) h[t] = 0u;
+    if (threadIdx.x < 2) { found[threadIdx.x][0] = 0ull; found[threadIdx.x][1] = 0ull; }
+    if (threadIdx.x == 0) nfin = 0;
+    __syncthreads();
+    for (unsigned long long i = threadIdx.x; i < nc; i += blockDim.x) atomicAdd(&h[cand_bin(c[i], lo, scale)], 1u);
+    __syncthreads();
+    const unsigned long long r0 = k0 - below, r1 = k1 - below;
+    block_find_bin(h, FAST_NBINS, r0, wsum, found[0]);
+    block_find_bin(h, FAST_NBINS, r1, wsum, found[1]);
+    const int ba = (int)found[0][0], bb = (int)found[1][0];
+    const unsigned long long base_a = found[0][1];
+    for (unsigned long long i = threadIdx.x; i < nc; i += blockDim.x) {
+        const double r = c[i];
+        const int bin = cand_bin(r, lo, scale);
+        if (bin >= ba && bin <= bb) {
+            const unsigned int slot = atomicAdd(&nfin, 1u);
+            if (slot < SEG_FINCAP) fin[slot] = r;
+        }
+    }
+    __syncthreads();
+    const unsigned int nf = nfin;
+    if (nf > SEG_FINCAP || r1 - base_a >= nf) {                       // ties piled up in the middle bins
+        if (threadIdx.x == 0) { o[0] = 0.; o[1] = 0.; o[2] = 0.; o[3] = 0.; }
+        return;
+    }
+    unsigned int m2 = 1;
+    while (m2 < nf) m2 <<= 1;
+    for (unsigned int t = nf + threadIdx.x; t < m2; t += blockDim.x) fin[t] = __longlong_as_double(0x7ff0000000000000ll);
+    __syncthreads();
+    block_bitonic_sort(fin, m2);
+    if (threadIdx.x == 0) {
+        const double va = fin[r0 - base_a], vb = fin[r1 - base_a];
+        o[0] = ((va + vb) / 2.) * 2.; o[1] = va; o[2] = vb; o[3] = 1.;
     }
 }
 
@@ -1776,6 +2138,160 @@ int pxf_gather_rows(const double *const *rows_in, double *const *rows_out, int32
     k_gather_rows<<<grid_for(count, PXF_BLOCK, 8), PXF_BLOCK, 0, s>>>(h, nrows, reinterpret_cast<const long long *>(idx), count);
     count_launch();
     return check_launch("k_gather_rows");
+}
+
+// ---- segmented bundles ------------------------------------------------------------------------
+static int seg_args(int64_t num, const int64_t *seg_start_dev, int32_t nseg, const char *what)
+{
+    if (num < 0 || !seg_start_dev || nseg < 1) { set_error("%s: bad argument", what); return PXF_ERR_INVALID; }
+    return need_device();
+}
+
+int pxf_segment_counts(const uint8_t *flags, int64_t num, const int64_t *seg_start_dev, int32_t nseg,
+                       int64_t *counts_dev, pxf_stream_t stream)
+{
+    int rc = seg_args(num, seg_start_dev, nseg, "pxf_segment_counts");
+    if (rc) return rc;
+    if (!counts_dev || (num > 0 && !flags)) { set_error("pxf_segment_counts: bad argument"); return PXF_ERR_INVALID; }
+    cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
+    PXF_CUDA(cudaMemsetAsync(counts_dev, 0, (size_t)nseg * 8, s));
+    if (num == 0) return PXF_OK;
+    k_seg_counts<<<grid_for(num, SEGSUM_TILE, 4), PXF_BLOCK, 0, s>>>(flags, num, reinterpret_cast<const long long *>(seg_start_dev),
+                                                                    nseg, reinterpret_cast<unsigned long long *>(counts_dev));
+    count_launch();
+    return check_launch("k_seg_counts");
+}
+
+size_t pxf_sums_segmented_scratch_bytes(int64_t num, int32_t nseg)
+{
+    const int64_t ntiles = (num > 0 ? num : 0) / SEGSUM_TILE + 1;
+    return (size_t)(ntiles + (nseg > 0 ? nseg : 0)) * NSUM * sizeof(double);
+}
+
+int pxf_sums_segmented(int32_t mode, const double *x, const double *y, const double *z, const double *l, const double *m,
+                       const double *n, const double *w, int64_t num, const int64_t *seg_start_dev, int32_t nseg,
+                       const double *ab_dev, double *out_dev, void *scratch, pxf_stream_t stream)
+{
+    int rc = seg_args(num, seg_start_dev, nseg, "pxf_sums_segmented");
+    if (rc) return rc;
+    const bool ip = mode == PXF_SUMS_IMAGEPLANE || mode == PXF_SUMS_IMAGEPLANE_Z;
+    const bool zz = mode == PXF_SUMS_IMAGEPLANE_Z || mode == PXF_SUMS_POINT;
+    if (!out_dev || !scratch || (num > 0 && (!x || !y || (ip && (!l || !m || !n)) || (zz && !z))) ||
+        ((mode == PXF_SUMS_RMS || mode == PXF_SUMS_POINT) && !ab_dev) || mode < PXF_SUMS_CENTROID || mode > PXF_SUMS_POINT) {
+        set_error("pxf_sums_segmented: bad argument");
+        return PXF_ERR_INVALID;
+    }
+    cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
+    const long long *ss = reinterpret_cast<const long long *>(seg_start_dev);
+    double *partial = static_cast<double *>(scratch);
+    const int ns = mode == PXF_SUMS_CENTROID ? 4 : ((mode == PXF_SUMS_RMS || mode == PXF_SUMS_POINT) ? 2 : 9);
+    if (num > 0) {
+        uintptr_t al = reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(y) | reinterpret_cast<uintptr_t>(w);
+        if (zz) al |= reinterpret_cast<uintptr_t>(z);
+        if (ip) al |= reinterpret_cast<uintptr_t>(l) | reinterpret_cast<uintptr_t>(m) | reinterpret_cast<uintptr_t>(n);
+        const bool v2 = (al & 15) == 0;
+        const int grid = grid_for(num, SEGSUM_TILE, 4);
+#define PXF_SEGSUMS_GO(M)                                                                                          \
+        do {                                                                                                       \
+            if (v2) k_sums_seg<M, true><<<grid, PXF_BLOCK, 0, s>>>(x, y, z, l, m, n, w, num, ss, nseg, ab_dev, partial);   \
+            else k_sums_seg<M, false><<<grid, PXF_BLOCK, 0, s>>>(x, y, z, l, m, n, w, num, ss, nseg, ab_dev, partial);    \
+        } while (0)
+        if (mode == PXF_SUMS_CENTROID) PXF_SEGSUMS_GO(PXF_SUMS_CENTROID);
+        else if (mode == PXF_SUMS_RMS) PXF_SEGSUMS_GO(PXF_SUMS_RMS);
+        else if (mode == PXF_SUMS_IMAGEPLANE) PXF_SEGSUMS_GO(PXF_SUMS_IMAGEPLANE);
+        else if (mode == PXF_SUMS_IMAGEPLANE_Z) PXF_SEGSUMS_GO(PXF_SUMS_IMAGEPLANE_Z);
+        else PXF_SEGSUMS_GO(PXF_SUMS_POINT);
+#undef PXF_SEGSUMS_GO
+        count_launch();
+    }
+    k_sums_seg_fold<<<nseg, PXF_BLOCK, 0, s>>>(partial, ss, ns, out_dev);
+    count_launch();
+    return check_launch("k_sums_seg");
+}
+
+int pxf_centroids_segmented(const double *sums_dev, int32_t nseg, double *cxy_dev, pxf_stream_t stream)
+{
+    if (!sums_dev || !cxy_dev || nseg < 1) { set_error("pxf_centroids_segmented: bad argument"); return PXF_ERR_INVALID; }
+    int rc = need_device();
+    if (rc) return rc;
+    k_centroids_seg<<<grid_for(nseg, PXF_BLOCK, 4), PXF_BLOCK, 0, reinterpret_cast<cudaStream_t>(stream)>>>(sums_dev, nseg, cxy_dev);
+    count_launch();
+    return check_launch("k_centroids_seg");
+}
+
+struct HpdSegWs { double *cxy, *lohi, *cand; unsigned long long *counters; int *state; void *fallback; };
+static size_t hpdseg_carve(HpdSegWs &w, char *base, int64_t num, int32_t nseg)
+{
+    size_t off = 0;
+    w.cxy = (double *)(base + off); off += a256((size_t)nseg * 16);
+    w.lohi = (double *)(base + off); off += a256((size_t)nseg * 16);
+    w.counters = (unsigned long long *)(base + off); off += a256((size_t)nseg * 24);
+    w.state = (int *)(base + off); off += a256((size_t)nseg * 4);
+    w.fallback = base + off; off += a256(pxf_hpd_workspace_bytes(0));
+    w.cand = (double *)(base + off); off += a256((size_t)(num / SEG_CAND_DIV + 1) * 8);
+    return off;
+}
+
+size_t pxf_hpd_segmented_workspace_bytes(int64_t num, int32_t nseg, int32_t weighted)
+{
+    HpdSegWs w;
+    if (num < 0) num = 0;
+    if (nseg < 1) nseg = 1;
+    if (weighted) return hpd_weighted_segmented_bytes(num) + 256;
+    return hpdseg_carve(w, nullptr, num, nseg) + 256;
+}
+
+int pxf_hpd_segmented(const double *x, const double *y, const double *w, int64_t num, const int64_t *seg_start_dev,
+                      int32_t nseg, const double *sums_dev, double *out_dev, void *workspace, int32_t mode,
+                      pxf_stream_t stream)
+{
+    int rc = seg_args(num, seg_start_dev, nseg, "pxf_hpd_segmented");
+    if (rc) return rc;
+    if (!sums_dev || !out_dev || !workspace || (num > 0 && (!x || !y)) || (mode != 0 && mode != 1)) {
+        set_error("pxf_hpd_segmented: bad argument");
+        return PXF_ERR_INVALID;
+    }
+    cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
+    const long long *ss = reinterpret_cast<const long long *>(seg_start_dev);
+    if (w) return hpd_weighted_segmented(x, y, w, num, ss, nseg, sums_dev, out_dev, workspace, s);
+    HpdSegWs ws;
+    hpdseg_carve(ws, static_cast<char *>(workspace), num, nseg);
+    if (mode == 1) {
+        // every segment through the five-pass select on its slice (reads the layout back: a testing aid)
+        int64_t *hs = static_cast<int64_t *>(malloc((size_t)(nseg + 1) * 8));
+        if (!hs) { set_error("pxf_hpd_segmented: out of host memory"); return PXF_ERR_INVALID; }
+        cudaError_t e = cudaMemcpyAsync(hs, seg_start_dev, (size_t)(nseg + 1) * 8, cudaMemcpyDeviceToHost, s);
+        if (e == cudaSuccess) e = cudaStreamSynchronize(s);
+        if (e != cudaSuccess) { free(hs); set_error("pxf_hpd_segmented: %s", cudaGetErrorString(e)); return PXF_ERR_CUDA; }
+        for (int sg = 0; sg < nseg && rc == 0; sg++) {
+            const int64_t a = hs[sg], cnt = hs[sg + 1] - hs[sg];
+            rc = pxf_hpd_from_sums_dev(cnt > 0 ? x + a : x, cnt > 0 ? y + a : y, cnt, sums_dev + 16 * (int64_t)sg,
+                                       out_dev + 4 * (int64_t)sg, ws.fallback, 1, stream);
+        }
+        free(hs);
+        return rc;
+    }
+    static bool smem_set[64] = {};
+    if (first_on_device(smem_set)) {
+        PXF_CUDA(cudaFuncSetAttribute(k_hpdseg_prepare, cudaFuncAttributeMaxDynamicSharedMemorySize, SEG_DIRECT * 8));
+        PXF_CUDA(cudaFuncSetAttribute(k_hpdseg_finish, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                      SEG_FINCAP * 8 + FAST_NBINS * 4));
+    }
+    int64_t ra, rb;
+    pxf_bracket_sample_ranks(SEG_DIRECT, &ra, &rb);
+    k_hpdseg_prepare<<<nseg, 1024, SEG_DIRECT * 8, s>>>(x, y, ss, sums_dev, (int)ra, (int)rb, ws.cxy, ws.lohi, ws.counters,
+                                                         ws.state, out_dev);
+    count_launch();
+    if (num > 0) {
+        const bool v2 = ((reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(y)) & 15) == 0;
+        const int grid = grid_for(num, SEGCOL_TILE, 4);
+        if (v2) k_hpdseg_collect<true><<<grid, PXF_BLOCK, 0, s>>>(x, y, num, ss, nseg, ws.state, ws.cxy, ws.lohi, ws.cand, ws.counters);
+        else k_hpdseg_collect<false><<<grid, PXF_BLOCK, 0, s>>>(x, y, num, ss, nseg, ws.state, ws.cxy, ws.lohi, ws.cand, ws.counters);
+        count_launch();
+    }
+    k_hpdseg_finish<<<nseg, 1024, SEG_FINCAP * 8 + FAST_NBINS * 4, s>>>(ss, ws.state, ws.counters, ws.lohi, ws.cand, out_dev);
+    count_launch();
+    return check_launch("pxf_hpd_segmented");
 }
 
 }  // extern "C"

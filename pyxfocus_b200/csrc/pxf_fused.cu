@@ -192,17 +192,7 @@ k_program_seg(const RowPtrs P, const RowPtrs Q, const int64_t num, uint8_t *__re
     const int words = nops * (int)(sizeof(FusedOp) / 8);
     for (int64_t t0 = (int64_t)blockIdx.x * SEG_TILE; t0 < num; t0 += (int64_t)gridDim.x * SEG_TILE) {
         const int64_t t1 = t0 + SEG_TILE < num ? t0 + SEG_TILE : num;
-        int lo = 0, hi = nseg - 1;                     // last segment starting at or before t0
-        while (lo < hi) {
-            const int mid = (lo + hi + 1) >> 1;
-            if (seg_start[mid] <= t0) lo = mid; else hi = mid - 1;
-        }
-        int seg = lo;
-        int64_t pos = t0;
-        while (pos < t1 && seg < nseg) {
-            int64_t send = seg_start[seg + 1];
-            if (send <= pos) { seg++; continue; }      // empty segment
-            if (send > t1) send = t1;
+        seg_tile_pieces(t0, t1, seg_start, nseg, [&](int seg, int64_t pos, int64_t send) {
             if (seg != staged) {                       // block-uniform
                 __syncthreads();
                 const double *src = reinterpret_cast<const double *>(ops + (int64_t)seg * nops);
@@ -220,9 +210,7 @@ k_program_seg(const RowPtrs P, const RowPtrs Q, const int64_t num, uint8_t *__re
                 fstore1(a, Q, SM, i);
                 if (alive) alive[i] = keep ? 1 : 0;
             }
-            pos = send;
-            seg++;
-        }
+        });
     }
 }
 

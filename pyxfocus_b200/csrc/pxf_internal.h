@@ -34,6 +34,11 @@ inline bool first_on_device(bool (&seen)[64])
 // Persistent grid: SM count x resident CTAs, capped by the work available.
 int grid_for(int64_t work_items, int per_block, int ctas_per_sm);
 
+// Weighted HPD of every segment of a segmented bundle (pxf_sort.cu; the entry point is pxf_hpd_segmented).
+size_t hpd_weighted_segmented_bytes(int64_t num);
+int hpd_weighted_segmented(const double *x, const double *y, const double *w, int64_t num, const long long *seg_start,
+                           int nseg, const double *sums, double *out, void *workspace, cudaStream_t s);
+
 inline int check_launch(const char *what)
 {
     cudaError_t e = cudaGetLastError();

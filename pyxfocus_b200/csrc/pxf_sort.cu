@@ -609,6 +609,193 @@ static int onesweep_passes(const double *keys_in, u64 *kA, u64 *kB, u32 *vA, u32
 }
 
 
+// ------------------------------------------------------------------ segmented weighted HPD
+// analyses.hpd(rays, weights) of every segment of a segmented bundle: radii about each segment's centroid, ONE
+// stable sort by (segment, radius) -- the radius digits first, then a stable sort of the segment ids, so every
+// segment's rays end up in its own slice [seg_start[s], seg_start[s+1]) in radius order, ties in input order as
+// in the single-bundle sort -- then one CTA per segment: cumulative weights restarted at the segment, its max,
+// and the first minimisers of |cdf/max - .75| and |cdf/max - .25|.
+#define HPDW_SEG_TILE 4096
+__global__ void __launch_bounds__(SORT_THREADS)
+k_rho_seg(const double *__restrict__ x, const double *__restrict__ y, int64_t num, const long long *__restrict__ seg_start,
+          int nseg, const double *__restrict__ sums, double *__restrict__ rho)
+{
+    for (int64_t t0 = (int64_t)blockIdx.x * HPDW_SEG_TILE; t0 < num; t0 += (int64_t)gridDim.x * HPDW_SEG_TILE) {
+        const int64_t t1 = t0 + HPDW_SEG_TILE < num ? t0 + HPDW_SEG_TILE : num;
+        seg_tile_pieces(t0, t1, seg_start, nseg, [&](int seg, int64_t a, int64_t b) {
+            const double cx = sums[16 * (int64_t)seg + 1] / sums[16 * (int64_t)seg];
+            const double cy = sums[16 * (int64_t)seg + 2] / sums[16 * (int64_t)seg];
+            for (int64_t i = a + threadIdx.x; i < b; i += blockDim.x) rho[i] = sqrt(sq(x[i] - cx) + sq(y[i] - cy));
+        });
+    }
+}
+
+// key[i] = segment of ray idx[i] (exact as a double)
+__global__ void __launch_bounds__(SORT_THREADS)
+k_seg_of(const long long *__restrict__ idx, int64_t num, const long long *__restrict__ seg_start, int nseg,
+         double *__restrict__ key)
+{
+    const int64_t tid = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    const int64_t nthr = (int64_t)gridDim.x * blockDim.x;
+    for (int64_t i = tid; i < num; i += nthr) {
+        const long long r = idx[i];
+        int lo = 0, hi = nseg - 1;                      // last segment starting at or before r
+        while (lo < hi) {
+            const int mid = (lo + hi + 1) >> 1;
+            if (seg_start[mid] <= r) lo = mid; else hi = mid - 1;
+        }
+        key[i] = (double)lo;
+    }
+}
+
+__global__ void __launch_bounds__(SORT_THREADS)
+k_seg_compose(const long long *__restrict__ idx1, const double *__restrict__ rs1, const long long *__restrict__ idx2,
+              int64_t num, long long *__restrict__ idx, double *__restrict__ rs)
+{
+    const int64_t tid = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    const int64_t nthr = (int64_t)gridDim.x * blockDim.x;
+    for (int64_t i = tid; i < num; i += nthr) {
+        const long long j = idx2[i];
+        idx[i] = idx1[j];
+        rs[i] = rs1[j];
+    }
+}
+
+#define HPDW_SEG_THREADS 1024
+__global__ void __launch_bounds__(HPDW_SEG_THREADS)
+k_hpdw_seg(const double *__restrict__ w, const long long *__restrict__ idx, const double *__restrict__ rs,
+           const long long *__restrict__ seg_start, const double *__restrict__ sums, double *__restrict__ cdf,
+           double *__restrict__ out)
+{
+    constexpr int NW = HPDW_SEG_THREADS / 32;
+    __shared__ double wtot[NW];
+    __shared__ double carry, mxs;
+    __shared__ double shv[2][NW];
+    __shared__ long long shi[2][NW];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int s = blockIdx.x;
+    const long long a = seg_start[s], b = seg_start[s + 1];
+    double *o = out + 4 * (int64_t)s;
+    const double nanv = __longlong_as_double(0x7ff8000000000000ll);
+    if (b == a || sums[16 * (int64_t)s] == 0.) {       // no rays / no weight: documented as NaN
+        if (threadIdx.x == 0) { o[0] = nanv; o[1] = nanv; o[2] = nanv; o[3] = 1.; }
+        return;
+    }
+    if (threadIdx.x == 0) carry = 0.;
+    __syncthreads();
+    // inclusive scan of w[idx[i]] over the slice (block scan with a running carry, as k_scan_apply) and its max
+    double m = -__longlong_as_double(0x7ff0000000000000ll);
+    bool nan = false;
+    for (long long t0 = a; t0 < b; t0 += HPDW_SEG_THREADS) {
+        const long long i = t0 + threadIdx.x;
+        const double v = i < b ? w[idx[i]] : 0.;
+        double incl = v;
+#pragma unroll
+        for (int q = 1; q < 32; q <<= 1) {
+            const double t = __shfl_up_sync(0xffffffffu, incl, q);
+            if (lane >= q) incl += t;
+        }
+        if (lane == 31) wtot[warp] = incl;
+        __syncthreads();
+        double base = carry;
+        for (int q = 0; q < warp; q++) base += wtot[q];
+        if (i < b) {
+            const double c = base + incl;
+            cdf[i] = c;
+            if (c != c) nan = true;
+            else if (c > m) m = c;
+        }
+        __syncthreads();
+        if (threadIdx.x == HPDW_SEG_THREADS - 1) carry = base + incl;
+        __syncthreads();
+    }
+    if (nan) m = nanv;
+#pragma unroll
+    for (int q = 16; q > 0; q >>= 1) {
+        const double ov = __shfl_down_sync(0xffffffffu, m, q);
+        if (ov != ov || (m == m && ov > m)) m = ov;
+    }
+    if (lane == 0) wtot[warp] = m;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        double r = wtot[0];
+        for (int q = 1; q < NW; q++) {
+            const double ov = wtot[q];
+            if (ov != ov || (r == r && ov > r)) r = ov;
+        }
+        mxs = r;
+    }
+    __syncthreads();
+    const double mx = mxs;
+    double bv[2] = {__longlong_as_double(0x7ff0000000000000ll), __longlong_as_double(0x7ff0000000000000ll)};
+    long long bi[2] = {0x7fffffffffffffffll, 0x7fffffffffffffffll};
+    for (long long i = a + threadIdx.x; i < b; i += HPDW_SEG_THREADS) {
+        const double c = cdf[i] / mx;
+        const double d0 = fabs(c - .75), d1 = fabs(c - .25);
+        if (am_better(d0, i, bv[0], bi[0])) { bv[0] = d0; bi[0] = i; }
+        if (am_better(d1, i, bv[1], bi[1])) { bv[1] = d1; bi[1] = i; }
+    }
+#pragma unroll
+    for (int c = 0; c < 2; c++) {
+#pragma unroll
+        for (int q = 16; q > 0; q >>= 1) {
+            const double ov = __shfl_down_sync(0xffffffffu, bv[c], q);
+            const long long oi = __shfl_down_sync(0xffffffffu, bi[c], q);
+            if (am_better(ov, oi, bv[c], bi[c])) { bv[c] = ov; bi[c] = oi; }
+        }
+        if (lane == 0) { shv[c][warp] = bv[c]; shi[c][warp] = bi[c]; }
+    }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        long long ii[2];
+        for (int c = 0; c < 2; c++) {
+            double v = shv[c][0];
+            long long i = shi[c][0];
+            for (int q = 1; q < NW; q++)
+                if (am_better(shv[c][q], shi[c][q], v, i)) { v = shv[c][q]; i = shi[c][q]; }
+            ii[c] = i;
+        }
+        const double r75 = rs[ii[0]], r25 = rs[ii[1]];
+        o[0] = r75 - r25; o[1] = r75; o[2] = r25; o[3] = 1.;
+    }
+}
+
+size_t hpd_weighted_segmented_bytes(int64_t num)
+{
+    const size_t n = (size_t)(num > 0 ? num : 1);
+    return 7 * align256(n * 8) + align256(pxf_sort_scratch_bytes(num)) + 256;
+}
+
+int hpd_weighted_segmented(const double *x, const double *y, const double *w, int64_t num, const long long *seg_start,
+                           int nseg, const double *sums, double *out, void *workspace, cudaStream_t s)
+{
+    const size_t n = (size_t)(num > 0 ? num : 1);
+    char *p = static_cast<char *>(workspace);
+    double *rho = (double *)p; p += align256(n * 8);      // radii, then the segment keys, then the cdf
+    double *rs1 = (double *)p; p += align256(n * 8);
+    long long *idx1 = (long long *)p; p += align256(n * 8);
+    double *kout = (double *)p; p += align256(n * 8);
+    long long *idx2 = (long long *)p; p += align256(n * 8);
+    long long *idx = (long long *)p; p += align256(n * 8);
+    double *rs = (double *)p; p += align256(n * 8);
+    void *sort_scr = p;
+    pxf_stream_t st = reinterpret_cast<pxf_stream_t>(s);
+    int rc;
+    if (num > 0) {
+        k_rho_seg<<<grid_for(num, HPDW_SEG_TILE, 4), SORT_THREADS, 0, s>>>(x, y, num, seg_start, nseg, sums, rho);
+        count_launch();
+        if ((rc = pxf_argsort(rho, num, rs1, reinterpret_cast<int64_t *>(idx1), sort_scr, st))) return rc;
+        k_seg_of<<<grid_for(num, SORT_THREADS * 4, 8), SORT_THREADS, 0, s>>>(idx1, num, seg_start, nseg, rho);
+        count_launch();
+        if ((rc = pxf_argsort(rho, num, kout, reinterpret_cast<int64_t *>(idx2), sort_scr, st))) return rc;
+        k_seg_compose<<<grid_for(num, SORT_THREADS * 4, 8), SORT_THREADS, 0, s>>>(idx1, rs1, idx2, num, idx, rs);
+        count_launch();
+    }
+    k_hpdw_seg<<<nseg, HPDW_SEG_THREADS, 0, s>>>(w, idx, rs, seg_start, sums, rho, out);
+    count_launch();
+    return check_launch("pxf_hpd_segmented (weighted)");
+}
+
 }  // namespace pxf
 
 using namespace pxf;

@@ -483,6 +483,47 @@ def config2_fast(n=10_000_000, arcmin=None, aperture=None, rng="numpy", rng_seed
     return [config2_point_fast(n, a / 60. * np.pi / 180., aperture, rng, rng_seed, device) for a in arcmin]
 
 
+def config2_sweep_fast(n=10_000_000, arcmin=None, aperture=None, rng="numpy", rng_seed=0, device=None,
+                       R0=WS["R0"], Z0=WS["Z0"], psi=WS["psi"], az=WS["az"], sources=None):
+    """``config2_fast`` as ONE bundle: the source is drawn once and replicated per field point (config2_fast reuses
+    the same draws at every point), one segmented launch traces all points with a per-segment kick, and every
+    analysis runs per segment (``segments=``) in a number of launches that does not depend on the point count.
+    Returns the same list of per-point dicts; ``rays`` is each point's view of the joint bundle."""
+    pxf = _pxf()
+    from pyxfocus_b200._call import bundle_alloc, bundle_split
+    anal = pxf.analyses
+    arcmin = np.linspace(0., 30., 31) if arcmin is None else np.asarray(arcmin, dtype=np.float64)
+    aperture = ws_aperture(product_api(device)) if aperture is None else aperture
+    a0, a1 = aperture
+    K = len(arcmin)
+    seed(rng_seed)
+    src = (sources or pxf.sources).subannulus(a0, a1, az / R0, n, **_source_kw(rng, rng_seed, device))
+    dev = src[1].device
+    rays = bundle_alloc(K * n, dev)
+    for r, s_ in zip(rays, src):
+        r.view(K, n).copy_(s_.unsqueeze(0).expand(K, n))
+    del src
+    segs = pxf.Segments([n] * K, device=dev)
+    alpha = pxf.conicsolve.woltparam(R0, Z0)[0]
+    # the recorded form of config2_point_fast's chain (transform arguments negated, as transformations.transform does)
+    progs = [pxf.Program().transform(-0., -0., Z0, -0., -0., -0.).wsprimary(alpha, Z0, psi)
+             .kick(np.sin(a / 60. * np.pi / 180.), 0., -1.).reflect().wssecondary(alpha, Z0, psi).reflect().flat()
+             for a in arcmin]
+    pxf.SegmentedProgram(progs, segs.sizes(), device=dev).run(rays)
+    s9 = anal.imageplane_sums(rays, at_z0=True, segments=segs)
+    d2 = anal.findimageplane(rays, 20., 100, sums=s9, segments=segs)
+    d3 = anal.findimageplane(rays, 1., 100, sums=s9, moved=d2, segments=segs)
+    pxf.SegmentedProgram([pxf.Program().transform(-0., -0., -d2[k], -0., -0., -0.)
+                          .transform(-0., -0., -d3[k], -0., -0., -0.).flat() for k in range(K)],
+                         segs.sizes(), device=dev).run(rays)
+    hpd_scan, rms_scan = anal.hpd(rays, segments=segs), anal.rmsCentroid(rays, segments=segs)
+    f = pxf.surfaces.focusI(rays, segments=segs)
+    hpd, rms = anal.hpd(rays, segments=segs), anal.rmsCentroid(rays, segments=segs)
+    views = bundle_split(rays, [n] * K)
+    return [dict(rays=views[k], f=float(f[k]), d2=float(d2[k]), d3=float(d3[k]), hpd_scan=float(hpd_scan[k]),
+                 rms_scan=float(rms_scan[k]), hpd=float(hpd[k]), rms=float(rms[k])) for k in range(K)]
+
+
 def config3_fast(n=100_000_000, rng="numpy", rng_seed=0, device=None, want_idx=True, sources=None):
     pxf = _pxf()
     src = sources or pxf.sources

@@ -310,6 +310,74 @@ class FanAux:
         return k
 
 
+class Segments:
+    """Layout of a segmented bundle: segment k is rays ``start[k]:start[k+1]`` (``start`` host int64, nseg+1 entries,
+    ``start[0] == 0``) with a device copy ``start_dev``.  The per-segment analyses (``segments=`` of ``analyses`` and
+    ``surfaces.focus*``) take one; ``SegmentedProgram.segments`` is the layout a segmented trace ran with."""
+
+    def __init__(self, sizes, device=None):
+        import numpy as np
+        sz = np.asarray(sizes)
+        if sz.ndim != 1 or sz.shape[0] < 1:
+            raise ValueError("segments need a 1-D list of at least one size")
+        if not np.issubdtype(sz.dtype, np.integer) and not np.all(np.equal(np.mod(sz, 1), 0)):
+            raise ValueError("segment sizes must be integers")
+        sz = sz.astype(np.int64)
+        if (sz < 0).any():
+            raise ValueError("segment sizes must be non-negative")
+        start = np.zeros(sz.shape[0] + 1, dtype=np.int64)
+        start[1:] = np.cumsum(sz)
+        self.start = start
+        if device is None:
+            device = torch.device("cuda", torch.cuda.current_device() if torch.cuda.is_available() else 0)
+        self.device = torch.device(device)
+        self._dev = None
+
+    @classmethod
+    def _from(cls, start, start_dev):
+        seg = cls.__new__(cls)
+        seg.start, seg._dev, seg.device = start, start_dev, start_dev.device
+        return seg
+
+    @property
+    def start_dev(self):
+        if self._dev is None:
+            self._dev = torch.from_numpy(self.start).to(self.device)
+        return self._dev
+
+    @property
+    def nseg(self):
+        return self.start.shape[0] - 1
+
+    @property
+    def num(self):
+        return int(self.start[-1])
+
+    def sizes(self):
+        import numpy as np
+        return np.diff(self.start)
+
+    def check(self, num, device):
+        """Raise ValueError unless these segments describe a bundle of ``num`` rays on ``device``."""
+        if num != self.num:
+            raise ValueError("bundle has %d rays, the segments add up to %d" % (num, self.num))
+        if torch.device(device) != self.device:
+            raise ValueError("segments live on %s, the bundle on %s" % (self.device, device))
+
+    def after(self, alive):
+        """The segments of ``transformations.compact(rays, alive)``: survivors counted per segment on the device, one
+        read-back of nseg int64; compaction keeps the order, so the new starts are their exclusive scan."""
+        import numpy as np
+        if not isinstance(alive, torch.Tensor) or alive.dtype != torch.uint8 or alive.dim() != 1:
+            raise ValueError("alive must be a 1-D uint8 tensor")
+        self.check(alive.shape[0], alive.device)
+        counts = torch.empty(self.nseg, dtype=torch.int64, device=alive.device)
+        with torch.cuda.device(alive.device):
+            _lib.check(_lib.lib().pxf_segment_counts(alive.contiguous().data_ptr(), alive.shape[0], self.start_dev.data_ptr(),
+                                                     self.nseg, counts.data_ptr(), stream_ptr(alive.device)))
+        return Segments(counts.cpu().numpy(), device=alive.device)
+
+
 class SegmentedProgram:
     """One launch for a bundle made of segments that run the same routines with different scalars -- a nested
     mirror assembly, one shell per segment (the reference loops over shells in Python,
@@ -351,6 +419,7 @@ class SegmentedProgram:
         dev = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
         self.table_dev = self.table_host.to(dev)
         self.seg_start_dev = torch.from_numpy(start).to(dev)
+        self.segments = Segments._from(start, self.seg_start_dev)
 
     def run(self, rays, alive=None, out=None):
         dev = rays[1].device

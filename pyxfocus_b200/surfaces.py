@@ -254,10 +254,30 @@ def ellipsoidSecondaryLL(rays, R0, F, S, psi, zmax, zmin, dphi, coeff, axial, az
     return
 
 
-def focus(rays, fn, weights=None, nr=None, coords=None):
+def _move_segments(rays, dz, segments, nr):
+    # every segment by its own dz: transform(rays, 0, 0, dz[k], 0, 0, 0) + flat, as the recorder would record them
+    from .program import Program, SegmentedProgram
+    progs = []
+    for d in dz:
+        p = Program().transform(-0., -0., -float(d), -0., -0., -0.)
+        progs.append(p.flatopd(nr) if nr is not None else p.flat())
+    SegmentedProgram(progs, segments.sizes(), device=rays[1].device).run(rays)
+
+
+def focus(rays, fn, weights=None, nr=None, coords=None, segments=None):
     """Two-pass best focus (surfaces.py:502-510).  Each "move the plane, trace to it" pair runs as one fused
-    kernel (same bits as the two calls)."""
-    from .program import fused, recorder_for
+    kernel (same bits as the two calls).  ``segments``: every segment is moved by its own dz (one segmented launch
+    per pass) and the dz of every segment is returned (np.ndarray[nseg]); not with ``coords``."""
+    from .program import fused, flush, recorder_for
+    if segments is not None:
+        if coords is not None:
+            raise ValueError("focus: coords= cannot follow per-segment moves")
+        flush(rays)
+        dz1 = fn(rays, weights=weights, segments=segments)
+        _move_segments(rays, dz1, segments, nr)
+        dz2 = fn(rays, weights=weights, segments=segments)
+        _move_segments(rays, dz2, segments, nr)
+        return dz1 + dz2
     own = recorder_for(rays) is None
     dz1 = fn(rays, weights=weights)
     if own:
@@ -278,19 +298,19 @@ def focus(rays, fn, weights=None, nr=None, coords=None):
     return dz1 + dz2
 
 
-def focusI(rays, weights=None, nr=None, coords=None):
+def focusI(rays, weights=None, nr=None, coords=None, segments=None):
     """Best focus from the analytic image plane (surfaces.py:518-519)."""
-    return focus(rays, analyticImagePlane, weights=weights, nr=nr, coords=coords)
+    return focus(rays, analyticImagePlane, weights=weights, nr=nr, coords=coords, segments=segments)
 
 
-def focusY(rays, weights=None, nr=None, coords=None):
+def focusY(rays, weights=None, nr=None, coords=None, segments=None):
     """Best line focus in y (surfaces.py:512-513)."""
-    return focus(rays, analyticYPlane, weights=weights, nr=nr, coords=coords)
+    return focus(rays, analyticYPlane, weights=weights, nr=nr, coords=coords, segments=segments)
 
 
-def focusX(rays, weights=None, nr=None, coords=None):
+def focusX(rays, weights=None, nr=None, coords=None, segments=None):
     """Best line focus in x (surfaces.py:515-516)."""
-    return focus(rays, analyticXPlane, weights=weights, nr=nr, coords=coords)
+    return focus(rays, analyticXPlane, weights=weights, nr=nr, coords=coords, segments=segments)
 
 
 def _need_orders(rorder, aorder):
