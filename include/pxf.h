@@ -372,6 +372,20 @@ int pxf_segmented_table_fill(const pxf_op *ops, int32_t nops, int32_t nseg, cons
 int pxf_trace_program_segmented(double *const rays_in[10], double *const rays_out[10], int64_t num,
                                 const void *table_host, const void *table_dev, uint8_t *alive,
                                 pxf_stream_t stream);
+/* Segmented programs with one Zernike surface per segment (a figure-error Monte Carlo, or shells that each have a
+ * measured figure): every segment's op list has its PXF_OP_ZERNSURF at the same position, with the same opd flag
+ * (p[1]); the term count, radial order (<= 7), rad and nr may differ.  pxf_segmented_table_fill refuses such lists;
+ * this pair takes them (and any list the plain pair takes).
+ *   zern_tables_host: nseg consecutive tables of pxf_zern_table_bytes() bytes, table s filled by pxf_zern_table_fill
+ *   for segment s (NULL is accepted when no op is a PXF_OP_ZERNSURF).  They are copied into the segmented table, so it
+ *   stays self-contained: upload it unchanged and pass both copies to pxf_trace_program_segmented, which stages the
+ *   segment's Zernike table next to its op table -- still ONE launch.  The op's p[0] (device table address) is not
+ *   used; its nmax p[2] is taken from the table.
+ *   Returns PXF_ERR_UNSUPPORTED for a table of radial order > 7 and for PXF_OP_GRATFAN / PXF_OP_ROTX_REMAINING,
+ *   PXF_ERR_INVALID for segments that differ in opcode sequence or opd flag, or for missing tables. */
+size_t pxf_segmented_table_bytes_zern(int32_t nops, int32_t nseg);
+int pxf_segmented_table_fill_zern(const pxf_op *ops, int32_t nops, int32_t nseg, const int64_t *seg_start,
+                                  const void *zern_tables_host, void *table_host);
 
 /* ======================= vignetting / compaction ======================== */
 /* flags[i] = (l^2+m^2+n^2 > .1), the default predicate of transformations.vignette

@@ -223,16 +223,18 @@ PXF_DEV void chain_body(const RowPtrs &P, const RowPtrs &Q, const int64_t num, u
 }
 
 // Segmented form (nested assemblies): the bundle is walked in tiles of CHAIN_SEG_TILE consecutive rays; a CTA stages
-// the parameter pack of the segment its tile lies in (re-staged only when the segment changes).
+// the parameter pack of the segment its tile lies in (re-staged only when the segment changes).  ZERN: zern holds one
+// Zernike table per segment, staged with the pack.
 #define CHAIN_SEG_TILE (PXF_BLOCK * 8)
-template <class C, class CP, unsigned LMc, unsigned SMc>
+template <class C, class CP, bool ZERN, unsigned LMc, unsigned SMc>
 PXF_DEV void chain_seg_body(const RowPtrs &P, const RowPtrs &Q, const int64_t num, uint8_t *__restrict__ alive,
                             const long long *__restrict__ seg_start, const CP *__restrict__ table, const int nseg,
-                            const unsigned LMr, const unsigned SMr)
+                            const unsigned LMr, const unsigned SMr, const ZernP *__restrict__ zern)
 {
     __shared__ __align__(16) CP sp;
+    __shared__ __align__(16) unsigned char zraw[ZERN ? sizeof(ZernP) : 16];
     const unsigned LM = LMc ? LMc : LMr, SM = SMc ? SMc : SMr;
-    const ChainCtx ctx = chain_ctx_none();
+    ChainCtx ctx = chain_ctx_none();
     int staged = -1;
     for (int64_t t0 = (int64_t)blockIdx.x * CHAIN_SEG_TILE; t0 < num; t0 += (int64_t)gridDim.x * CHAIN_SEG_TILE) {
         const int64_t t1 = t0 + CHAIN_SEG_TILE < num ? t0 + CHAIN_SEG_TILE : num;
@@ -252,13 +254,26 @@ PXF_DEV void chain_seg_body(const RowPtrs &P, const RowPtrs &Q, const int64_t nu
                 const double *src = reinterpret_cast<const double *>(table + seg);
                 double *dst = reinterpret_cast<double *>(&sp);
                 for (int t = threadIdx.x; t < (int)(sizeof(CP) / 8); t += blockDim.x) dst[t] = src[t];
+                if (ZERN) {
+                    const double *zsrc = reinterpret_cast<const double *>(zern + seg);
+                    double *zdst = reinterpret_cast<double *>(zraw);
+                    for (int t = threadIdx.x; t < (int)(sizeof(ZernP) / 8); t += blockDim.x) zdst[t] = zsrc[t];
+                }
                 __syncthreads();
                 staged = seg;
             }
             for (int64_t i = pos + threadIdx.x; i < send; i += blockDim.x) {
                 Ray a;
                 fload1(a, P, LM, i);
-                const bool keep = C::run(a, sp, ctx);
+                // ZERN: the staged pack and table are addressed per ray through an opaque zero.  Hoisted out of this
+                // loop their loads would hold ~90 more registers than the fused Zernike kernel does (ptxas, no cap:
+                // 242 vs 150) and spill at its 3 CTAs/SM.  Without ZERN, z is the constant 0.
+                int z = 0;
+                if (ZERN) {
+                    asm volatile("" : "+r"(z));
+                    ctx.zt = reinterpret_cast<const ZernP *>(zraw) + z;
+                }
+                const bool keep = C::run(a, (&sp)[z], ctx);
                 fstore1(a, Q, SM, i);
                 if (alive) alive[i] = keep ? 1 : 0;
             }

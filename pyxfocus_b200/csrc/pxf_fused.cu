@@ -177,17 +177,25 @@ k_program(const RowPtrs P, const RowPtrs Q, const int64_t num, uint8_t *__restri
 // 260 shells (measured 12 ms of launches for 1e7 rays).  Here one persistent grid walks the bundle in tiles of
 // SEG_TILE consecutive rays; a CTA stages the op table of the segment its tile lies in into shared memory
 // (re-staged only when the segment changes; a tile that straddles segments is processed piecewise).
+// A program with a PXF_OP_ZERNSURF op carries one Zernike table per segment (zern_off: their offset in the table,
+// 0 = none); the table of the segment is staged next to its op table.
 #define SEG_TILE (PXF_BLOCK * 8)
-struct SegHeader { unsigned load_mask, store_mask; int nops, nseg; int chain_id, jit_pack_bytes, pad[2]; };
+struct SegHeader { unsigned load_mask, store_mask; int nops, nseg; int chain_id, jit_pack_bytes; long long zern_off; };
+static_assert(sizeof(ZernP) % 16 == 0, "per-segment Zernike tables are laid out back to back, 16-byte aligned");
 
-template <int MINB>
+// shared-memory offset of the staged Zernike table: behind the op table, 16-byte aligned
+__host__ __device__ __forceinline__ int seg_zern_smem_offset(int nops) { return (nops * (int)sizeof(FusedOp) + 15) & ~15; }
+
+// ZERN: zern = nseg Zernike tables, one per segment (the Zernike instantiation of run_op, as k_program<.., true>)
+template <int MINB, bool ZERN = false>
 __global__ void __launch_bounds__(PXF_BLOCK, MINB)
 k_program_seg(const RowPtrs P, const RowPtrs Q, const int64_t num, uint8_t *__restrict__ alive,
               const long long *__restrict__ seg_start, const FusedOp *__restrict__ ops, const int nops, const int nseg,
-              const unsigned LM, const unsigned SM)
+              const unsigned LM, const unsigned SM, const ZernP *__restrict__ zern)
 {
     extern __shared__ __align__(16) unsigned char seg_smem[];
     FusedOp *sops = reinterpret_cast<FusedOp *>(seg_smem);
+    ZernP *zt = ZERN ? reinterpret_cast<ZernP *>(seg_smem + seg_zern_smem_offset(nops)) : nullptr;
     int staged = -1;
     const int words = nops * (int)(sizeof(FusedOp) / 8);
     for (int64_t t0 = (int64_t)blockIdx.x * SEG_TILE; t0 < num; t0 += (int64_t)gridDim.x * SEG_TILE) {
@@ -198,6 +206,11 @@ k_program_seg(const RowPtrs P, const RowPtrs Q, const int64_t num, uint8_t *__re
                 const double *src = reinterpret_cast<const double *>(ops + (int64_t)seg * nops);
                 double *dst = reinterpret_cast<double *>(sops);
                 for (int t = threadIdx.x; t < words; t += blockDim.x) dst[t] = src[t];
+                if (ZERN) {
+                    const double *zsrc = reinterpret_cast<const double *>(zern + seg);
+                    double *zdst = reinterpret_cast<double *>(zt);
+                    for (int t = threadIdx.x; t < (int)(sizeof(ZernP) / 8); t += blockDim.x) zdst[t] = zsrc[t];
+                }
                 __syncthreads();
                 staged = seg;
             }
@@ -206,7 +219,7 @@ k_program_seg(const RowPtrs P, const RowPtrs Q, const int64_t num, uint8_t *__re
                 fload1(a, P, LM, i);
                 bool keep = true;
                 for (int k = 0; k < nops; k++)
-                    if (!run_op(a, sops[k])) { keep = false; break; }
+                    if (!run_op<ZERN>(a, sops[k], zt)) { keep = false; break; }
                 fstore1(a, Q, SM, i);
                 if (alive) alive[i] = keep ? 1 : 0;
             }
@@ -507,8 +520,24 @@ extern "C" size_t pxf_segmented_table_bytes(int32_t nops, int32_t nseg)
 }
 static size_t seg_chain_offset(int nops, int nseg) { return seg_align(seg_ops_offset(nseg) + (size_t)nseg * nops * sizeof(FusedOp)); }
 
-extern "C" int pxf_segmented_table_fill(const pxf_op *ops, int32_t nops, int32_t nseg, const int64_t *seg_start,
-                                        void *table_host)
+static bool is_vignette(int code)
+{
+    return code == PXF_OP_VIGNETTE_MAG || code == PXF_OP_VIGNETTE_BOX || code == PXF_OP_VIGNETTE_ABS ||
+           code == PXF_OP_VIGNETTE_RHOGT;
+}
+
+// Zernike tables of a segmented program: behind everything pxf_segmented_table_bytes lays out, one per segment
+static size_t seg_zern_offset(int nops, int nseg) { return seg_align(pxf_segmented_table_bytes(nops, nseg)); }
+
+extern "C" size_t pxf_segmented_table_bytes_zern(int32_t nops, int32_t nseg)
+{
+    if (nops < 1 || nseg < 1) return 0;
+    return seg_zern_offset(nops, nseg) + (size_t)nseg * sizeof(ZernP);
+}
+
+// zern_tables: nseg tables of pxf_zern_table_fill (NULL: the program may not have a PXF_OP_ZERNSURF op)
+static int seg_table_fill(const pxf_op *ops, int nops, int nseg, const int64_t *seg_start, const void *zern_tables,
+                          bool zern_ok, void *table_host)
 {
     if (!ops || !seg_start || !table_host || nops < 1 || nops > PXF_MAX_OPS || nseg < 1) {
         set_error("pxf_segmented_table_fill: bad argument");
@@ -517,17 +546,49 @@ extern "C" int pxf_segmented_table_fill(const pxf_op *ops, int32_t nops, int32_t
     if (seg_start[0] != 0) { set_error("segmented program: seg_start[0] must be 0"); return PXF_ERR_INVALID; }
     for (int sgm = 0; sgm < nseg; sgm++)
         if (seg_start[sgm + 1] < seg_start[sgm]) { set_error("segmented program: seg_start must be non-decreasing"); return PXF_ERR_INVALID; }
+    bool zern = false;
+    if (zern_ok) {
+        for (size_t k = 0; k < (size_t)nseg * nops; k++) {
+            if (ops[k].code == PXF_OP_GRATFAN || ops[k].code == PXF_OP_ROTX_REMAINING) {
+                set_error("segmented program: PXF_OP_GRATFAN / PXF_OP_ROTX_REMAINING are not supported");
+                return PXF_ERR_UNSUPPORTED;
+            }
+            if (ops[k].code == PXF_OP_ZERNSURF) zern = true;
+        }
+        if (zern && !zern_tables) { set_error("segmented program: PXF_OP_ZERNSURF needs one Zernike table per segment"); return PXF_ERR_INVALID; }
+    }
     char *base = static_cast<char *>(table_host);
     SegHeader *h = reinterpret_cast<SegHeader *>(base);
     memset(h, 0, seg_align(sizeof(SegHeader)));
     memcpy(base + seg_align(sizeof(SegHeader)), seg_start, (size_t)(nseg + 1) * 8);
     FusedOp *dst = reinterpret_cast<FusedOp *>(base + seg_ops_offset(nseg));
+    ZernP *zdst = zern ? reinterpret_cast<ZernP *>(base + seg_zern_offset(nops, nseg)) : nullptr;
     h->nops = nops; h->nseg = nseg;
     for (int sgm = 0; sgm < nseg; sgm++) {
+        pxf_op sops[PXF_MAX_OPS];
+        memcpy(sops, ops + (size_t)sgm * nops, (size_t)nops * sizeof(pxf_op));
+        if (zern) {
+            // the segment's own table, copied into this one (the op's device address p[0] is not used)
+            memcpy(zdst + sgm, static_cast<const char *>(zern_tables) + (size_t)sgm * sizeof(ZernP), sizeof(ZernP));
+            const int nmax = zdst[sgm].nmax;
+            if (nmax < 0 || nmax > 7) {
+                set_error("segmented program: segment %d: PXF_OP_ZERNSURF supports radial orders <= 7 (table has %d)", sgm, nmax);
+                return PXF_ERR_UNSUPPORTED;
+            }
+            for (int k = 0; k < nops; k++)
+                if (sops[k].code == PXF_OP_ZERNSURF) {
+                    const ZernP *any = zdst + sgm;       // build_program only checks that a table is there
+                    memcpy(&sops[k].p[0], &any, sizeof(any));
+                    sops[k].p[2] = (double)nmax;
+                }
+        }
         FusedProgram fp;
-        int rc = build_program(fp, ops + (size_t)sgm * nops, nops);
+        int rc = build_program(fp, sops, nops);
         if (rc) return rc;
-        if (fp.zern || fp.uses_aux) { set_error("segmented program: PXF_OP_ZERNSURF / PXF_OP_GRATFAN are not supported"); return PXF_ERR_UNSUPPORTED; }
+        if ((fp.zern && !zern_ok) || fp.uses_aux) {
+            set_error("segmented program: PXF_OP_ZERNSURF needs pxf_segmented_table_fill_zern; PXF_OP_GRATFAN is not supported");
+            return PXF_ERR_UNSUPPORTED;
+        }
         if (sgm > 0)
             for (int k = 0; k < nops; k++)
                 if (fp.ops[k].code != dst[k].code || fp.ops[k].row != dst[k].row) {   // dst[0..nops) = segment 0
@@ -538,12 +599,12 @@ extern "C" int pxf_segmented_table_fill(const pxf_op *ops, int32_t nops, int32_t
         h->store_mask |= fp.store_mask;
         memcpy(dst + (size_t)sgm * nops, fp.ops, (size_t)nops * sizeof(FusedOp));
     }
+    if (zern) h->zern_off = (long long)seg_zern_offset(nops, nseg);
     // a statically specialised kernel for the canonical chains: one parameter pack per segment behind the op table
     h->chain_id = seg_chain_fill(dst, nops, nseg, base + seg_chain_offset(nops, nseg));
     bool vig = false;
     for (int k = 0; k < nops; k++)
-        if (dst[k].code == PXF_OP_VIGNETTE_MAG || dst[k].code == PXF_OP_VIGNETTE_BOX || dst[k].code == PXF_OP_VIGNETTE_ABS ||
-            dst[k].code == PXF_OP_VIGNETTE_RHOGT) vig = true;
+        if (is_vignette(dst[k].code)) vig = true;
     if (h->chain_id == 0 || vig) {
         // any other op list: parameter packs for a kernel specialised at run time (pxf_jit.cu)
         const size_t pb = jit_seg_fill(dst, nops, nseg, base + seg_chain_offset(nops, nseg));
@@ -551,6 +612,18 @@ extern "C" int pxf_segmented_table_fill(const pxf_op *ops, int32_t nops, int32_t
         else if (vig) h->chain_id = 0;
     }
     return PXF_OK;
+}
+
+extern "C" int pxf_segmented_table_fill(const pxf_op *ops, int32_t nops, int32_t nseg, const int64_t *seg_start,
+                                        void *table_host)
+{
+    return seg_table_fill(ops, nops, nseg, seg_start, nullptr, false, table_host);
+}
+
+extern "C" int pxf_segmented_table_fill_zern(const pxf_op *ops, int32_t nops, int32_t nseg, const int64_t *seg_start,
+                                             const void *zern_tables_host, void *table_host)
+{
+    return seg_table_fill(ops, nops, nseg, seg_start, zern_tables_host, true, table_host);
 }
 
 extern "C" int pxf_trace_program_segmented(double *const rays_in[10], double *const rays_out[10], int64_t num,
@@ -579,26 +652,42 @@ extern "C" int pxf_trace_program_segmented(double *const rays_in[10], double *co
     const FusedOp *hops = reinterpret_cast<const FusedOp *>(static_cast<const char *>(table_host) + seg_ops_offset(nseg));
     bool vig = false;
     for (int k = 0; k < nops; k++)
-        if (hops[k].code == PXF_OP_VIGNETTE_MAG || hops[k].code == PXF_OP_VIGNETTE_BOX || hops[k].code == PXF_OP_VIGNETTE_ABS ||
-            hops[k].code == PXF_OP_VIGNETTE_RHOGT) vig = true;
+        if (is_vignette(hops[k].code)) vig = true;
     if (vig && !alive) { set_error("program with a VIGNETTE op needs an alive array"); return PXF_ERR_INVALID; }
     const char *db = static_cast<const char *>(table_dev);
     const long long *dstart = reinterpret_cast<const long long *>(db + seg_align(sizeof(SegHeader)));
     const FusedOp *dops = reinterpret_cast<const FusedOp *>(db + seg_ops_offset(nseg));
-    const size_t smem = (size_t)nops * sizeof(FusedOp);
+    const ZernP *dzern = h->zern_off ? reinterpret_cast<const ZernP *>(db + h->zern_off) : nullptr;
     cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
     if (h->chain_id == 1 && !vig) {
         int rc = seg_chain_launch(h->chain_id, P, Q, num, alive, dstart, db + seg_chain_offset(nops, nseg), nseg, LM, SM, s);
         if (rc != PXF_ERR_UNSUPPORTED) return rc;
     }
     if (h->chain_id == 2) {
-        int rc = jit_seg_launch(hops, nops, P, Q, num, alive, dstart, db + seg_chain_offset(nops, nseg), nseg, LM, SM, s);
+        int rc = jit_seg_launch(hops, nops, P, Q, num, alive, dstart, db + seg_chain_offset(nops, nseg), nseg, LM, SM,
+                                dzern, s);
         if (rc != PXF_ERR_UNSUPPORTED) return rc;
     }
-    int nb = 0;
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, k_program_seg<4>, PXF_BLOCK, smem) != cudaSuccess || nb <= 0) { cudaGetLastError(); nb = 2; }
-    const int grid = grid_for(num, SEG_TILE, nb);
-    k_program_seg<4><<<grid, PXF_BLOCK, smem, s>>>(P, Q, num, alive, dstart, dops, nops, nseg, LM, SM);
+    auto go = [&](auto kern, size_t smem) {
+        int nb = 0;
+        if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, kern, PXF_BLOCK, smem) != cudaSuccess || nb <= 0) { cudaGetLastError(); nb = 2; }
+        const int grid = grid_for(num, SEG_TILE, nb);
+        kern<<<grid, PXF_BLOCK, smem, s>>>(P, Q, num, alive, dstart, dops, nops, nseg, LM, SM, dzern);
+    };
+    if (dzern) {
+        // the segment's Zernike table is staged behind its op table; register cap as for k_program<zernike>
+        // (PXF_ZERNPROG_MINB, resident CTAs per SM)
+        static int zm = -1;
+        if (zm < 0) { const char *e = getenv("PXF_ZERNPROG_MINB"); zm = e ? atoi(e) : 3; }
+        const size_t smem = (size_t)seg_zern_smem_offset(nops) + sizeof(ZernP);
+        if (zm == 1) go(k_program_seg<1, true>, smem);
+        else if (zm == 2) go(k_program_seg<2, true>, smem);
+        else go(k_program_seg<3, true>, smem);
+        count_launch();
+        note_kernel("k_program_seg<zernike> (interpreter)");
+        return check_launch("k_program_seg<zernike>");
+    }
+    go(k_program_seg<4>, (size_t)nops * sizeof(FusedOp));
     count_launch();
     note_kernel("k_program_seg (interpreter)");
     return check_launch("k_program_seg");

@@ -176,9 +176,10 @@ struct JitSpec {
             snprintf(buf, sizeof(buf),
                      "extern \"C\" __global__ void __launch_bounds__(PXF_BLOCK, %d)\n"
                      "pxf_jit_chain(const RowPtrs P, const RowPtrs Q, const long long num, unsigned char *alive,\n"
-                     "              const long long *seg_start, const CP *table, const int nseg, const unsigned LM, const unsigned SM)\n"
-                     "{\n    chain_seg_body<C, CP, %uu, %uu>(P, Q, num, alive, seg_start, table, nseg, LM, SM);\n}\n",
-                     minb, LM, SM);
+                     "              const long long *seg_start, const CP *table, const int nseg, const unsigned LM, const unsigned SM,\n"
+                     "              const ZernP *zern)\n"
+                     "{\n    chain_seg_body<C, CP, %s, %uu, %uu>(P, Q, num, alive, seg_start, table, nseg, LM, SM, zern);\n}\n",
+                     minb, zern ? "true" : "false", LM, SM);
         }
         return s + buf;
     }
@@ -369,28 +370,31 @@ int jit_launch_chain(const RowPtrs &P, const RowPtrs &Q, int64_t num, const Fuse
 }
 
 // ---- segmented form: the per-segment parameter packs are built when the table is filled
+// register cap (resident CTAs per SM): the Zernike form needs the budget of the fused Zernike kernel
+static int seg_minb(const JitSpec &sp) { return sp.zern ? 3 : 4; }
 size_t jit_seg_pack_bytes(int nops) { return (size_t)nops * FOP_PARAM_DOUBLES * 8 + 8; }
 size_t jit_seg_fill(const FusedOp *ops, int nops, int nseg, void *dst)
 {
     JitSpec sp;
-    if (!jit_enabled() || !spec_from_ops(ops, nops, sp) || sp.zern) return 0;
+    if (!jit_enabled() || !spec_from_ops(ops, nops, sp)) return 0;
     unsigned char *out = static_cast<unsigned char *>(dst);
     for (int sgm = 0; sgm < nseg; sgm++) pack_params(ops + (size_t)sgm * nops, nops, out + (size_t)sgm * sp.cp_bytes);
     return sp.cp_bytes;
 }
 int jit_seg_launch(const FusedOp *ops0, int nops, const RowPtrs &P, const RowPtrs &Q, int64_t num, uint8_t *alive,
-                   const long long *seg_start_dev, const void *packs_dev, int nseg, unsigned LM, unsigned SM, cudaStream_t s)
+                   const long long *seg_start_dev, const void *packs_dev, int nseg, unsigned LM, unsigned SM,
+                   const ZernP *zern_dev, cudaStream_t s)
 {
     if (!jit_enabled()) return PXF_ERR_UNSUPPORTED;
     std::lock_guard<std::mutex> lock(g_mu);
     JitSpec sp;
-    if (!spec_from_ops(ops0, nops, sp) || sp.zern) return PXF_ERR_UNSUPPORTED;
-    sp.LM = LM; sp.SM = SM; sp.seg = true; sp.mode = 1; sp.minb = 4;
+    if (!spec_from_ops(ops0, nops, sp) || sp.zern != (zern_dev != nullptr)) return PXF_ERR_UNSUPPORTED;
+    sp.LM = LM; sp.SM = SM; sp.seg = true; sp.mode = 1; sp.minb = seg_minb(sp);
     JitEntry *e = get_kernel(sp, num >= jit_min_rays());
     if (!e) return PXF_ERR_UNSUPPORTED;
     const int grid = grid_for(num, CHAIN_SEG_TILE, sp.minb);
     long long n = num;
-    void *args[] = {(void *)&P, (void *)&Q, &n, &alive, &seg_start_dev, &packs_dev, &nseg, &LM, &SM};
+    void *args[] = {(void *)&P, (void *)&Q, &n, &alive, &seg_start_dev, &packs_dev, &nseg, &LM, &SM, &zern_dev};
     cudaError_t rc = cudaLaunchKernel(reinterpret_cast<const void *>(e->kern), dim3(grid), dim3(PXF_BLOCK), args, 0, s);
     if (rc != cudaSuccess) { set_error("specialised segmented chain launch: %s", cudaGetErrorString(rc)); return PXF_ERR_CUDA; }
     count_launch();
@@ -409,7 +413,7 @@ int jit_precompile(const FusedProgram &fp0, bool segmented)
     if (segmented) {
         for (int oop = 0; oop < 2; oop++) {
             sp.LM = fp0.load_mask; sp.SM = fp0.store_mask | (oop ? fp0.load_mask : 0u);
-            sp.seg = true; sp.mode = 1; sp.minb = 4;
+            sp.seg = true; sp.mode = 1; sp.minb = seg_minb(sp);
             if (get_cubin(sp, true)) have++;
         }
         return have;

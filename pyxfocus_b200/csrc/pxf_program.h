@@ -53,7 +53,8 @@ int jit_launch_chain(const RowPtrs &P, const RowPtrs &Q, int64_t num, const Fuse
 size_t jit_seg_pack_bytes(int nops);
 size_t jit_seg_fill(const FusedOp *ops, int nops, int nseg, void *dst);     // returns bytes per segment pack, 0 = none
 int jit_seg_launch(const FusedOp *ops0, int nops, const RowPtrs &P, const RowPtrs &Q, int64_t num, uint8_t *alive,
-                   const long long *seg_start_dev, const void *packs_dev, int nseg, unsigned LM, unsigned SM, cudaStream_t s);
+                   const long long *seg_start_dev, const void *packs_dev, int nseg, unsigned LM, unsigned SM,
+                   const ZernP *zern_dev, cudaStream_t s);    // zern_dev: one Zernike table per segment (NULL: none)
 void note_kernel(const char *name);     // name of the last trace kernel launched (pxf_last_trace_kernel)
 
 // segmented specialised chains (pxf_chain.cu)

@@ -524,12 +524,13 @@ def config2_sweep_fast(n=10_000_000, arcmin=None, aperture=None, rng="numpy", rn
                  rms_scan=float(rms_scan[k]), hpd=float(hpd[k]), rms=float(rms[k])) for k in range(K)]
 
 
-def config3_fast(n=100_000_000, rng="numpy", rng_seed=0, device=None, want_idx=True, sources=None):
+def config3_fast(n=100_000_000, rng="numpy", rng_seed=0, device=None, want_idx=True, sources=None, coeff=None):
+    """``coeff``: the 36 Zernike coefficients (default: ``zernike_coeff(36, rng_seed)``, as ``config3``)."""
     pxf = _pxf()
     src = sources or pxf.sources
     tran, surf, anal = pxf.transformations, pxf.surfaces, pxf.analyses
     ro, ao = zernike_orders(7)
-    coeff = zernike_coeff(len(ro), rng_seed)
+    coeff = zernike_coeff(len(ro), rng_seed) if coeff is None else coeff
     seed(rng_seed)
     rays = src.subannulus(220., 220.6, 100. / 220., n, zhat=-1., **_source_kw(rng, rng_seed, device))
     with pxf.fused(rays):
@@ -553,6 +554,48 @@ def config3_fast(n=100_000_000, rng="numpy", rng_seed=0, device=None, want_idx=T
     if want_idx:
         out["idx"] = tran.surviving_indices(alive)
     return out
+
+
+def config3_program(coeff):
+    """The 14-op program ``config3_fast`` records, written out (transform arguments negated, as
+    ``transformations.transform`` passes them on): the same ops with the same scalars, so the same bits."""
+    pxf = _pxf()
+    ro, ao = zernike_orders(7)
+    return (pxf.Program().transform(-220.3, 0., 100., 0., 0., 0.).zernsurf(coeff, ro, ao, 62.5, 1.).reflect()
+            .transform(0., 0., 0., -np.pi, 0., 0.).flatopd(1.).transform(220.3, 0., 8600., 0., 0., 0.)
+            .wolterprimary(220., 8400., 1.).reflect().vignette_box(3, 8426., 8526.).vignette_abs(2, 50.)
+            .woltersecondary(220., 8400., 1.).reflect().vignette_mag().flat())
+
+
+def config3_tolerance_fast(n, coeffs, rng="numpy", rng_seed=0, device=None, sources=None):
+    """A figure-error Monte Carlo of config 3 as ONE bundle: one realisation per coefficient vector in ``coeffs``
+    (e.g. ``zernike_coeff(36, seed_k)``).  The source is drawn once and replicated per realisation (the loop of
+    ``config3_fast(coeff=c_k)`` draws the same rays every time), one segmented launch traces every realisation
+    through its own Zernike surface, one compaction drops the vignetted rays, and ``hpd`` / ``rmsCentroid`` run per
+    segment.  Returns one dict per realisation with the keys of ``config3_fast``: ``rays`` is the realisation's view
+    of the compacted bundle, ``idx`` the surviving indices within its own n rays."""
+    pxf = _pxf()
+    from pyxfocus_b200._call import bundle_alloc, bundle_split
+    tran, anal = pxf.transformations, pxf.analyses
+    K = len(coeffs)
+    seed(rng_seed)
+    src = (sources or pxf.sources).subannulus(220., 220.6, 100. / 220., n, zhat=-1.,
+                                               **_source_kw(rng, rng_seed, device))
+    dev = src[1].device
+    rays = bundle_alloc(K * n, dev)
+    for r, s_ in zip(rays, src):
+        r.view(K, n).copy_(s_.unsqueeze(0).expand(K, n))
+    del src
+    segs = pxf.Segments([n] * K, device=dev)
+    alive = pxf.SegmentedProgram([config3_program(c) for c in coeffs], segs.sizes(), device=dev).run(rays)
+    after = segs.after(alive)
+    surv = tran.compact(rays, alive)
+    idx = tran.surviving_indices(alive)
+    hpd, rms = anal.hpd(surv, segments=after), anal.rmsCentroid(surv, segments=after)
+    kept = after.sizes()
+    views = bundle_split(surv, kept)
+    return [dict(rays=views[k], hpd=float(hpd[k]), rms=float(rms[k]),
+                 idx=idx[after.start[k]:after.start[k + 1]] - k * n) for k in range(K)]
 
 
 def config4_fast(n_per_shell=1000, M=72, order=-3, wave=2.4, rng="numpy", rng_seed=0, device=None, offX=0., offY=0.,
@@ -670,6 +713,8 @@ def baseline_programs():
         (P().transform(1, 0, 1, 0, 0, 0).zernsurf(zernike_coeff(len(ro)), ro, ao, 62.5, 1.).reflect().transform(0, 0, 0, 1, 0, 0)
          .flatopd(1.).transform(1, 0, 1, 0, 0, 0).wolterprimary(220., 8400., 1.).reflect().vignette_box(3, 0, 1).vignette_abs(2, 1.)
          .woltersecondary(220., 8400., 1.).reflect().vignette_mag().flat(), False),
+        # config 3 as a figure-error Monte Carlo: one Zernike surface per segment (segmented)
+        (config3_program(zernike_coeff(len(ro))), True),
         # config 4: SPO shells (segmented), the grating fan, the way back, the outlier cut
         (P().transform(0, 0, 0, 0, 0, 1).spocone(700., .01).kickn(0, 0).reflect().spocone(700., .03).reflect()
          .transform(0, 0, 1, 0, 0, 0).transform(0, 0, 1, 0, 0, 0).flat(), True),

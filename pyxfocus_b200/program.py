@@ -387,7 +387,11 @@ class SegmentedProgram:
         seg = SegmentedProgram(progs, sizes)      # sizes[k] = rays of shell k, concatenated in this order
         seg.run(bundle)
 
-    The per-segment op tables are folded once on the host and uploaded once; ``run`` is a single kernel."""
+    The per-segment op tables are folded once on the host and uploaded once; ``run`` is a single kernel.
+
+    Every program may carry one ``zernsurf`` at the same position, each with its own terms, ``rad`` and ``nr`` (a
+    Monte Carlo over figure-error realisations, or a shell assembly with a measured figure per shell); the segment's
+    Zernike table is staged with its op table.  ``nr`` must be given for all segments or for none."""
 
     def __init__(self, programs, sizes, device=None):
         import numpy as np
@@ -413,9 +417,24 @@ class SegmentedProgram:
                 for j, v in enumerate(p):
                     o.p[j] = v
         L = _lib.lib()
-        nbytes = int(L.pxf_segmented_table_bytes(nops, self.nseg))
-        self.table_host = torch.empty(nbytes, dtype=torch.uint8)
-        _lib.check(L.pxf_segmented_table_fill(arr, nops, self.nseg, start.ctypes.data, self.table_host.data_ptr()))
+        zpos = [k for k, (c, _) in enumerate(programs[0].ops) if c == OP["ZERNSURF"]]
+        if zpos:
+            kz = zpos[0]
+            for p in programs:
+                if kz not in p._tables:
+                    raise ValueError("a zernsurf op needs the table Program.zernsurf records")
+                if p.ops[kz][1][1] != programs[0].ops[kz][1][1]:
+                    raise ValueError("every segment's zernsurf must give nr, or none may (tracezernOPD vs tracezern)")
+            # one host table per segment, back to back (include/pxf.h, pxf_segmented_table_fill_zern)
+            zt = torch.cat([p._tables[kz] for p in programs])
+            nbytes = int(L.pxf_segmented_table_bytes_zern(nops, self.nseg))
+            self.table_host = torch.empty(nbytes, dtype=torch.uint8)
+            _lib.check(L.pxf_segmented_table_fill_zern(arr, nops, self.nseg, start.ctypes.data, zt.data_ptr(),
+                                                       self.table_host.data_ptr()))
+        else:
+            nbytes = int(L.pxf_segmented_table_bytes(nops, self.nseg))
+            self.table_host = torch.empty(nbytes, dtype=torch.uint8)
+            _lib.check(L.pxf_segmented_table_fill(arr, nops, self.nseg, start.ctypes.data, self.table_host.data_ptr()))
         dev = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
         self.table_dev = self.table_host.to(dev)
         self.seg_start_dev = torch.from_numpy(start).to(dev)
