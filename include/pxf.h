@@ -289,8 +289,17 @@ enum {
     PXF_OP_GRATFAN = 24,       /* p: ang,hubdist,l,dpermm,order,wave ; the fanned radial-grating array of
                                   examples/arcus/sector.py:636-700 as ONE per-ray loop (see pxf_trace_program_aux).
                                   wave = NaN: per-ray wavelengths from aux.wave (radgratW), else scalar (radgrat). */
-    PXF_OP_ROTX_REMAINING = 25 /* p: ang,total ; apply transform(0,0,0,ang,0,0) (total - aux.count[i]) times: the
+    PXF_OP_ROTX_REMAINING = 25, /* p: ang,total ; apply transform(0,0,0,ang,0,0) (total - aux.count[i]) times: the
                                   whole-bundle rotations a ray still receives after it met its grating */
+    PXF_OP_LLSURF = 26         /* p: table (a DEVICE copy of what pxf_ll_table_fill wrote, its address bit-cast into
+                                  the double), highest order as returned by the fill (it must be that value: the
+                                  specialised kernels evaluate the terms up to the order p[1] rounds to -- 3, 5 or
+                                  7 -- so a smaller p[1] drops terms on that path, silently, and not in the
+                                  interpreter, which evaluates all 8x8).  A Legendre-Legendre shell
+                                  (wolterprimLL / woltersecLL / ellipsoidWoltLL, the kind is in the table) with the
+                                  bits of pxf_wolterprimll / pxf_woltersecll / pxf_ellipsoidwoltll.  Orders <= 7 only;
+                                  at most two per program, and not in a program with PXF_OP_ZERNSURF or
+                                  PXF_OP_GRATFAN (PXF_ERR_UNSUPPORTED).                                          */
 };
 typedef struct pxf_op {
     int32_t code;
@@ -308,6 +317,15 @@ typedef struct pxf_op {
 size_t pxf_zern_table_bytes(void);
 int32_t pxf_zern_table_fill(const double *coeff, const int32_t *rorder, const int32_t *aorder, int32_t arrsize,
                             double rad, int32_t opd, double nr, void *table_host);
+/* Table for a PXF_OP_LLSURF op: folds the term list exactly as pxf_wolterprimll (kind 0; psi and S unused),
+ * pxf_woltersecll (kind 1; S unused) or pxf_ellipsoidwoltll (kind 2) do, into pxf_ll_table_bytes() bytes of HOST
+ * memory: the scalars and the coefficient matrix as an 8x8 block, zero beyond the orders present.  The caller uploads
+ * them unchanged.  Returns the highest axial / azimuthal order (0..7), or -1 for an invalid term list or an order
+ * above 7 (those run through the stand-alone routines). */
+size_t pxf_ll_table_bytes(void);
+int32_t pxf_ll_table_fill(int32_t kind, double r0, double z0, double psi, double S, double zmax, double zmin,
+                          double dphi, const double *coeff, const int32_t *axial, const int32_t *az, int32_t cnum,
+                          void *table_host);
 int pxf_trace_program(double *const rays[10], int64_t num, const pxf_op *ops, int32_t nops,
                       uint8_t *alive, pxf_stream_t stream);
 /* Per-ray side arrays of the ops that need them (all device pointers, each nullable unless an op uses it):
@@ -339,7 +357,7 @@ int pxf_trace_program_aux(double *const rays_in[10], double *const rays_out[10],
  *   pxf_jit_compile      compile (no GPU needed) the kernels a program will want -- in place / out of place, with /
  *                        without the centroid sums; segmented != 0: the segmented form.  Returns the number of
  *                        kernels now available (0: NVRTC missing or the compilation failed), -1: invalid program.
- *                        PXF_OP_ZERNSURF: any non-null table address will do; aux may be NULL.
+ *                        PXF_OP_ZERNSURF / PXF_OP_LLSURF: any non-null table address will do; aux may be NULL.
  *   pxf_jit_status       "ok" or why the interpreter is being used, plus counters
  *   pxf_last_trace_kernel  name of the kernel the last trace on this process launched                          */
 int32_t pxf_jit_compile(const pxf_op *ops, int32_t nops, int32_t segmented, const pxf_program_aux *aux);
@@ -386,6 +404,21 @@ int pxf_trace_program_segmented(double *const rays_in[10], double *const rays_ou
 size_t pxf_segmented_table_bytes_zern(int32_t nops, int32_t nseg);
 int pxf_segmented_table_fill_zern(const pxf_op *ops, int32_t nops, int32_t nseg, const int64_t *seg_start,
                                   const void *zern_tables_host, void *table_host);
+/* Segmented programs with Legendre-Legendre shells (a figure-error Monte Carlo of a Wolter-I pair, or shells that each
+ * have a measured figure): every segment's op list has its PXF_OP_LLSURF ops (one or two) at the same positions.
+ * Kinds, term lists and orders (<= 7) may differ between segments.  pxf_segmented_table_fill and
+ * pxf_segmented_table_fill_zern refuse such lists; this pair takes them (and any list the plain pair takes).
+ *   ll_tables_host: nseg * (LL ops per program) tables of pxf_ll_table_bytes() bytes, segment-major and in op order,
+ *   each filled by pxf_ll_table_fill (NULL is accepted when no op is a PXF_OP_LLSURF).  They are copied into the
+ *   segmented table (pxf_segmented_table_bytes_ll has room for two per segment), so it stays self-contained: upload
+ *   it unchanged and pass both copies to pxf_trace_program_segmented -- still ONE launch.  The op's p[0] (device
+ *   table address) is not used; at each LL position every segment is evaluated at the largest order of any segment
+ *   there, which gives the same bits as its own order.
+ *   Returns PXF_ERR_UNSUPPORTED for an order above 7, a third LL op and PXF_OP_GRATFAN / PXF_OP_ROTX_REMAINING,
+ *   PXF_ERR_INVALID for segments that differ in opcode sequence, or for missing tables. */
+size_t pxf_segmented_table_bytes_ll(int32_t nops, int32_t nseg);
+int pxf_segmented_table_fill_ll(const pxf_op *ops, int32_t nops, int32_t nseg, const int64_t *seg_start,
+                                const void *ll_tables_host, void *table_host);
 
 /* ======================= vignetting / compaction ======================== */
 /* flags[i] = (l^2+m^2+n^2 > .1), the default predicate of transformations.vignette

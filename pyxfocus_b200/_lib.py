@@ -199,6 +199,10 @@ SIGNATURES = {
     "pxf_segmented_table_fill": (_c.c_int, [_vp, _i32, _i32, _vp, _vp]),
     "pxf_segmented_table_bytes_zern": (_sz, [_i32, _i32]),
     "pxf_segmented_table_fill_zern": (_c.c_int, [_vp, _i32, _i32, _vp, _vp, _vp]),
+    "pxf_ll_table_bytes": (_sz, []),
+    "pxf_ll_table_fill": (_i32, [_i32, _d, _d, _d, _d, _d, _d, _d, _vp, _vp, _vp, _i32, _vp]),
+    "pxf_segmented_table_bytes_ll": (_sz, [_i32, _i32]),
+    "pxf_segmented_table_fill_ll": (_c.c_int, [_vp, _i32, _i32, _vp, _vp, _vp]),
     "pxf_trace_program_segmented": (_c.c_int, [_vp, _vp, _i64, _vp, _vp, _vp, _st]),
     "pxf_source_from_uniform": (_c.c_int, [_i32, _vp, _i64, _dp, _dp, _d, _d, _d, _d, _st]),
     "pxf_source_grid": (_c.c_int, [_i32, _vp, _i64, _i64, _i64, _i64, _d, _d, _d, _st]),

@@ -16,6 +16,7 @@ struct NoP { double unused; };
 // what an op may need besides the ray and its parameters
 struct ChainCtx {
     const ZernP *zt;          // Zernike table staged in shared memory (PXF_OP_ZERNSURF)
+    const LLTab *llt;         // LL tables staged in shared memory, by slot (PXF_OP_LLSURF)
     int64_t i;                // index of the ray in the bundle (side arrays)
     const double *aux_wave;   // pxf_program_aux
     int *aux_count;
@@ -23,7 +24,7 @@ struct ChainCtx {
 };
 PXF_DEV ChainCtx chain_ctx_none()
 {
-    ChainCtx c; c.zt = nullptr; c.i = 0; c.aux_wave = nullptr; c.aux_count = nullptr; c.aux_count_max = nullptr;
+    ChainCtx c; c.zt = nullptr; c.llt = nullptr; c.i = 0; c.aux_wave = nullptr; c.aux_count = nullptr; c.aux_count_max = nullptr;
     return c;
 }
 
@@ -115,6 +116,20 @@ struct CZernSurf {
         return true;
     }
 };
+// LLSURF: q = {N, slot}; the table comes through the context.  Both are template arguments: N is the op's order as
+// make_ll rounds it (3, 5, 7), read from the zero-padded 8x8 block with static offsets -- the same bits as the
+// per-routine kernel of that order (pxf_ray.cuh, LLTab)
+struct LLOpP { double n, slot; };
+template <int N, int SLOT> struct CLLSurf {
+    using P = LLOpP;
+    static constexpr int CODE = 26;
+    PXF_DEV static bool apply(Ray &r, const P &, const ChainCtx &ctx)
+    {
+        const LLTab &t = ctx.llt[SLOT];
+        op_ll<N, PXF_LL_PROG_MAXN + 1>(r, t.s, t.C);
+        return true;
+    }
+};
 struct CGratFan {
     using P = GratFanP;
     static constexpr int CODE = 24;
@@ -164,13 +179,14 @@ template <class Op, class... Rest> struct Chain<Op, Rest...> {
 
 // ---- kernel bodies for the run-time specialised chains ----
 // MODE 2: two rays per thread-iteration (double2 rows), 1: one ray (also the path for unaligned rows).
-// LMc/SMc: the program's row masks as compile-time constants.
-template <class C, class CP, int MODE, bool ZERN, unsigned LMc, unsigned SMc>
+// LMc/SMc: the program's row masks as compile-time constants.  NLL: the number of PXF_OP_LLSURF ops (tables ll0, ll1).
+template <class C, class CP, int MODE, bool ZERN, int NLL, unsigned LMc, unsigned SMc>
 PXF_DEV void chain_body(const RowPtrs &P, const RowPtrs &Q, const int64_t num, uint8_t *__restrict__ alive,
                         double *__restrict__ partials, const CP &prm, const ZernP *__restrict__ zern_dev,
-                        const double *__restrict__ aux_wave, int *__restrict__ aux_count, int *__restrict__ aux_count_max)
+                        const double *__restrict__ aux_wave, int *__restrict__ aux_count, int *__restrict__ aux_count_max,
+                        const LLTab *__restrict__ ll0, const LLTab *__restrict__ ll1)
 {
-    __shared__ __align__(16) unsigned char zraw[ZERN ? sizeof(ZernP) : 16];
+    __shared__ __align__(16) unsigned char zraw[ZERN ? sizeof(ZernP) : NLL ? NLL * sizeof(LLTab) : 16];
     ChainCtx ctx = chain_ctx_none();
     ctx.aux_wave = aux_wave; ctx.aux_count = aux_count; ctx.aux_count_max = aux_count_max;
     if (ZERN && zern_dev) {
@@ -179,6 +195,14 @@ PXF_DEV void chain_body(const RowPtrs &P, const RowPtrs &Q, const int64_t num, u
         for (int t = threadIdx.x; t < (int)(sizeof(ZernP) / 8); t += blockDim.x) dst[t] = src[t];
         __syncthreads();
         ctx.zt = reinterpret_cast<const ZernP *>(zraw);
+    }
+    if (NLL) {
+        double *dst = reinterpret_cast<double *>(zraw);
+        for (int j = 0; j < NLL; j++) {
+            const double *src = reinterpret_cast<const double *>(j ? ll1 : ll0);
+            for (int t = threadIdx.x; t < (int)(sizeof(LLTab) / 8); t += blockDim.x) dst[j * (int)(sizeof(LLTab) / 8) + t] = src[t];
+        }
+        __syncthreads();
     }
     double cnt = 0., sx = 0., sy = 0.;
     const int64_t tid = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -213,6 +237,14 @@ PXF_DEV void chain_body(const RowPtrs &P, const RowPtrs &Q, const int64_t num, u
             Ray a;
             fload1(a, P, LMc, i);
             ctx.i = i;
+            // NLL (one ray per thread): the staged tables are addressed per ray through an opaque zero, as in
+            // chain_seg_body.  Hoisted out of the loop, their scalars and coefficients stay in registers (ptxas for the
+            // LL pair at N = 5, no cap: 254 registers against 154 with the re-addressing).
+            if (NLL) {
+                int z = 0;
+                asm volatile("" : "+r"(z));
+                ctx.llt = reinterpret_cast<const LLTab *>(zraw) + z;
+            }
             const bool ka = C::run(a, prm, ctx);
             fstore1(a, Q, SMc, i);
             if (alive) alive[i] = ka ? 1 : 0;
@@ -224,15 +256,17 @@ PXF_DEV void chain_body(const RowPtrs &P, const RowPtrs &Q, const int64_t num, u
 
 // Segmented form (nested assemblies): the bundle is walked in tiles of CHAIN_SEG_TILE consecutive rays; a CTA stages
 // the parameter pack of the segment its tile lies in (re-staged only when the segment changes).  ZERN: zern holds one
-// Zernike table per segment, staged with the pack.
+// Zernike table per segment, staged with the pack.  NLL: ll holds NLL LL tables per segment (segment-major), staged
+// likewise.
 #define CHAIN_SEG_TILE (PXF_BLOCK * 8)
-template <class C, class CP, bool ZERN, unsigned LMc, unsigned SMc>
+template <class C, class CP, bool ZERN, int NLL, unsigned LMc, unsigned SMc>
 PXF_DEV void chain_seg_body(const RowPtrs &P, const RowPtrs &Q, const int64_t num, uint8_t *__restrict__ alive,
                             const long long *__restrict__ seg_start, const CP *__restrict__ table, const int nseg,
-                            const unsigned LMr, const unsigned SMr, const ZernP *__restrict__ zern)
+                            const unsigned LMr, const unsigned SMr, const ZernP *__restrict__ zern,
+                            const LLTab *__restrict__ ll)
 {
     __shared__ __align__(16) CP sp;
-    __shared__ __align__(16) unsigned char zraw[ZERN ? sizeof(ZernP) : 16];
+    __shared__ __align__(16) unsigned char zraw[ZERN ? sizeof(ZernP) : NLL ? NLL * sizeof(LLTab) : 16];
     const unsigned LM = LMc ? LMc : LMr, SM = SMc ? SMc : SMr;
     ChainCtx ctx = chain_ctx_none();
     int staged = -1;
@@ -259,6 +293,11 @@ PXF_DEV void chain_seg_body(const RowPtrs &P, const RowPtrs &Q, const int64_t nu
                     double *zdst = reinterpret_cast<double *>(zraw);
                     for (int t = threadIdx.x; t < (int)(sizeof(ZernP) / 8); t += blockDim.x) zdst[t] = zsrc[t];
                 }
+                if (NLL) {
+                    const double *lsrc = reinterpret_cast<const double *>(ll + (int64_t)seg * NLL);
+                    double *ldst = reinterpret_cast<double *>(zraw);
+                    for (int t = threadIdx.x; t < NLL * (int)(sizeof(LLTab) / 8); t += blockDim.x) ldst[t] = lsrc[t];
+                }
                 __syncthreads();
                 staged = seg;
             }
@@ -267,12 +306,12 @@ PXF_DEV void chain_seg_body(const RowPtrs &P, const RowPtrs &Q, const int64_t nu
                 fload1(a, P, LM, i);
                 // ZERN: the staged pack and table are addressed per ray through an opaque zero.  Hoisted out of this
                 // loop their loads would hold ~90 more registers than the fused Zernike kernel does (ptxas, no cap:
-                // 242 vs 150) and spill at its 3 CTAs/SM.  Without ZERN, z is the constant 0.
+                // 242 vs 150) and spill at its 3 CTAs/SM.  NLL: likewise (the LL pair at N = 5, no cap: 255 registers
+                // and spills, against 154 with the re-addressing).  Otherwise z is the constant 0.
                 int z = 0;
-                if (ZERN) {
-                    asm volatile("" : "+r"(z));
-                    ctx.zt = reinterpret_cast<const ZernP *>(zraw) + z;
-                }
+                if (ZERN || NLL) asm volatile("" : "+r"(z));
+                if (ZERN) ctx.zt = reinterpret_cast<const ZernP *>(zraw) + z;
+                if (NLL) ctx.llt = reinterpret_cast<const LLTab *>(zraw) + z;
                 const bool keep = C::run(a, (&sp)[z], ctx);
                 fstore1(a, Q, SM, i);
                 if (alive) alive[i] = keep ? 1 : 0;

@@ -31,9 +31,11 @@ PXF_DEV void count_max_update(int *dst, int k)
 // i: the ray's index in the bundle (side arrays); aux_*: FusedProgram::aux_* (null unless the program uses them)
 // AUX: whether this instantiation carries the side-array ops (the grating fan: asin + a data-dependent loop) -- like
 // ZERN they get their own kernel so that every other program keeps its register budget
-template <bool ZERN = false, bool AUX = false>
+// LL: whether it carries the Legendre-Legendre shells (PXF_OP_LLSURF); llt: their tables in shared memory, by slot
+template <bool ZERN = false, bool AUX = false, bool LL = false>
 PXF_DEV bool run_op(Ray &r, const FusedOp &op, const ZernP *zt = nullptr, int64_t i = 0,
-                    const double *aux_wave = nullptr, int *aux_count = nullptr, int *aux_count_max = nullptr)
+                    const double *aux_wave = nullptr, int *aux_count = nullptr, int *aux_count_max = nullptr,
+                    const LLTab *llt = nullptr)
 {
     switch (op.code) {
         case PXF_OP_KICKN: op_kickn(r, *reinterpret_cast<const KickNP *>(op.q)); break;
@@ -96,6 +98,11 @@ PXF_DEV bool run_op(Ray &r, const FusedOp &op, const ZernP *zt = nullptr, int64_
                 if (zt) op_tracezern<7>(r, zt->rad, zt->nr, zt->tol, zt->nmax, op.q[1] != 0., reinterpret_cast<const double *>(zt->e));
             }
             break;
+        case PXF_OP_LLSURF:
+            // every table is an 8x8 block padded with zeros: the order-7 evaluation gives the bits of the per-routine
+            // kernel of the table's own order (pxf_ray.cuh, LLTab)
+            if constexpr (LL) op_ll<PXF_LL_PROG_MAXN, PXF_LL_PROG_MAXN + 1>(r, llt[op.row].s, llt[op.row].C);
+            break;
         case PXF_OP_KICK: {
             r.l = r.l + op.q[0];
             r.m = r.m + op.q[1];
@@ -107,29 +114,41 @@ PXF_DEV bool run_op(Ray &r, const FusedOp &op, const ZernP *zt = nullptr, int64_
     return true;
 }
 
-template <bool ZERN = false, bool AUX = false>
-PXF_DEV bool run_program(Ray &r, const FusedProgram &prog, const ZernP *zt = nullptr, int64_t i = 0)
+template <bool ZERN = false, bool AUX = false, bool LL = false>
+PXF_DEV bool run_program(Ray &r, const FusedProgram &prog, const ZernP *zt = nullptr, int64_t i = 0,
+                         const LLTab *llt = nullptr)
 {
     for (int k = 0; k < prog.nops; k++)
-        if (!run_op<ZERN, AUX>(r, prog.ops[k], zt, i, prog.aux_wave, prog.aux_count, prog.aux_count_max)) return false;
+        if (!run_op<ZERN, AUX, LL>(r, prog.ops[k], zt, i, prog.aux_wave, prog.aux_count, prog.aux_count_max, llt))
+            return false;
     return true;
 }
 
-template <bool VEC2, int MINB = 1, bool ZERN = false, bool AUX = false>
+template <bool VEC2, int MINB = 1, bool ZERN = false, bool AUX = false, bool LL = false>
 __global__ void __launch_bounds__(PXF_BLOCK, MINB)
 k_program(const RowPtrs P, const RowPtrs Q, const int64_t num, uint8_t *__restrict__ alive,
           double *__restrict__ partials, const __grid_constant__ FusedProgram prog)
 {
     double cnt = 0., sx = 0., sy = 0.;
-    // the Zernike table of a PXF_OP_ZERNSURF op, staged once per CTA
-    __shared__ __align__(16) unsigned char zraw[ZERN ? sizeof(ZernP) : 16];
+    // the Zernike table of a PXF_OP_ZERNSURF op, or the tables of the PXF_OP_LLSURF ops, staged once per CTA
+    __shared__ __align__(16) unsigned char zraw[ZERN ? sizeof(ZernP) : LL ? PXF_PROG_MAX_LL * sizeof(LLTab) : 16];
     const ZernP *zt = nullptr;
+    const LLTab *llt = nullptr;
     if (ZERN && prog.zern) {
         const double *src = reinterpret_cast<const double *>(prog.zern);
         double *dst = reinterpret_cast<double *>(zraw);
         for (int t = threadIdx.x; t < (int)(sizeof(ZernP) / 8); t += blockDim.x) dst[t] = src[t];
         __syncthreads();
         zt = reinterpret_cast<const ZernP *>(zraw);
+    }
+    if (LL) {
+        double *dst = reinterpret_cast<double *>(zraw);
+        for (int j = 0; j < prog.nll; j++) {
+            const double *src = reinterpret_cast<const double *>(prog.ll[j]);
+            for (int t = threadIdx.x; t < (int)(sizeof(LLTab) / 8); t += blockDim.x) dst[j * (sizeof(LLTab) / 8) + t] = src[t];
+        }
+        __syncthreads();
+        llt = reinterpret_cast<const LLTab *>(zraw);
     }
     // P: rows read, Q: rows written (Q == P for the in-place f2py semantics)
     const unsigned LM = prog.load_mask, SM = prog.store_mask;
@@ -141,8 +160,8 @@ k_program(const RowPtrs P, const RowPtrs Q, const int64_t num, uint8_t *__restri
             const int64_t i = q << 1;
             Ray a, b;
             fload2(a, b, P, LM, i);
-            const bool ka = run_program<ZERN, AUX>(a, prog, zt, i);
-            const bool kb = run_program<ZERN, AUX>(b, prog, zt, i + 1);
+            const bool ka = run_program<ZERN, AUX, LL>(a, prog, zt, i, llt);
+            const bool kb = run_program<ZERN, AUX, LL>(b, prog, zt, i + 1, llt);
             fstore2(a, b, Q, SM, i);
             if (alive) { alive[i] = ka ? 1 : 0; alive[i + 1] = kb ? 1 : 0; }
             if (ka) { cnt += 1.; sx += a.x; sy += a.y; }
@@ -152,7 +171,7 @@ k_program(const RowPtrs P, const RowPtrs Q, const int64_t num, uint8_t *__restri
             const int64_t i = num - 1;
             Ray a;
             fload1(a, P, LM, i);
-            const bool ka = run_program<ZERN, AUX>(a, prog, zt, i);
+            const bool ka = run_program<ZERN, AUX, LL>(a, prog, zt, i, llt);
             fstore1(a, Q, SM, i);
             if (alive) alive[i] = ka ? 1 : 0;
             if (ka) { cnt += 1.; sx += a.x; sy += a.y; }
@@ -161,7 +180,7 @@ k_program(const RowPtrs P, const RowPtrs Q, const int64_t num, uint8_t *__restri
         for (int64_t i = tid; i < num; i += nthr) {
             Ray a;
             fload1(a, P, LM, i);
-            const bool ka = run_program<ZERN, AUX>(a, prog, zt, i);
+            const bool ka = run_program<ZERN, AUX, LL>(a, prog, zt, i, llt);
             fstore1(a, Q, SM, i);
             if (alive) alive[i] = ka ? 1 : 0;
             if (ka) { cnt += 1.; sx += a.x; sy += a.y; }
@@ -178,24 +197,32 @@ k_program(const RowPtrs P, const RowPtrs Q, const int64_t num, uint8_t *__restri
 // SEG_TILE consecutive rays; a CTA stages the op table of the segment its tile lies in into shared memory
 // (re-staged only when the segment changes; a tile that straddles segments is processed piecewise).
 // A program with a PXF_OP_ZERNSURF op carries one Zernike table per segment (zern_off: their offset in the table,
-// 0 = none); the table of the segment is staged next to its op table.
+// 0 = none); the table of the segment is staged next to its op table.  A program with nll PXF_OP_LLSURF ops carries
+// nll LL tables per segment (ll_off), staged the same way.
 #define SEG_TILE (PXF_BLOCK * 8)
-struct SegHeader { unsigned load_mask, store_mask; int nops, nseg; int chain_id, jit_pack_bytes; long long zern_off; };
+struct SegHeader {
+    unsigned load_mask, store_mask; int nops, nseg; int chain_id, jit_pack_bytes; long long zern_off;
+    long long ll_off; int nll, unused;
+};
 static_assert(sizeof(ZernP) % 16 == 0, "per-segment Zernike tables are laid out back to back, 16-byte aligned");
+static_assert(sizeof(LLTab) % 8 == 0, "per-segment LL tables are laid out back to back, whole doubles");
 
-// shared-memory offset of the staged Zernike table: behind the op table, 16-byte aligned
+// shared-memory offset of the staged Zernike or LL tables: behind the op table, 16-byte aligned
 __host__ __device__ __forceinline__ int seg_zern_smem_offset(int nops) { return (nops * (int)sizeof(FusedOp) + 15) & ~15; }
 
 // ZERN: zern = nseg Zernike tables, one per segment (the Zernike instantiation of run_op, as k_program<.., true>)
-template <int MINB, bool ZERN = false>
+// LL: ll = nseg * nll LL tables, segment-major (the LL instantiation of run_op, as k_program<.., LL = true>)
+template <int MINB, bool ZERN = false, bool LL = false>
 __global__ void __launch_bounds__(PXF_BLOCK, MINB)
 k_program_seg(const RowPtrs P, const RowPtrs Q, const int64_t num, uint8_t *__restrict__ alive,
               const long long *__restrict__ seg_start, const FusedOp *__restrict__ ops, const int nops, const int nseg,
-              const unsigned LM, const unsigned SM, const ZernP *__restrict__ zern)
+              const unsigned LM, const unsigned SM, const ZernP *__restrict__ zern, const LLTab *__restrict__ ll,
+              const int nll)
 {
     extern __shared__ __align__(16) unsigned char seg_smem[];
     FusedOp *sops = reinterpret_cast<FusedOp *>(seg_smem);
     ZernP *zt = ZERN ? reinterpret_cast<ZernP *>(seg_smem + seg_zern_smem_offset(nops)) : nullptr;
+    LLTab *llt = LL ? reinterpret_cast<LLTab *>(seg_smem + seg_zern_smem_offset(nops)) : nullptr;
     int staged = -1;
     const int words = nops * (int)(sizeof(FusedOp) / 8);
     for (int64_t t0 = (int64_t)blockIdx.x * SEG_TILE; t0 < num; t0 += (int64_t)gridDim.x * SEG_TILE) {
@@ -211,6 +238,11 @@ k_program_seg(const RowPtrs P, const RowPtrs Q, const int64_t num, uint8_t *__re
                     double *zdst = reinterpret_cast<double *>(zt);
                     for (int t = threadIdx.x; t < (int)(sizeof(ZernP) / 8); t += blockDim.x) zdst[t] = zsrc[t];
                 }
+                if (LL) {
+                    const double *lsrc = reinterpret_cast<const double *>(ll + (int64_t)seg * nll);
+                    double *ldst = reinterpret_cast<double *>(llt);
+                    for (int t = threadIdx.x; t < nll * (int)(sizeof(LLTab) / 8); t += blockDim.x) ldst[t] = lsrc[t];
+                }
                 __syncthreads();
                 staged = seg;
             }
@@ -219,7 +251,7 @@ k_program_seg(const RowPtrs P, const RowPtrs Q, const int64_t num, uint8_t *__re
                 fload1(a, P, LM, i);
                 bool keep = true;
                 for (int k = 0; k < nops; k++)
-                    if (!run_op<ZERN>(a, sops[k], zt)) { keep = false; break; }
+                    if (!run_op<ZERN, false, LL>(a, sops[k], zt, 0, nullptr, nullptr, nullptr, llt)) { keep = false; break; }
                 fstore1(a, Q, SM, i);
                 if (alive) alive[i] = keep ? 1 : 0;
             }
@@ -251,6 +283,7 @@ static void op_masks(int code, int row, unsigned &use, unsigned &st, unsigned &k
         case PXF_OP_VIGNETTE_RHOGT: use = R_X | R_Y; st = 0; kill = 0; break;
         case PXF_OP_GRATFAN: case PXF_OP_ROTX_REMAINING: use = R_NINE; st = R_NINE; kill = 0; break;
         case PXF_OP_ZERNSURF: use = R_POS | R_DIR | (row ? R_OPD : 0u); st = R_POS | R_NRM | (row ? R_OPD : 0u); kill = R_POS | R_NRM; break;
+        case PXF_OP_LLSURF: use = R_POS | R_DIR; st = R_POS | R_NRM; kill = R_POS | R_NRM; break;
         default: use = 0; st = 0; kill = 0; break;
     }
 }
@@ -331,6 +364,27 @@ int build_program(FusedProgram &fp, const pxf_op *ops, int nops, const pxf_progr
                 f.row = p[1] != 0. ? 1 : 0;            // opd flag: decides whether row 0 is touched
                 break;
             }
+            case PXF_OP_LLSURF: {
+                const LLTab *tab;
+                memcpy(&tab, &p[0], sizeof(tab));
+                if (!tab) { set_error("program: PXF_OP_LLSURF needs a device table"); return PXF_ERR_INVALID; }
+                if (!(p[1] >= 0. && p[1] <= PXF_LL_PROG_MAXN)) {
+                    set_error("program: PXF_OP_LLSURF supports Legendre orders <= %d (use pxf_wolterprimll and the other "
+                              "stand-alone routines)", PXF_LL_PROG_MAXN);
+                    return PXF_ERR_UNSUPPORTED;
+                }
+                if (fp.nll == PXF_PROG_MAX_LL) {
+                    set_error("program: at most %d PXF_OP_LLSURF ops per program", PXF_PROG_MAX_LL);
+                    return PXF_ERR_UNSUPPORTED;
+                }
+                // q: the order N the specialised kernels evaluate (make_ll's rounding), the table slot
+                const int top = (int)p[1];
+                f.q[0] = top <= 3 ? 3. : top <= 5 ? 5. : 7.;
+                f.q[1] = (double)fp.nll;
+                f.row = fp.nll;
+                fp.ll[fp.nll++] = tab;
+                break;
+            }
             default: set_error("program: unknown opcode %d", o.code); return PXF_ERR_INVALID;
         }
         if (o.code == PXF_OP_VIGNETTE_MAG || o.code == PXF_OP_VIGNETTE_BOX || o.code == PXF_OP_VIGNETTE_ABS ||
@@ -346,6 +400,10 @@ int build_program(FusedProgram &fp, const pxf_op *ops, int nops, const pxf_progr
             fp.const_mask |= R_Z | R_NRM;
             fp.const_val[3] = 0.; fp.const_val[7] = 0.; fp.const_val[8] = 0.; fp.const_val[9] = 1.;
         }
+    }
+    if (fp.nll && (fp.zern || fp.uses_aux)) {
+        set_error("program: Legendre-Legendre shells cannot share a program with a Zernike surface or a grating fan");
+        return PXF_ERR_UNSUPPORTED;
     }
     if (fp.has_vignette) fp.const_mask = 0;
     // Backward liveness: a row is read from HBM only if some op consumes its incoming value
@@ -436,12 +494,25 @@ int launch_program(double *const rays[10], int64_t num, const FusedProgram &fp, 
         else if (zm == 2) go(k_program<false, 2, true>, num);
         else go(k_program<false, 3, true>, num);
     }
+    else if (fp.nll) {
+        // one ray per thread; PXF_LLPROG_MINB (tuning): register cap for 1 / 2 / 3 / 4 resident CTAs per SM.  Measured
+        // on the LL pair (36 terms per mirror) at 5e7 rays, out of place, one B200 at 1000 W: 11.6 / 13.7 / 20.2 / 28.2
+        // ms (1: 212 registers, no spills; 2-4 spill 0.4-0.8 KB); with 16 / 64 terms 11.9 / 12.7 ms at 1 CTA/SM
+        // (profiles/ll_program_bench_b200.json)
+        static int lm = -1;
+        if (lm < 0) { const char *e = getenv("PXF_LLPROG_MINB"); lm = e ? atoi(e) : 1; }
+        if (lm == 2) go(k_program<false, 2, false, false, true>, num);
+        else if (lm == 3) go(k_program<false, 3, false, false, true>, num);
+        else if (lm == 4) go(k_program<false, 4, false, false, true>, num);
+        else go(k_program<false, 1, false, false, true>, num);
+    }
     else if (aligned && variant == 0) go(k_program<true, 1>, (num + 1) >> 1);
     else if (variant == 3) go(k_program<false, 3>, num);
     else if (variant == 1) go(k_program<false, 1>, num);
     else go(k_program<false, 4>, num);
     count_launch();
-    note_kernel(fp.zern ? "k_program<zernike> (interpreter)" : (fp.uses_aux ? "k_program<aux> (interpreter)" : "k_program (interpreter)"));
+    note_kernel(fp.zern ? "k_program<zernike> (interpreter)" : fp.uses_aux ? "k_program<aux> (interpreter)" :
+                fp.nll ? "k_program<ll> (interpreter)" : "k_program (interpreter)");
     return check_launch("k_program");
 }
 
@@ -508,6 +579,38 @@ extern "C" int32_t pxf_zern_table_fill(const double *coeff, const int32_t *rorde
     return n;
 }
 
+extern "C" size_t pxf_ll_table_bytes(void) { return sizeof(LLTab); }
+
+extern "C" int32_t pxf_ll_table_fill(int32_t kind, double r0, double z0, double psi, double S, double zmax, double zmin,
+                                     double dphi, const double *coeff, const int32_t *axial, const int32_t *az,
+                                     int32_t cnum, void *table_host)
+{
+    if (!coeff || !axial || !az || cnum <= 0 || !table_host || kind < 0 || kind > 2) {
+        set_error("pxf_ll_table_fill: bad argument");
+        return -1;
+    }
+    // folded by the routine of the stand-alone kernels, so every scalar and coefficient has the same bits
+    LLP q;
+    if (make_ll(q, kind, r0, z0, psi, S, zmax, zmin, dphi, coeff, axial, az, cnum) < 0) {
+        set_error("pxf_ll_table_fill: invalid Legendre orders (need 0 <= order <= %d)", PXF_LL_MAXN);
+        return -1;
+    }
+    const int top = q.s.nz > q.s.nt ? q.s.nz : q.s.nt;
+    if (top > PXF_LL_PROG_MAXN) {
+        set_error("pxf_ll_table_fill: programs hold Legendre orders <= %d (this list has %d; use the stand-alone routine)",
+                  PXF_LL_PROG_MAXN, top);
+        return -1;
+    }
+    LLTab t;
+    memset(&t, 0, sizeof(t));
+    t.s = q.s;
+    const int N = q.s.stride - 1;
+    for (int a = 0; a <= N; a++)
+        for (int b = 0; b <= N; b++) t.C[a * (PXF_LL_PROG_MAXN + 1) + b] = q.C[a * q.s.stride + b];
+    memcpy(table_host, &t, sizeof(t));
+    return top;
+}
+
 // ---- segmented programs -------------------------------------------------------------------------
 static size_t seg_align(size_t v) { return (v + 15) & ~(size_t)15; }
 static size_t seg_ops_offset(int nseg) { return seg_align(sizeof(SegHeader)) + seg_align((size_t)(nseg + 1) * 8); }
@@ -535,10 +638,23 @@ extern "C" size_t pxf_segmented_table_bytes_zern(int32_t nops, int32_t nseg)
     return seg_zern_offset(nops, nseg) + (size_t)nseg * sizeof(ZernP);
 }
 
-// zern_tables: nseg tables of pxf_zern_table_fill (NULL: the program may not have a PXF_OP_ZERNSURF op)
-static int seg_table_fill(const pxf_op *ops, int nops, int nseg, const int64_t *seg_start, const void *zern_tables,
-                          bool zern_ok, void *table_host)
+// LL tables of a segmented program: at the same place, room for PXF_PROG_MAX_LL per segment
+extern "C" size_t pxf_segmented_table_bytes_ll(int32_t nops, int32_t nseg)
 {
+    if (nops < 1 || nseg < 1) return 0;
+    return seg_zern_offset(nops, nseg) + (size_t)nseg * PXF_PROG_MAX_LL * sizeof(LLTab);
+}
+
+// Which per-segment tables a fill takes: none, one Zernike table, or one LL table per PXF_OP_LLSURF op
+enum SegTables { SEG_PLAIN, SEG_ZERN, SEG_LL };
+
+// tables: nseg tables of pxf_zern_table_fill (SEG_ZERN), nseg * nll tables of pxf_ll_table_fill (SEG_LL), segment-major;
+// NULL: the program may not have such an op
+static int seg_table_fill(const pxf_op *ops, int nops, int nseg, const int64_t *seg_start, const void *tables,
+                          SegTables kind, void *table_host)
+{
+    const bool zern_ok = kind == SEG_ZERN, ll_ok = kind == SEG_LL;
+    const void *zern_tables = zern_ok ? tables : nullptr;
     if (!ops || !seg_start || !table_host || nops < 1 || nops > PXF_MAX_OPS || nseg < 1) {
         set_error("pxf_segmented_table_fill: bad argument");
         return PXF_ERR_INVALID;
@@ -547,23 +663,53 @@ static int seg_table_fill(const pxf_op *ops, int nops, int nseg, const int64_t *
     for (int sgm = 0; sgm < nseg; sgm++)
         if (seg_start[sgm + 1] < seg_start[sgm]) { set_error("segmented program: seg_start must be non-decreasing"); return PXF_ERR_INVALID; }
     bool zern = false;
-    if (zern_ok) {
+    if (zern_ok || ll_ok) {
         for (size_t k = 0; k < (size_t)nseg * nops; k++) {
             if (ops[k].code == PXF_OP_GRATFAN || ops[k].code == PXF_OP_ROTX_REMAINING) {
                 set_error("segmented program: PXF_OP_GRATFAN / PXF_OP_ROTX_REMAINING are not supported");
                 return PXF_ERR_UNSUPPORTED;
             }
-            if (ops[k].code == PXF_OP_ZERNSURF) zern = true;
+            if (ops[k].code == PXF_OP_ZERNSURF && zern_ok) zern = true;
         }
         if (zern && !zern_tables) { set_error("segmented program: PXF_OP_ZERNSURF needs one Zernike table per segment"); return PXF_ERR_INVALID; }
     }
+    // LL ops: their positions in segment 0's list (the others must match, checked with the opcode sequence below)
+    int llpos[PXF_PROG_MAX_LL], nll = 0;
+    for (size_t k = 0; k < (size_t)nseg * nops; k++)
+        if (ops[k].code == PXF_OP_LLSURF && !ll_ok) {
+            set_error("segmented program: PXF_OP_LLSURF needs pxf_segmented_table_fill_ll");
+            return PXF_ERR_UNSUPPORTED;
+        }
+    for (int k = 0; k < nops; k++)
+        if (ops[k].code == PXF_OP_LLSURF) {
+            if (nll == PXF_PROG_MAX_LL) { set_error("program: at most %d PXF_OP_LLSURF ops per program", PXF_PROG_MAX_LL); return PXF_ERR_UNSUPPORTED; }
+            llpos[nll++] = k;
+        }
+    if (nll && !tables) { set_error("segmented program: PXF_OP_LLSURF needs one LL table per op and segment"); return PXF_ERR_INVALID; }
     char *base = static_cast<char *>(table_host);
     SegHeader *h = reinterpret_cast<SegHeader *>(base);
     memset(h, 0, seg_align(sizeof(SegHeader)));
     memcpy(base + seg_align(sizeof(SegHeader)), seg_start, (size_t)(nseg + 1) * 8);
     FusedOp *dst = reinterpret_cast<FusedOp *>(base + seg_ops_offset(nseg));
     ZernP *zdst = zern ? reinterpret_cast<ZernP *>(base + seg_zern_offset(nops, nseg)) : nullptr;
+    LLTab *ldst = nll ? reinterpret_cast<LLTab *>(base + seg_zern_offset(nops, nseg)) : nullptr;
     h->nops = nops; h->nseg = nseg;
+    // the segment's own LL tables, copied into this one; every segment evaluates position j at the largest order
+    // any segment has there (the zero padding makes that the same bits)
+    int lln[PXF_PROG_MAX_LL] = {0, 0};
+    if (nll) {
+        memcpy(ldst, tables, (size_t)nseg * nll * sizeof(LLTab));
+        for (size_t t = 0; t < (size_t)nseg * nll; t++) {
+            const LLS &ls = ldst[t].s;
+            const int top = ls.nz > ls.nt ? ls.nz : ls.nt;
+            if (ls.kind < 0 || ls.kind > 2 || ls.nz < 0 || ls.nt < 0 || top > PXF_LL_PROG_MAXN) {
+                set_error("segmented program: segment %d: PXF_OP_LLSURF supports Legendre orders <= %d (table has %d)",
+                          (int)(t / nll), PXF_LL_PROG_MAXN, top);
+                return PXF_ERR_UNSUPPORTED;
+            }
+            if (top > lln[t % nll]) lln[t % nll] = top;
+        }
+    }
     for (int sgm = 0; sgm < nseg; sgm++) {
         pxf_op sops[PXF_MAX_OPS];
         memcpy(sops, ops + (size_t)sgm * nops, (size_t)nops * sizeof(pxf_op));
@@ -582,6 +728,12 @@ static int seg_table_fill(const pxf_op *ops, int nops, int nseg, const int64_t *
                     sops[k].p[2] = (double)nmax;
                 }
         }
+        for (int j = 0; j < nll; j++)
+            if (sops[llpos[j]].code == PXF_OP_LLSURF) {
+                const LLTab *any = ldst + (size_t)sgm * nll + j;
+                memcpy(&sops[llpos[j]].p[0], &any, sizeof(any));
+                sops[llpos[j]].p[1] = (double)lln[j];
+            }
         FusedProgram fp;
         int rc = build_program(fp, sops, nops);
         if (rc) return rc;
@@ -600,6 +752,7 @@ static int seg_table_fill(const pxf_op *ops, int nops, int nseg, const int64_t *
         memcpy(dst + (size_t)sgm * nops, fp.ops, (size_t)nops * sizeof(FusedOp));
     }
     if (zern) h->zern_off = (long long)seg_zern_offset(nops, nseg);
+    if (nll) { h->ll_off = (long long)seg_zern_offset(nops, nseg); h->nll = nll; }
     // a statically specialised kernel for the canonical chains: one parameter pack per segment behind the op table
     h->chain_id = seg_chain_fill(dst, nops, nseg, base + seg_chain_offset(nops, nseg));
     bool vig = false;
@@ -617,13 +770,19 @@ static int seg_table_fill(const pxf_op *ops, int nops, int nseg, const int64_t *
 extern "C" int pxf_segmented_table_fill(const pxf_op *ops, int32_t nops, int32_t nseg, const int64_t *seg_start,
                                         void *table_host)
 {
-    return seg_table_fill(ops, nops, nseg, seg_start, nullptr, false, table_host);
+    return seg_table_fill(ops, nops, nseg, seg_start, nullptr, SEG_PLAIN, table_host);
 }
 
 extern "C" int pxf_segmented_table_fill_zern(const pxf_op *ops, int32_t nops, int32_t nseg, const int64_t *seg_start,
                                              const void *zern_tables_host, void *table_host)
 {
-    return seg_table_fill(ops, nops, nseg, seg_start, zern_tables_host, true, table_host);
+    return seg_table_fill(ops, nops, nseg, seg_start, zern_tables_host, SEG_ZERN, table_host);
+}
+
+extern "C" int pxf_segmented_table_fill_ll(const pxf_op *ops, int32_t nops, int32_t nseg, const int64_t *seg_start,
+                                           const void *ll_tables_host, void *table_host)
+{
+    return seg_table_fill(ops, nops, nseg, seg_start, ll_tables_host, SEG_LL, table_host);
 }
 
 extern "C" int pxf_trace_program_segmented(double *const rays_in[10], double *const rays_out[10], int64_t num,
@@ -658,6 +817,8 @@ extern "C" int pxf_trace_program_segmented(double *const rays_in[10], double *co
     const long long *dstart = reinterpret_cast<const long long *>(db + seg_align(sizeof(SegHeader)));
     const FusedOp *dops = reinterpret_cast<const FusedOp *>(db + seg_ops_offset(nseg));
     const ZernP *dzern = h->zern_off ? reinterpret_cast<const ZernP *>(db + h->zern_off) : nullptr;
+    const LLTab *dll = h->ll_off ? reinterpret_cast<const LLTab *>(db + h->ll_off) : nullptr;
+    const int nll = dll ? h->nll : 0;
     cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
     if (h->chain_id == 1 && !vig) {
         int rc = seg_chain_launch(h->chain_id, P, Q, num, alive, dstart, db + seg_chain_offset(nops, nseg), nseg, LM, SM, s);
@@ -665,14 +826,14 @@ extern "C" int pxf_trace_program_segmented(double *const rays_in[10], double *co
     }
     if (h->chain_id == 2) {
         int rc = jit_seg_launch(hops, nops, P, Q, num, alive, dstart, db + seg_chain_offset(nops, nseg), nseg, LM, SM,
-                                dzern, s);
+                                dzern, dll, s);
         if (rc != PXF_ERR_UNSUPPORTED) return rc;
     }
     auto go = [&](auto kern, size_t smem) {
         int nb = 0;
         if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, kern, PXF_BLOCK, smem) != cudaSuccess || nb <= 0) { cudaGetLastError(); nb = 2; }
         const int grid = grid_for(num, SEG_TILE, nb);
-        kern<<<grid, PXF_BLOCK, smem, s>>>(P, Q, num, alive, dstart, dops, nops, nseg, LM, SM, dzern);
+        kern<<<grid, PXF_BLOCK, smem, s>>>(P, Q, num, alive, dstart, dops, nops, nseg, LM, SM, dzern, dll, nll);
     };
     if (dzern) {
         // the segment's Zernike table is staged behind its op table; register cap as for k_program<zernike>
@@ -686,6 +847,19 @@ extern "C" int pxf_trace_program_segmented(double *const rays_in[10], double *co
         count_launch();
         note_kernel("k_program_seg<zernike> (interpreter)");
         return check_launch("k_program_seg<zernike>");
+    }
+    if (dll) {
+        // the segment's LL tables are staged behind its op table; register cap as for k_program<ll> (PXF_LLPROG_MINB)
+        static int lm = -1;
+        if (lm < 0) { const char *e = getenv("PXF_LLPROG_MINB"); lm = e ? atoi(e) : 1; }
+        const size_t smem = (size_t)seg_zern_smem_offset(nops) + (size_t)nll * sizeof(LLTab);
+        if (lm == 2) go(k_program_seg<2, false, true>, smem);
+        else if (lm == 3) go(k_program_seg<3, false, true>, smem);
+        else if (lm == 4) go(k_program_seg<4, false, true>, smem);
+        else go(k_program_seg<1, false, true>, smem);
+        count_launch();
+        note_kernel("k_program_seg<ll> (interpreter)");
+        return check_launch("k_program_seg<ll>");
     }
     go(k_program_seg<4>, (size_t)nops * sizeof(FusedOp));
     count_launch();

@@ -55,6 +55,7 @@ static const OpDesc OPS[] = {
     {PXF_OP_VIGNETTE_RHOGT, "CVignetteRhoGt", sizeof(CVignetteRhoGt::P), false},
     {PXF_OP_GRATFAN, "CGratFan", sizeof(CGratFan::P), false},
     {PXF_OP_ROTX_REMAINING, "CRotxRemaining", sizeof(CRotxRemaining::P), false},
+    {PXF_OP_LLSURF, "CLLSurf", sizeof(LLOpP), false},
 };
 static const OpDesc *op_desc(int code)
 {
@@ -136,9 +137,10 @@ static Nvrtc g_nvrtc;
 
 // ---------------------------------------------------------------- signatures and source text
 struct JitSpec {
-    std::vector<int> codes, rows;
+    std::vector<int> codes;
+    std::vector<std::string> targs;     // template arguments of each functor ("" / "<row>" / "<N, slot>")
     unsigned LM = 0, SM = 0;
-    int mode = 2, minb = 3;
+    int mode = 2, minb = 3, nll = 0;
     bool zern = false, seg = false;
     size_t cp_bytes = 8;
     std::string chain_type() const
@@ -148,14 +150,14 @@ struct JitSpec {
             const OpDesc *d = op_desc(codes[k]);
             if (k) t += ", ";
             t += d->name;
-            if (d->row) t += "<" + std::to_string(rows[k]) + ">";
+            t += targs[k];
         }
         return t;
     }
     std::string signature() const
     {
-        char buf[96];
-        snprintf(buf, sizeof(buf), "v3;seg%d;m%d;b%d;z%d;L%u;S%u;", seg ? 1 : 0, mode, minb, zern ? 1 : 0, LM, SM);
+        char buf[112];
+        snprintf(buf, sizeof(buf), "v4;seg%d;m%d;b%d;z%d;l%d;L%u;S%u;", seg ? 1 : 0, mode, minb, zern ? 1 : 0, nll, LM, SM);
         return std::string(buf) + chain_type();
     }
     std::string source() const
@@ -169,17 +171,18 @@ struct JitSpec {
                      "extern \"C\" __global__ void __launch_bounds__(PXF_BLOCK, %d)\n"
                      "pxf_jit_chain(const RowPtrs P, const RowPtrs Q, const long long num, unsigned char *alive, double *partials,\n"
                      "              const ZernP *zern, const double *aux_wave, int *aux_count, int *aux_count_max,\n"
-                     "              const __grid_constant__ CP prm)\n"
-                     "{\n    chain_body<C, CP, %d, %s, %uu, %uu>(P, Q, num, alive, partials, prm, zern, aux_wave, aux_count, aux_count_max);\n}\n",
-                     minb, mode, zern ? "true" : "false", LM, SM);
+                     "              const LLTab *ll0, const LLTab *ll1, const __grid_constant__ CP prm)\n"
+                     "{\n    chain_body<C, CP, %d, %s, %d, %uu, %uu>(P, Q, num, alive, partials, prm, zern, aux_wave, aux_count,\n"
+                     "                                          aux_count_max, ll0, ll1);\n}\n",
+                     minb, mode, zern ? "true" : "false", nll, LM, SM);
         } else {
             snprintf(buf, sizeof(buf),
                      "extern \"C\" __global__ void __launch_bounds__(PXF_BLOCK, %d)\n"
                      "pxf_jit_chain(const RowPtrs P, const RowPtrs Q, const long long num, unsigned char *alive,\n"
                      "              const long long *seg_start, const CP *table, const int nseg, const unsigned LM, const unsigned SM,\n"
-                     "              const ZernP *zern)\n"
-                     "{\n    chain_seg_body<C, CP, %s, %uu, %uu>(P, Q, num, alive, seg_start, table, nseg, LM, SM, zern);\n}\n",
-                     minb, zern ? "true" : "false", LM, SM);
+                     "              const ZernP *zern, const LLTab *ll)\n"
+                     "{\n    chain_seg_body<C, CP, %s, %d, %uu, %uu>(P, Q, num, alive, seg_start, table, nseg, LM, SM, zern, ll);\n}\n",
+                     minb, zern ? "true" : "false", nll, LM, SM);
         }
         return s + buf;
     }
@@ -187,14 +190,21 @@ struct JitSpec {
 
 static bool spec_from_ops(const FusedOp *ops, int nops, JitSpec &sp)
 {
-    sp.codes.clear(); sp.rows.clear();
+    sp.codes.clear(); sp.targs.clear();
     sp.cp_bytes = 8;
     sp.zern = false;
+    sp.nll = 0;
     for (int k = 0; k < nops; k++) {
         const OpDesc *d = op_desc(ops[k].code);
         if (!d) return false;
         sp.codes.push_back(ops[k].code);
-        sp.rows.push_back(ops[k].row);
+        std::string ta;
+        if (d->row) ta = "<" + std::to_string(ops[k].row) + ">";
+        if (ops[k].code == PXF_OP_LLSURF) {
+            ta = "<" + std::to_string((int)ops[k].q[0]) + ", " + std::to_string(ops[k].row) + ">";
+            sp.nll++;
+        }
+        sp.targs.push_back(ta);
         sp.cp_bytes += d->bytes;
         if (ops[k].code == PXF_OP_ZERNSURF) sp.zern = true;
     }
@@ -334,12 +344,17 @@ static int64_t jit_min_rays()
 static char g_last_kernel[512] = "";
 void note_kernel(const char *name) { snprintf(g_last_kernel, sizeof(g_last_kernel), "%s", name); }
 
+// LL chains: 2 resident CTAs per SM.  ptxas, the LL pair: N = 5 needs 154 registers uncapped and spills 100 B at
+// 2 CTAs/SM (692 B at 3); N = 7 needs 216 and spills 772 B at 2.  Measured at 5e7 rays on one B200 (1000 W): 4.9 /
+// 7.1 / 13.0 ms for N = 3 / 5 / 7 (profiles/ll_program_bench_b200.json)
+static const int LL_MINB = 2;
+
 static void fill_spec(JitSpec &sp, const FusedProgram &fp, bool aligned)
 {
     sp.LM = fp.load_mask; sp.SM = fp.store_mask;
     sp.seg = false;
-    sp.mode = (aligned && !sp.zern && !fp.uses_aux) ? 2 : 1;
-    sp.minb = 3;
+    sp.mode = (aligned && !sp.zern && !sp.nll && !fp.uses_aux) ? 2 : 1;
+    sp.minb = sp.nll ? LL_MINB : 3;
 }
 
 int jit_launch_chain(const RowPtrs &P, const RowPtrs &Q, int64_t num, const FusedProgram &fp, uint8_t *alive,
@@ -361,7 +376,8 @@ int jit_launch_chain(const RowPtrs &P, const RowPtrs &Q, int64_t num, const Fuse
     const ZernP *zern = fp.zern;
     const double *aw = fp.aux_wave;
     int *ac = fp.aux_count, *acm = fp.aux_count_max;
-    void *args[] = {(void *)&P, (void *)&Q, &n, &alive, &partials, &zern, &aw, &ac, &acm, cp.data()};
+    const LLTab *ll0 = fp.ll[0], *ll1 = fp.ll[1];
+    void *args[] = {(void *)&P, (void *)&Q, &n, &alive, &partials, &zern, &aw, &ac, &acm, &ll0, &ll1, cp.data()};
     cudaError_t rc = cudaLaunchKernel(reinterpret_cast<const void *>(e->kern), dim3(grid), dim3(PXF_BLOCK), args, 0, s);
     if (rc != cudaSuccess) { set_error("specialised chain launch: %s", cudaGetErrorString(rc)); return PXF_ERR_CUDA; }
     count_launch();
@@ -370,8 +386,9 @@ int jit_launch_chain(const RowPtrs &P, const RowPtrs &Q, int64_t num, const Fuse
 }
 
 // ---- segmented form: the per-segment parameter packs are built when the table is filled
-// register cap (resident CTAs per SM): the Zernike form needs the budget of the fused Zernike kernel
-static int seg_minb(const JitSpec &sp) { return sp.zern ? 3 : 4; }
+// register cap (resident CTAs per SM): the Zernike form needs the budget of the fused Zernike kernel, the LL form
+// that of the specialised LL chains
+static int seg_minb(const JitSpec &sp) { return sp.zern ? 3 : sp.nll ? LL_MINB : 4; }
 size_t jit_seg_pack_bytes(int nops) { return (size_t)nops * FOP_PARAM_DOUBLES * 8 + 8; }
 size_t jit_seg_fill(const FusedOp *ops, int nops, int nseg, void *dst)
 {
@@ -383,18 +400,19 @@ size_t jit_seg_fill(const FusedOp *ops, int nops, int nseg, void *dst)
 }
 int jit_seg_launch(const FusedOp *ops0, int nops, const RowPtrs &P, const RowPtrs &Q, int64_t num, uint8_t *alive,
                    const long long *seg_start_dev, const void *packs_dev, int nseg, unsigned LM, unsigned SM,
-                   const ZernP *zern_dev, cudaStream_t s)
+                   const ZernP *zern_dev, const LLTab *ll_dev, cudaStream_t s)
 {
     if (!jit_enabled()) return PXF_ERR_UNSUPPORTED;
     std::lock_guard<std::mutex> lock(g_mu);
     JitSpec sp;
-    if (!spec_from_ops(ops0, nops, sp) || sp.zern != (zern_dev != nullptr)) return PXF_ERR_UNSUPPORTED;
+    if (!spec_from_ops(ops0, nops, sp) || sp.zern != (zern_dev != nullptr) || (sp.nll > 0) != (ll_dev != nullptr))
+        return PXF_ERR_UNSUPPORTED;
     sp.LM = LM; sp.SM = SM; sp.seg = true; sp.mode = 1; sp.minb = seg_minb(sp);
     JitEntry *e = get_kernel(sp, num >= jit_min_rays());
     if (!e) return PXF_ERR_UNSUPPORTED;
     const int grid = grid_for(num, CHAIN_SEG_TILE, sp.minb);
     long long n = num;
-    void *args[] = {(void *)&P, (void *)&Q, &n, &alive, &seg_start_dev, &packs_dev, &nseg, &LM, &SM, &zern_dev};
+    void *args[] = {(void *)&P, (void *)&Q, &n, &alive, &seg_start_dev, &packs_dev, &nseg, &LM, &SM, &zern_dev, &ll_dev};
     cudaError_t rc = cudaLaunchKernel(reinterpret_cast<const void *>(e->kern), dim3(grid), dim3(PXF_BLOCK), args, 0, s);
     if (rc != cudaSuccess) { set_error("specialised segmented chain launch: %s", cudaGetErrorString(rc)); return PXF_ERR_CUDA; }
     count_launch();

@@ -439,7 +439,7 @@ struct OpLL {
     static constexpr int AUX = 0, SMEM = 0;
     PXF_DEV static const double *table(const Params &p) { return p.C; }
     // the coefficient matrix is read straight from the kernel parameter (constant bank, static offsets)
-    PXF_DEV static void apply(Ray &r, const Params &p, const double *, double, double) { op_ll<N>(r, p, p.C); }
+    PXF_DEV static void apply(Ray &r, const Params &p, const double *, double, double) { op_ll<N>(r, p.s, p.C); }
 };
 
 // ------------------------------------------------------------------ the kernel
@@ -625,7 +625,7 @@ static int launch_ll(RowPtrs P, int64_t num, const uint8_t *mask, int kind, doub
         return PXF_ERR_INVALID;
     }
     // one instantiation per padded order (the Horner scheme is fully unrolled, coefficients read with static offsets)
-    switch (q.stride - 1) {
+    switch (q.s.stride - 1) {
     case 3: return launch_op<OpLL<3>>(P, num, mask, nullptr, nullptr, q, stream);
     case 5: {
         // PXF_LL_VARIANT (tuning): 0 = two rays per thread capped for 2 CTAs/SM; 1/2 = one ray per thread capped for

@@ -245,17 +245,18 @@ inline int make_ll(LLP &q, int kind, double r0, double z0, double psi, double S,
                    double dphi, const double *coeff, const int32_t *axial, const int32_t *az, int cnum)
 {
     memset(&q, 0, sizeof(q));
-    q.kind = kind;
+    LLS &s = q.s;
+    s.kind = kind;
     int nz = 0, nt = 0;
     for (int a = 0; a < cnum; a++) {
         if (axial[a] < 0 || axial[a] > PXF_LL_MAXN || az[a] < 0 || az[a] > PXF_LL_MAXN) return -1;
         if (axial[a] > nz) nz = axial[a];
         if (az[a] > nt) nt = az[a];
     }
-    q.nz = nz; q.nt = nt;
+    s.nz = nz; s.nt = nt;
     const int top = nz > nt ? nz : nt;
     const int N = top <= 3 ? 3 : top <= 5 ? 5 : top <= 7 ? 7 : top <= 11 ? 11 : 15;
-    q.stride = N + 1;
+    s.stride = N + 1;
     // power-basis coefficients of P_0..P_15 from (n+1) P_{n+1} = (2n+1) x P_n - n P_{n-1} (dyadic rationals with
     // numerators < 2**53: exact), then  M[a][b] = sum_t coeff_t * L[axial_t][a] * L[az_t][b]  accumulated in long double
     static long double L[PXF_LL_MAXN + 1][PXF_LL_MAXN + 1];
@@ -274,27 +275,27 @@ inline int make_ll(LLP &q, int kind, double r0, double z0, double psi, double S,
         for (int a = 0; a <= axial[t]; a++)
             for (int b = 0; b <= az[t]; b++) M[a][b] += (long double)coeff[t] * L[axial[t]][a] * L[az[t]][b];
     for (int a = 0; a <= N; a++)
-        for (int b = 0; b <= N; b++) q.C[a * q.stride + b] = (double)M[a][b];
-    q.zmid = (zmax + zmin) / 2.;
-    q.zhalf = (zmax - zmin) / 2.;
-    q.dphi = dphi;
-    q.twoodphi = 2 / dphi;
-    q.zrange = zmax - zmin;
-    q.izhalf = 1 / q.zhalf;
-    q.twoozrange = 2 / q.zrange;
+        for (int b = 0; b <= N; b++) q.C[a * s.stride + b] = (double)M[a][b];
+    s.zmid = (zmax + zmin) / 2.;
+    s.zhalf = (zmax - zmin) / 2.;
+    s.dphi = dphi;
+    s.twoodphi = 2 / dphi;
+    s.zrange = zmax - zmin;
+    s.izhalf = 1 / s.zhalf;
+    s.twoozrange = 2 / s.zrange;
     if (kind == 0) {            // woltsurf.f95:235-241: thetah = 3.*alpha, thetap = alpha
         double alpha = .25 * atan(r0 / z0);
         double thetah = 3. * alpha, thetap = alpha;
         double p = z0 * tan(4 * alpha) * tan(thetap);
         double d = z0 * tan(4 * alpha) * tan(4 * alpha - thetah);
         double e = cos(4 * alpha) * (1 + tan(4 * alpha) * tan(thetah));
-        q.g0 = h_sq(p); q.g1 = 2 * p; q.g2 = 4 * h_sq(e) * p * d / (h_sq(e) - 1);
-        q.tol = h_tol10();
+        s.g0 = h_sq(p); s.g1 = 2 * p; s.g2 = 4 * h_sq(e) * p * d / (h_sq(e) - 1);
+        s.tol = h_tol10();
     } else if (kind == 1) {     // woltsurf.f95:307-312, tol 1.e-7 (:319)
         double p, d, e;
         vanspeybroeck(r0, z0, psi, p, d, e);
-        q.g0 = h_sq(e); q.g1 = 2 * h_sq(e); q.g2 = d;
-        q.tol = h_tol7();
+        s.g0 = h_sq(e); s.g1 = 2 * h_sq(e); s.g2 = d;
+        s.tol = h_tol7();
     } else {                    // woltsurf.f95:657-666
         double P = r0 / sin((psi * asin(r0 / z0) - asin(r0 / S)) / (1 + psi));
         double ff = (S + P) / 2.;
@@ -302,9 +303,9 @@ inline int make_ll(LLP &q, int kind, double r0, double z0, double psi, double S,
         double cq = h_sq(ff) * h_sq(ff - P);
         double aa = sqrt((-bq + sqrt(h_sq(bq) - 4 * cq)) / 2.);
         double bb = sqrt(h_sq(aa) - h_sq(ff));
-        q.g0 = ff - P + z0; q.g1 = h_sq(aa); q.g2 = h_sq(bb);
-        q.ig1 = 1 / q.g1; q.ig2 = 1 / q.g2;
-        q.tol = h_tol10();
+        s.g0 = ff - P + z0; s.g1 = h_sq(aa); s.g2 = h_sq(bb);
+        s.ig1 = 1 / s.g1; s.ig2 = 1 / s.g2;
+        s.tol = h_tol10();
     }
     return 0;
 }

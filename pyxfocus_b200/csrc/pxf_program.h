@@ -8,10 +8,11 @@
 namespace pxf {
 
 #define FOP_PARAM_DOUBLES 38   // sizeof(WSP)/8 is the largest folded parameter block
+#define PXF_PROG_MAX_LL 2      // Legendre-Legendre shells per program: a deformed primary and secondary
 
 struct FusedOp {
     int code;
-    int row;                 // VIGNETTE_BOX / ABS: bundle row index
+    int row;                 // VIGNETTE_BOX / ABS: bundle row index; LLSURF: table slot
     double q[FOP_PARAM_DOUBLES];
 };
 struct FusedProgram {
@@ -30,6 +31,9 @@ struct FusedProgram {
     int *aux_count_max;
     int uses_aux;            // some op reads or writes a side array (needs the ray index)
     FusedOp ops[PXF_MAX_OPS];
+    // device tables of the program's PXF_OP_LLSURF ops in op order (FusedOp::row = slot); staged in shared memory
+    const LLTab *ll[PXF_PROG_MAX_LL];
+    int nll;
 };
 
 static_assert(sizeof(WSP) <= FOP_PARAM_DOUBLES * 8, "WSP does not fit a fused op slot");
@@ -54,7 +58,8 @@ size_t jit_seg_pack_bytes(int nops);
 size_t jit_seg_fill(const FusedOp *ops, int nops, int nseg, void *dst);     // returns bytes per segment pack, 0 = none
 int jit_seg_launch(const FusedOp *ops0, int nops, const RowPtrs &P, const RowPtrs &Q, int64_t num, uint8_t *alive,
                    const long long *seg_start_dev, const void *packs_dev, int nseg, unsigned LM, unsigned SM,
-                   const ZernP *zern_dev, cudaStream_t s);    // zern_dev: one Zernike table per segment (NULL: none)
+                   const ZernP *zern_dev, const LLTab *ll_dev, cudaStream_t s);
+                   // zern_dev: one Zernike table per segment, ll_dev: the segment's LL tables, segment-major (NULL: none)
 void note_kernel(const char *name);     // name of the last trace kernel launched (pxf_last_trace_kernel)
 
 // segmented specialised chains (pxf_chain.cu)

@@ -598,6 +598,73 @@ def config3_tolerance_fast(n, coeffs, rng="numpy", rng_seed=0, device=None, sour
                  idx=idx[after.start[k]:after.start[k + 1]] - k * n) for k in range(K)]
 
 
+# ------------------------------------------------------------------ Legendre-Legendre Wolter-I pair
+# The geometry of the reference fixture for the LL shells (tests/golden/make_golden.py, singlePassAlignment.py style):
+# a 220 mm Wolter-I pair at 8400 mm, 0.25 rad of azimuth, the primary's figure on 8400..8500 mm, the secondary's on
+# 8300..8400 mm.
+def ll_orders(nmax=5):
+    """(axial, az) of every Legendre-Legendre term up to order ``nmax`` in both directions: (nmax+1)**2 terms."""
+    ax, az = np.meshgrid(np.arange(nmax + 1), np.arange(nmax + 1), indexing="ij")
+    return ax.ravel(), az.ravel()
+
+
+def ll_coeff(nterms=36, rng_seed=0, sigma=2.e-4):
+    """Random LL figure coefficients [mm] (one realisation of a figure error)."""
+    return np.random.default_rng(rng_seed).normal(0., sigma, nterms)
+
+
+def llpair_program(coeff_p, coeff_s, axial, az):
+    """The LL pair ``llpair_fast`` records, written out (transform arguments negated, as ``transformations.transform``
+    passes them on): the same ops with the same scalars, so the same bits."""
+    pxf = _pxf()
+    return (pxf.Program().transform(-0., -0., 8400., -0., -0., -0.)
+            .wolterprimll(220., 8400., 8500., 8400., .25, coeff_p, axial, az).reflect()
+            .woltersecll(220., 8400., 1., 8400., 8300., .25, coeff_s, axial, az).reflect().flat())
+
+
+def llpair_fast(n, coeff_p, coeff_s, axial, az, rng="numpy", rng_seed=0, device=None, sources=None):
+    """A Wolter-I pair whose primary and secondary carry Legendre-Legendre figure terms, traced to the focal plane
+    inside ``fused``: one launch for orders <= 7."""
+    pxf = _pxf()
+    src = sources or pxf.sources
+    tran, surf, anal = pxf.transformations, pxf.surfaces, pxf.analyses
+    seed(rng_seed)
+    rays = src.subannulus(220., 220.6, .25, n, zhat=-1., **_source_kw(rng, rng_seed, device))
+    with pxf.fused(rays):
+        tran.transform(rays, 0, 0, -8400., 0, 0, 0)
+        surf.primaryLL(rays, 220., 8400., 8500., 8400., .25, coeff_p, axial, az)
+        tran.reflect(rays)
+        surf.secondaryLL(rays, 220., 8400., 1., 8400., 8300., .25, coeff_s, axial, az)
+        tran.reflect(rays)
+        surf.flat(rays)
+    return dict(rays=rays, hpd=anal.hpd(rays), rms=anal.rmsCentroid(rays))
+
+
+def ll_tolerance_fast(n, realisations, axial, az, rng="numpy", rng_seed=0, device=None, sources=None):
+    """A figure-error Monte Carlo of the LL pair as ONE bundle: one realisation per (coeff_p, coeff_s) pair in
+    ``realisations``.  The source is drawn once and replicated per realisation (the loop of ``llpair_fast`` draws the
+    same rays every time), one segmented launch traces every realisation through its own pair of figures, and
+    ``hpd`` / ``rmsCentroid`` run per segment.  Returns one dict per realisation with the keys of ``llpair_fast``:
+    ``rays`` is the realisation's view of the joint bundle."""
+    pxf = _pxf()
+    from pyxfocus_b200._call import bundle_alloc, bundle_split
+    anal = pxf.analyses
+    K = len(realisations)
+    seed(rng_seed)
+    src = (sources or pxf.sources).subannulus(220., 220.6, .25, n, zhat=-1., **_source_kw(rng, rng_seed, device))
+    dev = src[1].device
+    rays = bundle_alloc(K * n, dev)
+    for r, s_ in zip(rays, src):
+        r.view(K, n).copy_(s_.unsqueeze(0).expand(K, n))
+    del src
+    segs = pxf.Segments([n] * K, device=dev)
+    pxf.SegmentedProgram([llpair_program(cp, cs, axial, az) for cp, cs in realisations], segs.sizes(),
+                         device=dev).run(rays)
+    hpd, rms = anal.hpd(rays, segments=segs), anal.rmsCentroid(rays, segments=segs)
+    views = bundle_split(rays, [n] * K)
+    return [dict(rays=views[k], hpd=float(hpd[k]), rms=float(rms[k])) for k in range(K)]
+
+
 def config4_fast(n_per_shell=1000, M=72, order=-3, wave=2.4, rng="numpy", rng_seed=0, device=None, offX=0., offY=0.,
                  sources=None):
     pxf = _pxf()
@@ -715,6 +782,9 @@ def baseline_programs():
          .woltersecondary(220., 8400., 1.).reflect().vignette_mag().flat(), False),
         # config 3 as a figure-error Monte Carlo: one Zernike surface per segment (segmented)
         (config3_program(zernike_coeff(len(ro))), True),
+        # the Legendre-Legendre Wolter-I pair (36 terms per mirror), single and as a figure-error Monte Carlo
+        (llpair_program(ll_coeff(36), ll_coeff(36, 1), *ll_orders(5)), False),
+        (llpair_program(ll_coeff(36), ll_coeff(36, 1), *ll_orders(5)), True),
         # config 4: SPO shells (segmented), the grating fan, the way back, the outlier cut
         (P().transform(0, 0, 0, 0, 0, 1).spocone(700., .01).kickn(0, 0).reflect().spocone(700., .03).reflect()
          .transform(0, 0, 1, 0, 0, 0).transform(0, 0, 1, 0, 0, 0).flat(), True),

@@ -32,8 +32,11 @@ from ._call import stream_ptr
 OP = dict(TRANSFORM=1, ITRANSFORM=2, REFLECT=3, REFRACT=4, RADGRAT=5, FLAT=6, FLATOPD=7, CONIC=8,
           CONICOPD=9, WOLTERPRIMARY=10, WOLTERPRIMARYOPD=11, WOLTERSECONDARY=12, WOLTERSINE=13,
           WSPRIMARY=14, WSSECONDARY=15, SPOCONE=16, VIGNETTE_MAG=17, VIGNETTE_BOX=18,
-          VIGNETTE_ABS=19, KICK=20, ZERNSURF=21, KICKN=22, VIGNETTE_RHOGT=23, GRATFAN=24, ROTX_REMAINING=25)
+          VIGNETTE_ABS=19, KICK=20, ZERNSURF=21, KICKN=22, VIGNETTE_RHOGT=23, GRATFAN=24, ROTX_REMAINING=25,
+          LLSURF=26)
 MAX_OPS = 24
+LL_MAX_ORDER = 7       # Legendre orders a fused program holds (higher orders run the stand-alone routines)
+LL_MAX_OPS = 2         # Legendre-Legendre shells per program
 _VIGNETTES = (OP["VIGNETTE_MAG"], OP["VIGNETTE_BOX"], OP["VIGNETTE_ABS"], OP["VIGNETTE_RHOGT"])
 _AUX_OPS = (OP["GRATFAN"], OP["ROTX_REMAINING"])
 
@@ -43,7 +46,7 @@ class Program:
 
     def __init__(self):
         self.ops = []
-        self._tables = {}        # op index -> host table (uint8 tensor) of a ZERNSURF op
+        self._tables = {}        # op index -> host table (uint8 tensor) of a ZERNSURF or LLSURF op
         self._dev_tables = {}    # (op index, device) -> its device copy
 
     def __len__(self):
@@ -119,6 +122,8 @@ class Program:
             raise ValueError("coeff, rorder, aorder must be 1-D arrays of one length")
         if any(code == OP["ZERNSURF"] for code, _ in self.ops):
             raise ValueError("a program carries at most one Zernike surface")
+        if any(code == OP["LLSURF"] for code, _ in self.ops):
+            raise NotImplementedError("a Zernike surface and Legendre-Legendre shells in one program are not supported")
         L = _lib.lib()
         tab = torch.empty(int(L.pxf_zern_table_bytes()), dtype=torch.uint8)
         nmax = int(L.pxf_zern_table_fill(c.ctypes.data, r.ctypes.data, a.ctypes.data, c.shape[0], float(rad),
@@ -129,6 +134,48 @@ class Program:
             raise NotImplementedError("fused Zernike surfaces support radial orders <= 7")
         self._tables[len(self.ops)] = tab
         return self.add(OP["ZERNSURF"], 0., 0. if nr is None else 1., float(nmax))
+
+    # --- Legendre-Legendre shells (woltsurf.f95:219-379, :643-718) ---
+    def wolterprimll(self, r0, z0, zmax, zmin, dphi, coeff, axial, az):
+        """wolterprimLL inside the program (arguments as ``woltsurf.wolterprimll``)."""
+        return self._ll(0, r0, z0, 1., 0., zmax, zmin, dphi, coeff, axial, az)
+
+    def woltersecll(self, r0, z0, psi, zmax, zmin, dphi, coeff, axial, az):
+        """woltersecLL inside the program (arguments as ``woltsurf.woltersecll``)."""
+        return self._ll(1, r0, z0, psi, 0., zmax, zmin, dphi, coeff, axial, az)
+
+    def ellipsoidwoltll(self, r0, z0, psi, S, zmax, zmin, dphi, coeff, axial, az):
+        """ellipsoidWoltLL inside the program (arguments as ``woltsurf.ellipsoidwoltll``)."""
+        return self._ll(2, r0, z0, psi, S, zmax, zmin, dphi, coeff, axial, az)
+
+    def _ll(self, kind, r0, z0, psi, S, zmax, zmin, dphi, coeff, axial, az):
+        # Legendre orders <= 7, at most two shells per program, none with a Zernike surface.  The term list is folded
+        # on the host exactly as for the stand-alone routine; the table is uploaded once per device and staged in
+        # shared memory by the kernel.
+        import numpy as np
+        c = np.ascontiguousarray(np.asarray(coeff, dtype=np.float64).ravel())
+        ax = np.asarray(axial).ravel()
+        a = np.asarray(az).ravel()
+        if not (c.shape == ax.shape == a.shape) or c.shape[0] == 0:
+            raise ValueError("coeff, axial, az must be 1-D arrays of one length")
+        if not (np.all(np.equal(np.mod(ax, 1), 0)) and np.all(np.equal(np.mod(a, 1), 0))) or ax.min() < 0 or a.min() < 0:
+            raise ValueError("Legendre orders must be non-negative integers")
+        ax, a = np.ascontiguousarray(ax, dtype=np.int32), np.ascontiguousarray(a, dtype=np.int32)
+        if max(ax.max(), a.max()) > LL_MAX_ORDER:
+            raise NotImplementedError("fused Legendre-Legendre shells support orders <= %d" % LL_MAX_ORDER)
+        if sum(code == OP["LLSURF"] for code, _ in self.ops) >= LL_MAX_OPS:
+            raise NotImplementedError("a program carries at most %d Legendre-Legendre shells" % LL_MAX_OPS)
+        if any(code == OP["ZERNSURF"] for code, _ in self.ops):
+            raise NotImplementedError("a Zernike surface and Legendre-Legendre shells in one program are not supported")
+        L = _lib.lib()
+        tab = torch.empty(int(L.pxf_ll_table_bytes()), dtype=torch.uint8)
+        top = int(L.pxf_ll_table_fill(kind, float(r0), float(z0), float(psi), float(S), float(zmax), float(zmin),
+                                      float(dphi), c.ctypes.data, ax.ctypes.data, a.ctypes.data, c.shape[0],
+                                      tab.data_ptr()))
+        if top < 0:
+            raise ValueError("invalid Legendre-Legendre term list: " + L.pxf_last_error().decode())
+        self._tables[len(self.ops)] = tab
+        return self.add(OP["LLSURF"], 0., float(top))
 
     # --- per-ray predicates (the ray stops at the op; use with ``alive``) ---
     def vignette_mag(self):
@@ -186,11 +233,11 @@ class Program:
                 arr[k].p[j] = v
             if k in self._tables:
                 if device is None:
-                    raise ValueError("a program with a Zernike surface needs a device")
+                    raise ValueError("a program with a Zernike surface or an LL shell needs a device")
                 key = (k, str(device))
                 if key not in self._dev_tables:
                     self._dev_tables[key] = self._tables[k].to(device)
-                # the table's device address travels bit-cast in p[0] (include/pxf.h, PXF_OP_ZERNSURF)
+                # the table's device address travels bit-cast in p[0] (include/pxf.h, PXF_OP_ZERNSURF / LLSURF)
                 arr[k].p[0] = struct.unpack("d", struct.pack("Q", self._dev_tables[key].data_ptr()))[0]
         return arr
 
@@ -391,7 +438,10 @@ class SegmentedProgram:
 
     Every program may carry one ``zernsurf`` at the same position, each with its own terms, ``rad`` and ``nr`` (a
     Monte Carlo over figure-error realisations, or a shell assembly with a measured figure per shell); the segment's
-    Zernike table is staged with its op table.  ``nr`` must be given for all segments or for none."""
+    Zernike table is staged with its op table.  ``nr`` must be given for all segments or for none.
+
+    Likewise every program may carry one or two Legendre-Legendre shells (``wolterprimll`` / ``woltersecll`` /
+    ``ellipsoidwoltll``) at the same positions, each segment with its own kind, terms and orders (<= 7)."""
 
     def __init__(self, programs, sizes, device=None):
         import numpy as np
@@ -418,7 +468,19 @@ class SegmentedProgram:
                     o.p[j] = v
         L = _lib.lib()
         zpos = [k for k, (c, _) in enumerate(programs[0].ops) if c == OP["ZERNSURF"]]
-        if zpos:
+        lpos = [k for k, (c, _) in enumerate(programs[0].ops) if c == OP["LLSURF"]]
+        if lpos:
+            for p in programs:
+                if any(k not in p._tables for k in lpos):
+                    raise ValueError("an LL op needs the table Program.wolterprimll / woltersecll / ellipsoidwoltll "
+                                     "records")
+            # the LL tables of every segment, segment-major and in op order (include/pxf.h, pxf_segmented_table_fill_ll)
+            lt = torch.cat([p._tables[k] for p in programs for k in lpos])
+            nbytes = int(L.pxf_segmented_table_bytes_ll(nops, self.nseg))
+            self.table_host = torch.empty(nbytes, dtype=torch.uint8)
+            _lib.check(L.pxf_segmented_table_fill_ll(arr, nops, self.nseg, start.ctypes.data, lt.data_ptr(),
+                                                     self.table_host.data_ptr()))
+        elif zpos:
             kz = zpos[0]
             for p in programs:
                 if kz not in p._tables:

@@ -23,7 +23,7 @@ from . import transformations as tran
 from . import woltsurf as wolt
 from . import zernsurf as zern
 from .analyses import analyticImagePlane, analyticXPlane, analyticYPlane
-from .program import flush, recorder_for
+from .program import LL_MAX_OPS, LL_MAX_ORDER, OP, flush, recorder_for
 
 
 def flat(rays, ind=None, nr=None):
@@ -57,7 +57,8 @@ def zernsurf(rays, coeff, rad, rorder=None, aorder=None, nr=None):
         raise NotImplementedError("pass rorder/aorder explicitly: the reference's default ordering lives in "
                                   "the third-party module utilities.imaging.zernikemod (not vendored)")
     prog = recorder_for(rays)
-    if prog is not None and np.max(np.asarray(rorder)) <= 7 and not any(c == 21 for c, _ in prog.ops):
+    if prog is not None and np.max(np.asarray(rorder)) <= 7 and not any(c in (OP["ZERNSURF"], OP["LLSURF"])
+                                                                        for c, _ in prog.ops):
         prog.zernsurf(coeff, rorder, aorder, rad, nr)       # radial orders <= 7: stays in the fused program
         return
     flush(rays)
@@ -204,9 +205,33 @@ def spoSecondary(rays, R0, F, d=.605, ind=None):
     return
 
 
+def _ll_recorder(rays, coeff, axial, az):
+    """The program recording for ``rays`` when it can hold one more Legendre-Legendre shell with these terms (orders
+    <= 7, fewer than two shells so far, no Zernike surface or grating fan), else None."""
+    prog = recorder_for(rays)
+    if prog is None:
+        return None
+    try:
+        c, ax, a = (np.asarray(v).ravel() for v in (coeff, axial, az))
+        ok = (c.shape[0] > 0 and c.shape == ax.shape == a.shape and np.all(np.equal(np.mod(ax, 1), 0))
+              and np.all(np.equal(np.mod(a, 1), 0)) and ax.min() >= 0 and a.min() >= 0
+              and max(ax.max(), a.max()) <= LL_MAX_ORDER)
+    except (TypeError, ValueError):
+        ok = False
+    codes = [code for code, _ in prog.ops]
+    if not ok or codes.count(OP["LLSURF"]) >= LL_MAX_OPS or any(
+            code in codes for code in (OP["ZERNSURF"], OP["GRATFAN"], OP["ROTX_REMAINING"])):
+        return None
+    return prog
+
+
 def secondaryLL(rays, r0, z0, psi, zmax, zmin, dphi, coeff, axial, az):
     """Wolter-I secondary with Legendre-Legendre figure terms, placed at the focus."""
     opd, x, y, z, l, m, n, ux, uy, uz = rays
+    prog = _ll_recorder(rays, coeff, axial, az)
+    if prog is not None:
+        prog.woltersecll(r0, z0, psi, zmax, zmin, dphi, coeff, axial, az)
+        return
     flush(rays)
     wolt.woltersecll(x, y, z, l, m, n, ux, uy, uz, r0, z0, psi, zmax, zmin, dphi, coeff, axial, az)
     return
@@ -215,6 +240,10 @@ def secondaryLL(rays, r0, z0, psi, zmax, zmin, dphi, coeff, axial, az):
 def primaryLL(rays, r0, z0, zmax, zmin, dphi, coeff, axial, az):
     """Wolter-I primary with Legendre-Legendre figure terms, placed at the focus."""
     opd, x, y, z, l, m, n, ux, uy, uz = rays
+    prog = _ll_recorder(rays, coeff, axial, az)
+    if prog is not None:
+        prog.wolterprimll(r0, z0, zmax, zmin, dphi, coeff, axial, az)
+        return
     flush(rays)
     wolt.wolterprimll(x, y, z, l, m, n, ux, uy, uz, r0, z0, zmax, zmin, dphi, coeff, axial, az)
     return
@@ -241,6 +270,10 @@ def ellipsoidSecondary(rays, R0, F, S, psi):
 def ellipsoidPrimaryLL(rays, R0, F, S, psi, zmax, zmin, dphi, coeff, axial, az):
     """Ellipsoid primary with Legendre-Legendre figure terms."""
     opd, x, y, z, l, m, n, ux, uy, uz = rays
+    prog = _ll_recorder(rays, coeff, axial, az)
+    if prog is not None:
+        prog.ellipsoidwoltll(R0, F, psi, S, zmax, zmin, dphi, coeff, axial, az)
+        return
     flush(rays)
     wolt.ellipsoidwoltll(x, y, z, l, m, n, ux, uy, uz, R0, F, psi, S, zmax, zmin, dphi, coeff, axial, az)
     return

@@ -1,0 +1,42 @@
+"""Executed by tests/test_gpu_ll_program.py in two processes -- PXF_JIT=0 (interpreter only) and PXF_JIT_MIN_RAYS=0
+(every program specialised at run time) -- and prints one line per case: name, sha256 of the traced rows and alive
+flags, and the kernel that ran.  The digests must be identical."""
+import hashlib
+import os
+import sys
+
+import numpy as np
+import torch
+
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.join(ROOT, "tests"))
+import pyxfocus_b200 as pxf  # noqa: E402
+from ll_cases import LAYOUT, SINGLE, seg_program, single_name, single_program, source  # noqa: E402
+from util import to_dev  # noqa: E402
+
+
+def digest(rows, alive):
+    h = hashlib.sha256()
+    for t in rows + ([alive] if alive is not None else []):
+        h.update(t.cpu().numpy().tobytes())
+    return h.hexdigest()[:24]
+
+
+def main():
+    for oop in (False, True):
+        progs = [seg_program(pxf, k) for k in range(len(LAYOUT))]
+        rays = to_dev(source(int(np.sum(LAYOUT)), seed=1))
+        out = [torch.zeros_like(r) for r in rays] if oop else None
+        alive = pxf.SegmentedProgram(progs, LAYOUT).run(rays, out=out)
+        print("seg_oop%d %s %s" % (int(oop), digest(out if oop else rays, alive),
+                                   pxf.last_trace_kernel().replace(" ", "_")), flush=True)
+    for case in SINGLE:
+        rays = to_dev(source(20_000, seed=2))
+        alive = single_program(pxf, *case).run(rays)
+        print("%s %s %s" % (single_name(*case), digest(rays, alive), pxf.last_trace_kernel().replace(" ", "_")),
+              flush=True)
+
+
+if __name__ == "__main__":
+    main()
