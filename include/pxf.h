@@ -291,7 +291,7 @@ enum {
                                   wave = NaN: per-ray wavelengths from aux.wave (radgratW), else scalar (radgrat). */
     PXF_OP_ROTX_REMAINING = 25, /* p: ang,total ; apply transform(0,0,0,ang,0,0) (total - aux.count[i]) times: the
                                   whole-bundle rotations a ray still receives after it met its grating */
-    PXF_OP_LLSURF = 26         /* p: table (a DEVICE copy of what pxf_ll_table_fill wrote, its address bit-cast into
+    PXF_OP_LLSURF = 26,        /* p: table (a DEVICE copy of what pxf_ll_table_fill wrote, its address bit-cast into
                                   the double), highest order as returned by the fill (it must be that value: the
                                   specialised kernels evaluate the terms up to the order p[1] rounds to -- 3, 5 or
                                   7 -- so a smaller p[1] drops terms on that path, silently, and not in the
@@ -300,6 +300,20 @@ enum {
                                   bits of pxf_wolterprimll / pxf_woltersecll / pxf_ellipsoidwoltll.  Orders <= 7 only;
                                   at most two per program, and not in a program with PXF_OP_ZERNSURF or
                                   PXF_OP_GRATFAN (PXF_ERR_UNSUPPORTED).                                          */
+    /* The remaining scalar surfaces of surfacesf / woltsurf, with the bits of the stand-alone entry point of the
+     * same name (the scalars mean what they mean there).  A program that holds one of them together with
+     * PXF_OP_ZERNSURF, PXF_OP_LLSURF, PXF_OP_GRATFAN or PXF_OP_ROTX_REMAINING is refused (PXF_ERR_UNSUPPORTED). */
+    PXF_OP_TRACESPHERE = 27,   /* p: rad ; pxf_tracesphere (a ray that misses is zeroed and gets a NaN normal) */
+    PXF_OP_TRACESPHEREOPD = 28, /* p: rad,nr ; pxf_tracesphereopd                                        */
+    PXF_OP_TRACECYL = 29,      /* p: rad ; pxf_tracecyl (cylinder about y; misses as for the sphere)     */
+    PXF_OP_TRACECYLOPD = 30,   /* p: rad,nr ; pxf_tracecylopd                                           */
+    PXF_OP_CYLCONIC = 31,      /* p: rad,k ; pxf_cylconic                                               */
+    PXF_OP_PARAXIAL = 32,      /* p: F ; pxf_paraxial                                                   */
+    PXF_OP_PARAXIALY = 33,     /* p: F ; pxf_paraxialy (m only)                                         */
+    PXF_OP_TORUS = 34,         /* p: rin,rout ; pxf_torus                                               */
+    PXF_OP_WSPRIMARYBACK = 35, /* p: alpha,z0,psi,thick ; pxf_wsprimaryback (PXF_OPT_WS_* apply as to
+                                  PXF_OP_WSPRIMARY)                                                    */
+    PXF_OP_WSSECONDARYBACK = 36 /* p: alpha,z0,psi,thick ; pxf_wssecondaryback                         */
 };
 typedef struct pxf_op {
     int32_t code;
@@ -383,6 +397,8 @@ int pxf_trace_program_sums(double *const rays_in[10], double *const rays_out[10]
  *   pxf_segmented_table_fill folds the scalars into a host table (pxf_segmented_table_bytes bytes; seg_start
  *   has nseg+1 entries, seg_start[0] == 0); the caller uploads it unchanged to device memory and passes both
  *   copies to pxf_trace_program_segmented (the host copy is read for the row masks only).
+ *   The surface ops 27..36 (PXF_OP_TRACESPHERE .. PXF_OP_WSSECONDARYBACK) go through this pair; their scalars may
+ *   differ between segments.  The _zern and _ll fills refuse them (PXF_ERR_UNSUPPORTED).
  *   rays_out == NULL: in place. */
 size_t pxf_segmented_table_bytes(int32_t nops, int32_t nseg);
 int pxf_segmented_table_fill(const pxf_op *ops, int32_t nops, int32_t nseg, const int64_t *seg_start,
@@ -393,7 +409,7 @@ int pxf_trace_program_segmented(double *const rays_in[10], double *const rays_ou
 /* Segmented programs with one Zernike surface per segment (a figure-error Monte Carlo, or shells that each have a
  * measured figure): every segment's op list has its PXF_OP_ZERNSURF at the same position, with the same opd flag
  * (p[1]); the term count, radial order (<= 7), rad and nr may differ.  pxf_segmented_table_fill refuses such lists;
- * this pair takes them (and any list the plain pair takes).
+ * this pair takes them (and any list the plain pair takes, except one with ops 27..36).
  *   zern_tables_host: nseg consecutive tables of pxf_zern_table_bytes() bytes, table s filled by pxf_zern_table_fill
  *   for segment s (NULL is accepted when no op is a PXF_OP_ZERNSURF).  They are copied into the segmented table, so it
  *   stays self-contained: upload it unchanged and pass both copies to pxf_trace_program_segmented, which stages the
@@ -407,7 +423,8 @@ int pxf_segmented_table_fill_zern(const pxf_op *ops, int32_t nops, int32_t nseg,
 /* Segmented programs with Legendre-Legendre shells (a figure-error Monte Carlo of a Wolter-I pair, or shells that each
  * have a measured figure): every segment's op list has its PXF_OP_LLSURF ops (one or two) at the same positions.
  * Kinds, term lists and orders (<= 7) may differ between segments.  pxf_segmented_table_fill and
- * pxf_segmented_table_fill_zern refuse such lists; this pair takes them (and any list the plain pair takes).
+ * pxf_segmented_table_fill_zern refuse such lists; this pair takes them (and any list the plain pair takes, except one
+ * with ops 27..36).
  *   ll_tables_host: nseg * (LL ops per program) tables of pxf_ll_table_bytes() bytes, segment-major and in op order,
  *   each filled by pxf_ll_table_fill (NULL is accepted when no op is a PXF_OP_LLSURF).  They are copied into the
  *   segmented table (pxf_segmented_table_bytes_ll has room for two per segment), so it stays self-contained: upload

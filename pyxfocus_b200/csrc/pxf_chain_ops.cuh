@@ -73,6 +73,16 @@ struct KickP { double dl, dm, sn; };
 PXF_CHAIN_OP(CKick, 20, KickP,
              r.l = r.l + p.dl; r.m = r.m + p.dm; r.n = p.sn * sqrt(1. - sq(r.l) - sq(r.m)))
 PXF_CHAIN_OP(CKickN, 22, KickNP, op_kickn(r, p))
+PXF_CHAIN_OP(CTraceSphere, 27, SphereP, op_tracesphere(r, p))
+PXF_CHAIN_OP(CTraceSphereOpd, 28, SphereP, op_tracesphere(r, p))
+PXF_CHAIN_OP(CTraceCyl, 29, SphereP, op_tracecyl(r, p))
+PXF_CHAIN_OP(CTraceCylOpd, 30, SphereP, op_tracecyl(r, p))
+PXF_CHAIN_OP(CCylConic, 31, CylConicP, op_cylconic(r, p))
+PXF_CHAIN_OP(CParaxial, 32, ParaxialP, op_paraxial(r, p))
+PXF_CHAIN_OP(CParaxialY, 33, ParaxialP, op_paraxial(r, p))
+PXF_CHAIN_OP(CTorus, 34, TorusP, op_torus(r, p))
+PXF_CHAIN_OP(CWsPrimaryBack, 35, WSP, op_wsprimary_t<true>(r, p))
+PXF_CHAIN_OP(CWsSecondaryBack, 36, WSP, op_wssecondary_t<true>(r, p))
 #undef PXF_CHAIN_OP
 
 // predicates: the ray stops at the op when apply() returns false

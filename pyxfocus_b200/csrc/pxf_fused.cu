@@ -32,7 +32,8 @@ PXF_DEV void count_max_update(int *dst, int k)
 // AUX: whether this instantiation carries the side-array ops (the grating fan: asin + a data-dependent loop) -- like
 // ZERN they get their own kernel so that every other program keeps its register budget
 // LL: whether it carries the Legendre-Legendre shells (PXF_OP_LLSURF); llt: their tables in shared memory, by slot
-template <bool ZERN = false, bool AUX = false, bool LL = false>
+// SURF: whether it carries the remaining scalar surfaces (PXF_OP_TRACESPHERE .. PXF_OP_WSSECONDARYBACK)
+template <bool ZERN = false, bool AUX = false, bool LL = false, bool SURF = false>
 PXF_DEV bool run_op(Ray &r, const FusedOp &op, const ZernP *zt = nullptr, int64_t i = 0,
                     const double *aux_wave = nullptr, int *aux_count = nullptr, int *aux_count_max = nullptr,
                     const LLTab *llt = nullptr)
@@ -103,6 +104,30 @@ PXF_DEV bool run_op(Ray &r, const FusedOp &op, const ZernP *zt = nullptr, int64_
             // kernel of the table's own order (pxf_ray.cuh, LLTab)
             if constexpr (LL) op_ll<PXF_LL_PROG_MAXN, PXF_LL_PROG_MAXN + 1>(r, llt[op.row].s, llt[op.row].C);
             break;
+        case PXF_OP_TRACESPHERE:
+        case PXF_OP_TRACESPHEREOPD:
+            if constexpr (SURF) op_tracesphere(r, *reinterpret_cast<const SphereP *>(op.q));
+            break;
+        case PXF_OP_TRACECYL:
+        case PXF_OP_TRACECYLOPD:
+            if constexpr (SURF) op_tracecyl(r, *reinterpret_cast<const SphereP *>(op.q));
+            break;
+        case PXF_OP_CYLCONIC:
+            if constexpr (SURF) { const CylConicP p = *reinterpret_cast<const CylConicP *>(op.q); op_cylconic(r, p); }
+            break;
+        case PXF_OP_PARAXIAL:
+        case PXF_OP_PARAXIALY:
+            if constexpr (SURF) op_paraxial(r, *reinterpret_cast<const ParaxialP *>(op.q));
+            break;
+        case PXF_OP_TORUS:
+            if constexpr (SURF) { const TorusP p = *reinterpret_cast<const TorusP *>(op.q); op_torus(r, p); }
+            break;
+        case PXF_OP_WSPRIMARYBACK:
+            if constexpr (SURF) op_wsprimary_t<true>(r, *reinterpret_cast<const WSP *>(op.q));
+            break;
+        case PXF_OP_WSSECONDARYBACK:
+            if constexpr (SURF) op_wssecondary_t<true>(r, *reinterpret_cast<const WSP *>(op.q));
+            break;
         case PXF_OP_KICK: {
             r.l = r.l + op.q[0];
             r.m = r.m + op.q[1];
@@ -114,17 +139,17 @@ PXF_DEV bool run_op(Ray &r, const FusedOp &op, const ZernP *zt = nullptr, int64_
     return true;
 }
 
-template <bool ZERN = false, bool AUX = false, bool LL = false>
+template <bool ZERN = false, bool AUX = false, bool LL = false, bool SURF = false>
 PXF_DEV bool run_program(Ray &r, const FusedProgram &prog, const ZernP *zt = nullptr, int64_t i = 0,
                          const LLTab *llt = nullptr)
 {
     for (int k = 0; k < prog.nops; k++)
-        if (!run_op<ZERN, AUX, LL>(r, prog.ops[k], zt, i, prog.aux_wave, prog.aux_count, prog.aux_count_max, llt))
+        if (!run_op<ZERN, AUX, LL, SURF>(r, prog.ops[k], zt, i, prog.aux_wave, prog.aux_count, prog.aux_count_max, llt))
             return false;
     return true;
 }
 
-template <bool VEC2, int MINB = 1, bool ZERN = false, bool AUX = false, bool LL = false>
+template <bool VEC2, int MINB = 1, bool ZERN = false, bool AUX = false, bool LL = false, bool SURF = false>
 __global__ void __launch_bounds__(PXF_BLOCK, MINB)
 k_program(const RowPtrs P, const RowPtrs Q, const int64_t num, uint8_t *__restrict__ alive,
           double *__restrict__ partials, const __grid_constant__ FusedProgram prog)
@@ -160,8 +185,8 @@ k_program(const RowPtrs P, const RowPtrs Q, const int64_t num, uint8_t *__restri
             const int64_t i = q << 1;
             Ray a, b;
             fload2(a, b, P, LM, i);
-            const bool ka = run_program<ZERN, AUX, LL>(a, prog, zt, i, llt);
-            const bool kb = run_program<ZERN, AUX, LL>(b, prog, zt, i + 1, llt);
+            const bool ka = run_program<ZERN, AUX, LL, SURF>(a, prog, zt, i, llt);
+            const bool kb = run_program<ZERN, AUX, LL, SURF>(b, prog, zt, i + 1, llt);
             fstore2(a, b, Q, SM, i);
             if (alive) { alive[i] = ka ? 1 : 0; alive[i + 1] = kb ? 1 : 0; }
             if (ka) { cnt += 1.; sx += a.x; sy += a.y; }
@@ -171,7 +196,7 @@ k_program(const RowPtrs P, const RowPtrs Q, const int64_t num, uint8_t *__restri
             const int64_t i = num - 1;
             Ray a;
             fload1(a, P, LM, i);
-            const bool ka = run_program<ZERN, AUX, LL>(a, prog, zt, i, llt);
+            const bool ka = run_program<ZERN, AUX, LL, SURF>(a, prog, zt, i, llt);
             fstore1(a, Q, SM, i);
             if (alive) alive[i] = ka ? 1 : 0;
             if (ka) { cnt += 1.; sx += a.x; sy += a.y; }
@@ -180,7 +205,7 @@ k_program(const RowPtrs P, const RowPtrs Q, const int64_t num, uint8_t *__restri
         for (int64_t i = tid; i < num; i += nthr) {
             Ray a;
             fload1(a, P, LM, i);
-            const bool ka = run_program<ZERN, AUX, LL>(a, prog, zt, i, llt);
+            const bool ka = run_program<ZERN, AUX, LL, SURF>(a, prog, zt, i, llt);
             fstore1(a, Q, SM, i);
             if (alive) alive[i] = ka ? 1 : 0;
             if (ka) { cnt += 1.; sx += a.x; sy += a.y; }
@@ -202,7 +227,7 @@ k_program(const RowPtrs P, const RowPtrs Q, const int64_t num, uint8_t *__restri
 #define SEG_TILE (PXF_BLOCK * 8)
 struct SegHeader {
     unsigned load_mask, store_mask; int nops, nseg; int chain_id, jit_pack_bytes; long long zern_off;
-    long long ll_off; int nll, unused;
+    long long ll_off; int nll, surf;
 };
 static_assert(sizeof(ZernP) % 16 == 0, "per-segment Zernike tables are laid out back to back, 16-byte aligned");
 static_assert(sizeof(LLTab) % 8 == 0, "per-segment LL tables are laid out back to back, whole doubles");
@@ -212,7 +237,8 @@ __host__ __device__ __forceinline__ int seg_zern_smem_offset(int nops) { return 
 
 // ZERN: zern = nseg Zernike tables, one per segment (the Zernike instantiation of run_op, as k_program<.., true>)
 // LL: ll = nseg * nll LL tables, segment-major (the LL instantiation of run_op, as k_program<.., LL = true>)
-template <int MINB, bool ZERN = false, bool LL = false>
+// SURF: the remaining scalar surfaces (as k_program<.., SURF = true>)
+template <int MINB, bool ZERN = false, bool LL = false, bool SURF = false>
 __global__ void __launch_bounds__(PXF_BLOCK, MINB)
 k_program_seg(const RowPtrs P, const RowPtrs Q, const int64_t num, uint8_t *__restrict__ alive,
               const long long *__restrict__ seg_start, const FusedOp *__restrict__ ops, const int nops, const int nseg,
@@ -251,7 +277,7 @@ k_program_seg(const RowPtrs P, const RowPtrs Q, const int64_t num, uint8_t *__re
                 fload1(a, P, LM, i);
                 bool keep = true;
                 for (int k = 0; k < nops; k++)
-                    if (!run_op<ZERN, false, LL>(a, sops[k], zt, 0, nullptr, nullptr, nullptr, llt)) { keep = false; break; }
+                    if (!run_op<ZERN, false, LL, SURF>(a, sops[k], zt, 0, nullptr, nullptr, nullptr, llt)) { keep = false; break; }
                 fstore1(a, Q, SM, i);
                 if (alive) alive[i] = keep ? 1 : 0;
             }
@@ -284,8 +310,22 @@ static void op_masks(int code, int row, unsigned &use, unsigned &st, unsigned &k
         case PXF_OP_GRATFAN: case PXF_OP_ROTX_REMAINING: use = R_NINE; st = R_NINE; kill = 0; break;
         case PXF_OP_ZERNSURF: use = R_POS | R_DIR | (row ? R_OPD : 0u); st = R_POS | R_NRM | (row ? R_OPD : 0u); kill = R_POS | R_NRM; break;
         case PXF_OP_LLSURF: use = R_POS | R_DIR; st = R_POS | R_NRM; kill = R_POS | R_NRM; break;
+        // a ray that misses the sphere / cylinder is zeroed, direction included: the direction is stored, not killed
+        case PXF_OP_TRACESPHERE: case PXF_OP_TRACECYL: use = R_POS | R_DIR; st = R_NINE; kill = R_POS | R_NRM; break;
+        case PXF_OP_TRACESPHEREOPD: case PXF_OP_TRACECYLOPD:
+            use = R_POS | R_DIR | R_OPD; st = R_NINE | R_OPD; kill = R_POS | R_NRM; break;
+        case PXF_OP_CYLCONIC: case PXF_OP_TORUS: use = R_POS | R_DIR; st = R_POS | R_NRM; kill = R_POS | R_NRM; break;
+        case PXF_OP_PARAXIAL: use = R_X | R_Y | R_L | R_M; st = R_L | R_M; kill = R_L | R_M; break;
+        case PXF_OP_PARAXIALY: use = R_Y | R_M; st = R_M; kill = R_M; break;
+        case PXF_OP_WSPRIMARYBACK: case PXF_OP_WSSECONDARYBACK: use = R_NINE; st = R_POS | R_NRM; kill = R_POS; break;
         default: use = 0; st = 0; kill = 0; break;
     }
+}
+
+static bool is_surface_op(int code) { return code >= PXF_OP_TRACESPHERE && code <= PXF_OP_WSSECONDARYBACK; }
+static bool is_table_or_aux_op(int code)
+{
+    return code == PXF_OP_ZERNSURF || code == PXF_OP_LLSURF || code == PXF_OP_GRATFAN || code == PXF_OP_ROTX_REMAINING;
 }
 
 int build_program(FusedProgram &fp, const pxf_op *ops, int nops, const pxf_program_aux *aux)
@@ -293,6 +333,19 @@ int build_program(FusedProgram &fp, const pxf_op *ops, int nops, const pxf_progr
     if (!ops || nops < 1 || nops > PXF_MAX_OPS) { set_error("program: need 1..%d ops", PXF_MAX_OPS); return PXF_ERR_INVALID; }
     memset(&fp, 0, sizeof(fp));
     fp.nops = nops;
+    // the remaining scalar surfaces run in an interpreter of their own, which holds no table or side-array op: refused
+    // before anything else is checked, so the verdict does not depend on the order of the ops
+    bool surf = false, other = false;
+    for (int k = 0; k < nops; k++) {
+        surf = surf || is_surface_op(ops[k].code);
+        other = other || is_table_or_aux_op(ops[k].code);
+    }
+    if (surf && other) {
+        set_error("program: the sphere / cylinder / cylconic / paraxial / torus / W-S back-surface ops cannot share a "
+                  "program with a Zernike surface, a Legendre-Legendre shell or a grating fan");
+        return PXF_ERR_UNSUPPORTED;
+    }
+    fp.surf = surf ? 1 : 0;
     if (aux) { fp.aux_wave = aux->wave; fp.aux_count = aux->count; fp.aux_count_max = aux->count_max; }
     unsigned store = 0;
     for (int k = 0; k < nops; k++) {
@@ -316,6 +369,14 @@ int build_program(FusedProgram &fp, const pxf_op *ops, int nops, const pxf_progr
             case PXF_OP_WOLTERSINE: { WolterSineP t = make_woltersine(p[0], p[1], p[2], p[3]); memcpy(f.q, &t, sizeof(t)); break; }
             case PXF_OP_WSPRIMARY: case PXF_OP_WSSECONDARY: { WSP t = make_ws(p[0], p[1], p[2]); memcpy(f.q, &t, sizeof(t)); break; }
             case PXF_OP_SPOCONE: { SpoP t = make_spo(p[0], p[1]); memcpy(f.q, &t, sizeof(t)); break; }
+            // folded as the stand-alone entry points of pxf_ops.cu fold them
+            case PXF_OP_TRACESPHERE: case PXF_OP_TRACECYL: { SphereP t = make_sphere(p[0], false, 0.); memcpy(f.q, &t, sizeof(t)); break; }
+            case PXF_OP_TRACESPHEREOPD: case PXF_OP_TRACECYLOPD: { SphereP t = make_sphere(p[0], true, p[1]); memcpy(f.q, &t, sizeof(t)); break; }
+            case PXF_OP_CYLCONIC: { CylConicP t = make_cylconic(p[0], p[1]); memcpy(f.q, &t, sizeof(t)); break; }
+            case PXF_OP_PARAXIAL: { ParaxialP t{p[0], 0, 0}; memcpy(f.q, &t, sizeof(t)); break; }
+            case PXF_OP_PARAXIALY: { ParaxialP t{p[0], 1, 0}; memcpy(f.q, &t, sizeof(t)); break; }
+            case PXF_OP_TORUS: { TorusP t = make_torus(p[0], p[1]); memcpy(f.q, &t, sizeof(t)); break; }
+            case PXF_OP_WSPRIMARYBACK: case PXF_OP_WSSECONDARYBACK: { WSP t = make_ws(p[0], p[1], p[2], p[3]); memcpy(f.q, &t, sizeof(t)); break; }
             case PXF_OP_VIGNETTE_BOX:
                 f.row = (int)p[0];
                 if (f.row < 0 || f.row > 9) { set_error("program: bad row in VIGNETTE_BOX"); return PXF_ERR_INVALID; }
@@ -439,6 +500,13 @@ int build_program(FusedProgram &fp, const pxf_op *ops, int nops, const pxf_progr
     return PXF_OK;
 }
 
+// Register cap (resident CTAs per SM) of the interpreter of the remaining scalar surfaces, k_program<surf> and
+// k_program_seg<surf>.  ptxas: 120 registers uncapped (1 and 2 CTAs/SM are the same kernel), 80 with 0.1 KB of spills at
+// 3, 64 with 0.2 KB at 4.  Measured at 5e7 rays, out of place, on one B200 (1000 W), caps 2 / 3 / 4: tracesphere 5.55 /
+// 4.88 / 5.39 ms, paraxial 4.73 / 4.23 / 4.59, wssecondaryback 7.74 / 6.93 / 7.18, torus 3.11 / 3.59 / 3.51, the
+// 1000-segment lens 17.4 / 13.8 / 15.2 (profiles/surface_ops_bench_b200.json)
+#define SURF_MINB 3
+
 int launch_program(double *const rays[10], int64_t num, const FusedProgram &fp, uint8_t *alive, cudaStream_t s,
                    double *const rays_out[10], double *partials, int *grid_out)
 {
@@ -506,13 +574,17 @@ int launch_program(double *const rays[10], int64_t num, const FusedProgram &fp, 
         else if (lm == 4) go(k_program<false, 4, false, false, true>, num);
         else go(k_program<false, 1, false, false, true>, num);
     }
+    else if (fp.surf) {
+        // one ray per thread, capped for SURF_MINB resident CTAs per SM (see its definition)
+        go(k_program<false, SURF_MINB, false, false, false, true>, num);
+    }
     else if (aligned && variant == 0) go(k_program<true, 1>, (num + 1) >> 1);
     else if (variant == 3) go(k_program<false, 3>, num);
     else if (variant == 1) go(k_program<false, 1>, num);
     else go(k_program<false, 4>, num);
     count_launch();
     note_kernel(fp.zern ? "k_program<zernike> (interpreter)" : fp.uses_aux ? "k_program<aux> (interpreter)" :
-                fp.nll ? "k_program<ll> (interpreter)" : "k_program (interpreter)");
+                fp.nll ? "k_program<ll> (interpreter)" : fp.surf ? "k_program<surf> (interpreter)" : "k_program (interpreter)");
     return check_launch("k_program");
 }
 
@@ -675,11 +747,21 @@ static int seg_table_fill(const pxf_op *ops, int nops, int nseg, const int64_t *
     }
     // LL ops: their positions in segment 0's list (the others must match, checked with the opcode sequence below)
     int llpos[PXF_PROG_MAX_LL], nll = 0;
-    for (size_t k = 0; k < (size_t)nseg * nops; k++)
+    bool surf = false;
+    for (size_t k = 0; k < (size_t)nseg * nops; k++) {
         if (ops[k].code == PXF_OP_LLSURF && !ll_ok) {
             set_error("segmented program: PXF_OP_LLSURF needs pxf_segmented_table_fill_ll");
             return PXF_ERR_UNSUPPORTED;
         }
+        if (is_surface_op(ops[k].code)) {
+            if (zern_ok || ll_ok) {
+                set_error("segmented program: the sphere / cylinder / cylconic / paraxial / torus / W-S back-surface "
+                          "ops need pxf_segmented_table_fill");
+                return PXF_ERR_UNSUPPORTED;
+            }
+            surf = true;
+        }
+    }
     for (int k = 0; k < nops; k++)
         if (ops[k].code == PXF_OP_LLSURF) {
             if (nll == PXF_PROG_MAX_LL) { set_error("program: at most %d PXF_OP_LLSURF ops per program", PXF_PROG_MAX_LL); return PXF_ERR_UNSUPPORTED; }
@@ -693,7 +775,7 @@ static int seg_table_fill(const pxf_op *ops, int nops, int nseg, const int64_t *
     FusedOp *dst = reinterpret_cast<FusedOp *>(base + seg_ops_offset(nseg));
     ZernP *zdst = zern ? reinterpret_cast<ZernP *>(base + seg_zern_offset(nops, nseg)) : nullptr;
     LLTab *ldst = nll ? reinterpret_cast<LLTab *>(base + seg_zern_offset(nops, nseg)) : nullptr;
-    h->nops = nops; h->nseg = nseg;
+    h->nops = nops; h->nseg = nseg; h->surf = surf ? 1 : 0;
     // the segment's own LL tables, copied into this one; every segment evaluates position j at the largest order
     // any segment has there (the zero padding makes that the same bits)
     int lln[PXF_PROG_MAX_LL] = {0, 0};
@@ -860,6 +942,12 @@ extern "C" int pxf_trace_program_segmented(double *const rays_in[10], double *co
         count_launch();
         note_kernel("k_program_seg<ll> (interpreter)");
         return check_launch("k_program_seg<ll>");
+    }
+    if (h->surf) {
+        go(k_program_seg<SURF_MINB, false, false, true>, (size_t)nops * sizeof(FusedOp));
+        count_launch();
+        note_kernel("k_program_seg<surf> (interpreter)");
+        return check_launch("k_program_seg<surf>");
     }
     go(k_program_seg<4>, (size_t)nops * sizeof(FusedOp));
     count_launch();

@@ -56,6 +56,16 @@ static const OpDesc OPS[] = {
     {PXF_OP_GRATFAN, "CGratFan", sizeof(CGratFan::P), false},
     {PXF_OP_ROTX_REMAINING, "CRotxRemaining", sizeof(CRotxRemaining::P), false},
     {PXF_OP_LLSURF, "CLLSurf", sizeof(LLOpP), false},
+    {PXF_OP_TRACESPHERE, "CTraceSphere", sizeof(CTraceSphere::P), false},
+    {PXF_OP_TRACESPHEREOPD, "CTraceSphereOpd", sizeof(CTraceSphereOpd::P), false},
+    {PXF_OP_TRACECYL, "CTraceCyl", sizeof(CTraceCyl::P), false},
+    {PXF_OP_TRACECYLOPD, "CTraceCylOpd", sizeof(CTraceCylOpd::P), false},
+    {PXF_OP_CYLCONIC, "CCylConic", sizeof(CCylConic::P), false},
+    {PXF_OP_PARAXIAL, "CParaxial", sizeof(CParaxial::P), false},
+    {PXF_OP_PARAXIALY, "CParaxialY", sizeof(CParaxialY::P), false},
+    {PXF_OP_TORUS, "CTorus", sizeof(CTorus::P), false},
+    {PXF_OP_WSPRIMARYBACK, "CWsPrimaryBack", sizeof(CWsPrimaryBack::P), false},
+    {PXF_OP_WSSECONDARYBACK, "CWsSecondaryBack", sizeof(CWsSecondaryBack::P), false},
 };
 static const OpDesc *op_desc(int code)
 {

@@ -34,6 +34,7 @@ struct FusedProgram {
     // device tables of the program's PXF_OP_LLSURF ops in op order (FusedOp::row = slot); staged in shared memory
     const LLTab *ll[PXF_PROG_MAX_LL];
     int nll;
+    int surf;                // some op is one of the remaining scalar surfaces (PXF_OP_TRACESPHERE .. WSSECONDARYBACK)
 };
 
 static_assert(sizeof(WSP) <= FOP_PARAM_DOUBLES * 8, "WSP does not fit a fused op slot");

@@ -33,12 +33,16 @@ OP = dict(TRANSFORM=1, ITRANSFORM=2, REFLECT=3, REFRACT=4, RADGRAT=5, FLAT=6, FL
           CONICOPD=9, WOLTERPRIMARY=10, WOLTERPRIMARYOPD=11, WOLTERSECONDARY=12, WOLTERSINE=13,
           WSPRIMARY=14, WSSECONDARY=15, SPOCONE=16, VIGNETTE_MAG=17, VIGNETTE_BOX=18,
           VIGNETTE_ABS=19, KICK=20, ZERNSURF=21, KICKN=22, VIGNETTE_RHOGT=23, GRATFAN=24, ROTX_REMAINING=25,
-          LLSURF=26)
+          LLSURF=26, TRACESPHERE=27, TRACESPHEREOPD=28, TRACECYL=29, TRACECYLOPD=30, CYLCONIC=31, PARAXIAL=32,
+          PARAXIALY=33, TORUS=34, WSPRIMARYBACK=35, WSSECONDARYBACK=36)
 MAX_OPS = 24
 LL_MAX_ORDER = 7       # Legendre orders a fused program holds (higher orders run the stand-alone routines)
 LL_MAX_OPS = 2         # Legendre-Legendre shells per program
 _VIGNETTES = (OP["VIGNETTE_MAG"], OP["VIGNETTE_BOX"], OP["VIGNETTE_ABS"], OP["VIGNETTE_RHOGT"])
 _AUX_OPS = (OP["GRATFAN"], OP["ROTX_REMAINING"])
+# the remaining scalar surfaces (sphere .. W-S back surfaces) share no program with a table or side-array op
+SURFACE_OPS = tuple(range(OP["TRACESPHERE"], OP["WSSECONDARYBACK"] + 1))
+TABLE_AUX_OPS = (OP["ZERNSURF"], OP["LLSURF"]) + _AUX_OPS
 
 
 class Program:
@@ -109,6 +113,52 @@ class Program:
     def spocone(self, r0, tg):
         return self.add(OP["SPOCONE"], r0, tg)
 
+    # --- the remaining scalar surfaces (surfacesf.f95:57-246, :251-296, :423-508; woltsurf.f95:726-933) ---
+    def tracesphere(self, rad):
+        return self._surface(OP["TRACESPHERE"], rad)
+
+    def tracesphereopd(self, rad, nr):
+        return self._surface(OP["TRACESPHEREOPD"], rad, nr)
+
+    def tracecyl(self, rad):
+        return self._surface(OP["TRACECYL"], rad)
+
+    def tracecylopd(self, rad, nr):
+        return self._surface(OP["TRACECYLOPD"], rad, nr)
+
+    def cylconic(self, rad, k):
+        return self._surface(OP["CYLCONIC"], rad, k)
+
+    def paraxial(self, F):
+        return self._surface(OP["PARAXIAL"], F)
+
+    def paraxialy(self, F):
+        return self._surface(OP["PARAXIALY"], F)
+
+    def torus(self, rin, rout):
+        return self._surface(OP["TORUS"], rin, rout)
+
+    def wsprimaryback(self, alpha, z0, psi, thick):
+        return self._surface(OP["WSPRIMARYBACK"], alpha, z0, psi, thick)
+
+    def wssecondaryback(self, alpha, z0, psi, thick):
+        return self._surface(OP["WSSECONDARYBACK"], alpha, z0, psi, thick)
+
+    def can_hold_surface(self):
+        """Whether one of the ops above may join this program (none of ``TABLE_AUX_OPS`` is in it)."""
+        return not any(c in TABLE_AUX_OPS for c, _ in self.ops)
+
+    def _surface(self, code, *p):
+        if not self.can_hold_surface():
+            raise NotImplementedError("the sphere / cylinder / cylconic / paraxial / torus / W-S back-surface ops "
+                                      "cannot share a program with a Zernike surface, an LL shell or a grating fan")
+        return self.add(code, *p)
+
+    def _refuse_with_surfaces(self, what):
+        if any(c in SURFACE_OPS for c, _ in self.ops):
+            raise NotImplementedError("%s cannot share a program with the sphere / cylinder / cylconic / paraxial / "
+                                      "torus / W-S back-surface ops" % what)
+
     # --- zernsurf ---
     def zernsurf(self, coeff, rorder, aorder, rad, nr=None):
         """tracezern / tracezernOPD (zernsurf.f95:8-203) inside the program; radial orders <= 7, one Zernike surface
@@ -124,6 +174,7 @@ class Program:
             raise ValueError("a program carries at most one Zernike surface")
         if any(code == OP["LLSURF"] for code, _ in self.ops):
             raise NotImplementedError("a Zernike surface and Legendre-Legendre shells in one program are not supported")
+        self._refuse_with_surfaces("a Zernike surface")
         L = _lib.lib()
         tab = torch.empty(int(L.pxf_zern_table_bytes()), dtype=torch.uint8)
         nmax = int(L.pxf_zern_table_fill(c.ctypes.data, r.ctypes.data, a.ctypes.data, c.shape[0], float(rad),
@@ -167,6 +218,7 @@ class Program:
             raise NotImplementedError("a program carries at most %d Legendre-Legendre shells" % LL_MAX_OPS)
         if any(code == OP["ZERNSURF"] for code, _ in self.ops):
             raise NotImplementedError("a Zernike surface and Legendre-Legendre shells in one program are not supported")
+        self._refuse_with_surfaces("a Legendre-Legendre shell")
         L = _lib.lib()
         tab = torch.empty(int(L.pxf_ll_table_bytes()), dtype=torch.uint8)
         top = int(L.pxf_ll_table_fill(kind, float(r0), float(z0), float(psi), float(S), float(zmax), float(zmin),
@@ -204,6 +256,7 @@ class Program:
         lands between ``hubdist`` and ``l + hubdist`` from the hub, then reflected and diffracted.  ``wave``: a
         float [nm] (radgrat) or a per-ray CUDA tensor (radgratW).  ``run`` needs ``aux=FanAux(...)``: the per-ray
         grating index and its maximum come back there."""
+        self._refuse_with_surfaces("a grating fan")
         if isinstance(wave, torch.Tensor):
             self._wave = wave
             w = float("nan")
@@ -214,6 +267,7 @@ class Program:
     def rotx_remaining(self, ang, total):
         """transform(0,0,0,ang,0,0) applied (total - count[i]) times: the whole-bundle fan rotations a ray still
         receives after it met its grating (sector.py:693), with ``count`` from a previous ``gratfan``."""
+        self._refuse_with_surfaces("rotx_remaining")
         return self.add(OP["ROTX_REMAINING"], ang, total)
 
     def kick(self, dl, dm, sn):
@@ -441,7 +495,10 @@ class SegmentedProgram:
     Zernike table is staged with its op table.  ``nr`` must be given for all segments or for none.
 
     Likewise every program may carry one or two Legendre-Legendre shells (``wolterprimll`` / ``woltersecll`` /
-    ``ellipsoidwoltll``) at the same positions, each segment with its own kind, terms and orders (<= 7)."""
+    ``ellipsoidwoltll``) at the same positions, each segment with its own kind, terms and orders (<= 7).
+
+    The remaining scalar surfaces (``tracesphere`` .. ``wssecondaryback``) take their own scalars per segment (a
+    tolerance sweep over the radii of a lens pair, say); they share no program with a Zernike surface or an LL shell."""
 
     def __init__(self, programs, sizes, device=None):
         import numpy as np

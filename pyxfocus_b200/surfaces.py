@@ -23,7 +23,7 @@ from . import transformations as tran
 from . import woltsurf as wolt
 from . import zernsurf as zern
 from .analyses import analyticImagePlane, analyticXPlane, analyticYPlane
-from .program import LL_MAX_OPS, LL_MAX_ORDER, OP, flush, recorder_for
+from .program import LL_MAX_OPS, LL_MAX_ORDER, OP, SURFACE_OPS, flush, recorder_for
 
 
 def flat(rays, ind=None, nr=None):
@@ -57,7 +57,7 @@ def zernsurf(rays, coeff, rad, rorder=None, aorder=None, nr=None):
         raise NotImplementedError("pass rorder/aorder explicitly: the reference's default ordering lives in "
                                   "the third-party module utilities.imaging.zernikemod (not vendored)")
     prog = recorder_for(rays)
-    if prog is not None and np.max(np.asarray(rorder)) <= 7 and not any(c in (OP["ZERNSURF"], OP["LLSURF"])
+    if prog is not None and np.max(np.asarray(rorder)) <= 7 and not any(c in (OP["ZERNSURF"], OP["LLSURF"]) + SURFACE_OPS
                                                                         for c, _ in prog.ops):
         prog.zernsurf(coeff, rorder, aorder, rad, nr)       # radial orders <= 7: stays in the fused program
         return
@@ -137,6 +137,10 @@ def _ws(rays, which, r0, z0, psi, check, thick=None):
     opd, x, y, z, l, m, n, ux, uy, uz = rays
     a, p, d, e = con.woltparam(r0, z0)
     if thick is not None:
+        prog = _surface_recorder(rays) if check is not True else None
+        if prog is not None:
+            getattr(prog, which)(a, z0, psi, thick)
+            return
         flush(rays)
         if check is True:
             x0, y0, zz0 = x.clone(), y.clone(), z.clone()
@@ -205,9 +209,16 @@ def spoSecondary(rays, R0, F, d=.605, ind=None):
     return
 
 
+def _surface_recorder(rays):
+    """The program recording for ``rays`` when it can hold one of the remaining scalar surfaces (sphere, cylinder,
+    cylconic, paraxial lenses, torus, W-S back surfaces: no Zernike surface, LL shell or grating fan in it), else None."""
+    prog = recorder_for(rays)
+    return prog if prog is not None and prog.can_hold_surface() else None
+
+
 def _ll_recorder(rays, coeff, axial, az):
     """The program recording for ``rays`` when it can hold one more Legendre-Legendre shell with these terms (orders
-    <= 7, fewer than two shells so far, no Zernike surface or grating fan), else None."""
+    <= 7, fewer than two shells so far, no Zernike surface, grating fan or remaining scalar surface), else None."""
     prog = recorder_for(rays)
     if prog is None:
         return None
@@ -220,7 +231,7 @@ def _ll_recorder(rays, coeff, axial, az):
         ok = False
     codes = [code for code, _ in prog.ops]
     if not ok or codes.count(OP["LLSURF"]) >= LL_MAX_OPS or any(
-            code in codes for code in (OP["ZERNSURF"], OP["GRATFAN"], OP["ROTX_REMAINING"])):
+            code in codes for code in (OP["ZERNSURF"], OP["GRATFAN"], OP["ROTX_REMAINING"]) + SURFACE_OPS):
         return None
     return prog
 
@@ -375,6 +386,13 @@ def zernsurfrot(rays, coeff1, coeff2, rad, rot, rorder1=None, aorder1=None, rord
 def sphere(rays, rad, nr=None):
     """Sphere centred on the origin; the closer intersection is taken."""
     opd, x, y, z, l, m, n, ux, uy, uz = rays
+    prog = _surface_recorder(rays)
+    if prog is not None:
+        if nr is not None:
+            prog.tracesphereopd(rad, nr)
+        else:
+            prog.tracesphere(rad)
+        return
     flush(rays)
     if nr is not None:
         surf.tracesphereopd(opd, x, y, z, l, m, n, ux, uy, uz, rad, nr)
@@ -417,6 +435,10 @@ def oapCollimate(rays, efl, oapangle, nr=None):
 def torus(rays, rin, rout):
     """Torus: outer radius in the xy plane, inner radius orthogonal."""
     opd, x, y, z, l, m, n, ux, uy, uz = rays
+    prog = _surface_recorder(rays)
+    if prog is not None:
+        prog.torus(rin, rout)
+        return
     flush(rays)
     surf.torus(x, y, z, l, m, n, ux, uy, uz, rin, rout)
     return
@@ -425,6 +447,13 @@ def torus(rays, rin, rout):
 def cyl(rays, rad, nr=None):
     """Cylinder about the y axis through the origin."""
     opd, x, y, z, l, m, n, ux, uy, uz = rays
+    prog = _surface_recorder(rays)
+    if prog is not None:
+        if nr is not None:
+            prog.tracecylopd(rad, nr)
+        else:
+            prog.tracecyl(rad)
+        return
     flush(rays)
     if nr is not None:
         surf.tracecylopd(opd, x, y, z, l, m, n, ux, uy, uz, rad, nr)
@@ -436,6 +465,10 @@ def cyl(rays, rad, nr=None):
 def cylconic(rays, rad, k):
     """Cylindrical conic (sag in y, cylinder axis z)."""
     opd, x, y, z, l, m, n, ux, uy, uz = rays
+    prog = _surface_recorder(rays)
+    if prog is not None:
+        prog.cylconic(rad, k)
+        return
     flush(rays)
     surf.cylconic(x, y, z, l, m, n, ux, uy, uz, rad, k)
 
@@ -443,6 +476,10 @@ def cylconic(rays, rad, k):
 def paraxial(rays, F):
     """Ideal paraxial lens in the xy plane, optical axis z."""
     x, y, z, l, m, n, ux, uy, uz = rays[1:]
+    prog = _surface_recorder(rays)
+    if prog is not None:
+        prog.paraxial(F)
+        return
     flush(rays)
     surf.paraxial(x, y, z, l, m, n, ux, uy, uz, F)
     return
@@ -451,6 +488,10 @@ def paraxial(rays, F):
 def paraxialY(rays, F):
     """Ideal paraxial cylinder lens acting on y only."""
     x, y, z, l, m, n, ux, uy, uz = rays[1:]
+    prog = _surface_recorder(rays)
+    if prog is not None:
+        prog.paraxialy(F)
+        return
     flush(rays)
     surf.paraxialy(x, y, z, l, m, n, ux, uy, uz, F)
     return
