@@ -313,7 +313,18 @@ enum {
     PXF_OP_TORUS = 34,         /* p: rin,rout ; pxf_torus                                               */
     PXF_OP_WSPRIMARYBACK = 35, /* p: alpha,z0,psi,thick ; pxf_wsprimaryback (PXF_OPT_WS_* apply as to
                                   PXF_OP_WSPRIMARY)                                                    */
-    PXF_OP_WSSECONDARYBACK = 36 /* p: alpha,z0,psi,thick ; pxf_wssecondaryback                         */
+    PXF_OP_WSSECONDARYBACK = 36, /* p: alpha,z0,psi,thick ; pxf_wssecondaryback                        */
+    PXF_OP_ZERNPHASE = 37,     /* p: table (a DEVICE copy of what pxf_zern_table_fill wrote with opd = 0, its address
+                                  bit-cast into the double), wave, nmax as returned by the fill ; pxf_zernphase.
+                                  Radial orders <= 7 only.  A program's single Zernike-table op: refused
+                                  (PXF_ERR_UNSUPPORTED) next to PXF_OP_ZERNSURF, another PXF_OP_ZERNPHASE,
+                                  PXF_OP_LLSURF, PXF_OP_GRATFAN, PXF_OP_ROTX_REMAINING or ops 27..40.           */
+    /* Two more surfaces of the family of ops 27..36 (they may share a program with those, and are refused where those
+     * are).  Their parameter block is a table in DEVICE memory, its address bit-cast into p[0]; the table must stay
+     * alive as long as a program or segmented table refers to it. */
+    PXF_OP_CONICPLUS = 38,     /* p: table (pxf_conicplus_table_fill, opd = 0) ; pxf_conicplus                    */
+    PXF_OP_CONICPLUSOPD = 39,  /* p: table (pxf_conicplus_table_fill, opd = 1, nr) ; pxf_conicplusopd            */
+    PXF_OP_LEGSURF = 40        /* p: table (pxf_legsurf_table_fill) ; pxf_legsurf                                 */
 };
 typedef struct pxf_op {
     int32_t code;
@@ -340,6 +351,23 @@ size_t pxf_ll_table_bytes(void);
 int32_t pxf_ll_table_fill(int32_t kind, double r0, double z0, double psi, double S, double zmax, double zmin,
                           double dphi, const double *coeff, const int32_t *axial, const int32_t *az, int32_t cnum,
                           void *table_host);
+/* Table of the two Zernike sets of pxf_tracezernrot (the second evaluated at theta + rot), folded by the same two
+ * steps, into pxf_zern_table_bytes() bytes of HOST memory.  It is a PXF_OP_ZERNSURF table (opd flag 0): a rotated
+ * Zernike surface needs no opcode of its own.  Returns the highest radial order or -1. */
+int32_t pxf_zern_table_fill_rot(const double *coeff1, const int32_t *rorder1, const int32_t *aorder1, int32_t arrsize1,
+                                const double *coeff2, const int32_t *rorder2, const int32_t *aorder2, int32_t arrsize2,
+                                double rad, double rot, void *table_host);
+/* Table for a PXF_OP_CONICPLUS (opd = 0) / PXF_OP_CONICPLUSOPD (opd = 1) op: R, K and 0..16 polynomial terms folded
+ * exactly as pxf_conicplus[opd] does, into pxf_conicplus_table_bytes() bytes of HOST memory; the caller uploads them
+ * unchanged.  Returns the byte count, or -1 for more than 16 terms. */
+size_t pxf_conicplus_table_bytes(void);
+int32_t pxf_conicplus_table_fill(double R, double K, const double *p, int32_t np, int32_t opd, double nr,
+                                 void *table_host);
+/* Table for a PXF_OP_LEGSURF op: 0..48 terms with orders 0..15, folded exactly as pxf_legsurf does, into
+ * pxf_legsurf_table_bytes() bytes of HOST memory.  Returns the byte count, or -1 for an invalid term list. */
+size_t pxf_legsurf_table_bytes(void);
+int32_t pxf_legsurf_table_fill(double xwidth, double ywidth, double order, const double *coeff, const int32_t *xo,
+                               const int32_t *yo, int32_t nc, void *table_host);
 int pxf_trace_program(double *const rays[10], int64_t num, const pxf_op *ops, int32_t nops,
                       uint8_t *alive, pxf_stream_t stream);
 /* Per-ray side arrays of the ops that need them (all device pointers, each nullable unless an op uses it):
@@ -371,7 +399,8 @@ int pxf_trace_program_aux(double *const rays_in[10], double *const rays_out[10],
  *   pxf_jit_compile      compile (no GPU needed) the kernels a program will want -- in place / out of place, with /
  *                        without the centroid sums; segmented != 0: the segmented form.  Returns the number of
  *                        kernels now available (0: NVRTC missing or the compilation failed), -1: invalid program.
- *                        PXF_OP_ZERNSURF / PXF_OP_LLSURF: any non-null table address will do; aux may be NULL.
+ *                        Ops with a device table (PXF_OP_ZERNSURF, LLSURF, ZERNPHASE, CONICPLUS[OPD], LEGSURF): any
+ *                        non-null table address will do; aux may be NULL.
  *   pxf_jit_status       "ok" or why the interpreter is being used, plus counters
  *   pxf_last_trace_kernel  name of the kernel the last trace on this process launched                          */
 int32_t pxf_jit_compile(const pxf_op *ops, int32_t nops, int32_t segmented, const pxf_program_aux *aux);
@@ -398,7 +427,9 @@ int pxf_trace_program_sums(double *const rays_in[10], double *const rays_out[10]
  *   has nseg+1 entries, seg_start[0] == 0); the caller uploads it unchanged to device memory and passes both
  *   copies to pxf_trace_program_segmented (the host copy is read for the row masks only).
  *   The surface ops 27..36 (PXF_OP_TRACESPHERE .. PXF_OP_WSSECONDARYBACK) go through this pair; their scalars may
- *   differ between segments.  The _zern and _ll fills refuse them (PXF_ERR_UNSUPPORTED).
+ *   differ between segments.  So do PXF_OP_CONICPLUS / CONICPLUSOPD / LEGSURF: each segment's op carries the device
+ *   address of its own table, copied like any scalar, so those tables must outlive the segmented table.  The _zern
+ *   and _ll fills refuse ops 27..36 and 38..40 (PXF_ERR_UNSUPPORTED).
  *   rays_out == NULL: in place. */
 size_t pxf_segmented_table_bytes(int32_t nops, int32_t nseg);
 int pxf_segmented_table_fill(const pxf_op *ops, int32_t nops, int32_t nseg, const int64_t *seg_start,
@@ -409,7 +440,9 @@ int pxf_trace_program_segmented(double *const rays_in[10], double *const rays_ou
 /* Segmented programs with one Zernike surface per segment (a figure-error Monte Carlo, or shells that each have a
  * measured figure): every segment's op list has its PXF_OP_ZERNSURF at the same position, with the same opd flag
  * (p[1]); the term count, radial order (<= 7), rad and nr may differ.  pxf_segmented_table_fill refuses such lists;
- * this pair takes them (and any list the plain pair takes, except one with ops 27..36).
+ * this pair takes them (and any list the plain pair takes, except one with ops 27..36 or 38..40).
+ * PXF_OP_ZERNPHASE may take the place of PXF_OP_ZERNSURF: the same opcode in every segment, each with its own table
+ * and wave (p[1]); segments whose Zernike op differs in kind are refused (PXF_ERR_INVALID).
  *   zern_tables_host: nseg consecutive tables of pxf_zern_table_bytes() bytes, table s filled by pxf_zern_table_fill
  *   for segment s (NULL is accepted when no op is a PXF_OP_ZERNSURF).  They are copied into the segmented table, so it
  *   stays self-contained: upload it unchanged and pass both copies to pxf_trace_program_segmented, which stages the
@@ -424,7 +457,7 @@ int pxf_segmented_table_fill_zern(const pxf_op *ops, int32_t nops, int32_t nseg,
  * have a measured figure): every segment's op list has its PXF_OP_LLSURF ops (one or two) at the same positions.
  * Kinds, term lists and orders (<= 7) may differ between segments.  pxf_segmented_table_fill and
  * pxf_segmented_table_fill_zern refuse such lists; this pair takes them (and any list the plain pair takes, except one
- * with ops 27..36).
+ * with ops 27..36 or 38..40).
  *   ll_tables_host: nseg * (LL ops per program) tables of pxf_ll_table_bytes() bytes, segment-major and in op order,
  *   each filled by pxf_ll_table_fill (NULL is accepted when no op is a PXF_OP_LLSURF).  They are copied into the
  *   segmented table (pxf_segmented_table_bytes_ll has room for two per segment), so it stays self-contained: upload

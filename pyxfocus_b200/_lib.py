@@ -201,6 +201,11 @@ SIGNATURES = {
     "pxf_segmented_table_fill_zern": (_c.c_int, [_vp, _i32, _i32, _vp, _vp, _vp]),
     "pxf_ll_table_bytes": (_sz, []),
     "pxf_ll_table_fill": (_i32, [_i32, _d, _d, _d, _d, _d, _d, _d, _vp, _vp, _vp, _i32, _vp]),
+    "pxf_zern_table_fill_rot": (_i32, [_vp, _vp, _vp, _i32, _vp, _vp, _vp, _i32, _d, _d, _vp]),
+    "pxf_conicplus_table_bytes": (_sz, []),
+    "pxf_conicplus_table_fill": (_i32, [_d, _d, _vp, _i32, _i32, _d, _vp]),
+    "pxf_legsurf_table_bytes": (_sz, []),
+    "pxf_legsurf_table_fill": (_i32, [_d, _d, _d, _vp, _vp, _vp, _i32, _vp]),
     "pxf_segmented_table_bytes_ll": (_sz, [_i32, _i32]),
     "pxf_segmented_table_fill_ll": (_c.c_int, [_vp, _i32, _i32, _vp, _vp, _vp]),
     "pxf_trace_program_segmented": (_c.c_int, [_vp, _vp, _i64, _vp, _vp, _vp, _st]),

@@ -15,7 +15,7 @@ struct NoP { double unused; };
 
 // what an op may need besides the ray and its parameters
 struct ChainCtx {
-    const ZernP *zt;          // Zernike table staged in shared memory (PXF_OP_ZERNSURF)
+    const ZernP *zt;          // Zernike table staged in shared memory (PXF_OP_ZERNSURF / ZERNPHASE)
     const LLTab *llt;         // LL tables staged in shared memory, by slot (PXF_OP_LLSURF)
     int64_t i;                // index of the ray in the bundle (side arrays)
     const double *aux_wave;   // pxf_program_aux
@@ -83,6 +83,12 @@ PXF_CHAIN_OP(CParaxialY, 33, ParaxialP, op_paraxial(r, p))
 PXF_CHAIN_OP(CTorus, 34, TorusP, op_torus(r, p))
 PXF_CHAIN_OP(CWsPrimaryBack, 35, WSP, op_wsprimary_t<true>(r, p))
 PXF_CHAIN_OP(CWsSecondaryBack, 36, WSP, op_wssecondary_t<true>(r, p))
+// CONICPLUS[OPD] / LEGSURF: q = the device address of the folded block
+struct ConicPlusTabP { const ConicPlusP *t; };
+struct LegSurfTabP { const LegSurfP *t; };
+PXF_CHAIN_OP(CConicPlus, 38, ConicPlusTabP, op_conicplus(r, *p.t))
+PXF_CHAIN_OP(CConicPlusOpd, 39, ConicPlusTabP, op_conicplus(r, *p.t))
+PXF_CHAIN_OP(CLegSurf, 40, LegSurfTabP, op_legsurf(r, *p.t))
 #undef PXF_CHAIN_OP
 
 // predicates: the ray stops at the op when apply() returns false
@@ -123,6 +129,18 @@ struct CZernSurf {
     {
         const ZernP *zt = ctx.zt;
         if (zt) op_tracezern<7>(r, zt->rad, zt->nr, zt->tol, zt->nmax, p.with_opd != 0., reinterpret_cast<const double *>(zt->e));
+        return true;
+    }
+};
+// ZERNPHASE: q = {wave}; the table comes through the context, as for ZERNSURF
+struct ZernPhaseOpP { double wave; };
+struct CZernPhase {
+    using P = ZernPhaseOpP;
+    static constexpr int CODE = 37;
+    PXF_DEV static bool apply(Ray &r, const P &p, const ChainCtx &ctx)
+    {
+        const ZernP *zt = ctx.zt;
+        if (zt) op_zernphase<7>(r, zt->rad, p.wave, zt->nmax, reinterpret_cast<const double *>(zt->e));
         return true;
     }
 };

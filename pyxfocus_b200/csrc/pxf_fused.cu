@@ -33,7 +33,9 @@ PXF_DEV void count_max_update(int *dst, int k)
 // ZERN they get their own kernel so that every other program keeps its register budget
 // LL: whether it carries the Legendre-Legendre shells (PXF_OP_LLSURF); llt: their tables in shared memory, by slot
 // SURF: whether it carries the remaining scalar surfaces (PXF_OP_TRACESPHERE .. PXF_OP_WSSECONDARYBACK)
-template <bool ZERN = false, bool AUX = false, bool LL = false, bool SURF = false>
+// TAB: whether it also carries the surfaces read through a device table (PXF_OP_CONICPLUS[OPD], PXF_OP_LEGSURF)
+// ZPH: whether it carries the Zernike phase surface (PXF_OP_ZERNPHASE; zt as for ZERN)
+template <bool ZERN = false, bool AUX = false, bool LL = false, bool SURF = false, bool TAB = false, bool ZPH = false>
 PXF_DEV bool run_op(Ray &r, const FusedOp &op, const ZernP *zt = nullptr, int64_t i = 0,
                     const double *aux_wave = nullptr, int *aux_count = nullptr, int *aux_count_max = nullptr,
                     const LLTab *llt = nullptr)
@@ -128,6 +130,20 @@ PXF_DEV bool run_op(Ray &r, const FusedOp &op, const ZernP *zt = nullptr, int64_
         case PXF_OP_WSSECONDARYBACK:
             if constexpr (SURF) op_wssecondary_t<true>(r, *reinterpret_cast<const WSP *>(op.q));
             break;
+        // q[0]: the device address of the folded block (warp-uniform, read through L1)
+        case PXF_OP_CONICPLUS:
+        case PXF_OP_CONICPLUSOPD:
+            if constexpr (TAB) op_conicplus(r, **reinterpret_cast<const ConicPlusP *const *>(op.q));
+            break;
+        case PXF_OP_LEGSURF:
+            if constexpr (TAB) op_legsurf(r, **reinterpret_cast<const LegSurfP *const *>(op.q));
+            break;
+        case PXF_OP_ZERNPHASE:
+            // zt: the table in shared memory; q[0] = wave.  Same device code as pxf_zernphase (nmax <= 7)
+            if constexpr (ZPH) {
+                if (zt) op_zernphase<7>(r, zt->rad, op.q[0], zt->nmax, reinterpret_cast<const double *>(zt->e));
+            }
+            break;
         case PXF_OP_KICK: {
             r.l = r.l + op.q[0];
             r.m = r.m + op.q[1];
@@ -139,27 +155,28 @@ PXF_DEV bool run_op(Ray &r, const FusedOp &op, const ZernP *zt = nullptr, int64_
     return true;
 }
 
-template <bool ZERN = false, bool AUX = false, bool LL = false, bool SURF = false>
+template <bool ZERN = false, bool AUX = false, bool LL = false, bool SURF = false, bool TAB = false, bool ZPH = false>
 PXF_DEV bool run_program(Ray &r, const FusedProgram &prog, const ZernP *zt = nullptr, int64_t i = 0,
                          const LLTab *llt = nullptr)
 {
     for (int k = 0; k < prog.nops; k++)
-        if (!run_op<ZERN, AUX, LL, SURF>(r, prog.ops[k], zt, i, prog.aux_wave, prog.aux_count, prog.aux_count_max, llt))
+        if (!run_op<ZERN, AUX, LL, SURF, TAB, ZPH>(r, prog.ops[k], zt, i, prog.aux_wave, prog.aux_count, prog.aux_count_max, llt))
             return false;
     return true;
 }
 
-template <bool VEC2, int MINB = 1, bool ZERN = false, bool AUX = false, bool LL = false, bool SURF = false>
+template <bool VEC2, int MINB = 1, bool ZERN = false, bool AUX = false, bool LL = false, bool SURF = false,
+          bool TAB = false, bool ZPH = false>
 __global__ void __launch_bounds__(PXF_BLOCK, MINB)
 k_program(const RowPtrs P, const RowPtrs Q, const int64_t num, uint8_t *__restrict__ alive,
           double *__restrict__ partials, const __grid_constant__ FusedProgram prog)
 {
     double cnt = 0., sx = 0., sy = 0.;
-    // the Zernike table of a PXF_OP_ZERNSURF op, or the tables of the PXF_OP_LLSURF ops, staged once per CTA
-    __shared__ __align__(16) unsigned char zraw[ZERN ? sizeof(ZernP) : LL ? PXF_PROG_MAX_LL * sizeof(LLTab) : 16];
+    // the Zernike table of a PXF_OP_ZERNSURF / ZERNPHASE op, or the tables of the PXF_OP_LLSURF ops, staged once per CTA
+    __shared__ __align__(16) unsigned char zraw[(ZERN || ZPH) ? sizeof(ZernP) : LL ? PXF_PROG_MAX_LL * sizeof(LLTab) : 16];
     const ZernP *zt = nullptr;
     const LLTab *llt = nullptr;
-    if (ZERN && prog.zern) {
+    if ((ZERN || ZPH) && prog.zern) {
         const double *src = reinterpret_cast<const double *>(prog.zern);
         double *dst = reinterpret_cast<double *>(zraw);
         for (int t = threadIdx.x; t < (int)(sizeof(ZernP) / 8); t += blockDim.x) dst[t] = src[t];
@@ -185,8 +202,8 @@ k_program(const RowPtrs P, const RowPtrs Q, const int64_t num, uint8_t *__restri
             const int64_t i = q << 1;
             Ray a, b;
             fload2(a, b, P, LM, i);
-            const bool ka = run_program<ZERN, AUX, LL, SURF>(a, prog, zt, i, llt);
-            const bool kb = run_program<ZERN, AUX, LL, SURF>(b, prog, zt, i + 1, llt);
+            const bool ka = run_program<ZERN, AUX, LL, SURF, TAB, ZPH>(a, prog, zt, i, llt);
+            const bool kb = run_program<ZERN, AUX, LL, SURF, TAB, ZPH>(b, prog, zt, i + 1, llt);
             fstore2(a, b, Q, SM, i);
             if (alive) { alive[i] = ka ? 1 : 0; alive[i + 1] = kb ? 1 : 0; }
             if (ka) { cnt += 1.; sx += a.x; sy += a.y; }
@@ -196,7 +213,7 @@ k_program(const RowPtrs P, const RowPtrs Q, const int64_t num, uint8_t *__restri
             const int64_t i = num - 1;
             Ray a;
             fload1(a, P, LM, i);
-            const bool ka = run_program<ZERN, AUX, LL, SURF>(a, prog, zt, i, llt);
+            const bool ka = run_program<ZERN, AUX, LL, SURF, TAB, ZPH>(a, prog, zt, i, llt);
             fstore1(a, Q, SM, i);
             if (alive) alive[i] = ka ? 1 : 0;
             if (ka) { cnt += 1.; sx += a.x; sy += a.y; }
@@ -205,7 +222,7 @@ k_program(const RowPtrs P, const RowPtrs Q, const int64_t num, uint8_t *__restri
         for (int64_t i = tid; i < num; i += nthr) {
             Ray a;
             fload1(a, P, LM, i);
-            const bool ka = run_program<ZERN, AUX, LL, SURF>(a, prog, zt, i, llt);
+            const bool ka = run_program<ZERN, AUX, LL, SURF, TAB, ZPH>(a, prog, zt, i, llt);
             fstore1(a, Q, SM, i);
             if (alive) alive[i] = ka ? 1 : 0;
             if (ka) { cnt += 1.; sx += a.x; sy += a.y; }
@@ -237,8 +254,9 @@ __host__ __device__ __forceinline__ int seg_zern_smem_offset(int nops) { return 
 
 // ZERN: zern = nseg Zernike tables, one per segment (the Zernike instantiation of run_op, as k_program<.., true>)
 // LL: ll = nseg * nll LL tables, segment-major (the LL instantiation of run_op, as k_program<.., LL = true>)
-// SURF: the remaining scalar surfaces (as k_program<.., SURF = true>)
-template <int MINB, bool ZERN = false, bool LL = false, bool SURF = false>
+// SURF: the remaining scalar surfaces (as k_program<.., SURF = true>); TAB: and the table surfaces (TAB = true)
+// ZPH: zern = nseg Zernike tables of PXF_OP_ZERNPHASE ops (as k_program<.., ZPH = true>)
+template <int MINB, bool ZERN = false, bool LL = false, bool SURF = false, bool TAB = false, bool ZPH = false>
 __global__ void __launch_bounds__(PXF_BLOCK, MINB)
 k_program_seg(const RowPtrs P, const RowPtrs Q, const int64_t num, uint8_t *__restrict__ alive,
               const long long *__restrict__ seg_start, const FusedOp *__restrict__ ops, const int nops, const int nseg,
@@ -247,7 +265,7 @@ k_program_seg(const RowPtrs P, const RowPtrs Q, const int64_t num, uint8_t *__re
 {
     extern __shared__ __align__(16) unsigned char seg_smem[];
     FusedOp *sops = reinterpret_cast<FusedOp *>(seg_smem);
-    ZernP *zt = ZERN ? reinterpret_cast<ZernP *>(seg_smem + seg_zern_smem_offset(nops)) : nullptr;
+    ZernP *zt = (ZERN || ZPH) ? reinterpret_cast<ZernP *>(seg_smem + seg_zern_smem_offset(nops)) : nullptr;
     LLTab *llt = LL ? reinterpret_cast<LLTab *>(seg_smem + seg_zern_smem_offset(nops)) : nullptr;
     int staged = -1;
     const int words = nops * (int)(sizeof(FusedOp) / 8);
@@ -259,7 +277,7 @@ k_program_seg(const RowPtrs P, const RowPtrs Q, const int64_t num, uint8_t *__re
                 const double *src = reinterpret_cast<const double *>(ops + (int64_t)seg * nops);
                 double *dst = reinterpret_cast<double *>(sops);
                 for (int t = threadIdx.x; t < words; t += blockDim.x) dst[t] = src[t];
-                if (ZERN) {
+                if (ZERN || ZPH) {
                     const double *zsrc = reinterpret_cast<const double *>(zern + seg);
                     double *zdst = reinterpret_cast<double *>(zt);
                     for (int t = threadIdx.x; t < (int)(sizeof(ZernP) / 8); t += blockDim.x) zdst[t] = zsrc[t];
@@ -277,7 +295,7 @@ k_program_seg(const RowPtrs P, const RowPtrs Q, const int64_t num, uint8_t *__re
                 fload1(a, P, LM, i);
                 bool keep = true;
                 for (int k = 0; k < nops; k++)
-                    if (!run_op<ZERN, false, LL, SURF>(a, sops[k], zt, 0, nullptr, nullptr, nullptr, llt)) { keep = false; break; }
+                    if (!run_op<ZERN, false, LL, SURF, TAB, ZPH>(a, sops[k], zt, 0, nullptr, nullptr, nullptr, llt)) { keep = false; break; }
                 fstore1(a, Q, SM, i);
                 if (alive) alive[i] = keep ? 1 : 0;
             }
@@ -318,14 +336,38 @@ static void op_masks(int code, int row, unsigned &use, unsigned &st, unsigned &k
         case PXF_OP_PARAXIAL: use = R_X | R_Y | R_L | R_M; st = R_L | R_M; kill = R_L | R_M; break;
         case PXF_OP_PARAXIALY: use = R_Y | R_M; st = R_M; kill = R_M; break;
         case PXF_OP_WSPRIMARYBACK: case PXF_OP_WSSECONDARYBACK: use = R_NINE; st = R_POS | R_NRM; kill = R_POS; break;
+        case PXF_OP_CONICPLUS: use = R_POS | R_DIR; st = R_POS | R_NRM; kill = R_POS | R_NRM; break;
+        case PXF_OP_CONICPLUSOPD: use = R_POS | R_DIR | R_OPD; st = R_POS | R_NRM | R_OPD; kill = R_POS | R_NRM; break;
+        // the phase surfaces kick the direction they read (legsurf keeps the sign of n): nothing is killed
+        case PXF_OP_LEGSURF: use = R_X | R_Y | R_DIR; st = R_DIR; kill = 0; break;
+        case PXF_OP_ZERNPHASE: use = R_X | R_Y | R_DIR | R_OPD; st = R_DIR | R_OPD; kill = 0; break;
         default: use = 0; st = 0; kill = 0; break;
     }
 }
 
-static bool is_surface_op(int code) { return code >= PXF_OP_TRACESPHERE && code <= PXF_OP_WSSECONDARYBACK; }
+static bool is_table_surface_op(int code)
+{
+    return code == PXF_OP_CONICPLUS || code == PXF_OP_CONICPLUSOPD || code == PXF_OP_LEGSURF;
+}
+// the surface family: ops 27..36 and the table surfaces
+static bool is_surface_op(int code)
+{
+    return (code >= PXF_OP_TRACESPHERE && code <= PXF_OP_WSSECONDARYBACK) || is_table_surface_op(code);
+}
+// which of the interpreters of the newer table ops an op list needs (read from the ops, so that FusedProgram, the
+// parameter of every k_program, keeps its layout)
+static void new_table_kinds(const FusedOp *ops, int nops, bool &zphase, bool &tabsurf)
+{
+    zphase = tabsurf = false;
+    for (int k = 0; k < nops; k++) {
+        zphase = zphase || ops[k].code == PXF_OP_ZERNPHASE;
+        tabsurf = tabsurf || is_table_surface_op(ops[k].code);
+    }
+}
 static bool is_table_or_aux_op(int code)
 {
-    return code == PXF_OP_ZERNSURF || code == PXF_OP_LLSURF || code == PXF_OP_GRATFAN || code == PXF_OP_ROTX_REMAINING;
+    return code == PXF_OP_ZERNSURF || code == PXF_OP_LLSURF || code == PXF_OP_GRATFAN || code == PXF_OP_ROTX_REMAINING ||
+           code == PXF_OP_ZERNPHASE;
 }
 
 int build_program(FusedProgram &fp, const pxf_op *ops, int nops, const pxf_program_aux *aux)
@@ -336,13 +378,22 @@ int build_program(FusedProgram &fp, const pxf_op *ops, int nops, const pxf_progr
     // the remaining scalar surfaces run in an interpreter of their own, which holds no table or side-array op: refused
     // before anything else is checked, so the verdict does not depend on the order of the ops
     bool surf = false, other = false;
+    int zphase = 0, tables = 0;                // PXF_OP_ZERNPHASE ops; ops with a Zernike or LL table or a side array
     for (int k = 0; k < nops; k++) {
         surf = surf || is_surface_op(ops[k].code);
         other = other || is_table_or_aux_op(ops[k].code);
+        zphase += ops[k].code == PXF_OP_ZERNPHASE;
+        tables += is_table_or_aux_op(ops[k].code);
     }
     if (surf && other) {
-        set_error("program: the sphere / cylinder / cylconic / paraxial / torus / W-S back-surface ops cannot share a "
-                  "program with a Zernike surface, a Legendre-Legendre shell or a grating fan");
+        set_error("program: the sphere / cylinder / cylconic / paraxial / torus / W-S back-surface / conicplus / legsurf "
+                  "ops cannot share a program with a Zernike surface or phase, a Legendre-Legendre shell or a grating fan");
+        return PXF_ERR_UNSUPPORTED;
+    }
+    // the Zernike phase surface runs in an interpreter of its own, which holds no other table or side-array op
+    if (zphase && tables > 1) {
+        set_error("program: a Zernike phase surface cannot share a program with another Zernike surface or phase, a "
+                  "Legendre-Legendre shell or a grating fan");
         return PXF_ERR_UNSUPPORTED;
     }
     fp.surf = surf ? 1 : 0;
@@ -377,6 +428,23 @@ int build_program(FusedProgram &fp, const pxf_op *ops, int nops, const pxf_progr
             case PXF_OP_PARAXIALY: { ParaxialP t{p[0], 1, 0}; memcpy(f.q, &t, sizeof(t)); break; }
             case PXF_OP_TORUS: { TorusP t = make_torus(p[0], p[1]); memcpy(f.q, &t, sizeof(t)); break; }
             case PXF_OP_WSPRIMARYBACK: case PXF_OP_WSSECONDARYBACK: { WSP t = make_ws(p[0], p[1], p[2], p[3]); memcpy(f.q, &t, sizeof(t)); break; }
+            // the device table's address (folded by pxf_conicplus_table_fill / pxf_legsurf_table_fill)
+            case PXF_OP_CONICPLUS: case PXF_OP_CONICPLUSOPD: case PXF_OP_LEGSURF: {
+                const void *tab;
+                memcpy(&tab, &p[0], sizeof(tab));
+                if (!tab) { set_error("program: PXF_OP_CONICPLUS / CONICPLUSOPD / LEGSURF need a device table"); return PXF_ERR_INVALID; }
+                memcpy(f.q, &tab, sizeof(tab));
+                break;
+            }
+            case PXF_OP_ZERNPHASE: {
+                const ZernP *tab;
+                memcpy(&tab, &p[0], sizeof(tab));
+                if (!tab) { set_error("program: PXF_OP_ZERNPHASE needs a device table"); return PXF_ERR_INVALID; }
+                if (!(p[2] >= 0. && p[2] <= 7.)) { set_error("program: PXF_OP_ZERNPHASE supports radial orders <= 7 (use pxf_zernphase)"); return PXF_ERR_UNSUPPORTED; }
+                fp.zern = tab;
+                f.q[0] = p[1];                         // wave
+                break;
+            }
             case PXF_OP_VIGNETTE_BOX:
                 f.row = (int)p[0];
                 if (f.row < 0 || f.row > 9) { set_error("program: bad row in VIGNETTE_BOX"); return PXF_ERR_INVALID; }
@@ -506,6 +574,12 @@ int build_program(FusedProgram &fp, const pxf_op *ops, int nops, const pxf_progr
 // 4.88 / 5.39 ms, paraxial 4.73 / 4.23 / 4.59, wssecondaryback 7.74 / 6.93 / 7.18, torus 3.11 / 3.59 / 3.51, the
 // 1000-segment lens 17.4 / 13.8 / 15.2 (profiles/surface_ops_bench_b200.json)
 #define SURF_MINB 3
+// ... and of the interpreters with the table surfaces (k_program<tabsurf>, the surface family plus conicplus / legsurf)
+// and with the Zernike phase surface (k_program<zphase>), and their segmented forms.  Not swept: the cap of
+// k_program<surf>, whose ops they hold, and of k_program<zernike> (PXF_ZERNPROG_MINB's default), whose table staging
+// they share.  ptxas at 3: 80 registers and 128 / 112 B of spill stores.
+#define TABSURF_MINB 3
+#define ZPHASE_MINB 3
 
 int launch_program(double *const rays[10], int64_t num, const FusedProgram &fp, uint8_t *alive, cudaStream_t s,
                    double *const rays_out[10], double *partials, int *grid_out)
@@ -548,9 +622,15 @@ int launch_program(double *const rays[10], int64_t num, const FusedProgram &fp, 
         if (grid_out) *grid_out = grid;
         kern<<<grid, PXF_BLOCK, 0, s>>>(P, Q, num, alive, partials, fp);
     };
+    bool zphase, tabsurf;
+    new_table_kinds(fp.ops, fp.nops, zphase, tabsurf);
     if (fp.uses_aux) {
         if (fp.zern) { set_error("program: a Zernike surface and a grating fan in one program are not supported"); return PXF_ERR_UNSUPPORTED; }
         go(k_program<false, 3, false, true>, num);
+    }
+    else if (zphase) {
+        // one ray per thread, capped for ZPHASE_MINB resident CTAs per SM
+        go(k_program<false, ZPHASE_MINB, false, false, false, false, false, true>, num);
     }
     else if (fp.zern) {
         // one ray per thread; PXF_ZERNPROG_MINB (tuning): register cap for 1 / 2 / 3 resident CTAs per SM.  Measured on
@@ -574,6 +654,10 @@ int launch_program(double *const rays[10], int64_t num, const FusedProgram &fp, 
         else if (lm == 4) go(k_program<false, 4, false, false, true>, num);
         else go(k_program<false, 1, false, false, true>, num);
     }
+    else if (tabsurf) {
+        // one ray per thread, capped for TABSURF_MINB resident CTAs per SM
+        go(k_program<false, TABSURF_MINB, false, false, false, true, true>, num);
+    }
     else if (fp.surf) {
         // one ray per thread, capped for SURF_MINB resident CTAs per SM (see its definition)
         go(k_program<false, SURF_MINB, false, false, false, true>, num);
@@ -583,8 +667,10 @@ int launch_program(double *const rays[10], int64_t num, const FusedProgram &fp, 
     else if (variant == 1) go(k_program<false, 1>, num);
     else go(k_program<false, 4>, num);
     count_launch();
-    note_kernel(fp.zern ? "k_program<zernike> (interpreter)" : fp.uses_aux ? "k_program<aux> (interpreter)" :
-                fp.nll ? "k_program<ll> (interpreter)" : fp.surf ? "k_program<surf> (interpreter)" : "k_program (interpreter)");
+    note_kernel(zphase ? "k_program<zphase> (interpreter)" : fp.zern ? "k_program<zernike> (interpreter)" :
+                fp.uses_aux ? "k_program<aux> (interpreter)" : fp.nll ? "k_program<ll> (interpreter)" :
+                tabsurf ? "k_program<tabsurf> (interpreter)" : fp.surf ? "k_program<surf> (interpreter)" :
+                "k_program (interpreter)");
     return check_launch("k_program");
 }
 
@@ -683,6 +769,54 @@ extern "C" int32_t pxf_ll_table_fill(int32_t kind, double r0, double z0, double 
     return top;
 }
 
+// the two make_zern steps of pxf_tracezernrot, in that order
+extern "C" int32_t pxf_zern_table_fill_rot(const double *coeff1, const int32_t *rorder1, const int32_t *aorder1,
+                                           int32_t arrsize1, const double *coeff2, const int32_t *rorder2,
+                                           const int32_t *aorder2, int32_t arrsize2, double rad, double rot,
+                                           void *table_host)
+{
+    if (!coeff1 || !rorder1 || !aorder1 || arrsize1 <= 0 || !coeff2 || !rorder2 || !aorder2 || arrsize2 <= 0 || !table_host) {
+        set_error("pxf_zern_table_fill_rot: bad argument");
+        return -1;
+    }
+    ZernP z;
+    if (make_zern(z, coeff1, rorder1, aorder1, arrsize1, rad, false, 0.) < 0 ||
+        make_zern(z, coeff2, rorder2, aorder2, arrsize2, rad, false, 0., rot, true) < 0) {
+        set_error("pxf_zern_table_fill_rot: invalid Zernike table");
+        return -1;
+    }
+    memcpy(table_host, &z, sizeof(z));
+    return z.nmax;
+}
+
+extern "C" size_t pxf_conicplus_table_bytes(void) { return sizeof(ConicPlusP); }
+
+extern "C" int32_t pxf_conicplus_table_fill(double R, double K, const double *p, int32_t np, int32_t opd, double nr,
+                                            void *table_host)
+{
+    ConicPlusP q;
+    if (!table_host || (np > 0 && !p) || make_conicplus(q, R, K, p, np, opd != 0, opd != 0 ? nr : 0.) < 0) {
+        set_error("pxf_conicplus_table_fill: need 0..%d polynomial terms", PXF_CONICPLUS_MAXP);
+        return -1;
+    }
+    memcpy(table_host, &q, sizeof(q));
+    return (int32_t)sizeof(q);
+}
+
+extern "C" size_t pxf_legsurf_table_bytes(void) { return sizeof(LegSurfP); }
+
+extern "C" int32_t pxf_legsurf_table_fill(double xwidth, double ywidth, double order, const double *coeff,
+                                          const int32_t *xo, const int32_t *yo, int32_t nc, void *table_host)
+{
+    LegSurfP q;
+    if (!table_host || !coeff || !xo || !yo || make_legsurf(q, xwidth, ywidth, order, coeff, xo, yo, nc) < 0) {
+        set_error("pxf_legsurf_table_fill: need 0..%d terms with orders 0..%d", PXF_LEGSURF_MAXC, PXF_LEGSURF_MAXN);
+        return -1;
+    }
+    memcpy(table_host, &q, sizeof(q));
+    return (int32_t)sizeof(q);
+}
+
 // ---- segmented programs -------------------------------------------------------------------------
 static size_t seg_align(size_t v) { return (v + 15) & ~(size_t)15; }
 static size_t seg_ops_offset(int nseg) { return seg_align(sizeof(SegHeader)) + seg_align((size_t)(nseg + 1) * 8); }
@@ -741,9 +875,9 @@ static int seg_table_fill(const pxf_op *ops, int nops, int nseg, const int64_t *
                 set_error("segmented program: PXF_OP_GRATFAN / PXF_OP_ROTX_REMAINING are not supported");
                 return PXF_ERR_UNSUPPORTED;
             }
-            if (ops[k].code == PXF_OP_ZERNSURF && zern_ok) zern = true;
+            if ((ops[k].code == PXF_OP_ZERNSURF || ops[k].code == PXF_OP_ZERNPHASE) && zern_ok) zern = true;
         }
-        if (zern && !zern_tables) { set_error("segmented program: PXF_OP_ZERNSURF needs one Zernike table per segment"); return PXF_ERR_INVALID; }
+        if (zern && !zern_tables) { set_error("segmented program: PXF_OP_ZERNSURF / ZERNPHASE need one Zernike table per segment"); return PXF_ERR_INVALID; }
     }
     // LL ops: their positions in segment 0's list (the others must match, checked with the opcode sequence below)
     int llpos[PXF_PROG_MAX_LL], nll = 0;
@@ -755,8 +889,8 @@ static int seg_table_fill(const pxf_op *ops, int nops, int nseg, const int64_t *
         }
         if (is_surface_op(ops[k].code)) {
             if (zern_ok || ll_ok) {
-                set_error("segmented program: the sphere / cylinder / cylconic / paraxial / torus / W-S back-surface "
-                          "ops need pxf_segmented_table_fill");
+                set_error("segmented program: the sphere / cylinder / cylconic / paraxial / torus / W-S back-surface / "
+                          "conicplus / legsurf ops need pxf_segmented_table_fill");
                 return PXF_ERR_UNSUPPORTED;
             }
             surf = true;
@@ -800,11 +934,11 @@ static int seg_table_fill(const pxf_op *ops, int nops, int nseg, const int64_t *
             memcpy(zdst + sgm, static_cast<const char *>(zern_tables) + (size_t)sgm * sizeof(ZernP), sizeof(ZernP));
             const int nmax = zdst[sgm].nmax;
             if (nmax < 0 || nmax > 7) {
-                set_error("segmented program: segment %d: PXF_OP_ZERNSURF supports radial orders <= 7 (table has %d)", sgm, nmax);
+                set_error("segmented program: segment %d: PXF_OP_ZERNSURF / ZERNPHASE support radial orders <= 7 (table has %d)", sgm, nmax);
                 return PXF_ERR_UNSUPPORTED;
             }
             for (int k = 0; k < nops; k++)
-                if (sops[k].code == PXF_OP_ZERNSURF) {
+                if (sops[k].code == PXF_OP_ZERNSURF || sops[k].code == PXF_OP_ZERNPHASE) {
                     const ZernP *any = zdst + sgm;       // build_program only checks that a table is there
                     memcpy(&sops[k].p[0], &any, sizeof(any));
                     sops[k].p[2] = (double)nmax;
@@ -820,7 +954,8 @@ static int seg_table_fill(const pxf_op *ops, int nops, int nseg, const int64_t *
         int rc = build_program(fp, sops, nops);
         if (rc) return rc;
         if ((fp.zern && !zern_ok) || fp.uses_aux) {
-            set_error("segmented program: PXF_OP_ZERNSURF needs pxf_segmented_table_fill_zern; PXF_OP_GRATFAN is not supported");
+            set_error("segmented program: PXF_OP_ZERNSURF / ZERNPHASE need pxf_segmented_table_fill_zern; PXF_OP_GRATFAN is "
+                      "not supported");
             return PXF_ERR_UNSUPPORTED;
         }
         if (sgm > 0)
@@ -891,9 +1026,10 @@ extern "C" int pxf_trace_program_segmented(double *const rays_in[10], double *co
         if ((SM & (1u << k)) && !Q.p[k]) { set_error("segmented program: null output row pointer (row %d)", k); return PXF_ERR_INVALID; }
     }
     const FusedOp *hops = reinterpret_cast<const FusedOp *>(static_cast<const char *>(table_host) + seg_ops_offset(nseg));
-    bool vig = false;
+    bool vig = false, zph, tab;
     for (int k = 0; k < nops; k++)
         if (is_vignette(hops[k].code)) vig = true;
+    new_table_kinds(hops, nops, zph, tab);
     if (vig && !alive) { set_error("program with a VIGNETTE op needs an alive array"); return PXF_ERR_INVALID; }
     const char *db = static_cast<const char *>(table_dev);
     const long long *dstart = reinterpret_cast<const long long *>(db + seg_align(sizeof(SegHeader)));
@@ -917,6 +1053,13 @@ extern "C" int pxf_trace_program_segmented(double *const rays_in[10], double *co
         const int grid = grid_for(num, SEG_TILE, nb);
         kern<<<grid, PXF_BLOCK, smem, s>>>(P, Q, num, alive, dstart, dops, nops, nseg, LM, SM, dzern, dll, nll);
     };
+    if (dzern && zph) {
+        // the segment's Zernike table is staged behind its op table; register cap as for k_program<zphase>
+        go(k_program_seg<ZPHASE_MINB, false, false, false, false, true>, (size_t)seg_zern_smem_offset(nops) + sizeof(ZernP));
+        count_launch();
+        note_kernel("k_program_seg<zphase> (interpreter)");
+        return check_launch("k_program_seg<zphase>");
+    }
     if (dzern) {
         // the segment's Zernike table is staged behind its op table; register cap as for k_program<zernike>
         // (PXF_ZERNPROG_MINB, resident CTAs per SM)
@@ -942,6 +1085,12 @@ extern "C" int pxf_trace_program_segmented(double *const rays_in[10], double *co
         count_launch();
         note_kernel("k_program_seg<ll> (interpreter)");
         return check_launch("k_program_seg<ll>");
+    }
+    if (tab) {
+        go(k_program_seg<TABSURF_MINB, false, false, true, true>, (size_t)nops * sizeof(FusedOp));
+        count_launch();
+        note_kernel("k_program_seg<tabsurf> (interpreter)");
+        return check_launch("k_program_seg<tabsurf>");
     }
     if (h->surf) {
         go(k_program_seg<SURF_MINB, false, false, true>, (size_t)nops * sizeof(FusedOp));

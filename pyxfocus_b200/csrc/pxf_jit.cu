@@ -66,6 +66,10 @@ static const OpDesc OPS[] = {
     {PXF_OP_TORUS, "CTorus", sizeof(CTorus::P), false},
     {PXF_OP_WSPRIMARYBACK, "CWsPrimaryBack", sizeof(CWsPrimaryBack::P), false},
     {PXF_OP_WSSECONDARYBACK, "CWsSecondaryBack", sizeof(CWsSecondaryBack::P), false},
+    {PXF_OP_ZERNPHASE, "CZernPhase", sizeof(CZernPhase::P), false},
+    {PXF_OP_CONICPLUS, "CConicPlus", sizeof(CConicPlus::P), false},
+    {PXF_OP_CONICPLUSOPD, "CConicPlusOpd", sizeof(CConicPlusOpd::P), false},
+    {PXF_OP_LEGSURF, "CLegSurf", sizeof(CLegSurf::P), false},
 };
 static const OpDesc *op_desc(int code)
 {
@@ -216,7 +220,7 @@ static bool spec_from_ops(const FusedOp *ops, int nops, JitSpec &sp)
         }
         sp.targs.push_back(ta);
         sp.cp_bytes += d->bytes;
-        if (ops[k].code == PXF_OP_ZERNSURF) sp.zern = true;
+        if (ops[k].code == PXF_OP_ZERNSURF || ops[k].code == PXF_OP_ZERNPHASE) sp.zern = true;
     }
     return true;
 }
@@ -359,11 +363,23 @@ void note_kernel(const char *name) { snprintf(g_last_kernel, sizeof(g_last_kerne
 // 7.1 / 13.0 ms for N = 3 / 5 / 7 (profiles/ll_program_bench_b200.json)
 static const int LL_MINB = 2;
 
+// Chains with a conicplus run one ray per thread: its Newton loop over up to 16 powers does not gain from a second ray
+// in flight, and the pair costs registers.  The aspheric singlet of profiles/table_surface_ops_bench.py (sphere,
+// conicplus with 8 terms, 5e7 rays) on one B200 (1000 W): 11.80 ms with two rays per thread, 8.68 ms with one, at
+// 3 CTAs/SM; reading the conicplus block from shared memory or from a register copy instead of through L1 changed
+// either by less than 1 %.
+static bool has_conicplus(const FusedProgram &fp)
+{
+    for (int k = 0; k < fp.nops; k++)
+        if (fp.ops[k].code == PXF_OP_CONICPLUS || fp.ops[k].code == PXF_OP_CONICPLUSOPD) return true;
+    return false;
+}
+
 static void fill_spec(JitSpec &sp, const FusedProgram &fp, bool aligned)
 {
     sp.LM = fp.load_mask; sp.SM = fp.store_mask;
     sp.seg = false;
-    sp.mode = (aligned && !sp.zern && !sp.nll && !fp.uses_aux) ? 2 : 1;
+    sp.mode = (aligned && !sp.zern && !sp.nll && !fp.uses_aux && !has_conicplus(fp)) ? 2 : 1;
     sp.minb = sp.nll ? LL_MINB : 3;
 }
 

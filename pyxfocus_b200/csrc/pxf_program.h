@@ -24,7 +24,7 @@ struct FusedProgram {
     // of downloading them.  Empty when the program can stop rays early (vignette predicates).
     unsigned const_mask;
     double const_val[10];
-    const ZernP *zern;       // device table of the program's PXF_OP_ZERNSURF op (NULL: none); staged in shared memory
+    const ZernP *zern;       // device table of the program's PXF_OP_ZERNSURF or ZERNPHASE op (NULL: none); staged in shared memory
     // per-ray side arrays (pxf_program_aux): wavelengths / grating counts of PXF_OP_GRATFAN, PXF_OP_ROTX_REMAINING
     const double *aux_wave;
     int *aux_count;

@@ -34,15 +34,39 @@ OP = dict(TRANSFORM=1, ITRANSFORM=2, REFLECT=3, REFRACT=4, RADGRAT=5, FLAT=6, FL
           WSPRIMARY=14, WSSECONDARY=15, SPOCONE=16, VIGNETTE_MAG=17, VIGNETTE_BOX=18,
           VIGNETTE_ABS=19, KICK=20, ZERNSURF=21, KICKN=22, VIGNETTE_RHOGT=23, GRATFAN=24, ROTX_REMAINING=25,
           LLSURF=26, TRACESPHERE=27, TRACESPHEREOPD=28, TRACECYL=29, TRACECYLOPD=30, CYLCONIC=31, PARAXIAL=32,
-          PARAXIALY=33, TORUS=34, WSPRIMARYBACK=35, WSSECONDARYBACK=36)
+          PARAXIALY=33, TORUS=34, WSPRIMARYBACK=35, WSSECONDARYBACK=36, ZERNPHASE=37, CONICPLUS=38, CONICPLUSOPD=39,
+          LEGSURF=40)
 MAX_OPS = 24
 LL_MAX_ORDER = 7       # Legendre orders a fused program holds (higher orders run the stand-alone routines)
 LL_MAX_OPS = 2         # Legendre-Legendre shells per program
 _VIGNETTES = (OP["VIGNETTE_MAG"], OP["VIGNETTE_BOX"], OP["VIGNETTE_ABS"], OP["VIGNETTE_RHOGT"])
 _AUX_OPS = (OP["GRATFAN"], OP["ROTX_REMAINING"])
-# the remaining scalar surfaces (sphere .. W-S back surfaces) share no program with a table or side-array op
-SURFACE_OPS = tuple(range(OP["TRACESPHERE"], OP["WSSECONDARYBACK"] + 1))
-TABLE_AUX_OPS = (OP["ZERNSURF"], OP["LLSURF"]) + _AUX_OPS
+# the surfaces read through a device table of their own (conicplus, legsurf)
+TABLE_SURFACE_OPS = (OP["CONICPLUS"], OP["CONICPLUSOPD"], OP["LEGSURF"])
+# the surface family (sphere .. W-S back surfaces, conicplus, legsurf) shares no program with a table or side-array op
+SURFACE_OPS = tuple(range(OP["TRACESPHERE"], OP["WSSECONDARYBACK"] + 1)) + TABLE_SURFACE_OPS
+TABLE_AUX_OPS = (OP["ZERNSURF"], OP["LLSURF"]) + _AUX_OPS + (OP["ZERNPHASE"],)
+ZERN_MAX_ORDER = 7     # Zernike radial orders a fused program holds
+CONICPLUS_MAX_TERMS = 16   # polynomial terms of conicplus (surfacesf.f95:514-638)
+LEGSURF_MAX_TERMS = 48     # Legendre terms of legsurf ...
+LEGSURF_MAX_ORDER = 15     # ... and their orders (surfacesf.f95:642-668)
+
+
+def _host_array(a, dtype):
+    import numpy as np
+    if isinstance(a, torch.Tensor):
+        a = a.detach().cpu().numpy()
+    return np.ascontiguousarray(np.asarray(a).ravel(), dtype=dtype)
+
+
+def _zern_terms(coeff, rorder, aorder):
+    import numpy as np
+    c = np.ascontiguousarray(coeff, dtype=np.float64)
+    r = np.ascontiguousarray(rorder, dtype=np.int32)
+    a = np.ascontiguousarray(aorder, dtype=np.int32)
+    if not (c.shape == r.shape == a.shape) or c.ndim != 1 or c.shape[0] == 0:
+        raise ValueError("coeff, rorder, aorder must be 1-D arrays of one length")
+    return c, r, a
 
 
 class Program:
@@ -144,47 +168,114 @@ class Program:
     def wssecondaryback(self, alpha, z0, psi, thick):
         return self._surface(OP["WSSECONDARYBACK"], alpha, z0, psi, thick)
 
+    # --- surfaces with a folded table (surfacesf.f95:514-668): the table is uploaded once per device and read by
+    # the kernel through its address ---
+    def conicplus(self, R, K, p):
+        return self._table_surface(OP["CONICPLUS"], self._conicplus_table(R, K, p, 0, 0.))
+
+    def conicplusopd(self, R, K, p, nr):
+        return self._table_surface(OP["CONICPLUSOPD"], self._conicplus_table(R, K, p, 1, nr))
+
+    def legsurf(self, xwidth, ywidth, order, coeff, xo, yo):
+        c, a, b = _host_array(coeff, "float64"), _host_array(xo, "int32"), _host_array(yo, "int32")
+        if not (c.shape == a.shape == b.shape):
+            raise ValueError("coeff, xo, yo must have one length")
+        L = _lib.lib()
+        tab = torch.empty(int(L.pxf_legsurf_table_bytes()), dtype=torch.uint8)
+        if int(L.pxf_legsurf_table_fill(float(xwidth), float(ywidth), float(order), c.ctypes.data, a.ctypes.data,
+                                        b.ctypes.data, c.shape[0], tab.data_ptr())) < 0:
+            raise ValueError(L.pxf_last_error().decode())
+        return self._table_surface(OP["LEGSURF"], tab)
+
+    @staticmethod
+    def _conicplus_table(R, K, p, opd, nr):
+        pp = _host_array(p, "float64")
+        L = _lib.lib()
+        tab = torch.empty(int(L.pxf_conicplus_table_bytes()), dtype=torch.uint8)
+        if int(L.pxf_conicplus_table_fill(float(R), float(K), pp.ctypes.data, pp.shape[0], opd, float(nr),
+                                          tab.data_ptr())) < 0:
+            raise ValueError(L.pxf_last_error().decode())
+        return tab
+
+    def _table_surface(self, code, tab):
+        self._check_surface()
+        self._tables[len(self.ops)] = tab
+        return self.add(code, 0.)
+
     def can_hold_surface(self):
         """Whether one of the ops above may join this program (none of ``TABLE_AUX_OPS`` is in it)."""
         return not any(c in TABLE_AUX_OPS for c, _ in self.ops)
 
-    def _surface(self, code, *p):
+    def _check_surface(self):
         if not self.can_hold_surface():
-            raise NotImplementedError("the sphere / cylinder / cylconic / paraxial / torus / W-S back-surface ops "
-                                      "cannot share a program with a Zernike surface, an LL shell or a grating fan")
+            raise NotImplementedError("the sphere / cylinder / cylconic / paraxial / torus / W-S back-surface / "
+                                      "conicplus / legsurf ops cannot share a program with a Zernike surface or phase, "
+                                      "an LL shell or a grating fan")
+
+    def _surface(self, code, *p):
+        self._check_surface()
         return self.add(code, *p)
 
     def _refuse_with_surfaces(self, what):
         if any(c in SURFACE_OPS for c, _ in self.ops):
             raise NotImplementedError("%s cannot share a program with the sphere / cylinder / cylconic / paraxial / "
-                                      "torus / W-S back-surface ops" % what)
+                                      "torus / W-S back-surface / conicplus / legsurf ops" % what)
+        if any(c == OP["ZERNPHASE"] for c, _ in self.ops):
+            raise NotImplementedError("%s cannot share a program with a Zernike phase surface" % what)
 
     # --- zernsurf ---
     def zernsurf(self, coeff, rorder, aorder, rad, nr=None):
         """tracezern / tracezernOPD (zernsurf.f95:8-203) inside the program; radial orders <= 7, one Zernike surface
         per program.  The term list is folded on the host exactly as for the stand-alone routine; the table is
         uploaded once per device and staged in shared memory by the kernel."""
-        import numpy as np
-        c = np.ascontiguousarray(coeff, dtype=np.float64)
-        r = np.ascontiguousarray(rorder, dtype=np.int32)
-        a = np.ascontiguousarray(aorder, dtype=np.int32)
-        if not (c.shape == r.shape == a.shape) or c.ndim != 1 or c.shape[0] == 0:
-            raise ValueError("coeff, rorder, aorder must be 1-D arrays of one length")
+        c, r, a = _zern_terms(coeff, rorder, aorder)
+        self._check_zernsurf()
+        L = _lib.lib()
+        tab = torch.empty(int(L.pxf_zern_table_bytes()), dtype=torch.uint8)
+        nmax = int(L.pxf_zern_table_fill(c.ctypes.data, r.ctypes.data, a.ctypes.data, c.shape[0], float(rad),
+                                         0 if nr is None else 1, 0. if nr is None else float(nr), tab.data_ptr()))
+        return self._zern_op(OP["ZERNSURF"], tab, nmax, 0. if nr is None else 1.)
+
+    def tracezernrot(self, coeff1, rorder1, aorder1, coeff2, rorder2, aorder2, rad, rot):
+        """tracezernrot (zernsurf.f95:257-359) inside the program: both sets fold into one Zernike table, the second
+        rotated by ``rot``, and the program holds it as a ``zernsurf`` (the same rules apply)."""
+        c1, r1, a1 = _zern_terms(coeff1, rorder1, aorder1)
+        c2, r2, a2 = _zern_terms(coeff2, rorder2, aorder2)
+        self._check_zernsurf()
+        L = _lib.lib()
+        tab = torch.empty(int(L.pxf_zern_table_bytes()), dtype=torch.uint8)
+        nmax = int(L.pxf_zern_table_fill_rot(c1.ctypes.data, r1.ctypes.data, a1.ctypes.data, c1.shape[0],
+                                             c2.ctypes.data, r2.ctypes.data, a2.ctypes.data, c2.shape[0], float(rad),
+                                             float(rot), tab.data_ptr()))
+        return self._zern_op(OP["ZERNSURF"], tab, nmax, 0.)
+
+    def zernphase(self, coeff, rorder, aorder, rad, wave):
+        """zernphase (zernsurf.f95:206-250) inside the program; radial orders <= 7.  A program's only Zernike-table
+        op: it shares no program with a Zernike surface, an LL shell, a grating fan or the surface family."""
+        c, r, a = _zern_terms(coeff, rorder, aorder)
+        if not self.can_hold_surface() or any(code in SURFACE_OPS for code, _ in self.ops):
+            raise NotImplementedError("a Zernike phase surface cannot share a program with another Zernike surface or "
+                                      "phase, an LL shell, a grating fan or the sphere .. legsurf surface ops")
+        L = _lib.lib()
+        tab = torch.empty(int(L.pxf_zern_table_bytes()), dtype=torch.uint8)
+        nmax = int(L.pxf_zern_table_fill(c.ctypes.data, r.ctypes.data, a.ctypes.data, c.shape[0], float(rad), 0, 0.,
+                                         tab.data_ptr()))
+        return self._zern_op(OP["ZERNPHASE"], tab, nmax, float(wave))
+
+    def _check_zernsurf(self):
         if any(code == OP["ZERNSURF"] for code, _ in self.ops):
             raise ValueError("a program carries at most one Zernike surface")
         if any(code == OP["LLSURF"] for code, _ in self.ops):
             raise NotImplementedError("a Zernike surface and Legendre-Legendre shells in one program are not supported")
         self._refuse_with_surfaces("a Zernike surface")
-        L = _lib.lib()
-        tab = torch.empty(int(L.pxf_zern_table_bytes()), dtype=torch.uint8)
-        nmax = int(L.pxf_zern_table_fill(c.ctypes.data, r.ctypes.data, a.ctypes.data, c.shape[0], float(rad),
-                                         0 if nr is None else 1, 0. if nr is None else float(nr), tab.data_ptr()))
+
+    def _zern_op(self, code, tab, nmax, p1):
         if nmax < 0:
             raise ValueError("invalid Zernike term list")
-        if nmax > 7:
-            raise NotImplementedError("fused Zernike surfaces support radial orders <= 7")
+        if nmax > ZERN_MAX_ORDER:
+            raise NotImplementedError("fused Zernike surfaces support radial orders <= %d" % ZERN_MAX_ORDER)
         self._tables[len(self.ops)] = tab
-        return self.add(OP["ZERNSURF"], 0., 0. if nr is None else 1., float(nmax))
+        return self.add(code, 0., p1, float(nmax))
 
     # --- Legendre-Legendre shells (woltsurf.f95:219-379, :643-718) ---
     def wolterprimll(self, r0, z0, zmax, zmin, dphi, coeff, axial, az):
@@ -287,11 +378,11 @@ class Program:
                 arr[k].p[j] = v
             if k in self._tables:
                 if device is None:
-                    raise ValueError("a program with a Zernike surface or an LL shell needs a device")
+                    raise ValueError("a program with an op that carries a table needs a device")
                 key = (k, str(device))
                 if key not in self._dev_tables:
                     self._dev_tables[key] = self._tables[k].to(device)
-                # the table's device address travels bit-cast in p[0] (include/pxf.h, PXF_OP_ZERNSURF / LLSURF)
+                # the table's device address travels bit-cast in p[0] (include/pxf.h, PXF_OP_ZERNSURF, LLSURF, ...)
                 arr[k].p[0] = struct.unpack("d", struct.pack("Q", self._dev_tables[key].data_ptr()))[0]
         return arr
 
@@ -498,9 +589,16 @@ class SegmentedProgram:
     ``ellipsoidwoltll``) at the same positions, each segment with its own kind, terms and orders (<= 7).
 
     The remaining scalar surfaces (``tracesphere`` .. ``wssecondaryback``) take their own scalars per segment (a
-    tolerance sweep over the radii of a lens pair, say); they share no program with a Zernike surface or an LL shell."""
+    tolerance sweep over the radii of a lens pair, say); they share no program with a Zernike surface or an LL shell.
+    So do ``conicplus`` / ``conicplusopd`` / ``legsurf``, each segment with its own table (a tolerance Monte Carlo over
+    aspheric coefficients); the device copies of those tables are kept alive here.
+
+    ``zernphase`` may take the place of ``zernsurf`` (the same op in every segment, each with its own terms and
+    ``wave``), and a clocking sweep is a ``tracezernrot`` per segment whose ``rot`` differs."""
 
     def __init__(self, programs, sizes, device=None):
+        import struct
+
         import numpy as np
         if len(programs) != len(sizes) or not programs:
             raise ValueError("one program per segment")
@@ -523,8 +621,30 @@ class SegmentedProgram:
                 o.code = code
                 for j, v in enumerate(p):
                     o.p[j] = v
+        # (the device is looked up after the fill, which refuses a bad list first, unless tables go there before)
+        dev = None if device is None else torch.device(device)
+        # the tables of conicplus / legsurf ops are uploaded in one piece, kept here, and each segment's op carries the
+        # device address of its own (16-byte aligned)
+        tpos = [k for k, (c, _) in enumerate(programs[0].ops) if c in TABLE_SURFACE_OPS]
+        self._op_tables = None
+        if tpos:
+            if any(k not in prog._tables for prog in programs for k in tpos):
+                raise ValueError("a conicplus / legsurf op needs the table Program.conicplus / legsurf records")
+            if dev is None:
+                dev = torch.device("cuda", torch.cuda.current_device())
+            parts, offs = [], []
+            for prog in programs:
+                for k in tpos:
+                    t = prog._tables[k]
+                    offs.append(sum(p.numel() for p in parts))
+                    parts.append(torch.cat([t, torch.zeros(-t.numel() % 16, dtype=torch.uint8)]))
+            self._op_tables = torch.cat(parts).to(dev)
+            base = self._op_tables.data_ptr()
+            for j, off in enumerate(offs):
+                sgm, k = divmod(j, len(tpos))
+                arr[sgm * nops + tpos[k]].p[0] = struct.unpack("d", struct.pack("Q", base + off))[0]
         L = _lib.lib()
-        zpos = [k for k, (c, _) in enumerate(programs[0].ops) if c == OP["ZERNSURF"]]
+        zpos = [k for k, (c, _) in enumerate(programs[0].ops) if c in (OP["ZERNSURF"], OP["ZERNPHASE"])]
         lpos = [k for k, (c, _) in enumerate(programs[0].ops) if c == OP["LLSURF"]]
         if lpos:
             for p in programs:
@@ -541,8 +661,8 @@ class SegmentedProgram:
             kz = zpos[0]
             for p in programs:
                 if kz not in p._tables:
-                    raise ValueError("a zernsurf op needs the table Program.zernsurf records")
-                if p.ops[kz][1][1] != programs[0].ops[kz][1][1]:
+                    raise ValueError("a zernsurf / zernphase op needs the table Program.zernsurf / zernphase records")
+                if p.ops[kz][0] == OP["ZERNSURF"] and p.ops[kz][1][1] != programs[0].ops[kz][1][1]:
                     raise ValueError("every segment's zernsurf must give nr, or none may (tracezernOPD vs tracezern)")
             # one host table per segment, back to back (include/pxf.h, pxf_segmented_table_fill_zern)
             zt = torch.cat([p._tables[kz] for p in programs])
@@ -554,7 +674,8 @@ class SegmentedProgram:
             nbytes = int(L.pxf_segmented_table_bytes(nops, self.nseg))
             self.table_host = torch.empty(nbytes, dtype=torch.uint8)
             _lib.check(L.pxf_segmented_table_fill(arr, nops, self.nseg, start.ctypes.data, self.table_host.data_ptr()))
-        dev = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
+        if dev is None:
+            dev = torch.device("cuda", torch.cuda.current_device())
         self.table_dev = self.table_host.to(dev)
         self.seg_start_dev = torch.from_numpy(start).to(dev)
         self.segments = Segments._from(start, self.seg_start_dev)

@@ -23,7 +23,8 @@ from . import transformations as tran
 from . import woltsurf as wolt
 from . import zernsurf as zern
 from .analyses import analyticImagePlane, analyticXPlane, analyticYPlane
-from .program import LL_MAX_OPS, LL_MAX_ORDER, OP, SURFACE_OPS, flush, recorder_for
+from .program import (CONICPLUS_MAX_TERMS, LEGSURF_MAX_ORDER, LEGSURF_MAX_TERMS, LL_MAX_OPS, LL_MAX_ORDER, OP,
+                      SURFACE_OPS, ZERN_MAX_ORDER, flush, recorder_for)
 
 
 def flat(rays, ind=None, nr=None):
@@ -57,8 +58,7 @@ def zernsurf(rays, coeff, rad, rorder=None, aorder=None, nr=None):
         raise NotImplementedError("pass rorder/aorder explicitly: the reference's default ordering lives in "
                                   "the third-party module utilities.imaging.zernikemod (not vendored)")
     prog = recorder_for(rays)
-    if prog is not None and np.max(np.asarray(rorder)) <= 7 and not any(c in (OP["ZERNSURF"], OP["LLSURF"]) + SURFACE_OPS
-                                                                        for c, _ in prog.ops):
+    if _zernsurf_recorder(prog, rorder):
         prog.zernsurf(coeff, rorder, aorder, rad, nr)       # radial orders <= 7: stays in the fused program
         return
     flush(rays)
@@ -209,6 +209,12 @@ def spoSecondary(rays, R0, F, d=.605, ind=None):
     return
 
 
+def _zernsurf_recorder(prog, *rorders):
+    """Whether ``prog`` (a recording program or None) can hold one more Zernike surface of these radial orders."""
+    return (prog is not None and max(np.max(np.asarray(r)) for r in rorders) <= ZERN_MAX_ORDER and
+            not any(c in (OP["ZERNSURF"], OP["LLSURF"], OP["ZERNPHASE"]) + SURFACE_OPS for c, _ in prog.ops))
+
+
 def _surface_recorder(rays):
     """The program recording for ``rays`` when it can hold one of the remaining scalar surfaces (sphere, cylinder,
     cylconic, paraxial lenses, torus, W-S back surfaces: no Zernike surface, LL shell or grating fan in it), else None."""
@@ -231,7 +237,7 @@ def _ll_recorder(rays, coeff, axial, az):
         ok = False
     codes = [code for code, _ in prog.ops]
     if not ok or codes.count(OP["LLSURF"]) >= LL_MAX_OPS or any(
-            code in codes for code in (OP["ZERNSURF"], OP["GRATFAN"], OP["ROTX_REMAINING"]) + SURFACE_OPS):
+            code in codes for code in (OP["ZERNSURF"], OP["ZERNPHASE"], OP["GRATFAN"], OP["ROTX_REMAINING"]) + SURFACE_OPS):
         return None
     return prog
 
@@ -367,6 +373,11 @@ def zernphase(rays, coeff, rad, wave, rorder=None, aorder=None):
     """Zernike phase surface: wavelength in mm, radius in mm, coeff in mm."""
     opd, x, y, z, l, m, n, ux, uy, uz = rays
     _need_orders(rorder, aorder)
+    prog = recorder_for(rays)
+    if (prog is not None and np.max(np.asarray(rorder)) <= ZERN_MAX_ORDER and prog.can_hold_surface()
+            and not any(c in SURFACE_OPS for c, _ in prog.ops)):
+        prog.zernphase(coeff, rorder, aorder, rad, wave)    # radial orders <= 7: stays in the fused program
+        return
     flush(rays)
     zern.zernphase(opd, x, y, z, l, m, n, ux, uy, uz, coeff, np.array(rorder), np.array(aorder), rad, wave)
     return
@@ -377,6 +388,10 @@ def zernsurfrot(rays, coeff1, coeff2, rad, rot, rorder1=None, aorder1=None, rord
     opd, x, y, z, l, m, n, ux, uy, uz = rays
     _need_orders(rorder1, aorder1)
     _need_orders(rorder2, aorder2)
+    prog = recorder_for(rays)
+    if _zernsurf_recorder(prog, rorder1, rorder2):
+        prog.tracezernrot(coeff1, rorder1, aorder1, coeff2, rorder2, aorder2, rad, rot)
+        return
     flush(rays)
     zern.tracezernrot(x, y, z, l, m, n, ux, uy, uz, coeff1, np.array(rorder1), np.array(aorder1),
                       coeff2, np.array(rorder2), np.array(aorder2), rad, rot)
@@ -412,6 +427,13 @@ def tanSphere(rays, rad, nr=None):
 def conicplus(rays, R, K, p, nr=None):
     """Conic of curvature radius R and conic constant K plus even polynomial terms p."""
     opd, x, y, z, l, m, n, ux, uy, uz = rays
+    prog = _surface_recorder(rays)
+    if prog is not None and np.size(p) <= CONICPLUS_MAX_TERMS:
+        if nr is not None:
+            prog.conicplusopd(R, K, p, nr)
+        else:
+            prog.conicplus(R, K, p)
+        return
     flush(rays)
     if nr is not None:
         surf.conicplusopd(opd, x, y, z, l, m, n, ux, uy, uz, R, K, p, nr)
@@ -500,10 +522,23 @@ def paraxialY(rays, F):
 def legSurf(rays, xwidth, ywidth, order, coeff, xo, yo):
     """Diffract from a phase surface given by 2-D Legendre coefficients (rays already on the xy plane)."""
     x, y, z, l, m, n, ux, uy, uz = rays[1:]
+    prog = _surface_recorder(rays)
+    if prog is not None and _legsurf_terms_ok(coeff, xo, yo):
+        prog.legsurf(xwidth, ywidth, order, coeff, xo, yo)
+        return
     flush(rays)
     surf.legsurf(x, y, z, l, m, n, ux, uy, uz, xwidth, ywidth, order,
                  np.asarray(coeff).flatten(), np.asarray(xo).flatten(), np.asarray(yo).flatten())
     return
+
+
+def _legsurf_terms_ok(coeff, xo, yo):
+    """Whether the term list is one the table fill takes (else the stand-alone routine reports the error)."""
+    c, a, b = (np.asarray(v).ravel() for v in (coeff, xo, yo))
+    if c.shape != a.shape or c.shape != b.shape or c.shape[0] > LEGSURF_MAX_TERMS:
+        return False
+    orders = np.concatenate([a, b]).astype(np.int32)
+    return orders.size == 0 or (orders.min() >= 0 and orders.max() <= LEGSURF_MAX_ORDER)
 
 
 # The reference's three tangent-plane placements still use its pre-`rays` module-global call style
