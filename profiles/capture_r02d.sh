@@ -1,9 +1,6 @@
 #!/bin/bash
-# r02d: parity of the rewritten LL / Zernike / W-S clamp paths, their launch variants, then the captures
+# r02d: parity of the rewritten LL / Zernike / W-S clamp paths, then the captures
 O=gpurun_out; mkdir -p $O
 timeout 900 python -m pytest tests -m gpu -q -x -k "legendre or zern or ws or golden or fused or surfaces or config" > $O/r02d_gputest.log 2>&1; echo "pytest rc=$?" >> $O/r02d_gputest.log
 tail -3 $O/r02d_gputest.log
-for v in 0 1 2 3 4; do echo "PXF_ZERN_VARIANT=$v"; PXF_ZERN_VARIANT=$v python profiles/routine_probe.py tracezern 5e7 4; done > $O/r02d_variants.txt 2>&1
-for v in 0 1 2 3; do echo "PXF_LL_VARIANT=$v"; PXF_LL_VARIANT=$v python profiles/routine_probe.py wolterprimll 5e7 4; done >> $O/r02d_variants.txt 2>&1
-cat $O/r02d_variants.txt
 bash profiles/capture_routines.sh r02d

@@ -1,11 +1,7 @@
 #!/bin/bash
-# r02k: one-sweep sort tile-shape sweep (PXF_SORT_VARIANT), parity on the default
+# r02k: one-sweep sort parity and timing
 O=gpurun_out; mkdir -p $O
 timeout 900 python -m pytest tests/test_gpu_parity.py -m gpu -q -k "sort or weighted" > $O/r02k_gputest.log 2>&1; echo "pytest rc=$?" >> $O/r02k_gputest.log
 tail -4 $O/r02k_gputest.log
-for v in 0 1 2 3 4; do
-  echo "== PXF_SORT_VARIANT=$v" >> $O/r02k_sort_variants.txt
-  PXF_SORT_VARIANT=$v timeout 300 python profiles/sort_probe.py 5e7 4 >> $O/r02k_sort_variants.txt 2>&1
-done
-PXF_SORT_VARIANT=0 timeout 300 python profiles/sort_probe.py 2e8 3 >> $O/r02k_sort_variants.txt 2>&1
-cat $O/r02k_sort_variants.txt
+timeout 300 python profiles/sort_probe.py 2e8 3 > $O/r02k_sort.txt 2>&1
+cat $O/r02k_sort.txt

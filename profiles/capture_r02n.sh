@@ -1,10 +1,5 @@
 #!/bin/bash
-# r02n: sort after the full-tile fast path: parity, timing of variants 0/4
+# r02n: sort after the full-tile fast path: parity
 O=gpurun_out; mkdir -p $O; rm -f $O/r02n_sort_variants.txt
 timeout 900 python -m pytest tests/test_gpu_parity.py -m gpu -q -k "sort or weighted" > $O/r02n_gputest.log 2>&1; echo "pytest rc=$?" >> $O/r02n_gputest.log
 tail -4 $O/r02n_gputest.log
-for v in 0 4 1; do
-  echo "== PXF_SORT_VARIANT=$v" >> $O/r02n_sort_variants.txt
-  PXF_SORT_VARIANT=$v timeout 300 python profiles/sort_probe.py 5e7 4 >> $O/r02n_sort_variants.txt 2>&1
-done
-grep -v "call [01]:" $O/r02n_sort_variants.txt

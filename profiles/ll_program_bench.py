@@ -8,7 +8,7 @@ Workloads (same seeded inputs for both paths; every timing ends in a device sync
      five-launch sequence that ``fused`` ran before LL ops existed (transform | wolterprimll | reflect | woltersecll |
      reflect + flat) against ONE Program.run.  The first launch of the sequence and the program read the source
      bundle and write a second one, so every repetition does the same work; the results are compared bit for bit.
-     The interpreter (PXF_JIT=0) is timed in child processes for each register cap PXF_LLPROG_MINB = 1..4.
+     The interpreter (PXF_JIT=0, registers capped for 1 CTA/SM) is timed once, in a child process.
   M  figure-error Monte Carlo: 1000 realisations x 1e5 rays (36 terms per mirror), trace + hpd + rmsCentroid each.
      The loop of examples.llpair_fast against examples.ll_tolerance_fast; ray counts and hpd / rms are compared.
 Each entry reports the median and the spread (min, max) of R repetitions in ms, rays/s at the median, the libpxf
@@ -72,18 +72,14 @@ def trace(pxf, num, reps, with_routines=True):
     return {"rays": num, "cases": [pair_case(pxf, src, out, work, order, reps, with_routines) for order in (5, 3, 7)]}
 
 
-def interpreter_caps(scale, reps):
-    """P with the interpreter only, one child process per register cap (the caps are read once per process)."""
-    res = {}
-    for minb in (1, 2, 3, 4):
-        env = dict(os.environ, PXF_JIT="0", PXF_LLPROG_MINB=str(minb))
-        p = subprocess.run([sys.executable, os.path.abspath(__file__), "--child-interp", "--scale", str(scale),
-                            "--reps", str(reps)], env=env, capture_output=True, text=True, timeout=3000)
-        if p.returncode != 0:
-            res[str(minb)] = {"error": p.stderr[-2000:]}
-            continue
-        res[str(minb)] = json.loads(p.stdout.strip().splitlines()[-1])
-    return res
+def interpreter(scale, reps):
+    """P with the interpreter only, in a child process (PXF_JIT is read once per process)."""
+    env = dict(os.environ, PXF_JIT="0")
+    p = subprocess.run([sys.executable, os.path.abspath(__file__), "--child-interp", "--scale", str(scale),
+                        "--reps", str(reps)], env=env, capture_output=True, text=True, timeout=3000)
+    if p.returncode != 0:
+        return {"error": p.stderr[-2000:]}
+    return json.loads(p.stdout.strip().splitlines()[-1])
 
 
 def montecarlo(pxf, K, n, reps_loop, reps_seg):
@@ -124,12 +120,11 @@ def main():
     torch.cuda.set_device(0)
     if a.child_interp:
         r = trace(pxf, int(5e7 * a.scale), a.reps, with_routines=False)
-        print(json.dumps({"PXF_LLPROG_MINB": os.environ.get("PXF_LLPROG_MINB"),
-                          "cases": [{"max_order": c["max_order"], **c["program"]} for c in r["cases"]]}))
+        print(json.dumps({"cases": [{"max_order": c["max_order"], **c["program"]} for c in r["cases"]]}))
         return
     res = {"info": device_info()}
     res["P_trace"] = trace(pxf, int(5e7 * a.scale), a.reps)
-    res["P_interpreter_by_register_cap"] = interpreter_caps(a.scale, a.reps)
+    res["P_interpreter"] = interpreter(a.scale, a.reps)
     res["M_montecarlo"] = montecarlo(pxf, 1000, int(1e5 * a.scale), max(3, a.reps // 2), a.reps)
     res["jit_status"] = pxf.jit_status()
     txt = json.dumps(res, indent=1)

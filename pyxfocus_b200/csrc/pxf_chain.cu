@@ -36,17 +36,20 @@ template <class Op, class... Rest> struct ChainHost<Op, Rest...> {
 };
 
 // ---- kernel -------------------------------------------------------------------------------
-// MODE 1: one ray per thread-iteration (8-byte accesses, also the path for unaligned rows)
+// MODE 1: one ray per thread-iteration (8-byte accesses, the path for unaligned rows)
 // MODE 2: two rays per thread-iteration (double2 accesses), traced one after the other
-// PF    : software prefetch -- the loads of the NEXT iteration are issued before the current
-//         rays are traced, so every warp keeps ~1.5-3 KB of loads in flight during its compute
+// PF    : (MODE 1) software prefetch -- the loads of the NEXT iteration are issued before the current
+//         ray is traced, so every warp keeps ~1.5-3 KB of loads in flight during its compute
 //         phase.  Without it the kernel is limited by bytes in flight: a warp is either waiting
 //         for its loads or computing, and with ~70 % of the time spent computing too few loads
 //         are outstanding to keep HBM busy (measured: 4.1 ms vs 2.6 ms for the same traffic
 //         with trivial compute, profiles/r01_notes.md).
 // LMc/SMc: row masks known at compile time (0 = use the runtime masks LM/SM), so that rows the
 //         chain never loads cost no registers in the prefetch buffer.
-// MINB  : resident CTAs per SM the register allocation must allow.
+// Registers are capped for 3 resident CTAs per SM.  Tuned on B200 (profiles/r01_notes.md): on aligned rows two
+// rays in sequence, 3 CTAs/SM, no prefetch is the fastest shape; a bulk-async variant that streams the rows
+// into a shared-memory ring (cp.async.bulk, one producer thread) removes every load stall and is no faster.
+#define CHAIN_MINB 3
 template <unsigned M>
 PXF_DEV void cload1(Ray &r, const RowPtrs &P, unsigned LM, int64_t i)
 {
@@ -77,8 +80,8 @@ PXF_DEV void cstore2(const Ray &a, const Ray &b, const RowPtrs &P, unsigned SM, 
     fstore2(a, b, P, M ? M : SM, i);
 }
 
-template <class C, class CP, int MODE, bool PF, int MINB, unsigned LMc, unsigned SMc>
-__global__ void __launch_bounds__(PXF_BLOCK, MINB)
+template <class C, class CP, int MODE, bool PF, unsigned LMc, unsigned SMc>
+__global__ void __launch_bounds__(PXF_BLOCK, CHAIN_MINB)
 k_chain(const RowPtrs P, const RowPtrs Q, const int64_t num, uint8_t *__restrict__ alive,
         double *__restrict__ partials, const unsigned LM, const unsigned SM, const __grid_constant__ CP prm)
 {
@@ -88,22 +91,16 @@ k_chain(const RowPtrs P, const RowPtrs Q, const int64_t num, uint8_t *__restrict
     if (MODE >= 2) {
         const int64_t npair = num >> 1;
         int64_t q = tid;
-        Ray cur[2], nxt[2];
-        if (PF && q < npair) cload2<LMc>(cur[0], cur[1], P, LM, q << 1);
+        Ray cur[2];
         while (q < npair) {
             const int64_t qn = q + nthr;
-            if (PF) {
-                if (qn < npair) cload2<LMc>(nxt[0], nxt[1], P, LM, qn << 1);
-            } else {
-                cload2<LMc>(cur[0], cur[1], P, LM, q << 1);
-            }
+            cload2<LMc>(cur[0], cur[1], P, LM, q << 1);
             C::run(cur[0], prm);
             C::run(cur[1], prm);
             const int64_t i = q << 1;
             cstore2<SMc>(cur[0], cur[1], Q, SM, i);
             if (alive) { alive[i] = 1; alive[i + 1] = 1; }
             cnt += 2.; sx += cur[0].x; sx += cur[1].x; sy += cur[0].y; sy += cur[1].y;
-            if (PF) { cur[0] = nxt[0]; cur[1] = nxt[1]; }
             q = qn;
         }
         if ((num & 1) && tid == 0) {
@@ -137,172 +134,17 @@ k_chain(const RowPtrs P, const RowPtrs Q, const int64_t num, uint8_t *__restrict
     if (partials) centroid_block_reduce(cnt, sx, sy, partials);
 }
 
-// ---- bulk-async (TMA) pipelined variant ------------------------------------------------------
-// The register-file variants above are limited by bytes in flight: a warp either waits for its
-// own loads or computes, and with ~70 % of its time in the fp64 Newton loops too few loads are
-// outstanding to keep HBM busy -- memory time and compute time ADD (2.6 ms + 1.6 ms measured)
-// instead of overlapping.  Here the loads are decoupled from the warps: one elected thread per CTA
-// streams 256-ray tiles of the live-in rows into an NST-deep shared-memory ring with 1-D bulk
-// copies (cp.async.bulk, completion on an mbarrier), NST-1 tiles ahead of the compute, so the
-// bytes in flight per SM are CTAs x (NST-1) x rows x 2 KB whatever the warps are doing.  Each
-// thread then traces ONE ray (lowest register pressure => more resident warps for the fp64 pipe)
-// and stores its rows directly (stores do not stall the issuing warp).
-PXF_DEV uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
-PXF_DEV void mbar_init(uint32_t bar, uint32_t count)
-{
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count) : "memory");
-}
-PXF_DEV void mbar_expect_tx(uint32_t bar, uint32_t bytes)
-{
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-PXF_DEV void mbar_arrive(uint32_t bar)
-{
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
-}
-PXF_DEV void mbar_wait(uint32_t bar, uint32_t parity)
-{
-    uint32_t done;
-    do {
-        asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-                     "selp.u32 %0, 1, 0, p;\n\t}"
-                     : "=r"(done) : "r"(bar), "r"(parity) : "memory");
-    } while (!done);
-}
-PXF_DEV void bulk_g2s(uint32_t dst, const void *src, uint32_t bytes, uint32_t bar)
-{
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                 ::"r"(dst), "l"(src), "r"(bytes), "r"(bar) : "memory");
-}
-
-template <class C, class CP, int NST, int MINB, unsigned LMc, unsigned SMc>
-__global__ void __launch_bounds__(PXF_BLOCK, MINB)
-k_chain_tma(const RowPtrs P, const RowPtrs Q, const int64_t num, uint8_t *__restrict__ alive,
-            double *__restrict__ partials, const unsigned LM, const unsigned SM, const __grid_constant__ CP prm)
-{
-    extern __shared__ __align__(128) unsigned char ring_raw[];
-    const unsigned lm = LMc ? LMc : LM;
-    const int nrow = __popc(lm);
-    const uint32_t stage_bytes = (uint32_t)nrow * PXF_BLOCK * 8u;
-    double *ring = reinterpret_cast<double *>(ring_raw);                        // [NST][nrow][PXF_BLOCK]
-    const uint32_t ring_s = smem_u32(ring_raw);
-    const uint32_t bar_s = ring_s + NST * stage_bytes;                          // full[NST], empty[NST]
-    const int lane = threadIdx.x & 31;
-    const int64_t ntile = num / PXF_BLOCK;                                      // full tiles only
-    const int64_t mine = ntile > blockIdx.x ? (ntile - blockIdx.x + gridDim.x - 1) / gridDim.x : 0;
-
-    if (threadIdx.x == 0) {
-        for (int s = 0; s < NST; s++) {
-            mbar_init(bar_s + 8u * s, 1);
-            mbar_init(bar_s + 8u * (NST + s), PXF_BLOCK / 32);
-        }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    __syncthreads();
-
-    auto issue = [&](int64_t k) {
-        const int s = (int)(k % NST);
-        const int64_t base = ((int64_t)blockIdx.x + k * gridDim.x) * PXF_BLOCK;
-        const uint32_t full = bar_s + 8u * s;
-        mbar_expect_tx(full, stage_bytes);
-        uint32_t dst = ring_s + s * stage_bytes;
-#pragma unroll
-        for (int r = 0; r < 10; r++)
-            if ((lm >> r) & 1u) {
-                bulk_g2s(dst, P.p[r] + base, PXF_BLOCK * 8u, full);
-                dst += PXF_BLOCK * 8u;
-            }
-    };
-    if (threadIdx.x == 0)
-        for (int64_t k = 0; k < NST && k < mine; k++) issue(k);
-
-    double cnt = 0., sx = 0., sy = 0.;
-    for (int64_t k = 0; k < mine; k++) {
-        const int s = (int)(k % NST);
-        // refill the stage every warp finished reading one tile ago
-        if (threadIdx.x == 0 && k >= 1 && k - 1 + NST < mine) {
-            mbar_wait(bar_s + 8u * (NST + (int)((k - 1) % NST)), (uint32_t)(((k - 1) / NST) & 1));
-            issue(k - 1 + NST);
-        }
-        __syncwarp();
-        mbar_wait(bar_s + 8u * s, (uint32_t)((k / NST) & 1));
-        const double *st = ring + (size_t)s * nrow * PXF_BLOCK + threadIdx.x;
-        Ray r;
-        {
-            double v[10];
-            int slot = 0;
-#pragma unroll
-            for (int q = 0; q < 10; q++) {
-                v[q] = 0.;
-                if ((lm >> q) & 1u) { v[q] = st[slot * PXF_BLOCK]; slot++; }
-            }
-            r.opd = v[0]; r.x = v[1]; r.y = v[2]; r.z = v[3]; r.l = v[4]; r.m = v[5]; r.n = v[6];
-            r.ux = v[7]; r.uy = v[8]; r.uz = v[9];
-        }
-        __syncwarp();
-        if (lane == 0) mbar_arrive(bar_s + 8u * (NST + s));
-        const int64_t i = ((int64_t)blockIdx.x + k * gridDim.x) * PXF_BLOCK + threadIdx.x;
-        const bool ka = C::run(r, prm);
-        cstore1<SMc>(r, Q, SM, i);
-        if (alive) alive[i] = ka ? 1 : 0;
-        if (ka) { cnt += 1.; sx += r.x; sy += r.y; }
-    }
-    // ragged tail (< one tile): plain loads, by the CTA whose turn it would be
-    const int64_t rem = num - ntile * PXF_BLOCK;
-    if (rem > 0 && blockIdx.x == (unsigned)(ntile % gridDim.x) && threadIdx.x < rem) {
-        const int64_t i = ntile * PXF_BLOCK + threadIdx.x;
-        Ray r;
-        cload1<LMc>(r, P, LM, i);
-        const bool ka = C::run(r, prm);
-        cstore1<SMc>(r, Q, SM, i);
-        if (alive) alive[i] = ka ? 1 : 0;
-        if (ka) { cnt += 1.; sx += r.x; sy += r.y; }
-    }
-    if (partials) centroid_block_reduce(cnt, sx, sy, partials);
-}
-
-template <class C, class CP, int NST, int MINB, unsigned LMc, unsigned SMc>
-static int launch_tma(const RowPtrs &P, const RowPtrs &Q, int64_t num, uint8_t *alive, unsigned LM, unsigned SM,
-                      const CP &cp, cudaStream_t s, double *partials, int *grid_out)
-{
-    static int ctas = 0;
-    auto kern = k_chain_tma<C, CP, NST, MINB, LMc, SMc>;
-    const unsigned lm = LMc ? LMc : LM;
-    int nrow = 0;
-    for (int r = 0; r < 10; r++) nrow += (lm >> r) & 1u;
-    const size_t smem = (size_t)NST * nrow * PXF_BLOCK * 8 + 2 * NST * 8;
-    static bool seen[64] = {};
-    if (first_on_device(seen) || ctas == 0 || LMc == 0) {
-        // (runtime masks: the ring size depends on the live rows, so re-query; the attribute is per device)
-        if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 10 * NST * PXF_BLOCK * 8 + 2 * NST * 8) != cudaSuccess) {
-            cudaGetLastError();
-            return PXF_ERR_UNSUPPORTED;
-        }
-        int nb = 0;
-        if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, kern, PXF_BLOCK, smem) != cudaSuccess || nb <= 0) {
-            cudaGetLastError();
-            return PXF_ERR_UNSUPPORTED;
-        }
-        ctas = nb;
-    }
-    const int grid = grid_for(num, PXF_BLOCK, ctas);
-    if (grid_out) *grid_out = grid;
-    kern<<<grid, PXF_BLOCK, smem, s>>>(P, Q, num, alive, partials, LM, SM, cp);
-    count_launch();
-    return check_launch("k_chain_tma");
-}
-
-template <class C, class CP, int MODE, bool PF, int MINB, unsigned LMc, unsigned SMc>
-static int launch_variant(const RowPtrs &P, const RowPtrs &Q, int64_t num, uint8_t *alive, unsigned LM, unsigned SM,
+template <class C, class CP, int MODE, bool PF, unsigned LMc, unsigned SMc>
+static int launch_k_chain(const RowPtrs &P, const RowPtrs &Q, int64_t num, uint8_t *alive, unsigned LM, unsigned SM,
                           const CP &cp, cudaStream_t s, double *partials, int *grid_out)
 {
     static int ctas = 0;
-    auto kern = k_chain<C, CP, MODE, PF, MINB, LMc, SMc>;
+    auto kern = k_chain<C, CP, MODE, PF, LMc, SMc>;
     if (ctas == 0) {
         int nb = 0;
         if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, kern, PXF_BLOCK, 0) != cudaSuccess || nb <= 0) {
             cudaGetLastError();
-            nb = MINB;
+            nb = CHAIN_MINB;
         }
         ctas = nb;
     }
@@ -314,21 +156,9 @@ static int launch_variant(const RowPtrs &P, const RowPtrs &Q, int64_t num, uint8
     return check_launch("k_chain");
 }
 
-// PXF_CHAIN_VARIANT=<mode><minb><pf> (e.g. 231 = two rays in sequence, 3 CTAs/SM, prefetch)
-// overrides the tuned default of the tunable chain; for tuning only.
-static int variant_override()
-{
-    static int v = -1;
-    if (v < 0) {
-        const char *e = getenv("PXF_CHAIN_VARIANT");
-        v = e ? atoi(e) : 0;
-    }
-    return v;
-}
-
 // LMc/SMc: the row masks this chain has when traced in place or out of place (checked against
 // build_program's liveness result at run time; any other masks take the runtime-mask kernel).
-template <bool TUNABLE, unsigned LMc, unsigned SMc, class... Ops>
+template <unsigned LMc, unsigned SMc, class... Ops>
 static int try_chain(const RowPtrs &P, const RowPtrs &Q, int64_t num, const FusedProgram &fp, uint8_t *alive,
                      bool aligned, cudaStream_t s, double *partials, int *grid_out)
 {
@@ -339,43 +169,20 @@ static int try_chain(const RowPtrs &P, const RowPtrs &Q, int64_t num, const Fuse
     memset(&cp, 0, sizeof(cp));
     ChainHost<Ops...>::fill(cp, fp.ops);
     const unsigned LM = fp.load_mask, SM = fp.store_mask;
-    const bool stat = LMc != 0 && LM == LMc && SM == SMc;
-#define PXF_LV(MODE, PF, MINB)                                                                              \
-    (stat ? launch_variant<C, CP, MODE, PF, MINB, LMc, SMc>(P, Q, num, alive, LM, SM, cp, s, partials, grid_out) \
-          : launch_variant<C, CP, MODE, false, MINB, 0u, 0u>(P, Q, num, alive, LM, SM, cp, s, partials, grid_out))
-#define PXF_TV(NST, MINB)                                                                                  \
-    (stat ? launch_tma<C, CP, NST, MINB, LMc, SMc>(P, Q, num, alive, LM, SM, cp, s, partials, grid_out)     \
-          : launch_tma<C, CP, NST, MINB, 0u, 0u>(P, Q, num, alive, LM, SM, cp, s, partials, grid_out))
     {
         std::string nm = "k_chain<Chain<";
         const char *names[] = {Ops::NAME...};
         for (size_t k = 0; k < sizeof...(Ops); k++) { if (k) nm += ", "; nm += names[k]; }
         note_kernel((nm + ">> (built into libpxf)").c_str());
     }
-    if (!aligned) return PXF_LV(1, true, 3);
-    if constexpr (TUNABLE) {
-        switch (variant_override()) {
-            case 432: return PXF_TV(2, 3);
-            case 433: return PXF_TV(3, 3);
-            case 434: return PXF_TV(4, 3);
-            case 442: return PXF_TV(2, 4);
-            case 443: return PXF_TV(3, 4);
-            case 444: return PXF_TV(4, 4);
-            case 446: return PXF_TV(6, 4);
-            case 453: return PXF_TV(3, 5);
-            case 130: return PXF_LV(1, false, 3);
-            case 131: return PXF_LV(1, true, 3);
-            case 141: return PXF_LV(1, true, 4);
-            case 220: return PXF_LV(2, false, 2);
-            case 221: return PXF_LV(2, true, 2);
-            case 230: return PXF_LV(2, false, 3);
-            case 231: return PXF_LV(2, true, 3);
-            default: break;
+    if constexpr (LMc != 0) {
+        if (LM == LMc && SM == SMc) {
+            if (!aligned) return launch_k_chain<C, CP, 1, true, LMc, SMc>(P, Q, num, alive, LM, SM, cp, s, partials, grid_out);
+            return launch_k_chain<C, CP, 2, false, LMc, SMc>(P, Q, num, alive, LM, SM, cp, s, partials, grid_out);
         }
     }
-    return PXF_LV(2, false, 3);      // tuned on B200 (profiles/r01_notes.md): two rays in sequence, 3 CTAs/SM, no prefetch
-#undef PXF_LV
-#undef PXF_TV
+    if (!aligned) return launch_k_chain<C, CP, 1, false, 0u, 0u>(P, Q, num, alive, LM, SM, cp, s, partials, grid_out);
+    return launch_k_chain<C, CP, 2, false, 0u, 0u>(P, Q, num, alive, LM, SM, cp, s, partials, grid_out);
 }
 
 int launch_chain(const RowPtrs &P, const RowPtrs &Q, int64_t num, const FusedProgram &fp, uint8_t *alive,
@@ -389,29 +196,31 @@ int launch_chain(const RowPtrs &P, const RowPtrs &Q, int64_t num, const FusedPro
     if (disabled || fp.has_vignette) return PXF_ERR_UNSUPPORTED;
     int rc;
     // Wolter-I pair to the focal plane (BASELINE config 1)
-    rc = try_chain<true, (R_POS | R_DIR), R_NINE, CTransform, CWolterPrimary, CReflect, CWolterSecondary, CReflect, CFlat>(P, Q, num, fp, alive, aligned, s, partials, grid_out);
+    rc = try_chain<(R_POS | R_DIR), R_NINE, CTransform, CWolterPrimary, CReflect, CWolterSecondary, CReflect, CFlat>(P, Q, num, fp, alive, aligned, s, partials, grid_out);
     if (rc != PXF_ERR_UNSUPPORTED) return rc;
-    rc = try_chain<false, 0u, 0u, CWolterPrimary, CReflect, CWolterSecondary, CReflect, CFlat>(P, Q, num, fp, alive, aligned, s, partials, grid_out);
+    rc = try_chain<0u, 0u, CWolterPrimary, CReflect, CWolterSecondary, CReflect, CFlat>(P, Q, num, fp, alive, aligned, s, partials, grid_out);
     if (rc != PXF_ERR_UNSUPPORTED) return rc;
-    rc = try_chain<false, 0u, 0u, CTransform, CWolterPrimary, CReflect, CWolterSecondary, CReflect>(P, Q, num, fp, alive, aligned, s, partials, grid_out);
+    rc = try_chain<0u, 0u, CTransform, CWolterPrimary, CReflect, CWolterSecondary, CReflect>(P, Q, num, fp, alive, aligned, s, partials, grid_out);
     if (rc != PXF_ERR_UNSUPPORTED) return rc;
     // Wolter-Schwarzschild pair with the field-angle kick (BASELINE config 2)
-    rc = try_chain<false, 0u, 0u, CTransform, CWsPrimary, CKick, CReflect, CWsSecondary, CReflect>(P, Q, num, fp, alive, aligned, s, partials, grid_out);
+    rc = try_chain<0u, 0u, CTransform, CWsPrimary, CKick, CReflect, CWsSecondary, CReflect>(P, Q, num, fp, alive, aligned, s, partials, grid_out);
     if (rc != PXF_ERR_UNSUPPORTED) return rc;
     // SPO primary/secondary pair (BASELINE config 4, per-shell part)
-    rc = try_chain<false, 0u, 0u, CTransform, CSpoCone, CReflect, CSpoCone, CReflect, CTransform>(P, Q, num, fp, alive, aligned, s, partials, grid_out);
+    rc = try_chain<0u, 0u, CTransform, CSpoCone, CReflect, CSpoCone, CReflect, CTransform>(P, Q, num, fp, alive, aligned, s, partials, grid_out);
     if (rc != PXF_ERR_UNSUPPORTED) return rc;
     // focus step: move the plane and trace to it (surfaces.focus, surfaces.py:502-510)
-    rc = try_chain<false, 0u, 0u, CTransform, CFlat>(P, Q, num, fp, alive, aligned, s, partials, grid_out);
+    rc = try_chain<0u, 0u, CTransform, CFlat>(P, Q, num, fp, alive, aligned, s, partials, grid_out);
     return rc;
 }
 
 // ---- segmented specialised chain (nested assemblies) --------------------------------------------
 // Same tiling as k_program_seg (pxf_fused.cu) with the op list known at compile time: the per-segment
 // parameter pack ChainP (not an op table) is staged in shared memory and the chain runs straight-line.
+// Registers capped for 4 resident CTAs per SM: measured at 2e7 rays, 260 shells, caps 2 / 3 / 4 / 5: 0.92 / 0.78 /
+// 0.72 / 0.76 ms.
 #define CSEG_TILE (PXF_BLOCK * 8)
-template <class C, class CP, int MINB>
-__global__ void __launch_bounds__(PXF_BLOCK, MINB)
+template <class C, class CP>
+__global__ void __launch_bounds__(PXF_BLOCK, 4)
 k_chain_seg(const RowPtrs P, const RowPtrs Q, const int64_t num, uint8_t *__restrict__ alive,
             const long long *__restrict__ seg_start, const CP *__restrict__ table, const int nseg,
             const unsigned LM, const unsigned SM)
@@ -482,19 +291,11 @@ int seg_chain_launch(int chain_id, const RowPtrs &P, const RowPtrs &Q, int64_t n
                      cudaStream_t s)
 {
     if (chain_id != 1) return PXF_ERR_UNSUPPORTED;
-    // PXF_SEG_MINB (tuning): resident CTAs per SM the register allocation is capped for
-    static int minb = -1;
-    if (minb < 0) { const char *e = getenv("PXF_SEG_MINB"); minb = e ? atoi(e) : 4; }    // measured at 2e7 rays, 260 shells: 0.92 / 0.78 / 0.72 / 0.76 ms for 2 / 3 / 4 / 5
-    auto go = [&](auto kern) {
-        int nb = 0;
-        if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, kern, PXF_BLOCK, 0) != cudaSuccess || nb <= 0) { cudaGetLastError(); nb = 3; }
-        const int grid = grid_for(num, CSEG_TILE, nb);
-        kern<<<grid, PXF_BLOCK, 0, s>>>(P, Q, num, alive, seg_start_dev, static_cast<const SegWolterP *>(table_dev), nseg, LM, SM);
-    };
-    if (minb == 2) go(k_chain_seg<SegWolter, SegWolterP, 2>);
-    else if (minb == 3) go(k_chain_seg<SegWolter, SegWolterP, 3>);
-    else if (minb == 5) go(k_chain_seg<SegWolter, SegWolterP, 5>);
-    else go(k_chain_seg<SegWolter, SegWolterP, 4>);
+    auto kern = k_chain_seg<SegWolter, SegWolterP>;
+    int nb = 0;
+    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, kern, PXF_BLOCK, 0) != cudaSuccess || nb <= 0) { cudaGetLastError(); nb = 3; }
+    const int grid = grid_for(num, CSEG_TILE, nb);
+    kern<<<grid, PXF_BLOCK, 0, s>>>(P, Q, num, alive, seg_start_dev, static_cast<const SegWolterP *>(table_dev), nseg, LM, SM);
     count_launch();
     note_kernel("k_chain_seg<Chain<CTransform,CWolterPrimary,CReflect,CWolterSecondary,CReflect,CFlat>>");
     return check_launch("k_chain_seg");

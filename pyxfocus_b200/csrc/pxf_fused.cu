@@ -3,7 +3,6 @@
 // device code as the per-routine kernels (pxf_ray.cuh), so the result is bit-identical to
 // issuing the routines one by one.  Every ray runs the same program, so the opcode switch is
 // warp-uniform; only Newton trip counts and vignetting diverge.
-#include <stdlib.h>
 #include "pxf_program.h"
 
 namespace pxf {
@@ -165,8 +164,8 @@ PXF_DEV bool run_program(Ray &r, const FusedProgram &prog, const ZernP *zt = nul
     return true;
 }
 
-template <bool VEC2, int MINB = 1, bool ZERN = false, bool AUX = false, bool LL = false, bool SURF = false,
-          bool TAB = false, bool ZPH = false>
+template <int MINB, bool ZERN = false, bool AUX = false, bool LL = false, bool SURF = false, bool TAB = false,
+          bool ZPH = false>
 __global__ void __launch_bounds__(PXF_BLOCK, MINB)
 k_program(const RowPtrs P, const RowPtrs Q, const int64_t num, uint8_t *__restrict__ alive,
           double *__restrict__ partials, const __grid_constant__ FusedProgram prog)
@@ -196,37 +195,13 @@ k_program(const RowPtrs P, const RowPtrs Q, const int64_t num, uint8_t *__restri
     const unsigned LM = prog.load_mask, SM = prog.store_mask;
     const int64_t tid = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     const int64_t nthr = (int64_t)gridDim.x * blockDim.x;
-    if (VEC2) {
-        const int64_t npair = num >> 1;
-        for (int64_t q = tid; q < npair; q += nthr) {
-            const int64_t i = q << 1;
-            Ray a, b;
-            fload2(a, b, P, LM, i);
-            const bool ka = run_program<ZERN, AUX, LL, SURF, TAB, ZPH>(a, prog, zt, i, llt);
-            const bool kb = run_program<ZERN, AUX, LL, SURF, TAB, ZPH>(b, prog, zt, i + 1, llt);
-            fstore2(a, b, Q, SM, i);
-            if (alive) { alive[i] = ka ? 1 : 0; alive[i + 1] = kb ? 1 : 0; }
-            if (ka) { cnt += 1.; sx += a.x; sy += a.y; }
-            if (kb) { cnt += 1.; sx += b.x; sy += b.y; }
-        }
-        if ((num & 1) && tid == 0) {
-            const int64_t i = num - 1;
-            Ray a;
-            fload1(a, P, LM, i);
-            const bool ka = run_program<ZERN, AUX, LL, SURF, TAB, ZPH>(a, prog, zt, i, llt);
-            fstore1(a, Q, SM, i);
-            if (alive) alive[i] = ka ? 1 : 0;
-            if (ka) { cnt += 1.; sx += a.x; sy += a.y; }
-        }
-    } else {
-        for (int64_t i = tid; i < num; i += nthr) {
-            Ray a;
-            fload1(a, P, LM, i);
-            const bool ka = run_program<ZERN, AUX, LL, SURF, TAB, ZPH>(a, prog, zt, i, llt);
-            fstore1(a, Q, SM, i);
-            if (alive) alive[i] = ka ? 1 : 0;
-            if (ka) { cnt += 1.; sx += a.x; sy += a.y; }
-        }
+    for (int64_t i = tid; i < num; i += nthr) {
+        Ray a;
+        fload1(a, P, LM, i);
+        const bool ka = run_program<ZERN, AUX, LL, SURF, TAB, ZPH>(a, prog, zt, i, llt);
+        fstore1(a, Q, SM, i);
+        if (alive) alive[i] = ka ? 1 : 0;
+        if (ka) { cnt += 1.; sx += a.x; sy += a.y; }
     }
     if (partials) centroid_block_reduce(cnt, sx, sy, partials);
 }
@@ -252,7 +227,7 @@ static_assert(sizeof(LLTab) % 8 == 0, "per-segment LL tables are laid out back t
 // shared-memory offset of the staged Zernike or LL tables: behind the op table, 16-byte aligned
 __host__ __device__ __forceinline__ int seg_zern_smem_offset(int nops) { return (nops * (int)sizeof(FusedOp) + 15) & ~15; }
 
-// ZERN: zern = nseg Zernike tables, one per segment (the Zernike instantiation of run_op, as k_program<.., true>)
+// ZERN: zern = nseg Zernike tables, one per segment (the Zernike instantiation of run_op, as k_program<.., ZERN = true>)
 // LL: ll = nseg * nll LL tables, segment-major (the LL instantiation of run_op, as k_program<.., LL = true>)
 // SURF: the remaining scalar surfaces (as k_program<.., SURF = true>); TAB: and the table surfaces (TAB = true)
 // ZPH: zern = nseg Zernike tables of PXF_OP_ZERNPHASE ops (as k_program<.., ZPH = true>)
@@ -576,10 +551,19 @@ int build_program(FusedProgram &fp, const pxf_op *ops, int nops, const pxf_progr
 #define SURF_MINB 3
 // ... and of the interpreters with the table surfaces (k_program<tabsurf>, the surface family plus conicplus / legsurf)
 // and with the Zernike phase surface (k_program<zphase>), and their segmented forms.  Not swept: the cap of
-// k_program<surf>, whose ops they hold, and of k_program<zernike> (PXF_ZERNPROG_MINB's default), whose table staging
-// they share.  ptxas at 3: 80 registers and 128 / 112 B of spill stores.
+// k_program<surf>, whose ops they hold, and of k_program<zernike> (ZERN_MINB), whose table staging they share.
+// ptxas at 3: 80 registers and 128 / 112 B of spill stores.
 #define TABSURF_MINB 3
 #define ZPHASE_MINB 3
+// ... of the Zernike interpreter, k_program<zernike> and k_program_seg<zernike>.  Measured on config 3's 14-op program at
+// 5e7 rays, caps 1 / 2 / 3 / 4: 9.40 / 6.28 / 6.01 / 6.28 ms; the same work as three launches (transform, tracezern,
+// 12-op tail) takes 7.0 ms
+#define ZERN_MINB 3
+// ... of the Legendre-Legendre interpreter, k_program<ll> and k_program_seg<ll>.  Measured on the LL pair (36 terms per
+// mirror) at 5e7 rays, out of place, one B200 at 1000 W, caps 1 / 2 / 3 / 4: 11.6 / 13.7 / 20.2 / 28.2 ms (1: 212
+// registers, no spills; 2-4 spill 0.4-0.8 KB); with 16 / 64 terms 11.9 / 12.7 ms at 1 CTA/SM
+// (profiles/ll_program_bench_b200.json)
+#define LL_MINB 1
 
 int launch_program(double *const rays[10], int64_t num, const FusedProgram &fp, uint8_t *alive, cudaStream_t s,
                    double *const rays_out[10], double *partials, int *grid_out)
@@ -610,15 +594,11 @@ int launch_program(double *const rays[10], int64_t num, const FusedProgram &fp, 
         rc = jit_launch_chain(P, Q, num, fp, alive, aligned, s, partials, grid_out);
         if (rc != PXF_ERR_UNSUPPORTED) return rc;
     }
-    // PXF_PROGRAM_VARIANT (tuning): 0 = two rays per thread (double2 rows), 1/3/4 = one ray per thread with
-    // the register allocation capped for 1 / 3 / 4 resident CTAs per SM.  Measured on config 3's 12-op tail at
-    // 5e7 rays (profiles/r01h_notes.md): 3.82 / 3.75 / 3.27 / 3.00 ms for 0 / 1 / 3 / 4 (5 and 6 CTAs/SM spill: 4.6 / 5.7 ms).
-    static int variant = -1;
-    if (variant < 0) { const char *e = getenv("PXF_PROGRAM_VARIANT"); variant = e ? atoi(e) : 4; }
-    auto go = [&](auto kern, int64_t items) {
+    // every interpreter runs one ray per thread
+    auto go = [&](auto kern) {
         int nb = 0;
         if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, kern, PXF_BLOCK, 0) != cudaSuccess || nb <= 0) { cudaGetLastError(); nb = 2; }
-        const int grid = grid_for(items, PXF_BLOCK, nb);
+        const int grid = grid_for(num, PXF_BLOCK, nb);
         if (grid_out) *grid_out = grid;
         kern<<<grid, PXF_BLOCK, 0, s>>>(P, Q, num, alive, partials, fp);
     };
@@ -626,46 +606,17 @@ int launch_program(double *const rays[10], int64_t num, const FusedProgram &fp, 
     new_table_kinds(fp.ops, fp.nops, zphase, tabsurf);
     if (fp.uses_aux) {
         if (fp.zern) { set_error("program: a Zernike surface and a grating fan in one program are not supported"); return PXF_ERR_UNSUPPORTED; }
-        go(k_program<false, 3, false, true>, num);
+        go(k_program<3, false, true>);
     }
-    else if (zphase) {
-        // one ray per thread, capped for ZPHASE_MINB resident CTAs per SM
-        go(k_program<false, ZPHASE_MINB, false, false, false, false, false, true>, num);
-    }
-    else if (fp.zern) {
-        // one ray per thread; PXF_ZERNPROG_MINB (tuning): register cap for 1 / 2 / 3 resident CTAs per SM.  Measured on
-        // config 3's 14-op program at 5e7 rays: 9.40 / 6.28 / 6.01 ms (4: 6.28 ms); the same work as three launches
-        // (transform, tracezern, 12-op tail) takes 7.0 ms
-        static int zm = -1;
-        if (zm < 0) { const char *e = getenv("PXF_ZERNPROG_MINB"); zm = e ? atoi(e) : 3; }
-        if (zm == 1) go(k_program<false, 1, true>, num);
-        else if (zm == 2) go(k_program<false, 2, true>, num);
-        else go(k_program<false, 3, true>, num);
-    }
-    else if (fp.nll) {
-        // one ray per thread; PXF_LLPROG_MINB (tuning): register cap for 1 / 2 / 3 / 4 resident CTAs per SM.  Measured
-        // on the LL pair (36 terms per mirror) at 5e7 rays, out of place, one B200 at 1000 W: 11.6 / 13.7 / 20.2 / 28.2
-        // ms (1: 212 registers, no spills; 2-4 spill 0.4-0.8 KB); with 16 / 64 terms 11.9 / 12.7 ms at 1 CTA/SM
-        // (profiles/ll_program_bench_b200.json)
-        static int lm = -1;
-        if (lm < 0) { const char *e = getenv("PXF_LLPROG_MINB"); lm = e ? atoi(e) : 1; }
-        if (lm == 2) go(k_program<false, 2, false, false, true>, num);
-        else if (lm == 3) go(k_program<false, 3, false, false, true>, num);
-        else if (lm == 4) go(k_program<false, 4, false, false, true>, num);
-        else go(k_program<false, 1, false, false, true>, num);
-    }
-    else if (tabsurf) {
-        // one ray per thread, capped for TABSURF_MINB resident CTAs per SM
-        go(k_program<false, TABSURF_MINB, false, false, false, true, true>, num);
-    }
-    else if (fp.surf) {
-        // one ray per thread, capped for SURF_MINB resident CTAs per SM (see its definition)
-        go(k_program<false, SURF_MINB, false, false, false, true>, num);
-    }
-    else if (aligned && variant == 0) go(k_program<true, 1>, (num + 1) >> 1);
-    else if (variant == 3) go(k_program<false, 3>, num);
-    else if (variant == 1) go(k_program<false, 1>, num);
-    else go(k_program<false, 4>, num);
+    else if (zphase) go(k_program<ZPHASE_MINB, false, false, false, false, false, true>);
+    else if (fp.zern) go(k_program<ZERN_MINB, true>);
+    else if (fp.nll) go(k_program<LL_MINB, false, false, true>);
+    else if (tabsurf) go(k_program<TABSURF_MINB, false, false, false, true, true>);
+    else if (fp.surf) go(k_program<SURF_MINB, false, false, false, true>);
+    // capped for 4 resident CTAs per SM.  Measured on config 3's 12-op tail at 5e7 rays (profiles/r01h_notes.md): two
+    // rays per thread (double2 rows) 3.82 ms; one ray per thread capped for 1 / 3 / 4 CTAs/SM 3.75 / 3.27 / 3.00 ms (5
+    // and 6 CTAs/SM spill: 4.6 / 5.7 ms)
+    else go(k_program<4>);
     count_launch();
     note_kernel(zphase ? "k_program<zphase> (interpreter)" : fp.zern ? "k_program<zernike> (interpreter)" :
                 fp.uses_aux ? "k_program<aux> (interpreter)" : fp.nll ? "k_program<ll> (interpreter)" :
@@ -1062,26 +1013,14 @@ extern "C" int pxf_trace_program_segmented(double *const rays_in[10], double *co
     }
     if (dzern) {
         // the segment's Zernike table is staged behind its op table; register cap as for k_program<zernike>
-        // (PXF_ZERNPROG_MINB, resident CTAs per SM)
-        static int zm = -1;
-        if (zm < 0) { const char *e = getenv("PXF_ZERNPROG_MINB"); zm = e ? atoi(e) : 3; }
-        const size_t smem = (size_t)seg_zern_smem_offset(nops) + sizeof(ZernP);
-        if (zm == 1) go(k_program_seg<1, true>, smem);
-        else if (zm == 2) go(k_program_seg<2, true>, smem);
-        else go(k_program_seg<3, true>, smem);
+        go(k_program_seg<ZERN_MINB, true>, (size_t)seg_zern_smem_offset(nops) + sizeof(ZernP));
         count_launch();
         note_kernel("k_program_seg<zernike> (interpreter)");
         return check_launch("k_program_seg<zernike>");
     }
     if (dll) {
-        // the segment's LL tables are staged behind its op table; register cap as for k_program<ll> (PXF_LLPROG_MINB)
-        static int lm = -1;
-        if (lm < 0) { const char *e = getenv("PXF_LLPROG_MINB"); lm = e ? atoi(e) : 1; }
-        const size_t smem = (size_t)seg_zern_smem_offset(nops) + (size_t)nll * sizeof(LLTab);
-        if (lm == 2) go(k_program_seg<2, false, true>, smem);
-        else if (lm == 3) go(k_program_seg<3, false, true>, smem);
-        else if (lm == 4) go(k_program_seg<4, false, true>, smem);
-        else go(k_program_seg<1, false, true>, smem);
+        // the segment's LL tables are staged behind its op table; register cap as for k_program<ll>
+        go(k_program_seg<LL_MINB, false, true>, (size_t)seg_zern_smem_offset(nops) + (size_t)nll * sizeof(LLTab));
         count_launch();
         note_kernel("k_program_seg<ll> (interpreter)");
         return check_launch("k_program_seg<ll>");

@@ -16,7 +16,6 @@
 //      circumcircle are scanned.  The final triangle contains q and has an empty circumcircle: it is the triangle
 //      of the Delaunay triangulation (unique in general position) that scipy/Qhull interpolates in;
 //   4. barycentric interpolation inside that triangle.
-#include <stdlib.h>
 #include <string.h>
 #include <vector>
 #include "pxf_internal.h"
@@ -1116,10 +1115,8 @@ static int interp_bin(const InterpScratch &w, const double *x, const double *y, 
 static int interp_rings(const InterpScratch &w, int64_t num, cudaStream_t s)
 {
     PXF_CUDA(cudaMemsetAsync(w.slow, 0, 4, s));
-    int rq_dt = GI_RQ_DT;
-    if (const char *e = getenv("PXF_GRID_RQ")) rq_dt = atoi(e);          // (tuning / debugging)
     k_dt_rings<<<(unsigned)((num + GI_THREADS - 1) / GI_THREADS), GI_THREADS, 0, s>>>(w.sx, w.sy, w.start, w.g, (int)num, w.R, w.nfail,
-                                                                                       w.slow, rq_dt);
+                                                                                       w.slow, GI_RQ_DT);
     k_dt_rings_warp<<<grid_for(num, 1, 4), GI_COOP_THREADS, 0, s>>>(w.sx, w.sy, w.start, w.g, (int)num, w.R, w.nfail, w.slow);
     count_launch(2);
     unsigned long long hf[4] = {0, 0, 0, 0};

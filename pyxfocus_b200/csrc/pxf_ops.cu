@@ -4,7 +4,6 @@
 // of SM-count x resident-CTA blocks striding over ray pairs.
 #include <stdarg.h>
 #include <atomic>
-#include <stdlib.h>
 #include <type_traits>
 #include "pxf_internal.h"
 #include "pxf_params.h"
@@ -154,7 +153,10 @@ struct OpReflect {
     static constexpr int AUX = 0, SMEM = 0;
     PXF_DEV static void apply(Ray &r, const Params &, const double *, double, double) { op_reflect(r); }
 };
+// one ray per thread, 4 CTAs/SM (measured: 1.408 / 1.283 / 1.229 / 1.300 / 1.408 ms; shapes as listed at OpMinB)
 struct OpRefract {
+    static constexpr int MINB = 4;
+    static constexpr bool SCALAR = true;
     using Params = RefractP;
     static constexpr unsigned LOAD = R_DIR | R_NRM, STORE = R_DIR | R_NRM;
     static constexpr int AUX = 0, SMEM = 0;
@@ -294,7 +296,10 @@ struct OpWolterPrimaryOpd {
     static constexpr int AUX = 0, SMEM = 0;
     PXF_DEV static void apply(Ray &r, const Params &p, const double *, double, double) { op_wolterprimary(r, p); }
 };
+// one ray per thread, 5 CTAs/SM (measured: 0.893 / 0.900 / 0.900 / 0.865 / 0.897 ms; shapes as listed at OpMinB)
 struct OpWolterSecondary {
+    static constexpr int MINB = 5;
+    static constexpr bool SCALAR = true;
     using Params = WolterP;
     static constexpr unsigned LOAD = R_POS | R_DIR, STORE = R_POS | R_NRM;
     static constexpr int AUX = 0, SMEM = 0;
@@ -306,36 +311,26 @@ struct OpWolterSine {
     static constexpr int AUX = 0, SMEM = 0;
     PXF_DEV static void apply(Ray &r, const Params &p, const double *, double, double) { op_woltersine(r, p); }
 };
-// MINB / SCALAR as for OpZern: the W-S Newton loops are latency bound at two rays per thread and 140 registers
-// (8 warps per SM, fp64 pipe 30 %: profiles/r02d_k_op_wsprimary.txt)
-template <int MINB_ = 1, bool SCALAR_ = false>
-struct OpWsPrimaryT {
-    static constexpr int MINB = MINB_;
-    static constexpr bool SCALAR = SCALAR_;
+// One ray per thread, 3 CTAs/SM: the W-S Newton loops are latency bound at two rays per thread and 140 registers
+// (8 warps per SM, fp64 pipe 30 %: profiles/r02d_k_op_wsprimary.txt).  Measured at 5e7 rays, primary / secondary: two
+// rays per thread uncapped 2.60 / 5.70 ms, capped for 2 CTAs/SM 1.68 / 3.59 ms; one ray per thread capped for 3 / 4 / 2
+// CTAs/SM 1.51 / 3.21, 1.76 / 3.21, 1.76 / 3.58 ms
+struct OpWsPrimary {
+    static constexpr int MINB = 3;
+    static constexpr bool SCALAR = true;
     using Params = WSP;
     static constexpr unsigned LOAD = R_NINE, STORE = R_POS | R_NRM;
     static constexpr int AUX = 0, SMEM = 0;
     PXF_DEV static void apply(Ray &r, const Params &p, const double *, double, double) { op_wsprimary(r, p); }
 };
-template <int MINB_ = 1, bool SCALAR_ = false>
-struct OpWsSecondaryT {
-    static constexpr int MINB = MINB_;
-    static constexpr bool SCALAR = SCALAR_;
+struct OpWsSecondary {
+    static constexpr int MINB = 3;
+    static constexpr bool SCALAR = true;
     using Params = WSP;
     static constexpr unsigned LOAD = R_NINE, STORE = R_POS | R_NRM;
     static constexpr int AUX = 0, SMEM = 0;
     PXF_DEV static void apply(Ray &r, const Params &p, const double *, double, double) { op_wssecondary(r, p); }
 };
-typedef OpWsPrimaryT<> OpWsPrimary;
-typedef OpWsSecondaryT<> OpWsSecondary;
-static int ws_variant()
-{
-    // PXF_WS_VARIANT (tuning): 0 = two rays per thread, uncapped; 1 = two rays, capped for 2 CTAs/SM; 2/3/4 = one ray
-    // per thread capped for 3/4/2 CTAs/SM
-    static int variant = -1;
-    if (variant < 0) { const char *e = getenv("PXF_WS_VARIANT"); variant = e ? atoi(e) : 2; }   // measured at 5e7 rays, primary / secondary: 2.60/5.70, 1.68/3.59, 1.51/3.21, 1.76/3.21, 1.76/3.58 ms for 0..4
-    return variant;
-}
 struct OpWsPrimaryBack {
     using Params = WSP;
     static constexpr unsigned LOAD = R_NINE, STORE = R_POS | R_NRM;
@@ -393,19 +388,26 @@ struct OpLegSurf {
     static constexpr int AUX = 0, SMEM = 0;
     PXF_DEV static void apply(Ray &r, const Params &p, const double *, double, double) { op_legsurf(r, p); }
 };
+// one ray per thread, 3 CTAs/SM (measured: 1.199 / 1.001 / 1.049 / 1.137 / 1.215 ms; shapes as listed at OpMinB)
 struct OpSpoCone {
+    static constexpr int MINB = 3;
+    static constexpr bool SCALAR = true;
     using Params = SpoP;
     static constexpr unsigned LOAD = R_NINE, STORE = R_NINE;
     static constexpr int AUX = 0, SMEM = 0;
     PXF_DEV static void apply(Ray &r, const Params &p, const double *, double, double) { op_spocone(r, p); }
 };
-// MINB: minimum resident CTAs per SM the register allocation is capped for; SCALAR: one ray per thread even
-// on aligned rows (the unrolled Zernike evaluation needs ~200 registers per ray: two rays per thread leave
-// 8 warps per SM to cover the fp64 latency)
-template <int NMAX, bool OPD, int MINB_ = 1, bool SCALAR_ = false>
+// nmax <= 7: one ray per thread even on aligned rows, 4 CTAs/SM (the unrolled Zernike evaluation needs ~200 registers
+// per ray: two rays per thread leave 8 warps per SM to cover the fp64 latency).  The Cartesian Horner form needs far
+// fewer live values than the polar one; measured, 36 terms at 5e7 rays: two rays per thread uncapped 1.81 ms, capped
+// for 2 CTAs/SM 1.35 ms; one ray per thread capped for 3 / 4 / 2 CTAs/SM 1.46 / 1.35 / 1.50 ms (profiles/r02_notes.md).
+// Higher orders: two rays per thread, uncapped (measured, profiles/r01h_notes.md: two rays per thread at ~240
+// registers = 8 warps/SM runs 3.69 ms per 5e7 rays; one ray per thread capped for 1/2/3 CTAs per SM 4.12/3.99/4.03
+// ms -- the evaluation is issue bound)
+template <int NMAX, bool OPD>
 struct OpZern {
-    static constexpr int MINB = MINB_;
-    static constexpr bool SCALAR = SCALAR_;
+    static constexpr int MINB = NMAX <= 7 ? 4 : 1;
+    static constexpr bool SCALAR = NMAX <= 7;
     using Params = ZernP;
     static constexpr unsigned LOAD = R_POS | R_DIR | (OPD ? R_OPD : 0u);
     static constexpr unsigned STORE = R_POS | R_NRM | (OPD ? R_OPD : 0u);
@@ -430,10 +432,13 @@ struct OpZernPhase {
     }
 };
 
-template <int N, int MINB_ = 2, bool SCALAR_ = false>
+// N = 5: one ray per thread, 4 CTAs/SM; the other orders: two rays per thread, 2 CTAs/SM.  Measured at N = 5, 36 terms
+// at 5e7 rays: two rays per thread capped for 2 CTAs/SM 2.68 ms; one ray per thread capped for 3 / 4 CTAs/SM 2.58 /
+// 2.55 ms; two rays per thread uncapped 3.74 ms
+template <int N>
 struct OpLL {
-    static constexpr int MINB = MINB_;
-    static constexpr bool SCALAR = SCALAR_;
+    static constexpr int MINB = N == 5 ? 4 : 2;
+    static constexpr bool SCALAR = N == 5;
     using Params = LLP;
     static constexpr unsigned LOAD = R_POS | R_DIR, STORE = R_POS | R_NRM;
     static constexpr int AUX = 0, SMEM = 0;
@@ -443,25 +448,15 @@ struct OpLL {
 };
 
 // ------------------------------------------------------------------ the kernel
+// Launch shape of a routine.  MINB: resident CTAs per SM the register allocation is capped for (default 1, uncapped);
+// SCALAR: one ray per thread even on aligned rows (default: two rays per thread with double2 accesses).  The
+// compute-bound routines were timed at 5e7 rays in five shapes, listed as "measured:" in this order: two rays per
+// thread uncapped / one ray per thread capped for 3 / 4 / 5 CTAs per SM / two rays per thread capped for 2 CTAs per
+// SM (profiles/r02l_op_variants.txt).  Where the fastest shape wins by less than 1 %, the routine keeps the default.
 template <class Op, class = void> struct OpMinB { static constexpr int v = 1; };
 template <class Op> struct OpMinB<Op, std::void_t<decltype(Op::MINB)>> { static constexpr int v = Op::MINB; };
 template <class Op, class = void> struct OpScalar { static constexpr bool v = false; };
 template <class Op> struct OpScalar<Op, std::void_t<decltype(Op::SCALAR)>> { static constexpr bool v = Op::SCALAR; };
-
-// The same routine with another launch shape: registers capped for MINB_ CTAs per SM, one ray per thread if SCALAR_
-template <class Op, int MINB_, bool SCALAR_>
-struct Shaped : Op {
-    static constexpr int MINB = MINB_;
-    static constexpr bool SCALAR = SCALAR_;
-};
-// PXF_OP_VARIANT (tuning, compute-bound per-routine kernels): 0 = two rays per thread, registers uncapped;
-// 1/2/3 = one ray per thread capped for 3/4/5 CTAs per SM; 4 = two rays per thread capped for 2 CTAs per SM
-static int op_variant(int dflt)
-{
-    static int v = -2;
-    if (v == -2) { const char *e = getenv("PXF_OP_VARIANT"); v = e ? atoi(e) : -1; }
-    return v >= 0 ? v : dflt;
-}
 
 template <class Op, bool MASKED, bool VEC2>
 __global__ void __launch_bounds__(PXF_BLOCK, OpMinB<Op>::v)
@@ -562,25 +557,13 @@ static int launch_op(RowPtrs P, int64_t num, const uint8_t *mask, const double *
     if constexpr (OpScalar<Op>::v) {
         if (mask) return launch3<Op, true, false>(P, num, mask, aux0, aux1, prm, s);
         return launch3<Op, false, false>(P, num, mask, aux0, aux1, prm, s);
-    }
-    if (mask) {
-        if (aligned) return launch3<Op, true, true>(P, num, mask, aux0, aux1, prm, s);
-        return launch3<Op, true, false>(P, num, mask, aux0, aux1, prm, s);
-    }
-    if (aligned) return launch3<Op, false, true>(P, num, mask, aux0, aux1, prm, s);
-    return launch3<Op, false, false>(P, num, mask, aux0, aux1, prm, s);
-}
-
-template <class Op>
-static int launch_shaped(int dflt, RowPtrs P, int64_t num, const uint8_t *mask, const typename Op::Params &prm,
-                         pxf_stream_t stream)
-{
-    switch (op_variant(dflt)) {
-    case 1: return launch_op<Shaped<Op, 3, true>>(P, num, mask, nullptr, nullptr, prm, stream);
-    case 2: return launch_op<Shaped<Op, 4, true>>(P, num, mask, nullptr, nullptr, prm, stream);
-    case 3: return launch_op<Shaped<Op, 5, true>>(P, num, mask, nullptr, nullptr, prm, stream);
-    case 4: return launch_op<Shaped<Op, 2, false>>(P, num, mask, nullptr, nullptr, prm, stream);
-    default: return launch_op<Op>(P, num, mask, nullptr, nullptr, prm, stream);
+    } else {
+        if (mask) {
+            if (aligned) return launch3<Op, true, true>(P, num, mask, aux0, aux1, prm, s);
+            return launch3<Op, true, false>(P, num, mask, aux0, aux1, prm, s);
+        }
+        if (aligned) return launch3<Op, false, true>(P, num, mask, aux0, aux1, prm, s);
+        return launch3<Op, false, false>(P, num, mask, aux0, aux1, prm, s);
     }
 }
 
@@ -596,20 +579,7 @@ static RowPtrs rows9(double *x, double *y, double *z, double *l, double *m, doub
 template <bool OPD>
 static int launch_zern(RowPtrs P, int64_t num, const uint8_t *mask, const ZernP &z, pxf_stream_t stream)
 {
-    // (measured, profiles/r01h_notes.md: two rays per thread at ~240 registers = 8 warps/SM runs 3.69 ms per 5e7
-    // rays; one ray per thread capped for 1/2/3 CTAs per SM 4.12/3.99/4.03 ms -- the evaluation is issue bound)
-    if (z.nmax <= 7) {
-        // PXF_ZERN_VARIANT (tuning; the Cartesian Horner form needs far fewer live values than the polar one):
-        // 0 = two rays per thread, uncapped registers; 1 = two rays, capped for 2 CTAs/SM; 2/3/4 = one ray per thread
-        // capped for 3/4/2 CTAs/SM
-        static int variant = -1;
-        if (variant < 0) { const char *e = getenv("PXF_ZERN_VARIANT"); variant = e ? atoi(e) : 3; }   // measured, 36 terms at 5e7 rays: 1.81 / 1.35 / 1.46 / 1.35 / 1.50 ms for 0..4 (profiles/r02_notes.md)
-        if (variant == 1) return launch_op<OpZern<7, OPD, 2, false>>(P, num, mask, nullptr, nullptr, z, stream);
-        if (variant == 2) return launch_op<OpZern<7, OPD, 3, true>>(P, num, mask, nullptr, nullptr, z, stream);
-        if (variant == 3) return launch_op<OpZern<7, OPD, 4, true>>(P, num, mask, nullptr, nullptr, z, stream);
-        if (variant == 4) return launch_op<OpZern<7, OPD, 2, true>>(P, num, mask, nullptr, nullptr, z, stream);
-        return launch_op<OpZern<7, OPD>>(P, num, mask, nullptr, nullptr, z, stream);
-    }
+    if (z.nmax <= 7) return launch_op<OpZern<7, OPD>>(P, num, mask, nullptr, nullptr, z, stream);
     if (z.nmax <= 11) return launch_op<OpZern<11, OPD>>(P, num, mask, nullptr, nullptr, z, stream);
     return launch_op<OpZern<15, OPD>>(P, num, mask, nullptr, nullptr, z, stream);
 }
@@ -627,16 +597,7 @@ static int launch_ll(RowPtrs P, int64_t num, const uint8_t *mask, int kind, doub
     // one instantiation per padded order (the Horner scheme is fully unrolled, coefficients read with static offsets)
     switch (q.s.stride - 1) {
     case 3: return launch_op<OpLL<3>>(P, num, mask, nullptr, nullptr, q, stream);
-    case 5: {
-        // PXF_LL_VARIANT (tuning): 0 = two rays per thread capped for 2 CTAs/SM; 1/2 = one ray per thread capped for
-        // 3/4 CTAs/SM; 3 = two rays per thread, uncapped
-        static int variant = -1;
-        if (variant < 0) { const char *e = getenv("PXF_LL_VARIANT"); variant = e ? atoi(e) : 2; }   // measured, 36 terms at 5e7 rays: 2.68 / 2.58 / 2.55 / 3.74 ms for 0..3
-        if (variant == 1) return launch_op<OpLL<5, 3, true>>(P, num, mask, nullptr, nullptr, q, stream);
-        if (variant == 2) return launch_op<OpLL<5, 4, true>>(P, num, mask, nullptr, nullptr, q, stream);
-        if (variant == 3) return launch_op<OpLL<5, 1, false>>(P, num, mask, nullptr, nullptr, q, stream);
-        return launch_op<OpLL<5>>(P, num, mask, nullptr, nullptr, q, stream);
-    }
+    case 5: return launch_op<OpLL<5>>(P, num, mask, nullptr, nullptr, q, stream);
     case 7: return launch_op<OpLL<7>>(P, num, mask, nullptr, nullptr, q, stream);
     case 11: return launch_op<OpLL<11>>(P, num, mask, nullptr, nullptr, q, stream);
     default: return launch_op<OpLL<15>>(P, num, mask, nullptr, nullptr, q, stream);
@@ -694,8 +655,7 @@ int pxf_refract(double *l, double *m, double *n, double *ux, double *uy, double 
 {
     RefractP p;
     p.ratio = n1 / n2;
-    // (measured, 5e7 rays, variants 0..4: 1.408 / 1.283 / 1.229 / 1.300 / 1.408 ms, profiles/r02l_op_variants.txt)
-    return launch_shaped<OpRefract>(2, rows9(nullptr, nullptr, nullptr, l, m, n, ux, uy, uz), num, mask, p, stream);
+    return launch_op<OpRefract>(rows9(nullptr, nullptr, nullptr, l, m, n, ux, uy, uz), num, mask, nullptr, nullptr, p, stream);
 }
 
 int pxf_pointto(const double *x, const double *y, const double *z, double *l, double *m, double *n, int64_t num,
@@ -742,10 +702,10 @@ int pxf_indangle(const double *l, const double *m, const double *n, const double
 int pxf_radgrat(const double *x, const double *y, double *l, double *m, double *n, double wave,
                 int64_t num, double dpermm, double order, const uint8_t *mask, pxf_stream_t stream)
 {
-    // (measured: 0.654 / 0.693 / 0.694 / 0.676 / 0.653 ms)
-    return launch_shaped<OpRadgrat>(0, rows9(const_cast<double *>(x), const_cast<double *>(y), nullptr, l, m, n,
-                                             nullptr, nullptr, nullptr),
-                                    num, mask, make_radgrat(wave, dpermm, order), stream);
+    // two rays per thread, uncapped (measured: 0.654 / 0.693 / 0.694 / 0.676 / 0.653 ms; shapes as listed at OpMinB)
+    return launch_op<OpRadgrat>(rows9(const_cast<double *>(x), const_cast<double *>(y), nullptr, l, m, n,
+                                      nullptr, nullptr, nullptr),
+                                num, mask, nullptr, nullptr, make_radgrat(wave, dpermm, order), stream);
 }
 
 int pxf_radgratw(const double *x, const double *y, double *l, double *m, double *n, const double *wave,
@@ -788,8 +748,9 @@ int pxf_conic(double *x, double *y, double *z, double *l, double *m, double *n,
               double *ux, double *uy, double *uz, int64_t num, double R, double K,
               const uint8_t *mask, pxf_stream_t stream)
 {
-    // (measured: 1.165 / 1.163 / 1.281 / 1.422 / 1.160 ms)
-    return launch_shaped<OpConic>(0, rows9(x, y, z, l, m, n, ux, uy, uz), num, mask, make_conic(R, K, false, 0.), stream);
+    // two rays per thread, uncapped (measured: 1.165 / 1.163 / 1.281 / 1.422 / 1.160 ms; shapes as listed at OpMinB)
+    return launch_op<OpConic>(rows9(x, y, z, l, m, n, ux, uy, uz), num, mask, nullptr, nullptr, make_conic(R, K, false, 0.),
+                              stream);
 }
 
 int pxf_conicopd(double *opd, double *x, double *y, double *z, double *l, double *m, double *n,
@@ -821,9 +782,8 @@ int pxf_woltersecondary(double *x, double *y, double *z, double *l, double *m, d
                         double *ux, double *uy, double *uz, int64_t num, double r0, double z0, double psi,
                         const uint8_t *mask, pxf_stream_t stream)
 {
-    // (measured: 0.893 / 0.900 / 0.900 / 0.865 / 0.897 ms)
-    return launch_shaped<OpWolterSecondary>(3, rows9(x, y, z, l, m, n, ux, uy, uz), num, mask,
-                                            make_wolter(r0, z0, psi, false, 0.), stream);
+    return launch_op<OpWolterSecondary>(rows9(x, y, z, l, m, n, ux, uy, uz), num, mask, nullptr, nullptr,
+                                        make_wolter(r0, z0, psi, false, 0.), stream);
 }
 
 int pxf_woltersine(double *x, double *y, double *z, double *l, double *m, double *n,
@@ -831,23 +791,16 @@ int pxf_woltersine(double *x, double *y, double *z, double *l, double *m, double
                    double r0, double z0, double amp, double freq,
                    const uint8_t *mask, pxf_stream_t stream)
 {
-    // (measured: 1.596 / 1.610 / 1.613 / 1.636 / 1.597 ms -- bound by the two sin/cos evaluations per Newton step)
-    return launch_shaped<OpWolterSine>(0, rows9(x, y, z, l, m, n, ux, uy, uz), num, mask,
-                                       make_woltersine(r0, z0, amp, freq), stream);
+    // two rays per thread, uncapped (measured: 1.596 / 1.610 / 1.613 / 1.636 / 1.597 ms; shapes as listed at OpMinB --
+    // bound by the two sin/cos evaluations per Newton step)
+    return launch_op<OpWolterSine>(rows9(x, y, z, l, m, n, ux, uy, uz), num, mask, nullptr, nullptr,
+                                   make_woltersine(r0, z0, amp, freq), stream);
 }
 
 int pxf_wsprimary(double *x, double *y, double *z, double *l, double *m, double *n,
                   double *ux, double *uy, double *uz, int64_t num, double alpha, double z0, double psi,
                   const uint8_t *mask, pxf_stream_t stream)
 {
-    if (ws_variant() == 1) return launch_op<OpWsPrimaryT<2, false>>(rows9(x, y, z, l, m, n, ux, uy, uz), num, mask, nullptr, nullptr,
-                                  make_ws(alpha, z0, psi), stream);
-    if (ws_variant() == 2) return launch_op<OpWsPrimaryT<3, true>>(rows9(x, y, z, l, m, n, ux, uy, uz), num, mask, nullptr, nullptr,
-                                  make_ws(alpha, z0, psi), stream);
-    if (ws_variant() == 3) return launch_op<OpWsPrimaryT<4, true>>(rows9(x, y, z, l, m, n, ux, uy, uz), num, mask, nullptr, nullptr,
-                                  make_ws(alpha, z0, psi), stream);
-    if (ws_variant() == 4) return launch_op<OpWsPrimaryT<2, true>>(rows9(x, y, z, l, m, n, ux, uy, uz), num, mask, nullptr, nullptr,
-                                  make_ws(alpha, z0, psi), stream);
     return launch_op<OpWsPrimary>(rows9(x, y, z, l, m, n, ux, uy, uz), num, mask, nullptr, nullptr,
                                   make_ws(alpha, z0, psi), stream);
 }
@@ -856,14 +809,6 @@ int pxf_wssecondary(double *x, double *y, double *z, double *l, double *m, doubl
                     double *ux, double *uy, double *uz, int64_t num, double alpha, double z0, double psi,
                     const uint8_t *mask, pxf_stream_t stream)
 {
-    if (ws_variant() == 1) return launch_op<OpWsSecondaryT<2, false>>(rows9(x, y, z, l, m, n, ux, uy, uz), num, mask, nullptr, nullptr,
-                                    make_ws(alpha, z0, psi), stream);
-    if (ws_variant() == 2) return launch_op<OpWsSecondaryT<3, true>>(rows9(x, y, z, l, m, n, ux, uy, uz), num, mask, nullptr, nullptr,
-                                    make_ws(alpha, z0, psi), stream);
-    if (ws_variant() == 3) return launch_op<OpWsSecondaryT<4, true>>(rows9(x, y, z, l, m, n, ux, uy, uz), num, mask, nullptr, nullptr,
-                                    make_ws(alpha, z0, psi), stream);
-    if (ws_variant() == 4) return launch_op<OpWsSecondaryT<2, true>>(rows9(x, y, z, l, m, n, ux, uy, uz), num, mask, nullptr, nullptr,
-                                    make_ws(alpha, z0, psi), stream);
     return launch_op<OpWsSecondary>(rows9(x, y, z, l, m, n, ux, uy, uz), num, mask, nullptr, nullptr,
                                     make_ws(alpha, z0, psi), stream);
 }
@@ -872,8 +817,7 @@ int pxf_spocone(double *x, double *y, double *z, double *l, double *m, double *n
                 double *ux, double *uy, double *uz, int64_t num, double R0, double tg,
                 const uint8_t *mask, pxf_stream_t stream)
 {
-    // (measured: 1.199 / 1.001 / 1.049 / 1.137 / 1.215 ms)
-    return launch_shaped<OpSpoCone>(1, rows9(x, y, z, l, m, n, ux, uy, uz), num, mask, make_spo(R0, tg), stream);
+    return launch_op<OpSpoCone>(rows9(x, y, z, l, m, n, ux, uy, uz), num, mask, nullptr, nullptr, make_spo(R0, tg), stream);
 }
 
 int pxf_wolterprimll(double *x, double *y, double *z, double *l, double *m, double *n,

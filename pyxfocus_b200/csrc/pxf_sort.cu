@@ -572,31 +572,20 @@ static Chunking make_chunking(int64_t num)
 
 static size_t align256(size_t v) { return (v + 255) & ~(size_t)255; }
 
-// Tile shape of the one-sweep pass: PXF_SORT_VARIANT (tuning) 0 = 512 threads x 12 keys, 2 CTAs/SM;
-// 1 = 256 x 12, 3 CTAs/SM; 2 = 512 x 16, 2 CTAs/SM; 3 = 1024 x 8, 1 CTA/SM; 4 = 256 x 16, 3 CTAs/SM
-static int sort_variant()
-{
-    static int v = -1;
-    if (v < 0) { const char *e = getenv("PXF_SORT_VARIANT"); v = e ? atoi(e) : 0; if (v < 0 || v > 4) v = 0; }
-    return v;
-}
-static size_t sort_tile_keys()
-{
-    switch (sort_variant()) {
-    case 1: return 256 * 12;
-    case 2: return 512 * 16;
-    case 3: return 1024 * 8;
-    case 4: return 256 * 16;
-    default: return 512 * 12;
-    }
-}
+// Tile shape of the one-sweep pass: 512 threads x 12 keys, 2 CTAs/SM.  Argsort of 5e7 keys, steady state, threads x keys
+// (CTAs/SM) 512 x 12 (2) / 256 x 12 (3) / 512 x 16 (2) / 1024 x 8 (1) / 256 x 16 (3): 4.16 / 4.60 / 5.60 / 5.02 / 4.24 ms
+// (profiles/r02k_sort_variants.txt); after the full-tile fast path 512 x 12 / 256 x 16 / 256 x 12: 3.49 / 3.47 / 3.94 ms
+// (profiles/r02n_sort_variants.txt)
+#define OS_T 512
+#define OS_I 12
+#define OS_B 2
 
-template <int T, int I, int B>
 static int onesweep_passes(const double *keys_in, u64 *kA, u64 *kB, u32 *vA, u32 *vB, double *keys_out, long long *idx_out,
                            int64_t num, int digits, SortPlan *plan, u64 *status, cudaStream_t s)
 {
+    constexpr int T = OS_T, I = OS_I;
     const size_t tiles = ((size_t)num + (size_t)T * I - 1) / ((size_t)T * I);
-    auto kern = k_onesweep<T, I, B>;
+    auto kern = k_onesweep<T, I, OS_B>;
     static bool smem_set[64] = {};
     if (first_on_device(smem_set))
         PXF_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(OsSmem<T, I>)));
@@ -805,7 +794,7 @@ extern "C" {
 size_t pxf_sort_scratch_bytes(int64_t num)
 {
     size_t n = (size_t)(num > 0 ? num : 1);
-    const size_t tiles = (n + 256 * 12 - 1) / (256 * 12);       // the smallest tile of any variant
+    const size_t tiles = (n + 256 * 12 - 1) / (256 * 12);       // 256 x 12-key tiles: room for any tile shape of 3072 keys or more
     return 2 * align256(n * 8) + 2 * align256(n * 4) + align256(tiles * 256 * 8) + align256(8 * 256 * 8 + 64) +
            align256(sizeof(SortPlan)) + 1024;
 }
@@ -823,7 +812,7 @@ int pxf_argsort_digits(const double *keys_in, int64_t num, double *keys_out, int
     if (num == 0) return PXF_OK;
     cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
     const size_t n = (size_t)num;
-    const size_t tiles = (n + sort_tile_keys() - 1) / sort_tile_keys();
+    const size_t tiles = (n + OS_T * OS_I - 1) / (OS_T * OS_I);
     char *p = static_cast<char *>(scratch);
     u64 *kA = (u64 *)p; p += align256(n * 8);
     u64 *kB = (u64 *)p; p += align256(n * 8);
@@ -838,14 +827,7 @@ int pxf_argsort_digits(const double *keys_in, int64_t num, double *keys_out, int
     k_sort_plan<<<1, 256, 0, s>>>(ghist, num, digits, plan);
     count_launch(2);
     long long *io = reinterpret_cast<long long *>(idx_out);
-    int rc;
-    switch (sort_variant()) {
-    case 1: rc = onesweep_passes<256, 12, 3>(keys_in, kA, kB, vA, vB, keys_out, io, num, digits, plan, status, s); break;
-    case 2: rc = onesweep_passes<512, 16, 2>(keys_in, kA, kB, vA, vB, keys_out, io, num, digits, plan, status, s); break;
-    case 3: rc = onesweep_passes<1024, 8, 1>(keys_in, kA, kB, vA, vB, keys_out, io, num, digits, plan, status, s); break;
-    case 4: rc = onesweep_passes<256, 16, 3>(keys_in, kA, kB, vA, vB, keys_out, io, num, digits, plan, status, s); break;
-    default: rc = onesweep_passes<512, 12, 2>(keys_in, kA, kB, vA, vB, keys_out, io, num, digits, plan, status, s); break;
-    }
+    const int rc = onesweep_passes(keys_in, kA, kB, vA, vB, keys_out, io, num, digits, plan, status, s);
     if (rc) return rc;
     k_sort_identity<<<grid_for(num, SORT_THREADS * 2, 8), SORT_THREADS, 0, s>>>(keys_in, num, plan, keys_out, io);
     count_launch();
