@@ -324,7 +324,16 @@ enum {
      * alive as long as a program or segmented table refers to it. */
     PXF_OP_CONICPLUS = 38,     /* p: table (pxf_conicplus_table_fill, opd = 0) ; pxf_conicplus                    */
     PXF_OP_CONICPLUSOPD = 39,  /* p: table (pxf_conicplus_table_fill, opd = 1, nr) ; pxf_conicplusopd            */
-    PXF_OP_LEGSURF = 40        /* p: table (pxf_legsurf_table_fill) ; pxf_legsurf                                 */
+    PXF_OP_LEGSURF = 40,       /* p: table (pxf_legsurf_table_fill) ; pxf_legsurf                                 */
+    /* The gratings with per-ray arrays.  Each array is a DEVICE double[num], its address bit-cast into the double, and
+     * indexed by the ray's index in the bundle the program runs on (in a segmented program: in the whole bundle, so
+     * segment s reads entries seg_start[s] .. seg_start[s+1]-1).  A null address is PXF_ERR_INVALID.  The arrays
+     * must stay alive as long as a program or segmented table refers to them.  These ops run in the side-array
+     * interpreter: a program that also holds PXF_OP_ZERNSURF, PXF_OP_ZERNPHASE, PXF_OP_LLSURF or ops 27..40 is
+     * refused (PXF_ERR_UNSUPPORTED), and so is pxf_host_trace_program, which has no device arrays to point at. */
+    PXF_OP_RADGRATW = 41,      /* p: wave (array), dpermm, order ; pxf_radgratw (the sign of n comes from y)       */
+    PXF_OP_GRAT = 42           /* p: d, order (array), wave (array) ; pxf_grat (l, m, n zeroed where
+                                  l^2+m^2 > 1 after the kick)                                                      */
 };
 typedef struct pxf_op {
     int32_t code;
@@ -430,6 +439,10 @@ int pxf_trace_program_sums(double *const rays_in[10], double *const rays_out[10]
  *   differ between segments.  So do PXF_OP_CONICPLUS / CONICPLUSOPD / LEGSURF: each segment's op carries the device
  *   address of its own table, copied like any scalar, so those tables must outlive the segmented table.  The _zern
  *   and _ll fills refuse ops 27..36 and 38..40 (PXF_ERR_UNSUPPORTED).
+ *   PXF_OP_RADGRATW / PXF_OP_GRAT go through this pair as well, with their scalars per segment.  Their arrays are
+ *   indexed by the ray's index in the WHOLE bundle (segment s reads entries seg_start[s] .. seg_start[s+1]-1); the
+ *   segments' ops may carry the same or different addresses, and the arrays must outlive the segmented table.  The
+ *   _zern and _ll fills refuse them (PXF_ERR_UNSUPPORTED).
  *   rays_out == NULL: in place. */
 size_t pxf_segmented_table_bytes(int32_t nops, int32_t nseg);
 int pxf_segmented_table_fill(const pxf_op *ops, int32_t nops, int32_t nseg, const int64_t *seg_start,

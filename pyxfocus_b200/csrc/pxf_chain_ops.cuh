@@ -89,6 +89,9 @@ struct LegSurfTabP { const LegSurfP *t; };
 PXF_CHAIN_OP(CConicPlus, 38, ConicPlusTabP, op_conicplus(r, *p.t))
 PXF_CHAIN_OP(CConicPlusOpd, 39, ConicPlusTabP, op_conicplus(r, *p.t))
 PXF_CHAIN_OP(CLegSurf, 40, LegSurfTabP, op_legsurf(r, *p.t))
+// RADGRATW / GRAT: q = the scalars and the device addresses of the per-ray arrays, read at the ray's index
+PXF_CHAIN_OP(CRadgratW, 41, RadgratWP, op_radgrat(r, p.g, p.wave[ctx.i], true))
+PXF_CHAIN_OP(CGrat, 42, GratOpP, op_grat(r, p.d, p.order[ctx.i], p.wave[ctx.i]))
 #undef PXF_CHAIN_OP
 
 // predicates: the ray stops at the op when apply() returns false
@@ -340,6 +343,7 @@ PXF_DEV void chain_seg_body(const RowPtrs &P, const RowPtrs &Q, const int64_t nu
                 if (ZERN || NLL) asm volatile("" : "+r"(z));
                 if (ZERN) ctx.zt = reinterpret_cast<const ZernP *>(zraw) + z;
                 if (NLL) ctx.llt = reinterpret_cast<const LLTab *>(zraw) + z;
+                ctx.i = i;                             // (the per-ray arrays are indexed in the whole bundle)
                 const bool keep = C::run(a, (&sp)[z], ctx);
                 fstore1(a, Q, SM, i);
                 if (alive) alive[i] = keep ? 1 : 0;

@@ -34,7 +34,9 @@ PXF_DEV void count_max_update(int *dst, int k)
 // SURF: whether it carries the remaining scalar surfaces (PXF_OP_TRACESPHERE .. PXF_OP_WSSECONDARYBACK)
 // TAB: whether it also carries the surfaces read through a device table (PXF_OP_CONICPLUS[OPD], PXF_OP_LEGSURF)
 // ZPH: whether it carries the Zernike phase surface (PXF_OP_ZERNPHASE; zt as for ZERN)
-template <bool ZERN = false, bool AUX = false, bool LL = false, bool SURF = false, bool TAB = false, bool ZPH = false>
+// GRAT: whether it carries the gratings with per-ray arrays (PXF_OP_RADGRATW / GRAT) without the fan; AUX carries them too
+template <bool ZERN = false, bool AUX = false, bool LL = false, bool SURF = false, bool TAB = false, bool ZPH = false,
+          bool GRAT = false>
 PXF_DEV bool run_op(Ray &r, const FusedOp &op, const ZernP *zt = nullptr, int64_t i = 0,
                     const double *aux_wave = nullptr, int *aux_count = nullptr, int *aux_count_max = nullptr,
                     const LLTab *llt = nullptr)
@@ -68,6 +70,19 @@ PXF_DEV bool run_op(Ray &r, const FusedOp &op, const ZernP *zt = nullptr, int64_
             op_radgrat(r, p, p.wave, false);
             break;
         }
+        // the arrays are read at the ray's index i, as the stand-alone kernels read them
+        case PXF_OP_RADGRATW:
+            if constexpr (AUX || GRAT) {
+                const RadgratWP &p = *reinterpret_cast<const RadgratWP *>(op.q);
+                op_radgrat(r, p.g, p.wave[i], true);
+            }
+            break;
+        case PXF_OP_GRAT:
+            if constexpr (AUX || GRAT) {
+                const GratOpP &p = *reinterpret_cast<const GratOpP *>(op.q);
+                op_grat(r, p.d, p.order[i], p.wave[i]);
+            }
+            break;
         case PXF_OP_FLAT: op_flat(r, false, 0.); break;
         case PXF_OP_FLATOPD: op_flat(r, true, op.q[0]); break;
         case PXF_OP_CONIC:
@@ -231,7 +246,9 @@ __host__ __device__ __forceinline__ int seg_zern_smem_offset(int nops) { return 
 // LL: ll = nseg * nll LL tables, segment-major (the LL instantiation of run_op, as k_program<.., LL = true>)
 // SURF: the remaining scalar surfaces (as k_program<.., SURF = true>); TAB: and the table surfaces (TAB = true)
 // ZPH: zern = nseg Zernike tables of PXF_OP_ZERNPHASE ops (as k_program<.., ZPH = true>)
-template <int MINB, bool ZERN = false, bool LL = false, bool SURF = false, bool TAB = false, bool ZPH = false>
+// GRAT: the gratings with per-ray arrays (PXF_OP_RADGRATW / GRAT), read at the ray's index in the whole bundle
+template <int MINB, bool ZERN = false, bool LL = false, bool SURF = false, bool TAB = false, bool ZPH = false,
+          bool GRAT = false>
 __global__ void __launch_bounds__(PXF_BLOCK, MINB)
 k_program_seg(const RowPtrs P, const RowPtrs Q, const int64_t num, uint8_t *__restrict__ alive,
               const long long *__restrict__ seg_start, const FusedOp *__restrict__ ops, const int nops, const int nseg,
@@ -270,7 +287,7 @@ k_program_seg(const RowPtrs P, const RowPtrs Q, const int64_t num, uint8_t *__re
                 fload1(a, P, LM, i);
                 bool keep = true;
                 for (int k = 0; k < nops; k++)
-                    if (!run_op<ZERN, false, LL, SURF, TAB, ZPH>(a, sops[k], zt, 0, nullptr, nullptr, nullptr, llt)) { keep = false; break; }
+                    if (!run_op<ZERN, false, LL, SURF, TAB, ZPH, GRAT>(a, sops[k], zt, i, nullptr, nullptr, nullptr, llt)) { keep = false; break; }
                 fstore1(a, Q, SM, i);
                 if (alive) alive[i] = keep ? 1 : 0;
             }
@@ -285,7 +302,9 @@ static void op_masks(int code, int row, unsigned &use, unsigned &st, unsigned &k
         case PXF_OP_TRANSFORM: case PXF_OP_ITRANSFORM: use = R_NINE; st = R_NINE; kill = R_NINE; break;
         case PXF_OP_REFLECT: use = R_DIR | R_NRM; st = R_DIR; kill = R_DIR; break;
         case PXF_OP_REFRACT: use = R_DIR | R_NRM; st = R_DIR | R_NRM; kill = 0; break;
-        case PXF_OP_RADGRAT: use = R_X | R_Y | R_DIR; st = R_DIR; kill = R_DIR; break;
+        case PXF_OP_RADGRAT: case PXF_OP_RADGRATW: use = R_X | R_Y | R_DIR; st = R_DIR; kill = R_DIR; break;
+        // a ray whose kick leaves l^2+m^2 > 1 gets l = m = n = 0: the direction is written either way
+        case PXF_OP_GRAT: use = R_DIR; st = R_DIR; kill = R_DIR; break;
         case PXF_OP_FLAT: use = R_POS | R_DIR; st = R_POS | R_NRM; kill = R_POS | R_NRM; break;
         case PXF_OP_FLATOPD: use = R_POS | R_DIR | R_OPD; st = R_POS | R_NRM | R_OPD; kill = R_POS | R_NRM; break;
         case PXF_OP_CONIC: case PXF_OP_SPOCONE: use = R_NINE; st = R_NINE; kill = 0; break;
@@ -339,6 +358,14 @@ static void new_table_kinds(const FusedOp *ops, int nops, bool &zphase, bool &ta
         tabsurf = tabsurf || is_table_surface_op(ops[k].code);
     }
 }
+// the gratings with per-ray arrays, which run in the side-array interpreters
+static bool is_array_op(int code) { return code == PXF_OP_RADGRATW || code == PXF_OP_GRAT; }
+static bool has_array_ops(const FusedOp *ops, int nops)
+{
+    for (int k = 0; k < nops; k++)
+        if (is_array_op(ops[k].code)) return true;
+    return false;
+}
 static bool is_table_or_aux_op(int code)
 {
     return code == PXF_OP_ZERNSURF || code == PXF_OP_LLSURF || code == PXF_OP_GRATFAN || code == PXF_OP_ROTX_REMAINING ||
@@ -352,13 +379,23 @@ int build_program(FusedProgram &fp, const pxf_op *ops, int nops, const pxf_progr
     fp.nops = nops;
     // the remaining scalar surfaces run in an interpreter of their own, which holds no table or side-array op: refused
     // before anything else is checked, so the verdict does not depend on the order of the ops
-    bool surf = false, other = false;
+    bool surf = false, other = false, arrays = false, zll = false;
     int zphase = 0, tables = 0;                // PXF_OP_ZERNPHASE ops; ops with a Zernike or LL table or a side array
     for (int k = 0; k < nops; k++) {
+        arrays = arrays || is_array_op(ops[k].code);
+        zll = zll || ops[k].code == PXF_OP_ZERNSURF || ops[k].code == PXF_OP_ZERNPHASE || ops[k].code == PXF_OP_LLSURF;
         surf = surf || is_surface_op(ops[k].code);
         other = other || is_table_or_aux_op(ops[k].code);
         zphase += ops[k].code == PXF_OP_ZERNPHASE;
         tables += is_table_or_aux_op(ops[k].code);
+    }
+    // the gratings with per-ray arrays run in the side-array interpreters, which hold no table op and no surface of the
+    // family: the combinations would need interpreters of their own
+    if (arrays && (surf || zll)) {
+        set_error("program: PXF_OP_RADGRATW / GRAT cannot share a program with a Zernike surface or phase, a "
+                  "Legendre-Legendre shell or the sphere / cylinder / cylconic / paraxial / torus / W-S back-surface / "
+                  "conicplus / legsurf ops");
+        return PXF_ERR_UNSUPPORTED;
     }
     if (surf && other) {
         set_error("program: the sphere / cylinder / cylconic / paraxial / torus / W-S back-surface / conicplus / legsurf "
@@ -387,6 +424,24 @@ int build_program(FusedProgram &fp, const pxf_op *ops, int nops, const pxf_progr
             case PXF_OP_REFRACT: { RefractP t; t.ratio = p[0] / p[1]; memcpy(f.q, &t, sizeof(t)); break; }
             case PXF_OP_RADGRAT: { RadgratP t = make_radgrat(p[0], p[1], p[2]); memcpy(f.q, &t, sizeof(t)); break; }
             case PXF_OP_FLATOPD: f.q[0] = p[0]; break;
+            // the arrays' device addresses, bit-cast into the doubles; folded as pxf_radgratw / pxf_grat fold the scalars
+            case PXF_OP_RADGRATW: {
+                RadgratWP t;
+                t.g = make_radgrat(0., p[1], p[2]);
+                memcpy(&t.wave, &p[0], sizeof(t.wave));
+                if (!t.wave) { set_error("program: PXF_OP_RADGRATW needs a device wave array"); return PXF_ERR_INVALID; }
+                memcpy(f.q, &t, sizeof(t));
+                break;
+            }
+            case PXF_OP_GRAT: {
+                GratOpP t;
+                t.d = p[0];
+                memcpy(&t.order, &p[1], sizeof(t.order));
+                memcpy(&t.wave, &p[2], sizeof(t.wave));
+                if (!t.order || !t.wave) { set_error("program: PXF_OP_GRAT needs device order and wave arrays"); return PXF_ERR_INVALID; }
+                memcpy(f.q, &t, sizeof(t));
+                break;
+            }
             case PXF_OP_CONIC: { ConicP t = make_conic(p[0], p[1], false, 0.); memcpy(f.q, &t, sizeof(t)); break; }
             case PXF_OP_CONICOPD: { ConicP t = make_conic(p[0], p[1], true, p[2]); memcpy(f.q, &t, sizeof(t)); break; }
             case PXF_OP_WOLTERPRIMARY: { WolterP t = make_wolter(p[0], p[1], p[2], false, 0.); memcpy(f.q, &t, sizeof(t)); break; }
@@ -604,7 +659,8 @@ int launch_program(double *const rays[10], int64_t num, const FusedProgram &fp, 
     };
     bool zphase, tabsurf;
     new_table_kinds(fp.ops, fp.nops, zphase, tabsurf);
-    if (fp.uses_aux) {
+    const bool arrays = has_array_ops(fp.ops, fp.nops);
+    if (fp.uses_aux || arrays) {
         if (fp.zern) { set_error("program: a Zernike surface and a grating fan in one program are not supported"); return PXF_ERR_UNSUPPORTED; }
         go(k_program<3, false, true>);
     }
@@ -619,7 +675,7 @@ int launch_program(double *const rays[10], int64_t num, const FusedProgram &fp, 
     else go(k_program<4>);
     count_launch();
     note_kernel(zphase ? "k_program<zphase> (interpreter)" : fp.zern ? "k_program<zernike> (interpreter)" :
-                fp.uses_aux ? "k_program<aux> (interpreter)" : fp.nll ? "k_program<ll> (interpreter)" :
+                (fp.uses_aux || arrays) ? "k_program<aux> (interpreter)" : fp.nll ? "k_program<ll> (interpreter)" :
                 tabsurf ? "k_program<tabsurf> (interpreter)" : fp.surf ? "k_program<surf> (interpreter)" :
                 "k_program (interpreter)");
     return check_launch("k_program");
@@ -1030,6 +1086,13 @@ extern "C" int pxf_trace_program_segmented(double *const rays_in[10], double *co
         count_launch();
         note_kernel("k_program_seg<tabsurf> (interpreter)");
         return check_launch("k_program_seg<tabsurf>");
+    }
+    if (has_array_ops(hops, nops)) {
+        // the plain interpreter's ops and the gratings with per-ray arrays; register cap as for k_program_seg
+        go(k_program_seg<4, false, false, false, false, false, true>, (size_t)nops * sizeof(FusedOp));
+        count_launch();
+        note_kernel("k_program_seg<grat> (interpreter)");
+        return check_launch("k_program_seg<grat>");
     }
     if (h->surf) {
         go(k_program_seg<SURF_MINB, false, false, true>, (size_t)nops * sizeof(FusedOp));

@@ -168,6 +168,12 @@ int pxf_host_trace_program_hint(double *const rows_host[10], int64_t num, const 
     FusedProgram fp;
     int rc = build_program(fp, ops, nops);
     if (rc) return rc;
+    for (int k = 0; k < fp.nops; k++)
+        if (fp.ops[k].code == PXF_OP_RADGRATW || fp.ops[k].code == PXF_OP_GRAT) {
+            // their arrays live on the device, and this entry point streams host rows through device buffers
+            set_error("pxf_host_trace_program: PXF_OP_RADGRATW / GRAT read device arrays; use pxf_trace_program");
+            return PXF_ERR_UNSUPPORTED;
+        }
     if (sm_count() <= 0) { set_error("no CUDA device available (libpxf has no CPU fallback)"); return PXF_ERR_CUDA; }
     const unsigned LM = fp.load_mask, SM = fp.store_mask, USED = LM | SM;
     for (int r = 0; r < 10; r++)

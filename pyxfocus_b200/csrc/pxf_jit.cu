@@ -70,6 +70,8 @@ static const OpDesc OPS[] = {
     {PXF_OP_CONICPLUS, "CConicPlus", sizeof(CConicPlus::P), false},
     {PXF_OP_CONICPLUSOPD, "CConicPlusOpd", sizeof(CConicPlusOpd::P), false},
     {PXF_OP_LEGSURF, "CLegSurf", sizeof(CLegSurf::P), false},
+    {PXF_OP_RADGRATW, "CRadgratW", sizeof(CRadgratW::P), false},
+    {PXF_OP_GRAT, "CGrat", sizeof(CGrat::P), false},
 };
 static const OpDesc *op_desc(int code)
 {

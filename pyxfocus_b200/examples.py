@@ -665,16 +665,11 @@ def ll_tolerance_fast(n, realisations, axial, az, rng="numpy", rng_seed=0, devic
     return [dict(rays=views[k], hpd=float(hpd[k]), rms=float(rms[k])) for k in range(K)]
 
 
-def config4_fast(n_per_shell=1000, M=72, order=-3, wave=2.4, rng="numpy", rng_seed=0, device=None, offX=0., offY=0.,
-                 sources=None):
-    pxf = _pxf()
-    src = sources or pxf.sources
+def _arcus_spo_fast(pxf, src, g, N, M, rng, rng_seed, dev, offX, offY):
+    """The M SPO shells of ``config4_fast`` in one segmented launch, traced to the plane of the outermost grating.
+    Returns the bundle and the per-ray area weights."""
     import torch
     from pyxfocus_b200._call import bundle_alloc, bundle_split
-    tran, surf, anal = pxf.transformations, pxf.surfaces, pxf.analyses
-    g = arcus_geometry(M)
-    N = int(n_per_shell)
-    dev = pxf.sources._device(device)
     per = [N] * M
     seed(rng_seed)
     rays = bundle_alloc(N * M, dev, zero=True)
@@ -685,13 +680,6 @@ def config4_fast(n_per_shell=1000, M=72, order=-3, wave=2.4, rng="numpy", rng_se
         pxf.sources.segments("subannulus", [(g.R[i], g.R[i] + .605, g.spanv[i], -1.) for i in range(M)], per,
                              seed=rng_seed, out=rays)
     weights = torch.cat([torch.full((N,), a / N, dtype=torch.float64, device=dev) for a in g.area])
-    if isinstance(wave, str):
-        if rng == "numpy":
-            wave = torch.as_tensor(np.random.uniform(3.6, 7.2, size=N * M), device=dev)
-        else:
-            gen = torch.Generator(device=dev)
-            gen.manual_seed(int(rng_seed))
-            wave = 3.6 + 3.6 * torch.rand(N * M, dtype=torch.float64, device=dev, generator=gen)
     # one launch for the M shells: SPO pair, to the focus frame, to the plane of the outermost grating
     # (Program.* take the scalars as the Fortran routine sees them: transform arguments negated, transformations.py:29)
     shells = [pxf.Program().transform(0, 0, 0, 0, 0, -g.ang)
@@ -699,6 +687,30 @@ def config4_fast(n_per_shell=1000, M=72, order=-3, wave=2.4, rng="numpy", rng_se
               .spocone(g.R[i], .75 * np.arctan((g.R[i] + .605 / 2) / g.focVec[i])).reflect()
               .transform(0, 0, g.focVec[i], 0, 0, 0).transform(0, 0, -g.H, 0, 0, 0).flat() for i in range(M)]
     pxf.SegmentedProgram(shells, per, device=dev).run(rays)
+    return rays, weights
+
+
+def _uniform_wave(num, rng, rng_seed, dev):
+    """config4's ``wave='uniform'``: per-ray wavelengths [nm] from uniform(3.6, 7.2)."""
+    import torch
+    if rng == "numpy":
+        return torch.as_tensor(np.random.uniform(3.6, 7.2, size=num), device=dev)
+    gen = torch.Generator(device=dev)
+    gen.manual_seed(int(rng_seed))
+    return 3.6 + 3.6 * torch.rand(num, dtype=torch.float64, device=dev, generator=gen)
+
+
+def config4_fast(n_per_shell=1000, M=72, order=-3, wave=2.4, rng="numpy", rng_seed=0, device=None, offX=0., offY=0.,
+                 sources=None):
+    pxf = _pxf()
+    src = sources or pxf.sources
+    tran, surf, anal = pxf.transformations, pxf.surfaces, pxf.analyses
+    g = arcus_geometry(M)
+    N = int(n_per_shell)
+    dev = pxf.sources._device(device)
+    rays, weights = _arcus_spo_fast(pxf, src, g, N, M, rng, rng_seed, dev, offX, offY)
+    if isinstance(wave, str):
+        wave = _uniform_wave(N * M, rng, rng_seed, dev)
     # the grating fan: frame changes + per-ray loop over the gratings (sector.py:650-707)
     outerrad, hubdist, angle, inc, l = g.outerrad, g.hubdist, g.angle, g.inc, g.lgrat
     ang = l * np.sin(inc - offX) / hubdist * .95
@@ -717,6 +729,35 @@ def config4_fast(n_per_shell=1000, M=72, order=-3, wave=2.4, rng="numpy", rng_se
     cx, cy = anal.centroid(surv, weights=w)
     return dict(rays=rays, surv=surv, kept=int(surv[1].shape[0]), dz=dz, gratings=i, cx=cx, cy=cy,
                 rmsY=anal.rmsY(surv, weights=w), hpdY=anal.hpdY(surv, weights=w))
+
+
+def config4_spectrum_fast(n_per_shell=1000, M=72, order=-3, rng="numpy", rng_seed=0, device=None, offX=0., offY=0.,
+                          sources=None, fuse=True):
+    """The SPO shells of ``config4_fast`` followed by a straight grating stage driven by a sampled spectrum: per-ray
+    wavelengths drawn as config4's ``wave='uniform'``, a radial grating (radgratW) in the plane of the outermost
+    grating with the CAT period (``dpermm_num`` = 160 nm) at the outermost module radius, back down to the focal
+    plane and ``flat``.  Inside ``fused`` the grating stage is one launch; ``fuse=False`` runs the same calls one by
+    one.  Returns the rays, the wavelengths, the best line focus in y and the weighted y RMS there."""
+    pxf = _pxf()
+    src = sources or pxf.sources
+    tran, surf, anal = pxf.transformations, pxf.surfaces, pxf.analyses
+    g = arcus_geometry(M)
+    N = int(n_per_shell)
+    dev = pxf.sources._device(device)
+    rays, weights = _arcus_spo_fast(pxf, src, g, N, M, rng, rng_seed, dev, offX, offY)
+    wave = _uniform_wave(N * M, rng, rng_seed, dev)
+
+    def grating_stage():
+        tran.radgrat(rays, g.dpermm_num / g.outerrad, order, wave)
+        tran.transform(rays, 0, 0, -g.H, 0, 0, 0)
+        surf.flat(rays)
+    if fuse:
+        with pxf.fused(rays):
+            grating_stage()
+    else:
+        grating_stage()
+    dz = surf.focusY(rays, weights=weights)
+    return dict(rays=rays, wave=wave, dz=dz, rmsY=anal.rmsY(rays, weights=weights))
 
 
 def config5_fast(n_per_shell=1000, nshell=260, offaxis=0., rng="numpy", rng_seed=0, device=None, first=0,

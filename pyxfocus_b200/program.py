@@ -35,7 +35,7 @@ OP = dict(TRANSFORM=1, ITRANSFORM=2, REFLECT=3, REFRACT=4, RADGRAT=5, FLAT=6, FL
           VIGNETTE_ABS=19, KICK=20, ZERNSURF=21, KICKN=22, VIGNETTE_RHOGT=23, GRATFAN=24, ROTX_REMAINING=25,
           LLSURF=26, TRACESPHERE=27, TRACESPHEREOPD=28, TRACECYL=29, TRACECYLOPD=30, CYLCONIC=31, PARAXIAL=32,
           PARAXIALY=33, TORUS=34, WSPRIMARYBACK=35, WSSECONDARYBACK=36, ZERNPHASE=37, CONICPLUS=38, CONICPLUSOPD=39,
-          LEGSURF=40)
+          LEGSURF=40, RADGRATW=41, GRAT=42)
 MAX_OPS = 24
 LL_MAX_ORDER = 7       # Legendre orders a fused program holds (higher orders run the stand-alone routines)
 LL_MAX_OPS = 2         # Legendre-Legendre shells per program
@@ -45,7 +45,11 @@ _AUX_OPS = (OP["GRATFAN"], OP["ROTX_REMAINING"])
 TABLE_SURFACE_OPS = (OP["CONICPLUS"], OP["CONICPLUSOPD"], OP["LEGSURF"])
 # the surface family (sphere .. W-S back surfaces, conicplus, legsurf) shares no program with a table or side-array op
 SURFACE_OPS = tuple(range(OP["TRACESPHERE"], OP["WSSECONDARYBACK"] + 1)) + TABLE_SURFACE_OPS
-TABLE_AUX_OPS = (OP["ZERNSURF"], OP["LLSURF"]) + _AUX_OPS + (OP["ZERNPHASE"],)
+# the gratings with per-ray arrays (radgratW, grat): the device address of each array travels in the op, at these p
+# slots, and is indexed by the ray's index in the bundle
+ARRAY_OPS = (OP["RADGRATW"], OP["GRAT"])
+_ARRAY_SLOTS = {OP["RADGRATW"]: (0,), OP["GRAT"]: (1, 2)}
+TABLE_AUX_OPS = (OP["ZERNSURF"], OP["LLSURF"]) + _AUX_OPS + (OP["ZERNPHASE"],) + ARRAY_OPS
 ZERN_MAX_ORDER = 7     # Zernike radial orders a fused program holds
 CONICPLUS_MAX_TERMS = 16   # polynomial terms of conicplus (surfacesf.f95:514-638)
 LEGSURF_MAX_TERMS = 48     # Legendre terms of legsurf ...
@@ -57,6 +61,23 @@ def _host_array(a, dtype):
     if isinstance(a, torch.Tensor):
         a = a.detach().cpu().numpy()
     return np.ascontiguousarray(np.asarray(a).ravel(), dtype=dtype)
+
+
+def _per_ray(v, what, scalar_ok):
+    """A per-ray array of a grating op as the program keeps it: a 1-D float64 CUDA tensor or numpy array (used as
+    given), or -- where ``scalar_ok`` -- a float, broadcast to the bundle when the program runs."""
+    import numpy as np
+    if isinstance(v, torch.Tensor):
+        if not v.is_cuda or v.dtype != torch.float64 or v.dim() != 1 or not v.is_contiguous():
+            raise ValueError("%s must be a contiguous 1-D float64 CUDA tensor" % what)
+        return v
+    if isinstance(v, np.ndarray):
+        if v.dtype != np.float64 or v.ndim != 1:
+            raise ValueError("%s must be a 1-D float64 array" % what)
+        return np.ascontiguousarray(v)
+    if scalar_ok and np.ndim(v) == 0:
+        return float(v)
+    raise ValueError("%s must be a CUDA float64 tensor or a numpy float64 array with one entry per ray" % what)
 
 
 def _zern_terms(coeff, rorder, aorder):
@@ -76,6 +97,8 @@ class Program:
         self.ops = []
         self._tables = {}        # op index -> host table (uint8 tensor) of a ZERNSURF or LLSURF op
         self._dev_tables = {}    # (op index, device) -> its device copy
+        self._arrays = {}        # op index -> per-ray arrays of a RADGRATW / GRAT op, in the order of _ARRAY_SLOTS
+        self._dev_arrays = {}    # (op index, slot, device[, num]) -> the device copy of a host array / a broadcast scalar
 
     def __len__(self):
         return len(self.ops)
@@ -101,6 +124,71 @@ class Program:
 
     def radgrat(self, wave, dpermm, order):
         return self.add(OP["RADGRAT"], wave, dpermm, order)
+
+    def radgratw(self, wave, dpermm, order):
+        """radgratW (transformationsf.f95:242-272): the radial grating with one wavelength per ray, the sign of n taken
+        from y.  ``wave``: a float64 CUDA tensor or numpy array with one entry per ray of the bundle the program runs
+        on (of the whole bundle in a ``SegmentedProgram``).  The program keeps a reference and reads it when it runs;
+        a host array is uploaded once per device."""
+        w = _per_ray(wave, "wave", False)
+        self._check_arrays("radgratw")
+        self._arrays[len(self.ops)] = [w]
+        return self.add(OP["RADGRATW"], 0., dpermm, order)
+
+    def grat(self, d, order, wave):
+        """grat (transformationsf.f95:277-305): the linear grating with grooves along +y, with a per-ray order and
+        wavelength (arrays as for ``radgratw``; a scalar is broadcast to every ray, as ``transformations.grat`` does)."""
+        o, w = _per_ray(order, "order", True), _per_ray(wave, "wave", True)
+        self._check_arrays("grat")
+        self._arrays[len(self.ops)] = [o, w]
+        return self.add(OP["GRAT"], d, 0., 0.)
+
+    def can_hold_arrays(self):
+        """Whether ``radgratw`` / ``grat`` may join this program: they run in the side-array interpreter, which holds
+        no Zernike surface or phase, LL shell or op of the surface family (``SURFACE_OPS``)."""
+        return not any(c in SURFACE_OPS or c in (OP["ZERNSURF"], OP["ZERNPHASE"], OP["LLSURF"]) for c, _ in self.ops)
+
+    def _check_arrays(self, what):
+        if not self.can_hold_arrays():
+            raise NotImplementedError("%s cannot share a program with a Zernike surface or phase, an LL shell or the "
+                                      "sphere / cylinder / cylconic / paraxial / torus / W-S back-surface / conicplus / "
+                                      "legsurf ops" % what)
+
+    def _refuse_with_arrays(self, what):
+        if any(c in ARRAY_OPS for c, _ in self.ops):
+            raise NotImplementedError("%s cannot share a program with radgratw / grat" % what)
+
+    def device_arrays(self, num, device):
+        """{op index: device tensors} of the per-ray arrays for a bundle of ``num`` rays on ``device``: CUDA tensors
+        as given, host arrays uploaded and scalars broadcast (each once per device).  Raises ValueError for an array
+        with another length or on another device."""
+        device = torch.device(device)
+        for k, vals in self._arrays.items():
+            for j in range(len(vals)):
+                self._check_array(k, j, num, device)
+        return {k: [self._device_array(k, j, num, device) for j in range(len(vals))]
+                for k, vals in self._arrays.items()}
+
+    def _check_array(self, k, j, num, device):
+        v = self._arrays[k][j]
+        code = self.ops[k][0]
+        what = "%s op %d, p[%d]" % ("radgratw" if code == OP["RADGRATW"] else "grat", k, _ARRAY_SLOTS[code][j])
+        if isinstance(v, float):
+            return
+        if v.shape[0] != num:
+            raise ValueError("%s: the array has %d entries, the bundle %d rays" % (what, v.shape[0], num))
+        if isinstance(v, torch.Tensor) and v.device != device:
+            raise ValueError("%s: the array lives on %s, the bundle on %s" % (what, v.device, device))
+
+    def _device_array(self, k, j, num, device):
+        v = self._arrays[k][j]
+        if isinstance(v, torch.Tensor):
+            return v
+        key = (k, j, str(device)) if not isinstance(v, float) else (k, j, str(device), int(num))
+        if key not in self._dev_arrays:
+            self._dev_arrays[key] = (torch.full((int(num),), v, dtype=torch.float64, device=device)
+                                     if isinstance(v, float) else torch.from_numpy(v).to(device))
+        return self._dev_arrays[key]
 
     # --- surfacesf ---
     def flat(self):
@@ -207,6 +295,9 @@ class Program:
         return not any(c in TABLE_AUX_OPS for c, _ in self.ops)
 
     def _check_surface(self):
+        if any(c in ARRAY_OPS for c, _ in self.ops):
+            raise NotImplementedError("the sphere / cylinder / cylconic / paraxial / torus / W-S back-surface / "
+                                      "conicplus / legsurf ops cannot share a program with radgratw / grat")
         if not self.can_hold_surface():
             raise NotImplementedError("the sphere / cylinder / cylconic / paraxial / torus / W-S back-surface / "
                                       "conicplus / legsurf ops cannot share a program with a Zernike surface or phase, "
@@ -268,6 +359,7 @@ class Program:
         if any(code == OP["LLSURF"] for code, _ in self.ops):
             raise NotImplementedError("a Zernike surface and Legendre-Legendre shells in one program are not supported")
         self._refuse_with_surfaces("a Zernike surface")
+        self._refuse_with_arrays("a Zernike surface")
 
     def _zern_op(self, code, tab, nmax, p1):
         if nmax < 0:
@@ -310,6 +402,7 @@ class Program:
         if any(code == OP["ZERNSURF"] for code, _ in self.ops):
             raise NotImplementedError("a Zernike surface and Legendre-Legendre shells in one program are not supported")
         self._refuse_with_surfaces("a Legendre-Legendre shell")
+        self._refuse_with_arrays("a Legendre-Legendre shell")
         L = _lib.lib()
         tab = torch.empty(int(L.pxf_ll_table_bytes()), dtype=torch.uint8)
         top = int(L.pxf_ll_table_fill(kind, float(r0), float(z0), float(psi), float(S), float(zmax), float(zmin),
@@ -369,7 +462,9 @@ class Program:
     def has_vignette(self):
         return any(c in _VIGNETTES for c, _ in self.ops)
 
-    def c_ops(self, device=None):
+    def c_ops(self, device=None, arrays=None):
+        """The ops as the C ABI takes them; ``arrays``: ``device_arrays`` of the bundle, whose addresses the RADGRATW /
+        GRAT ops carry."""
         import struct
         arr = (_lib.pxf_op * len(self.ops))()
         for k, (code, p) in enumerate(self.ops):
@@ -384,6 +479,11 @@ class Program:
                     self._dev_tables[key] = self._tables[k].to(device)
                 # the table's device address travels bit-cast in p[0] (include/pxf.h, PXF_OP_ZERNSURF, LLSURF, ...)
                 arr[k].p[0] = struct.unpack("d", struct.pack("Q", self._dev_tables[key].data_ptr()))[0]
+            if k in self._arrays:
+                if arrays is None:
+                    raise ValueError("a program with radgratw / grat needs the bundle's arrays (Program.device_arrays)")
+                for slot, t in zip(_ARRAY_SLOTS[code], arrays[k]):
+                    arr[k].p[slot] = struct.unpack("d", struct.pack("Q", t.data_ptr()))[0]
         return arr
 
     def precompile(self, segmented=False):
@@ -398,6 +498,8 @@ class Program:
                 arr[k].p[j] = v
             if k in self._tables:
                 arr[k].p[0] = struct.unpack("d", struct.pack("Q", 8))[0]      # any non-null table address
+            for slot in _ARRAY_SLOTS.get(code, ()):
+                arr[k].p[slot] = struct.unpack("d", struct.pack("Q", 8))[0]   # ... and array address
         n = int(_lib.lib().pxf_jit_compile(arr, len(self.ops), 1 if segmented else 0, None))
         if n < 0:
             _lib.check(1)
@@ -419,6 +521,8 @@ class Program:
             head.ops, tail.ops = self.ops[:MAX_OPS], self.ops[MAX_OPS:]
             head._tables = {k: v for k, v in self._tables.items() if k < MAX_OPS}
             tail._tables = {k - MAX_OPS: v for k, v in self._tables.items() if k >= MAX_OPS}
+            head._arrays = {k: v for k, v in self._arrays.items() if k < MAX_OPS}
+            tail._arrays = {k - MAX_OPS: v for k, v in self._arrays.items() if k >= MAX_OPS}
             if head.has_vignette() or tail.has_vignette():
                 raise ValueError("programs with vignette predicates are limited to %d ops" % MAX_OPS)
             if out is not None:
@@ -438,7 +542,10 @@ class Program:
         if self.has_vignette() and alive is None:
             alive = torch.empty(num, dtype=torch.uint8, device=dev)
         ptrs = (ctypes.c_void_p * 10)(*[(r.data_ptr() if r is not None else None) for r in rays])
-        ops = self.c_ops(dev)
+        arrays = self.device_arrays(num, dev) if self._arrays else None
+        if arrays is not None and num == 0:
+            return alive             # (an empty array has no address for the op to carry, and there is nothing to do)
+        ops = self.c_ops(dev, arrays)
         ap = alive.data_ptr() if alive is not None else None
         optrs = None
         if out is not None:
@@ -594,7 +701,12 @@ class SegmentedProgram:
     aspheric coefficients); the device copies of those tables are kept alive here.
 
     ``zernphase`` may take the place of ``zernsurf`` (the same op in every segment, each with its own terms and
-    ``wave``), and a clocking sweep is a ``tracezernrot`` per segment whose ``rot`` differs."""
+    ``wave``), and a clocking sweep is a ``tracezernrot`` per segment whose ``rot`` differs.
+
+    ``radgratw`` / ``grat`` take their scalars per segment; their arrays hold one entry per ray of the WHOLE bundle and
+    segment k reads entries ``start[k]:start[k+1]`` (a program may give its own array or share one; a scalar ``order``
+    / ``wave`` of ``grat`` is broadcast).  The arrays must live on the segmented program's device and are read when it
+    runs."""
 
     def __init__(self, programs, sizes, device=None):
         import struct
@@ -643,6 +755,30 @@ class SegmentedProgram:
             for j, off in enumerate(offs):
                 sgm, k = divmod(j, len(tpos))
                 arr[sgm * nops + tpos[k]].p[0] = struct.unpack("d", struct.pack("Q", base + off))[0]
+        # the per-ray arrays of radgratw / grat ops: each segment's op carries the addresses of its own program's arrays,
+        # which hold one entry per ray of the whole bundle (segment s reads entries start[s]:start[s+1])
+        apos = [k for k, (c, _) in enumerate(programs[0].ops) if c in ARRAY_OPS]
+        self._arrays = []
+        if apos:
+            if any(k not in prog._arrays for prog in programs for k in apos):
+                raise ValueError("a radgratw / grat op needs the arrays Program.radgratw / grat records")
+            if dev is None:
+                dev = torch.device("cuda", torch.cuda.current_device())
+            shared = {}        # (op index, array) -> one bundle-long array for the segments that give a scalar there
+            for sgm, prog in enumerate(programs):
+                for k in apos:
+                    for j, slot in enumerate(_ARRAY_SLOTS[prog.ops[k][0]]):
+                        prog._check_array(k, j, self.num, dev)
+                        v = prog._arrays[k][j]
+                        if isinstance(v, float):
+                            if (k, j) not in shared:
+                                shared[k, j] = torch.zeros(self.num, dtype=torch.float64, device=dev)
+                            t = shared[k, j]
+                            t[int(start[sgm]):int(start[sgm + 1])] = v
+                        else:
+                            t = prog._device_array(k, j, self.num, dev)
+                        self._arrays.append(t)
+                        arr[sgm * nops + k].p[slot] = struct.unpack("d", struct.pack("Q", t.data_ptr()))[0]
         L = _lib.lib()
         zpos = [k for k, (c, _) in enumerate(programs[0].ops) if c in (OP["ZERNSURF"], OP["ZERNPHASE"])]
         lpos = [k for k, (c, _) in enumerate(programs[0].ops) if c == OP["LLSURF"]]
@@ -731,6 +867,7 @@ def flush(rays):
         todo = Program()
         todo.ops, prog.ops = prog.ops, []
         todo._tables, prog._tables = prog._tables, {}
+        todo._arrays, prog._arrays = prog._arrays, {}
         alive = todo.run(rays)
         if alive is not None:
             prev = last_alive(rays)

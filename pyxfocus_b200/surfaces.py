@@ -23,8 +23,8 @@ from . import transformations as tran
 from . import woltsurf as wolt
 from . import zernsurf as zern
 from .analyses import analyticImagePlane, analyticXPlane, analyticYPlane
-from .program import (CONICPLUS_MAX_TERMS, LEGSURF_MAX_ORDER, LEGSURF_MAX_TERMS, LL_MAX_OPS, LL_MAX_ORDER, OP,
-                      SURFACE_OPS, ZERN_MAX_ORDER, flush, recorder_for)
+from .program import (ARRAY_OPS, CONICPLUS_MAX_TERMS, LEGSURF_MAX_ORDER, LEGSURF_MAX_TERMS, LL_MAX_OPS, LL_MAX_ORDER,
+                      OP, SURFACE_OPS, ZERN_MAX_ORDER, flush, recorder_for)
 
 
 def flat(rays, ind=None, nr=None):
@@ -212,7 +212,7 @@ def spoSecondary(rays, R0, F, d=.605, ind=None):
 def _zernsurf_recorder(prog, *rorders):
     """Whether ``prog`` (a recording program or None) can hold one more Zernike surface of these radial orders."""
     return (prog is not None and max(np.max(np.asarray(r)) for r in rorders) <= ZERN_MAX_ORDER and
-            not any(c in (OP["ZERNSURF"], OP["LLSURF"], OP["ZERNPHASE"]) + SURFACE_OPS for c, _ in prog.ops))
+            not any(c in (OP["ZERNSURF"], OP["LLSURF"], OP["ZERNPHASE"]) + SURFACE_OPS + ARRAY_OPS for c, _ in prog.ops))
 
 
 def _surface_recorder(rays):
@@ -237,7 +237,8 @@ def _ll_recorder(rays, coeff, axial, az):
         ok = False
     codes = [code for code, _ in prog.ops]
     if not ok or codes.count(OP["LLSURF"]) >= LL_MAX_OPS or any(
-            code in codes for code in (OP["ZERNSURF"], OP["ZERNPHASE"], OP["GRATFAN"], OP["ROTX_REMAINING"]) + SURFACE_OPS):
+            code in codes for code in (OP["ZERNSURF"], OP["ZERNPHASE"], OP["GRATFAN"], OP["ROTX_REMAINING"]) + SURFACE_OPS
+            + ARRAY_OPS):
         return None
     return prog
 

@@ -115,13 +115,21 @@ def refract(rays, n1, n2):
 def radgrat(rays, dpermm, order, wave, ind=None):
     """Infinite radial grating in the x-y plane (transformations.py:124-172).  A scalar
     ``wave`` uses ``radgrat`` (sign of n kept); an array (numpy or tensor) uses ``radgratw``
-    (sign taken from y), the reference's own dispatch (:146-149)."""
+    (sign taken from y), the reference's own dispatch (:146-149).  Inside ``fused`` an array with one
+    entry per ray is recorded (a device tensor is read when the program runs, a host array is copied now)."""
     x, y, z, l, m, n = rays[1:7]
     is_arr = isinstance(wave, (np.ndarray, torch.Tensor)) and np.ndim(wave) > 0
     if is_arr and np.size(wave) == 1 and ind is not None:
         # reference: type(wave)==ndarray picks radgratw but a size-1 array is passed whole (:156-159)
         wave = torch.as_tensor(wave, dtype=torch.float64).reshape(1).expand(x.shape[0]).contiguous()
     if is_arr:
+        prog = recorder_for(rays) if ind is None else None
+        if prog is not None and prog.can_hold_arrays():
+            # converted as the stand-alone call converts its intent(in) array (_call.Staged.input)
+            w = torch.as_tensor(wave).to(device=x.device, dtype=torch.float64).contiguous()
+            if w.dim() == 1 and w.shape[0] == x.shape[0]:
+                prog.radgratw(w, dpermm, order)
+                return
         flush(rays)
         tran.radgratw(x, y, l, m, n, wave, dpermm, order, mask=ind)
         return
@@ -136,15 +144,22 @@ def radgrat(rays, dpermm, order, wave, ind=None):
 
 def grat(rays, d, order, wave, ind=None):
     """Linear grating with grooves along +y (transformations.py:200-212).  ``order`` and
-    ``wave`` are per-ray arrays (scalars are broadcast)."""
+    ``wave`` are per-ray arrays (scalars are broadcast).  Recorded inside ``fused`` unless ``ind`` is
+    given."""
     x, y, z, l, m, n = rays[1:7]
-    flush(rays)
     num = x.shape[0]
 
     def vec(v):
         t = torch.as_tensor(v, dtype=torch.float64, device=x.device)
-        return t.expand(num).contiguous() if t.dim() == 0 else t
-    tran.grat(x, y, l, m, n, d, vec(order), vec(wave), mask=ind)
+        return t.expand(num).contiguous() if t.dim() == 0 else t.contiguous()
+    order, wave = vec(order), vec(wave)
+    prog = recorder_for(rays) if ind is None else None
+    if (prog is not None and prog.can_hold_arrays() and order.dim() == wave.dim() == 1
+            and order.shape[0] == wave.shape[0] == num):
+        prog.grat(d, order, wave)
+        return
+    flush(rays)
+    tran.grat(x, y, l, m, n, d, order, wave, mask=ind)
     return
 
 
